@@ -10,6 +10,10 @@ replica of the inputs and evaluates its own 201-offset slice of a grid N times a
 
     python bench.py --gpus N --steps K --warmup W            # the B200 engine
     python bench.py --impl reference --steps K --warmup W    # the CPU path on the host cores
+    python bench.py --steps K --warmup W --dump-outputs DIR  # also save the last timed step's curve
+
+The inputs are generated from fixed seeds and every grid call's RNG is keyed by its call number, so
+two runs with the same arguments compute on identical inputs and their dumps can be compared.
 """
 from __future__ import annotations
 
@@ -37,7 +41,9 @@ UNIT = "cells/s"
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10,
+                    help="timed steps of the headline grid and of the end-to-end path (the syncpoint and scale "
+                         "sections report the best of a fixed number of whole passes)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="C2")
@@ -47,7 +53,13 @@ def parse():
     ap.add_argument("--scale-configs", action="store_true", help="(kept for old command lines: now the default)")
     ap.add_argument("--no-scale", action="store_true",
                     help="skip C3 (strong scaling) and C4 with 900 syncpoints (about 25 s at N = 1)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the loss curve of the last one (float64, one value per "
+                         "offset of the whole grid) to DIR/presync_costs.npy")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return a
 
 
 def make_workload(name, n_gpus):
@@ -442,6 +454,9 @@ def run_b200(args):
         ev[i][1].record(stream)
         kernel_ms.append(prob.stats()["last_grid_kernel_ms"])
     barrier()
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "presync_costs.npy"), step.curve.cpu().numpy().astype(np.float64))
     clocks = sampler.stop()
     launches = prob.stats()["kernel_launches"] - launches0
     step_ms = [a.elapsed_time(b) for a, b in ev]
@@ -456,7 +471,7 @@ def run_b200(args):
     # inputs enter through rank 0 only (one validation / staging / PCIe upload instead of N through the
     # same host), its finished device state is replicated to the other ranks over NVLink (NCCL
     # broadcast into the engines' own buffers), then every rank evaluates its offsets.
-    e2e_steps = max(3, min(args.steps, 5))
+    e2e_steps = args.steps
     counts = np.full(w.n_frames, w.n_rays)
     st0 = prob.stats()
     bcast_bytes = 0

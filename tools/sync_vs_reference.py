@@ -16,9 +16,12 @@ and, as the yardstick, a SECOND build of the same unmodified reference sources i
 may contract a*b+c into FMAs (oracle/_ref/librssync_ref_fma.so, `make -C oracle ref_fma`; what a
 -march=native release build does).  It writes the distributions of |delay_spec - delay_ref| and of
 |delay_ref_fma - delay_ref| to profiles/: the second one is how far the reference moves away from
-ITSELF under an equally valid rounding of the same expressions.  CPU only.
+ITSELF under an equally valid rounding of the same expressions.  CPU only.  The windows' recorded
+results also go to tests/golden/sync_reference.json, which the test suite replays where the
+reference is not at hand (tests/recorded_reference.py).
 
 usage: python tools/sync_vs_reference.py [--windows 56] [--out profiles/r02_sync_vs_reference.json]
+                                         [--golden tests/golden/sync_reference.json]
 """
 import argparse
 import importlib
@@ -38,6 +41,7 @@ def main():
     ap.add_argument("--windows", type=int, default=56)
     ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r02_sync_vs_reference.json"))
     ap.add_argument("--threads", type=int, default=os.cpu_count() or 1)
+    ap.add_argument("--golden", default=os.path.join(ROOT, "tests", "golden", "sync_reference.json"))
     a = ap.parse_args()
     from oracle import loader, ref_loader
     if not ref_loader.available():
@@ -78,7 +82,7 @@ def main():
                 cr, dr = r.Sync(dr, fb, fb + win, td, 0.2)
                 if r2:
                     _, dr2 = r2.Sync(dr2, fb, fb + win, td, 0.2)
-            rows.append(dict(scene=si, frames=win + 1, first_frame=fb, start=start, chain=chain,
+            rows.append(dict(scene=si, workload=kw, call_no=call, frames=win + 1, first_frame=fb, start=start, chain=chain,
                              delay_spec=do, delay_ref=dr, cost_spec=co, cost_ref=cr,
                              abs_delay_diff=abs(do - dr), rel_cost_diff=abs(co - cr) / abs(cr),
                              delay_ref_fma=dr2 if r2 else None,
@@ -105,7 +109,29 @@ def main():
             frac_within_1e_6=float(np.mean(e <= 1e-6)), frac_within_1e_4=float(np.mean(e <= 1e-4)))
     with open(a.out, "w") as f:
         json.dump(dict(summary=summary, rows=rows), f, indent=1)
+    write_golden(rows, a.golden)
     print(json.dumps(summary, indent=1))
+
+
+def write_golden(rows, path):
+    """the replayable part of `rows` (workload arguments, window, start, chain, call number and both
+    results, floats as hex) in the format tests/recorded_reference.py reads"""
+    comment = ("Sync results of the unmodified rs-sync reference sources (compiled with -ffp-contract=off "
+               "against oracle/shim) and of the spec oracle, recorded by tools/sync_vs_reference.py "
+               "(profiles/r02_sync_vs_reference.json).  Each row: w = synth.make_workload('C1', **workload); "
+               "problem loaded with seed 100; set_rng(100, call_no); d = start; `chain` times "
+               "(cost, d) = Sync(d, frame_begin, frame_end, w.true_delay[0], 0.2).")
+    out = []
+    for r in rows:
+        h = lambda k: float(r[k]).hex()
+        out.append({"workload": r["workload"], "frame_begin": r["first_frame"],
+                    "frame_end": r["first_frame"] + r["frames"] - 1, "start_hex": h("start"), "chain": r["chain"],
+                    "call_no": r["call_no"], "delay_ref_hex": h("delay_ref"), "cost_ref_hex": h("cost_ref"),
+                    "delay_spec_hex": h("delay_spec"), "cost_spec_hex": h("cost_spec")})
+    with open(path, "w") as f:
+        f.write('{"comment": ' + json.dumps(comment) + ',\n "rows": [\n')
+        f.write(",\n".join("  " + json.dumps(r) for r in out))
+        f.write("\n ]}\n")
 
 
 if __name__ == "__main__":

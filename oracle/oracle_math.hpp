@@ -242,6 +242,13 @@ static inline double dot3(const double a[3], const double b[3]) {
     return fmad(a[2], b[2], fmad(a[1], b[1], a[0] * b[0]));
 }
 
+// one component x*y - p of the estimator's hypothesis cross product (core_private.cpp:45), p the
+// rounded product of the other pair: exactly 0 where the reference's rounded products cancel
+// (parallel rows: a duplicated ray gives the reference's zero hypothesis), fma(x, y, -p) otherwise.
+static inline double hyp_cross_term(double x, double y, double p) {
+    return (x * y == p) ? 0.0 : fmad(x, y, -p);
+}
+
 // safe_normalize (inline_utils.hpp:5-11): vectors with norm < 1e-12 are left unscaled.
 static inline void safe_normalize3(const double v[3], double out[3]) {
     double nrm = std::sqrt(dot3(v, v));

@@ -162,8 +162,8 @@ void guess_motion(const double* P, int n, int iters, uint64_t key, double best[3
         do { b = rng_index(key, it, k++, n); } while (b == a);  // :43
         const double* pa = P + 3 * a;
         const double* pb = P + 3 * b;
-        double c[3] = {fmad(pa[1], pb[2], -(pa[2] * pb[1])), fmad(pa[2], pb[0], -(pa[0] * pb[2])),
-                       fmad(pa[0], pb[1], -(pa[1] * pb[0]))};
+        double c[3] = {hyp_cross_term(pa[1], pb[2], pa[2] * pb[1]), hyp_cross_term(pa[2], pb[0], pa[0] * pb[2]),
+                       hyp_cross_term(pa[0], pb[1], pa[1] * pb[0])};
         double v[3];
         safe_normalize3(c, v);  // :45-46
         for (int i = 0; i < n; ++i) {

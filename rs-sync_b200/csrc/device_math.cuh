@@ -240,6 +240,15 @@ __device__ __forceinline__ double dot3(double a0, double a1, double a2, double b
     return fma(a2, b2, fma(a1, b1, a0 * b0));
 }
 
+// one component x*y - p of the estimator's hypothesis cross product (core_private.cpp:45), p the
+// rounded product of the other pair: fma(x, y, -p), except that it is exactly 0 where the
+// reference's rounded products cancel (x*y == p).  Two equal rows (a duplicated ray) then give the
+// reference's zero hypothesis, whose quartile 0 wins and whose non-finite residuals are the
+// reference's panic, instead of a direction made of the products' rounding errors.
+__device__ __forceinline__ double hyp_cross_term(double x, double y, double p) {
+    return (x * y == p) ? 0.0 : fma(x, y, -p);
+}
+
 // safe_normalize (inline_utils.hpp:5-11)
 __device__ __forceinline__ void safe_normalize3(double v0, double v1, double v2, double out[3]) {
     const double nrm = sqrt(dot3(v0, v1, v2, v0, v1, v2));

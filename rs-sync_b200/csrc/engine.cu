@@ -238,9 +238,11 @@ __device__ __forceinline__ void draw_hypothesis(const DeviceData& dd, const Fram
     RS_ASSERT(a < (uint32_t)fd.n && b < (uint32_t)fd.n && (unsigned)pa < (unsigned)fd.n && (unsigned)pb < (unsigned)fd.n);
     const double a0 = sP[pa], a1 = sP[NP + pa], a2 = sP[2 * NP + pa];
     const double b0 = sP[pb], b1 = sP[NP + pb], b2 = sP[2 * NP + pb];
-    const double c0 = fma(a1, b2, -(a2 * b1));
-    const double c1 = fma(a2, b0, -(a0 * b2));
-    const double c2 = fma(a0, b1, -(a1 * b0));
+    // where the reference's two rounded products cancel (parallel rows: a duplicated ray) its
+    // component is exactly 0, not the products' rounding error that fma leaves (hyp_cross_term)
+    const double c0 = hyp_cross_term(a1, b2, a2 * b1);
+    const double c1 = hyp_cross_term(a2, b0, a0 * b2);
+    const double c2 = hyp_cross_term(a0, b1, a1 * b0);
     safe_normalize3(c0, c1, c2, v);  // :45-46
 }
 

@@ -90,6 +90,28 @@ int rssync_set_track_pixels(rssync_problem* p, size_t n_frames, const int64_t* f
                             const size_t* counts, const double* frame_ts_a, const double* frame_ts_b,
                             const double* points_a, const double* points_b, const rssync_lens* lens,
                             double image_rows);
+/* rssync_set_track_batch with the per-ray buffers in device memory of the problem's (primary) device.
+ * frames / counts stay host arrays. `stream` (a cudaStream_t, may be NULL = legacy default) is the
+ * stream on which the caller produced the buffers: the library orders its reads after the work queued
+ * there, and has finished reading the buffers when the call returns, so the caller may overwrite or
+ * free them right afterwards (the reference's borrow contract, rssync.h:15-17).
+ * Results are bit-identical to rssync_set_track_batch on the same values.  A frame id given more than
+ * once: the last occurrence wins.  The first frame holding a non-finite value fails the call with the
+ * host form's code and message; the frames before it are applied, the others are not.  A count above
+ * 512, a null buffer with rays to read, or a buffer that is not device (or managed) memory of the
+ * problem's device: RSSYNC_E_INVALID, nothing applied.  The buffers need 8-byte alignment only. */
+int rssync_set_track_batch_device(rssync_problem* p, size_t n_frames, const int64_t* frames,
+                                  const size_t* counts, const double* ts_a, const double* ts_b,
+                                  const double* rays_a, const double* rays_b, void* stream);
+/* rssync_set_track_pixels with points_a / points_b in device memory; frames, counts, frame_ts_a,
+ * frame_ts_b and lens stay on the host. Same ordering / borrow contract.  As in the host form,
+ * everything is checked (frame timestamps first, then the points in frame order) before anything is
+ * applied; results are bit-identical to it. */
+int rssync_set_track_pixels_device(rssync_problem* p, size_t n_frames, const int64_t* frames,
+                                   const size_t* counts, const double* frame_ts_a,
+                                   const double* frame_ts_b, const double* points_a,
+                                   const double* points_b, const rssync_lens* lens,
+                                   double image_rows, void* stream);
 /* PreSync(initial_delay, frame_begin, frame_end, search_step, search_radius) -> {cost, delay}
  *                                                                  rssync.h:19-21 */
 int rssync_presync(rssync_problem* p, double initial_delay, int64_t frame_begin, int64_t frame_end,

@@ -18,6 +18,7 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <unordered_set>
 #include <utility>
 #include <vector>
 #if defined(__x86_64__)
@@ -1564,15 +1565,25 @@ int rssync_set_gyro_var(rssync_problem* p, const int64_t* ts, const double* quat
 
 namespace {
 
+// SetTrackResult's error texts.  The non-finite ones are the reference's panic texts, indexed in its
+// order of checks (core_private.cpp:199-202); the pixels forms report points_a / points_b as rays_a /
+// rays_b.
+const char* const kMsgNullBuffer = "set-track-result: null buffer";
+const char* const kMsgTooManyRays = "set-track-result: more than 512 rays in one frame is not supported";
+enum { kRaysA, kRaysB, kTsA, kTsB };
+const char* const kMsgNonFinite[4] = {
+    "set-track-result: non-finite numbers in rays_a", "set-track-result: non-finite numbers in rays_b",
+    "set-track-result: non-finite numbers in ts_a", "set-track-result: non-finite numbers in ts_b"};
+
 // SetTrackResult, stage 1: the reference's panic conditions, in its order (core_private.cpp:199-202)
 int validate_track(const double* ts_a, const double* ts_b, const double* rays_a, const double* rays_b,
                    size_t count, const char** msg) {
-    if (count && (!ts_a || !ts_b || !rays_a || !rays_b)) { *msg = "set-track-result: null buffer"; return RSSYNC_E_INVALID; }
-    if (count > (size_t)rs::kMaxRaysPerFrame) { *msg = "set-track-result: more than 512 rays in one frame is not supported"; return RSSYNC_E_INVALID; }
-    if (!all_finite(rays_a, 3 * count)) { *msg = "set-track-result: non-finite numbers in rays_a"; return RSSYNC_E_NONFINITE; }
-    if (!all_finite(rays_b, 3 * count)) { *msg = "set-track-result: non-finite numbers in rays_b"; return RSSYNC_E_NONFINITE; }
-    if (!all_finite(ts_a, count)) { *msg = "set-track-result: non-finite numbers in ts_a"; return RSSYNC_E_NONFINITE; }
-    if (!all_finite(ts_b, count)) { *msg = "set-track-result: non-finite numbers in ts_b"; return RSSYNC_E_NONFINITE; }
+    if (count && (!ts_a || !ts_b || !rays_a || !rays_b)) { *msg = kMsgNullBuffer; return RSSYNC_E_INVALID; }
+    if (count > (size_t)rs::kMaxRaysPerFrame) { *msg = kMsgTooManyRays; return RSSYNC_E_INVALID; }
+    if (!all_finite(rays_a, 3 * count)) { *msg = kMsgNonFinite[kRaysA]; return RSSYNC_E_NONFINITE; }
+    if (!all_finite(rays_b, 3 * count)) { *msg = kMsgNonFinite[kRaysB]; return RSSYNC_E_NONFINITE; }
+    if (!all_finite(ts_a, count)) { *msg = kMsgNonFinite[kTsA]; return RSSYNC_E_NONFINITE; }
+    if (!all_finite(ts_b, count)) { *msg = kMsgNonFinite[kTsB]; return RSSYNC_E_NONFINITE; }
     return RSSYNC_OK;
 }
 
@@ -1655,8 +1666,8 @@ inline bool copy_checked(double* dst, const double* src, size_t n, double* lo, d
 int stage_track(const double* ts_a, const double* ts_b, const double* rays_a, const double* rays_b,
                 size_t count, double* s_ts_a, double* s_ts_b, double* s_rays_a, double* s_rays_b,
                 double& ts_lo, double& ts_hi, const char** msg) {
-    if (count && (!ts_a || !ts_b || !rays_a || !rays_b)) { *msg = "set-track-result: null buffer"; return RSSYNC_E_INVALID; }
-    if (count > (size_t)rs::kMaxRaysPerFrame) { *msg = "set-track-result: more than 512 rays in one frame is not supported"; return RSSYNC_E_INVALID; }
+    if (count && (!ts_a || !ts_b || !rays_a || !rays_b)) { *msg = kMsgNullBuffer; return RSSYNC_E_INVALID; }
+    if (count > (size_t)rs::kMaxRaysPerFrame) { *msg = kMsgTooManyRays; return RSSYNC_E_INVALID; }
     double lo = count ? ts_a[0] : 0.0, hi = lo;
     const bool ok_ra = copy_checked(s_rays_a, rays_a, 3 * count, nullptr, nullptr);
     const bool ok_rb = copy_checked(s_rays_b, rays_b, 3 * count, nullptr, nullptr);
@@ -1665,10 +1676,10 @@ int stage_track(const double* ts_a, const double* ts_b, const double* rays_a, co
     ts_lo = lo;
     ts_hi = hi;
     // the reference's order of checks (core_private.cpp:199-202)
-    if (!ok_ra) { *msg = "set-track-result: non-finite numbers in rays_a"; return RSSYNC_E_NONFINITE; }
-    if (!ok_rb) { *msg = "set-track-result: non-finite numbers in rays_b"; return RSSYNC_E_NONFINITE; }
-    if (!ok_ta) { *msg = "set-track-result: non-finite numbers in ts_a"; return RSSYNC_E_NONFINITE; }
-    if (!ok_tb) { *msg = "set-track-result: non-finite numbers in ts_b"; return RSSYNC_E_NONFINITE; }
+    if (!ok_ra) { *msg = kMsgNonFinite[kRaysA]; return RSSYNC_E_NONFINITE; }
+    if (!ok_rb) { *msg = kMsgNonFinite[kRaysB]; return RSSYNC_E_NONFINITE; }
+    if (!ok_ta) { *msg = kMsgNonFinite[kTsA]; return RSSYNC_E_NONFINITE; }
+    if (!ok_tb) { *msg = kMsgNonFinite[kTsB]; return RSSYNC_E_NONFINITE; }
     return RSSYNC_OK;
 }
 
@@ -2108,7 +2119,187 @@ int rssync_set_track_batch(rssync_problem* p, size_t n_frames, const int64_t* fr
 
 }  // extern "C"
 
+namespace {
+
+// at = offsets of the frames' rays in the concatenated per-ray buffers (n_frames + 1 entries)
+int frame_offsets(rssync_problem* p, size_t n_frames, const size_t* counts, std::vector<size_t>& at) {
+    at.assign(n_frames + 1, 0);
+    for (size_t i = 0; i < n_frames; ++i) {
+        if (counts[i] > (size_t)rs::kMaxRaysPerFrame) { p->err = kMsgTooManyRays; return RSSYNC_E_INVALID; }
+        at[i + 1] = at[i] + counts[i];
+    }
+    return RSSYNC_OK;
+}
+
+// the pixels forms' lens profile, image height and counts
+int check_pixel_args(rssync_problem* p, size_t n_frames, const size_t* counts, const rssync_lens* lens,
+                     double image_rows, std::vector<size_t>& at) {
+    const double lv[9] = {lens->readout, lens->fx, lens->fy, lens->cx, lens->cy, lens->k1, lens->k2, lens->k3, lens->k4};
+    if (!all_finite(lv, 9) || !(image_rows > 0) || !std::isfinite(image_rows) || lens->fx == 0 || lens->fy == 0) {
+        p->err = "set-track-pixels: bad lens profile or image height";
+        return RSSYNC_E_INVALID;
+    }
+    return frame_offsets(p, n_frames, counts, at);
+}
+
+// the pixels forms' per-frame timestamps, checked before any point
+int check_frame_ts(rssync_problem* p, size_t n_frames, const double* frame_ts_a, const double* frame_ts_b) {
+    if (!all_finite(frame_ts_a, n_frames)) { p->err = kMsgNonFinite[kTsA]; return RSSYNC_E_NONFINITE; }
+    if (!all_finite(frame_ts_b, n_frames)) { p->err = kMsgNonFinite[kTsB]; return RSSYNC_E_NONFINITE; }
+    return RSSYNC_OK;
+}
+
+// The per-ray buffers of a *_device call: device (or managed) memory of the problem's device.  A plain
+// host pointer is reported as unregistered memory.
+int check_device_buffers(rssync_problem* p, std::initializer_list<const double*> bufs, size_t total) {
+    if (!total) return RSSYNC_OK;
+    for (const double* b : bufs) {
+        if (!b) { p->err = kMsgNullBuffer; return RSSYNC_E_INVALID; }
+        cudaPointerAttributes attr{};
+        const cudaError_t e = cudaPointerGetAttributes(&attr, b);
+        if (e != cudaSuccess) cudaGetLastError();  // (clears the error)
+        if (e != cudaSuccess || (attr.type != cudaMemoryTypeDevice && attr.type != cudaMemoryTypeManaged) ||
+            attr.device != p->device) {
+            p->err = "set-track-result: a per-ray buffer is not device memory of the problem's device";
+            return RSSYNC_E_INVALID;
+        }
+    }
+    return RSSYNC_OK;
+}
+
+// The device forms' per-call blocks, in the pinned h_stage and (mirrored) in d_stage, in doubles:
+//   [at: n + 1 int64][frame_ts: 2n][info: 3n (rs::StageInfo)][records: 4n (rs::PixelFrame)]
+// followed on the device by the staged per-ray data.  Per frame 8 bytes go up before the check, 24
+// come back, 32 go up after the placement (pixels form: 16 more up, the frame timestamps).
+struct DeviceStaging {
+    int64_t* h_at;
+    double* h_fts;
+    rs::StageInfo* h_info;
+    rs::PixelFrame* h_rec;
+    int64_t* d_at;
+    double* d_fts;
+    rs::StageInfo* d_info;
+    rs::PixelFrame* d_rec;
+    double* d_data;
+};
+
+// Before the check-and-stage kernel of a device form: order the problem's stream behind everything
+// that writes the arena (as the host forms do) and behind the work the caller has queued on `stream`,
+// and upload the frame offsets (and the pixels form's frame timestamps).
+int begin_device_staging(rssync_problem* p, const std::vector<size_t>& at, size_t data_doubles,
+                         const double* frame_ts_a, const double* frame_ts_b, void* stream, DeviceStaging& s) {
+    const size_t n = at.size() - 1;
+    CUDA_TRY(p, cudaSetDevice(p->device));
+    if (int rc = wait_arena_copies(p)) return rc;  // an earlier call's staging block is free again
+    // frames set one by one before this call are older than it: their upload goes first
+    if (!p->pending.empty()) {
+        if (int rc = flush(p)) return rc;
+    } else if (int rc = wait_in_flight(p)) {
+        return rc;
+    }
+    const size_t block = 10 * n + 1;
+    CUDA_TRY(p, p->h_stage.reserve(block));
+    CUDA_TRY(p, p->d_stage.reserve(block + data_doubles));
+    double* h = p->h_stage.ptr;
+    double* d = p->d_stage.ptr;
+    s = DeviceStaging{reinterpret_cast<int64_t*>(h), h + n + 1, reinterpret_cast<rs::StageInfo*>(h + 3 * n + 1),
+                      reinterpret_cast<rs::PixelFrame*>(h + 6 * n + 1), reinterpret_cast<int64_t*>(d), d + n + 1,
+                      reinterpret_cast<rs::StageInfo*>(d + 3 * n + 1), reinterpret_cast<rs::PixelFrame*>(d + 6 * n + 1),
+                      d + block};
+    for (size_t i = 0; i <= n; ++i) s.h_at[i] = (int64_t)at[i];
+    if (int rc = h2d(p, s.d_at, s.h_at, (n + 1) * sizeof(int64_t))) return rc;
+    if (frame_ts_a) {
+        for (size_t i = 0; i < n; ++i) {
+            s.h_fts[2 * i] = frame_ts_a[i];
+            s.h_fts[2 * i + 1] = frame_ts_b[i];
+        }
+        if (int rc = h2d(p, s.d_fts, s.h_fts, 2 * n * sizeof(double))) return rc;
+    }
+    if (!p->ev_order) CUDA_TRY(p, cudaEventCreateWithFlags(&p->ev_order, cudaEventDisableTiming));
+    CUDA_TRY(p, cudaEventRecord(p->ev_order, static_cast<cudaStream_t>(stream)));
+    CUDA_TRY(p, cudaStreamWaitEvent(p->stream, p->ev_order, 0));
+    return RSSYNC_OK;
+}
+
+// After the kernel: the per-frame verdicts come back (the one round trip of a device form).  Once
+// this returns nothing reads the caller's buffers any more.
+int read_stage_info(rssync_problem* p, size_t n, const DeviceStaging& s) {
+    CUDA_TRY(p, cudaGetLastError());
+    if (int rc = d2h(p, s.h_info, s.d_info, n * sizeof(rs::StageInfo))) return rc;
+    CUDA_TRY(p, cudaStreamSynchronize(p->stream));
+    if (const int line = rs::checked_assert_line()) {
+        p->err = "device-side assertion failed at engine.cu:" + std::to_string(line);
+        return RSSYNC_E_CUDA;
+    }
+    return RSSYNC_OK;
+}
+
+// After the ingest kernel: the arena holds the frames; the next call that reuses the staging blocks
+// waits for this point of the problem's stream
+int end_device_ingest(rssync_problem* p) {
+    CUDA_TRY(p, cudaGetLastError());
+    p->dev_used = std::max(p->dev_used, p->used);
+    if (!p->ev_arena) CUDA_TRY(p, cudaEventCreateWithFlags(&p->ev_arena, cudaEventDisableTiming));
+    CUDA_TRY(p, cudaEventRecord(p->ev_arena, p->stream));
+    p->arena_copy_pending = true;
+    return RSSYNC_OK;
+}
+
+}  // namespace
+
 extern "C" {
+
+// Bulk SetTrackResult from device memory.  The check, the timestamp bounds and the copy into the
+// staging buffer run on the device (stage_tracks_kernel), the sort and transpose in the same ingest
+// kernel as the host form's.  Frames before the first one holding a non-finite value are applied;
+// of a frame id given more than once among them, the last occurrence (n_frames rssync_set_track
+// calls in order).
+int rssync_set_track_batch_device(rssync_problem* p, size_t n_frames, const int64_t* frames,
+                                  const size_t* counts, const double* ts_a, const double* ts_b,
+                                  const double* rays_a, const double* rays_b, void* stream) {
+    RS_NVTX_RANGE();
+    if (!p || (n_frames && (!frames || !counts)) || n_frames > (size_t)INT32_MAX) return RSSYNC_E_INVALID;
+    std::vector<size_t> at;
+    if (int rc = frame_offsets(p, n_frames, counts, at)) return rc;
+    const size_t total = at[n_frames];
+    if (int rc = check_device_buffers(p, {rays_a, rays_b, ts_a, ts_b}, total)) return rc;
+    if (n_frames == 0) return RSSYNC_OK;
+    DeviceStaging s;
+    if (int rc = begin_device_staging(p, at, 8 * total, nullptr, nullptr, stream, s)) return rc;
+    rs::launch_stage_rays(s.d_at, (int)n_frames, (int64_t)total, rays_a, rays_b, ts_a, ts_b, s.d_data, s.d_info,
+                          p->stream);
+    if (int rc = read_stage_info(p, n_frames, s)) return rc;
+    size_t n_ok = n_frames;
+    for (size_t i = 0; i < n_frames; ++i)
+        if (s.h_info[i].bad) { n_ok = i; break; }
+    std::vector<char> last(n_ok, 0);  // the frame is the last occurrence of its id among the applied ones
+    {
+        std::unordered_set<int64_t> seen;
+        for (size_t i = n_ok; i-- > 0;) last[i] = seen.insert(frames[i]).second;
+    }
+    p->version++;
+    size_t k = 0;
+    for (size_t i = 0; i < n_ok; ++i) {
+        if (!last[i]) continue;
+        FrameDesc* fd = nullptr;
+        if (int rc = place_track(p, frames[i], counts[i], &fd, /*host_mirror=*/false)) return rc;
+        fd->ts_lo = s.h_info[i].lo;
+        fd->ts_hi = s.h_info[i].hi;
+        s.h_rec[k++] = rs::PixelFrame{fd->off, fd->n, (int64_t)at[i], 0.0, 0.0};
+    }
+    if (k) {
+        if (int rc = reserve_device_arena(p)) return rc;
+        if (int rc = h2d(p, s.d_rec, s.h_rec, k * sizeof(rs::PixelFrame))) return rc;
+        rs::launch_ingest_rays(s.d_rec, (int)k, s.d_data, s.d_data + total, s.d_data + 2 * total, s.d_data + 5 * total,
+                               p->d_rays.ptr, p->d_orig.ptr, p->d_pos.ptr, p->stream);
+        if (int rc = end_device_ingest(p)) return rc;
+    }
+    if (n_ok < n_frames) {
+        p->err = kMsgNonFinite[__builtin_ctz(s.h_info[n_ok].bad)];
+        return RSSYNC_E_NONFINITE;
+    }
+    return RSSYNC_OK;
+}
 
 // The per-frame tail of track_frames (core_testcode.cpp:134-161) on the device: pixel pairs in,
 // rays + rolling-shutter timestamps straight into the device arena (no host sort / transpose, half
@@ -2121,22 +2312,10 @@ int rssync_set_track_pixels(rssync_problem* p, size_t n_frames, const int64_t* f
     if (n_frames == 0) return RSSYNC_OK;
     if (!frames || !counts || !frame_ts_a || !frame_ts_b || !points_a || !points_b || !lens) return RSSYNC_E_INVALID;
     p->version++;
-    const double lv[9] = {lens->readout, lens->fx, lens->fy, lens->cx, lens->cy, lens->k1, lens->k2, lens->k3, lens->k4};
-    if (!all_finite(lv, 9) || !(image_rows > 0) || !std::isfinite(image_rows) || lens->fx == 0 || lens->fy == 0) {
-        p->err = "set-track-pixels: bad lens profile or image height";
-        return RSSYNC_E_INVALID;
-    }
-    std::vector<size_t> at(n_frames + 1, 0);
-    for (size_t i = 0; i < n_frames; ++i) {
-        if (counts[i] > (size_t)rs::kMaxRaysPerFrame) {
-            p->err = "set-track-result: more than 512 rays in one frame is not supported";
-            return RSSYNC_E_INVALID;
-        }
-        at[i + 1] = at[i] + counts[i];
-    }
+    std::vector<size_t> at;
+    if (int rc = check_pixel_args(p, n_frames, counts, lens, image_rows, at)) return rc;
     const size_t total = at[n_frames];
-    if (!all_finite(frame_ts_a, n_frames)) { p->err = "set-track-result: non-finite numbers in ts_a"; return RSSYNC_E_NONFINITE; }
-    if (!all_finite(frame_ts_b, n_frames)) { p->err = "set-track-result: non-finite numbers in ts_b"; return RSSYNC_E_NONFINITE; }
+    if (int rc = check_frame_ts(p, n_frames, frame_ts_a, frame_ts_b)) return rc;
     if (int rc = wait_arena_copies(p)) return rc;
     cudaSetDevice(p->device);
     if (int rc = wait_in_flight(p)) return rc;  // this ingest runs on the problem's stream
@@ -2166,7 +2345,7 @@ int rssync_set_track_pixels(rssync_problem* p, size_t n_frames, const int64_t* f
     });
     for (size_t i = 0; i < n_frames; ++i)
         if (bad[i]) {
-            p->err = bad[i] == 1 ? "set-track-result: non-finite numbers in rays_a" : "set-track-result: non-finite numbers in rays_b";
+            p->err = kMsgNonFinite[bad[i] == 1 ? kRaysA : kRaysB];
             return RSSYNC_E_NONFINITE;
         }
     std::vector<rs::PixelFrame> pf(n_frames);
@@ -2189,6 +2368,49 @@ int rssync_set_track_pixels(rssync_problem* p, size_t n_frames, const int64_t* f
     CUDA_TRY(p, cudaGetLastError());
     p->dev_used = std::max(p->dev_used, p->used);
     return RSSYNC_OK;
+}
+
+// rssync_set_track_pixels with the points in device memory: the check, the timestamp bounds and the
+// copy into the staging buffer run on the device (stage_tracks_kernel).  As in the host form,
+// everything is checked before anything is placed.
+int rssync_set_track_pixels_device(rssync_problem* p, size_t n_frames, const int64_t* frames,
+                                   const size_t* counts, const double* frame_ts_a, const double* frame_ts_b,
+                                   const double* points_a, const double* points_b, const rssync_lens* lens,
+                                   double image_rows, void* stream) {
+    RS_NVTX_RANGE();
+    if (!p) return RSSYNC_E_INVALID;
+    if (n_frames == 0) return RSSYNC_OK;
+    if (!frames || !counts || !frame_ts_a || !frame_ts_b || !lens || n_frames > (size_t)INT32_MAX)
+        return RSSYNC_E_INVALID;
+    std::vector<size_t> at;
+    if (int rc = check_pixel_args(p, n_frames, counts, lens, image_rows, at)) return rc;
+    const size_t total = at[n_frames];
+    if (int rc = check_device_buffers(p, {points_a, points_b}, total)) return rc;
+    if (int rc = check_frame_ts(p, n_frames, frame_ts_a, frame_ts_b)) return rc;
+    DeviceStaging s;
+    if (int rc = begin_device_staging(p, at, 4 * total, frame_ts_a, frame_ts_b, stream, s)) return rc;
+    rs::launch_stage_points(s.d_at, s.d_fts, (int)n_frames, (int64_t)total, points_a, points_b, lens->readout,
+                            image_rows, s.d_data, s.d_info, p->stream);
+    if (int rc = read_stage_info(p, n_frames, s)) return rc;
+    for (size_t i = 0; i < n_frames; ++i)
+        if (s.h_info[i].bad) {
+            p->err = kMsgNonFinite[(s.h_info[i].bad & 1u) ? kRaysA : kRaysB];
+            return RSSYNC_E_NONFINITE;
+        }
+    p->version++;
+    for (size_t i = 0; i < n_frames; ++i) {
+        FrameDesc* fd = nullptr;
+        if (int rc = place_track(p, frames[i], counts[i], &fd, /*host_mirror=*/false)) return rc;
+        fd->ts_lo = s.h_info[i].lo;
+        fd->ts_hi = s.h_info[i].hi;
+        s.h_rec[i] = rs::PixelFrame{fd->off, fd->n, (int64_t)at[i], frame_ts_a[i], frame_ts_b[i]};
+    }
+    if (int rc = reserve_device_arena(p)) return rc;
+    if (int rc = h2d(p, s.d_rec, s.h_rec, n_frames * sizeof(rs::PixelFrame))) return rc;
+    rs::LensDev L{lens->readout, lens->fx, lens->fy, lens->cx, lens->cy, lens->k1, lens->k2, lens->k3, lens->k4};
+    rs::launch_ingest_pixels(s.d_rec, (int)n_frames, s.d_data, s.d_data + 2 * total, L, image_rows, p->d_rays.ptr,
+                             p->d_orig.ptr, p->d_pos.ptr, p->stream);
+    return end_device_ingest(p);
 }
 
 int rssync_set_kernel_timing(rssync_problem* p, int enabled) {

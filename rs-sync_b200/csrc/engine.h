@@ -158,6 +158,28 @@ void launch_ingest_rays(const PixelFrame* d_frames, int n_frames, const double* 
                         const double* d_ts_b, const double* d_rays_a, const double* d_rays_b,
                         double* d_rays, int32_t* d_orig, int32_t* d_pos, cudaStream_t st);
 
+// ---- track buffers the caller holds in device memory (rssync_set_track_*_device) ---------------
+// What the check-and-stage kernel reports per frame; the host reads these back and places the frames.
+struct StageInfo {
+    uint32_t bad;  // bit b set: source buffer b of the frame holds a NaN or an infinity
+    uint32_t pad;
+    double lo, hi;  // smallest / largest timestamp of the frame (0, 0 for a frame without rays)
+};
+// One block per frame reads the frame's segment of every per-ray buffer once, copies it into the
+// staging buffer at the same offsets (the layout launch_ingest_rays / launch_ingest_pixels read) and
+// writes info[f].  d_at: n_frames + 1 offsets (in rays) of the frames in the buffers.
+// Rays form: src = {rays_a, rays_b, ts_a, ts_b} (3, 3, 1, 1 doubles per ray), the reference's order of
+// checks; d_stage holds ts_a, ts_b, rays_a, rays_b of `total` rays back to back; lo / hi over ts_a, ts_b.
+void launch_stage_rays(const int64_t* d_at, int n_frames, int64_t total, const double* rays_a,
+                       const double* rays_b, const double* ts_a, const double* ts_b, double* d_stage,
+                       StageInfo* d_info, cudaStream_t st);
+// Pixels form: src = {points_a, points_b} (2 doubles per point); d_stage holds points_a, points_b;
+// lo / hi over frame_ts + readout * (y / rows), the expression ingest_pixels_kernel uses.
+// d_frame_ts: ts_a, ts_b of each frame (2 per frame).
+void launch_stage_points(const int64_t* d_at, const double* d_frame_ts, int n_frames, int64_t total,
+                         const double* points_a, const double* points_b, double readout, double rows,
+                         double* d_stage, StageInfo* d_info, cudaStream_t st);
+
 // ---- stage probes (tests only) ---------------------------------------------------------------
 void launch_probe_problem_matrix(const DeviceData& dd, FrameDesc fd, double delay, double* d_P,
                                  cudaStream_t st);

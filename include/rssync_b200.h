@@ -200,6 +200,28 @@ int rssync_orientation_search_ex(rssync_problem* p, const double* timestamps_s, 
                                  double search_step, double search_radius, const uint64_t* call_nos,
                                  double* out_cost, double* out_delay);
 
+/* Rolling-shutter readout search: PreSync(initial_delay, frame_begin, frame_end, search_step, search_radius)
+ * at each of n_readouts candidate readouts (seconds, as rssync_lens.readout), without re-ingesting.  Every
+ * frame in [frame_begin, frame_end) must have been ingested by rssync_set_track_pixels(_device) and not
+ * been overwritten by a rays form or adopted since (else RSSYNC_E_STATE naming the frame): those keep
+ * y / image_rows of every ray on the device and their frame timestamps on the host.  Result j equals,
+ * bit for bit, rssync_presync on a problem that ingested the same pixels, lens, image rows and frame
+ * timestamps with lens.readout = readouts[j], keyed by RNG call number call_nos[j] (NULL: consecutive
+ * values of the problem's counter, which then advances by n_readouts); out_curves (n_readouts x D, or
+ * NULL) row j is that call's cost over rssync_presync_delays(initial_delay, search_step, search_radius).
+ * The problem's arena, frame table and gyro are left as they are.  A non-finite readout or n_readouts < 0:
+ * RSSYNC_E_INVALID; n_readouts == 0: nothing done.  Otherwise rssync_presync's errors.  A multi-device
+ * problem runs the whole search on devices[0]: the row fractions live there only, and sharding the
+ * readouts would mean replicating them and widening rssync_device_state_t, which this version does not. */
+int rssync_readout_search(rssync_problem* p, const double* readouts, int n_readouts, double initial_delay,
+                          int64_t frame_begin, int64_t frame_end, double search_step, double search_radius,
+                          const uint64_t* call_nos, double* out_cost, double* out_delay, double* out_curves);
+/* Apply a readout: re-time the pixel-ingested frames of [frame_begin, frame_end) in place, so that the
+ * problem holds, byte for byte, what ingesting them with lens.readout = readout gives (arena tiles, orig /
+ * pos, frame table) and every later call returns what it would return on that problem.  Frames ingested
+ * later use the lens of their own call.  Errors as rssync_readout_search's. */
+int rssync_set_readout(rssync_problem* p, double readout, int64_t frame_begin, int64_t frame_end);
+
 /* Pinned RNG of the randomised translation estimator (replaces the reference's
  * random_device-seeded mt19937, inline_utils.hpp:13-17).  Default seed 100, call counter 0; the
  * counter advances by one per PreSync / DebugPreSync / Sync call. */

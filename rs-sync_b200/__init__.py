@@ -41,6 +41,7 @@ C_ABI_SYMBOLS = [
     "rssync_probe_stage_copy", "rssync_probe_replication_plan",
     "rssync_set_loss_mode", "rssync_probe_spec_trig",
     "rssync_set_track_batch_device", "rssync_set_track_pixels_device",
+    "rssync_readout_search", "rssync_set_readout",
 ]
 # Itanium-ABI symbols of the C++ drop-in face (same set the reference's librssync_core exports)
 CXX_ABI_SYMBOLS = [
@@ -169,6 +170,9 @@ def load_library():
     L.rssync_orientation_search_ex.argtypes = [P, c_double_p, c_double_p, C.c_size_t, C.POINTER(C.c_char_p),
                                                C.c_int, C.c_double, C.c_int64, C.c_int64, C.c_double,
                                                C.c_double, C.POINTER(C.c_uint64), c_double_p, c_double_p]
+    L.rssync_readout_search.argtypes = [P, c_double_p, C.c_int, C.c_double, C.c_int64, C.c_int64, C.c_double,
+                                        C.c_double, C.POINTER(C.c_uint64), c_double_p, c_double_p, c_double_p]
+    L.rssync_set_readout.argtypes = [P, C.c_double, C.c_int64, C.c_int64]
     _lib = L
     return L
 
@@ -226,6 +230,34 @@ def integrate_gyro(timestamps_s, gyro_xyz, orientation=None):
     if rc:
         raise RsSyncError(rc, f"malformed gyro_orientation {orientation!r}")
     return out
+
+
+def estimate_readout(readouts, costs):
+    """The rolling-shutter readout at the vertex of the least-squares parabola through the points
+    (readouts[i], costs[i]) -- e.g. a coarse grid of candidates and readout_search's PreSync minima.
+    Raises ValueError when there are fewer than 3 distinct candidates, the fit is not convex, or the
+    vertex lies outside [min(readouts), max(readouts)]."""
+    r = np.asarray(readouts, dtype=np.float64).ravel()
+    c = np.asarray(costs, dtype=np.float64).ravel()
+    if r.shape != c.shape:
+        raise ValueError(f"{r.size} readouts but {c.size} costs")
+    if not (np.all(np.isfinite(r)) and np.all(np.isfinite(c))):
+        raise ValueError("readouts and costs must be finite")
+    if np.unique(r).size < 3:
+        raise ValueError("a parabola needs at least 3 distinct readouts")
+    # fit in centred, scaled coordinates: readouts are milliseconds in seconds, costs are large
+    mid, half = 0.5 * (r.max() + r.min()), 0.5 * (r.max() - r.min())
+    x = (r - mid) / half
+    a, b, _ = np.polyfit(x, c, 2)
+    # (a vertex inside the candidates has |b| <= 2 a: the margin only turns rounding noise on a straight
+    # line into "not convex")
+    if not a > 1e-9 * max(abs(b), float(np.ptp(c))):
+        raise ValueError("the least-squares parabola is not convex: no minimum inside the candidates")
+    v = mid + half * (-b / (2.0 * a))
+    if not (r.min() <= v <= r.max()):
+        raise ValueError(f"the parabola's vertex {v!r} lies outside the candidate readouts "
+                         f"[{r.min()!r}, {r.max()!r}]")
+    return float(v)
 
 
 def measure_fp64_peak():
@@ -447,6 +479,35 @@ class SyncProblem:
                                                         frame_begin, frame_end, search_step, search_radius, cn,
                                                         _dp(costs), _dp(delays)))
         return costs, delays
+
+    def readout_search(self, readouts, initial_delay, frame_begin, frame_end, search_step, search_radius,
+                       call_nos=None, curves=False):
+        """PreSync at every candidate rolling-shutter readout (seconds) over frames ingested from pixels,
+        without re-ingesting them (rssync_readout_search).  Returns (costs, delays), plus the n x D cost
+        curves over presync_delays(...) when curves=True.  call_nos: explicit RNG call number per readout
+        (the problem's counter is then left alone)."""
+        r = _f64(readouts).ravel()
+        n = r.shape[0]
+        costs, delays = np.empty(n), np.empty(n)
+        cn = None
+        if call_nos is not None:
+            cn_arr = np.ascontiguousarray(call_nos, dtype=np.uint64).ravel()
+            if cn_arr.shape[0] != n:
+                raise ValueError(f"{n} readouts but {cn_arr.shape[0]} call numbers")
+            cn = cn_arr.ctypes.data_as(C.POINTER(C.c_uint64))
+        cv = None
+        if curves:
+            D = self.L.rssync_presync_delays(initial_delay, search_step, search_radius, None, 0)
+            cv = np.empty((n, max(D, 0)))
+        self._check(self.L.rssync_readout_search(self.h, _dp(r), n, initial_delay, frame_begin, frame_end,
+                                                 search_step, search_radius, cn, _dp(costs), _dp(delays),
+                                                 _dp(cv) if curves else None))
+        return (costs, delays, cv) if curves else (costs, delays)
+
+    def set_readout(self, readout, frame_begin, frame_end):
+        """Re-time the pixel-ingested frames of [frame_begin, frame_end) at `readout` (seconds) in place,
+        as if they had been ingested with lens.readout = readout (rssync_set_readout)."""
+        self._check(self.L.rssync_set_readout(self.h, float(readout), int(frame_begin), int(frame_end)))
 
     def device_count(self):
         return self.L.rssync_device_count(self.h)

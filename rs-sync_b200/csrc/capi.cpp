@@ -309,6 +309,20 @@ struct rssync_problem {
     cudaEvent_t ev_sync_ready = nullptr;
     DevBuf<double> d_probe;
 
+    // rolling-shutter re-timing (rssync_readout_search, rssync_set_readout).  A frame ingested from pixels
+    // keeps its two frame timestamps here and, in d_rowq (2 doubles per arena ray, the caller's ray
+    // order), y_a / rows and y_b / rows of every ray; a frame placed by any other form since, and every
+    // frame of an adopted state, has no entry.  d_rowq is allocated by the first pixels ingest.
+    std::unordered_map<int64_t, std::pair<double, double>> retime;
+    DevBuf<double> d_rowq;
+    // the readout search's scratch: the selected frames re-timed into an arena of their own, their row
+    // extremes (4 doubles per frame), one frame table per readout, the curves and flag words
+    DevBuf<double> d_rt_rays, d_rt_ext, d_rt_costs;
+    DevBuf<int32_t> d_rt_orig, d_rt_pos;
+    DevBuf<rs::PixelFrame> d_rt_frames;
+    DevBuf<FrameDesc> d_rt_tables;
+    DevBuf<unsigned> d_rt_flags;
+
     std::vector<std::pair<double, int32_t>> sort_scratch;
     std::vector<double> trace_delay, trace_step;
     uint64_t h2d = 0, d2h = 0, sync_outer = 0, sync_evals = 0;
@@ -1477,6 +1491,9 @@ void rssync_destroy(rssync_problem* p) {
     p->d_var_ts.release(); p->d_var_in.release(); p->d_var_q.release(); p->d_var_y.release(); p->d_var_rhs.release();
     p->d_var_rec.release(); p->d_var_prefix.release(); p->d_elim.release(); p->d_os_costs.release();
     p->d_var_orients.release(); p->d_var_flags.release();
+    p->d_rowq.release(); p->d_rt_rays.release(); p->d_rt_ext.release(); p->d_rt_costs.release();
+    p->d_rt_orig.release(); p->d_rt_pos.release(); p->d_rt_frames.release(); p->d_rt_tables.release();
+    p->d_rt_flags.release();
     if (p->owns_stream && p->stream) { cudaStreamSynchronize(p->stream); cudaStreamDestroy(p->stream); }
     for (SyncLane& L : p->lanes) L.release();
     if (p->ev_sync_ready) cudaEventDestroy(p->ev_sync_ready);
@@ -1719,6 +1736,7 @@ int place_track(rssync_problem* p, int64_t frame, size_t count, FrameDesc** fd_o
         CUDA_TRY(p, p->h_pos.reserve(want, p->used));
     }
     if (it == p->frames.end()) it = p->frames.emplace_hint(pos, frame, FrameDesc{});
+    if (!p->retime.empty()) p->retime.erase(frame);  // the pixels forms enter it again after placing
     FrameDesc& fd = it->second;  // map nodes are stable: fill_track completes ts_lo / ts_hi
     fd = FrameDesc{frame, (int32_t)off, (int32_t)count, 0.0, 0.0};
     p->total_rays += count;
@@ -2245,6 +2263,12 @@ int end_device_ingest(rssync_problem* p) {
     return RSSYNC_OK;
 }
 
+// The row-fraction plane of the pixels forms, as large as the device arena (contents kept)
+int reserve_rowq(rssync_problem* p) {
+    CUDA_TRY(p, p->d_rowq.grow(2 * std::max<size_t>(p->d_orig.cap, 1), 2 * p->dev_used, p->stream));
+    return RSSYNC_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -2356,7 +2380,9 @@ int rssync_set_track_pixels(rssync_problem* p, size_t n_frames, const int64_t* f
         fd->ts_hi = hi[i];
         pf[i] = rs::PixelFrame{fd->off, fd->n, (int64_t)at[i], frame_ts_a[i], frame_ts_b[i]};
     }
+    for (size_t i = 0; i < n_frames; ++i) p->retime[frames[i]] = {frame_ts_a[i], frame_ts_b[i]};
     if (int rc = reserve_device_arena(p)) return rc;
+    if (int rc = reserve_rowq(p)) return rc;
     CUDA_TRY(p, p->d_pix.reserve(4 * total + 1));
     CUDA_TRY(p, p->d_pixframes.reserve(n_frames));
     if (int rc = h2d(p, p->d_pix.ptr, p->h_pix.ptr, 4 * total * sizeof(double))) return rc;
@@ -2364,7 +2390,7 @@ int rssync_set_track_pixels(rssync_problem* p, size_t n_frames, const int64_t* f
     CUDA_TRY(p, cudaStreamSynchronize(p->stream));  // pf is a local; the pinned staging buffer is reused
     rs::LensDev L{lens->readout, lens->fx, lens->fy, lens->cx, lens->cy, lens->k1, lens->k2, lens->k3, lens->k4};
     rs::launch_ingest_pixels(p->d_pixframes.ptr, (int)n_frames, p->d_pix.ptr, p->d_pix.ptr + 2 * total, L,
-                             image_rows, p->d_rays.ptr, p->d_orig.ptr, p->d_pos.ptr, p->stream);
+                             image_rows, p->d_rays.ptr, p->d_orig.ptr, p->d_pos.ptr, p->d_rowq.ptr, p->stream);
     CUDA_TRY(p, cudaGetLastError());
     p->dev_used = std::max(p->dev_used, p->used);
     return RSSYNC_OK;
@@ -2405,11 +2431,13 @@ int rssync_set_track_pixels_device(rssync_problem* p, size_t n_frames, const int
         fd->ts_hi = s.h_info[i].hi;
         s.h_rec[i] = rs::PixelFrame{fd->off, fd->n, (int64_t)at[i], frame_ts_a[i], frame_ts_b[i]};
     }
+    for (size_t i = 0; i < n_frames; ++i) p->retime[frames[i]] = {frame_ts_a[i], frame_ts_b[i]};
     if (int rc = reserve_device_arena(p)) return rc;
+    if (int rc = reserve_rowq(p)) return rc;
     if (int rc = h2d(p, s.d_rec, s.h_rec, n_frames * sizeof(rs::PixelFrame))) return rc;
     rs::LensDev L{lens->readout, lens->fx, lens->fy, lens->cx, lens->cy, lens->k1, lens->k2, lens->k3, lens->k4};
     rs::launch_ingest_pixels(s.d_rec, (int)n_frames, s.d_data, s.d_data + 2 * total, L, image_rows, p->d_rays.ptr,
-                             p->d_orig.ptr, p->d_pos.ptr, p->stream);
+                             p->d_orig.ptr, p->d_pos.ptr, p->d_rowq.ptr, p->stream);
     return end_device_ingest(p);
 }
 
@@ -2752,6 +2780,218 @@ int rssync_orientation_search_ex(rssync_problem* p, const double* timestamps_s, 
     return RSSYNC_OK;
 }
 
+}  // extern "C"
+
+namespace {
+
+int check_readouts(rssync_problem* p, const double* readouts, int n, const char* who) {
+    if (!all_finite(readouts, (size_t)n)) {
+        p->err = std::string(who) + ": readout must be finite";
+        return RSSYNC_E_INVALID;
+    }
+    return RSSYNC_OK;
+}
+
+// every frame of `sel` can be re-timed: it was ingested from pixels and not overwritten since
+int require_retime(rssync_problem* p, const std::vector<FrameDesc>& sel, const char* who) {
+    for (const FrameDesc& fd : sel)
+        if (!p->retime.count(fd.id)) {
+            p->err = std::string(who) + ": frame " + std::to_string(fd.id) +
+                     " has no row fractions to re-time (it was not ingested from pixels, or was overwritten or"
+                     " adopted since)";
+            return RSSYNC_E_STATE;
+        }
+    return RSSYNC_OK;
+}
+
+// The re-timing records of `sel`: source offset and frame timestamps, destination offset `dst[f]`
+std::vector<rs::PixelFrame> retime_records(const rssync_problem* p, const std::vector<FrameDesc>& sel,
+                                           const std::vector<int32_t>& dst) {
+    std::vector<rs::PixelFrame> rec(sel.size());
+    for (size_t f = 0; f < sel.size(); ++f) {
+        const std::pair<double, double>& ts = p->retime.at(sel[f].id);
+        rec[f] = rs::PixelFrame{dst[f], sel[f].n, (int64_t)sel[f].off, ts.first, ts.second};
+    }
+    return rec;
+}
+
+// A frame's timestamp bounds at readout r from its row-fraction extremes e = {min q_a, max q_a, min q_b,
+// max q_b}.  fl(ts + fl(r q)) is monotone in q -- non-decreasing for r >= 0, non-increasing for r < 0 --
+// so the smallest and largest timestamps are among the four ends, and these are the values a re-ingest's
+// bounds (the min / max over every ray) take.
+void retimed_bounds(const rs::PixelFrame& f, const double* e, double r, double& lo, double& hi) {
+    if (f.n == 0) { lo = hi = 0.0; return; }
+    const double a0 = f.ts_a + r * e[0], a1 = f.ts_a + r * e[1];
+    const double b0 = f.ts_b + r * e[2], b1 = f.ts_b + r * e[3];
+    lo = std::min(std::min(a0, a1), std::min(b0, b1));
+    hi = std::max(std::max(a0, a1), std::max(b0, b1));
+}
+
+const char* presync_panic_text(unsigned fl) {  // core_private.cpp:76-83
+    return (fl & rs::kFlagP)   ? "pre-sync: non-finite numbers in P"
+           : (fl & rs::kFlagM) ? "pre-sync: non-finite numbers in M"
+           : (fl & rs::kFlagR) ? "pre-sync: non-finite r"
+                               : "pre-sync: non-finite rho";
+}
+
+}  // namespace
+
+extern "C" {
+
+// PreSync at n_readouts rolling-shutter readouts without re-ingesting: the selected frames are re-timed
+// into a scratch arena (retime_frames_kernel) and the loss grid runs on it, per readout, back to back on
+// the problem's stream; one read-back at the end.  The problem's own arena, frame table and gyro are
+// not touched.  Runs on the primary device of a multi-device problem.
+int rssync_readout_search(rssync_problem* p, const double* readouts, int n_readouts, double initial,
+                          int64_t fb, int64_t fe, double step, double radius, const uint64_t* call_nos,
+                          double* out_cost, double* out_delay, double* out_curves) {
+    RS_NVTX_RANGE();
+    if (!p) return RSSYNC_E_INVALID;
+    if (n_readouts < 0) { p->err = "readout-search: negative readout count"; return RSSYNC_E_INVALID; }
+    if (n_readouts == 0) return RSSYNC_OK;
+    if (!readouts || !out_cost || !out_delay) { p->err = "readout-search: null buffer"; return RSSYNC_E_INVALID; }
+    if (int rc = check_readouts(p, readouts, n_readouts, "readout-search")) return rc;
+    if (int rc = require_gyro(p, "pre-sync")) return rc;
+    if (!(step > 0) || !std::isfinite(radius) || !std::isfinite(initial)) {
+        p->err = "pre-sync: search_step must be > 0 and the search window finite";
+        return RSSYNC_E_INVALID;
+    }
+    const int D = rssync_presync_delays(initial, step, radius, nullptr, 0);
+    if (D <= 0 || D > (1 << 28)) { p->err = "pre-sync: empty or oversized delay grid"; return RSSYNC_E_INVALID; }
+    std::vector<double> delays((size_t)D);
+    rssync_presync_delays(initial, step, radius, delays.data(), D);
+    std::vector<FrameDesc> sel;
+    int max_n = 0;
+    if (int rc = select_frames(p, fb, fe, sel, max_n, "pre-sync")) return rc;
+    if (int rc = require_retime(p, sel, "readout-search")) return rc;
+    const int F = (int)sel.size(), n = n_readouts;
+    if ((long long)F * D > (1LL << 34)) { p->err = "pre-sync: grid too large"; return RSSYNC_E_INVALID; }
+    std::vector<uint64_t> calls((size_t)n);
+    for (int j = 0; j < n; ++j) calls[(size_t)j] = call_nos ? call_nos[j] : p->call_no + (uint64_t)j;
+    if (!call_nos) p->call_no += (uint64_t)n;
+    CUDA_TRY(p, cudaSetDevice(p->device));
+    if (int rc = flush(p)) return rc;  // pending gyro and tracks; ordered behind ingests in flight
+    std::vector<double> costs((size_t)n * D, 0.0);  // no frames: the reference sums over none
+    std::vector<unsigned> flags((size_t)n * 2, 0u);
+    if (F > 0) {
+        cudaStream_t st = p->stream;
+        // the scratch arena holds the selected frames back to back
+        std::vector<int32_t> dst((size_t)F);
+        size_t rays = 0;
+        for (int f = 0; f < F; ++f) {
+            dst[(size_t)f] = (int32_t)rays;
+            rays += (size_t)(sel[(size_t)f].n + 31) / 32 * 32;
+        }
+        const std::vector<rs::PixelFrame> rec = retime_records(p, sel, dst);
+        CUDA_TRY(p, p->d_rt_rays.reserve(rays * 8));
+        CUDA_TRY(p, p->d_rt_orig.reserve(rays));
+        CUDA_TRY(p, p->d_rt_pos.reserve(rays));
+        CUDA_TRY(p, p->d_rt_frames.reserve((size_t)F));
+        CUDA_TRY(p, p->d_rt_ext.reserve((size_t)F * 4));
+        CUDA_TRY(p, p->d_rt_tables.reserve((size_t)n * F));
+        CUDA_TRY(p, p->d_rt_costs.reserve((size_t)n * D));
+        CUDA_TRY(p, p->d_rt_flags.reserve((size_t)n * 2));
+        CUDA_TRY(p, p->d_delays.reserve((size_t)D));
+        CUDA_TRY(p, p->d_framecost.reserve((size_t)F * D));
+        if (int rc = h2d(p, p->d_rt_frames.ptr, rec.data(), sizeof(rs::PixelFrame) * F)) return rc;
+        // the first readout's re-time also reports each frame's row extremes, from which the host takes
+        // every readout's frame bounds (the frame tables and the grids' staging windows)
+        rs::launch_retime_frames(p->d_rt_frames.ptr, F, p->d_rays.ptr, p->d_orig.ptr, p->d_rowq.ptr, readouts[0],
+                                 p->d_rt_rays.ptr, p->d_rt_orig.ptr, p->d_rt_pos.ptr, p->d_rt_ext.ptr, st);
+        CUDA_TRY(p, cudaGetLastError());
+        std::vector<double> ext((size_t)F * 4);
+        if (int rc = d2h(p, ext.data(), p->d_rt_ext.ptr, ext.size() * sizeof(double))) return rc;
+        CUDA_TRY(p, cudaStreamSynchronize(st));
+        std::vector<FrameDesc> tables((size_t)n * F);
+        std::vector<int> max_chunk((size_t)n);
+        for (int j = 0; j < n; ++j) {
+            double span = 0.0;
+            for (int f = 0; f < F; ++f) {
+                FrameDesc& fd = tables[(size_t)j * F + f];
+                fd = FrameDesc{sel[(size_t)f].id, dst[(size_t)f], sel[(size_t)f].n, 0.0, 0.0};
+                retimed_bounds(rec[(size_t)f], &ext[(size_t)f * 4], readouts[j], fd.ts_lo, fd.ts_hi);
+                span = std::max(span, fd.ts_hi - fd.ts_lo);
+            }
+            max_chunk[(size_t)j] = rs::presync_max_chunk(delays.data(), D, span, p->sr, max_n);
+        }
+        if (int rc = h2d(p, p->d_rt_tables.ptr, tables.data(), sizeof(FrameDesc) * tables.size())) return rc;
+        if (int rc = h2d(p, p->d_delays.ptr, delays.data(), sizeof(double) * D)) return rc;
+        CUDA_TRY(p, cudaMemsetAsync(p->d_rt_flags.ptr, 0, (size_t)n * 2 * sizeof(unsigned), st));
+        rs::DeviceData dd = p->device_data();
+        dd.rays = p->d_rt_rays.ptr;
+        dd.orig = p->d_rt_orig.ptr;
+        dd.pos = p->d_rt_pos.ptr;
+        for (int j = 0; j < n; ++j) {
+            if (j > 0)
+                rs::launch_retime_frames(p->d_rt_frames.ptr, F, p->d_rays.ptr, p->d_orig.ptr, p->d_rowq.ptr, readouts[j],
+                                         p->d_rt_rays.ptr, p->d_rt_orig.ptr, p->d_rt_pos.ptr, nullptr, st);
+            rs::launch_presync_grid(dd, p->d_rt_tables.ptr + (size_t)j * F, F, max_n, p->d_delays.ptr, D, p->seed,
+                                    rs::kStreamPreSync, calls[(size_t)j], 0, p->d_framecost.ptr,
+                                    p->d_rt_costs.ptr + (size_t)j * D, p->d_rt_flags.ptr + 2 * (size_t)j, st, nullptr,
+                                    nullptr, nullptr, nullptr, 0, max_chunk[(size_t)j], p->simplified);
+        }
+        CUDA_TRY(p, cudaGetLastError());
+        if (int rc = d2h(p, costs.data(), p->d_rt_costs.ptr, costs.size() * sizeof(double))) return rc;
+        if (int rc = d2h(p, flags.data(), p->d_rt_flags.ptr, flags.size() * sizeof(unsigned))) return rc;
+        CUDA_TRY(p, cudaStreamSynchronize(st));
+        if (const int line = rs::checked_assert_line()) {
+            p->err = "device-side assertion failed at engine.cu:" + std::to_string(line);
+            return RSSYNC_E_CUDA;
+        }
+        p->grid_tasks = (uint64_t)F * (uint64_t)D;
+        p->grid_exact_tasks = flags[(size_t)n * 2 - 1];
+    }
+    for (int j = 0; j < n; ++j) {
+        if (const unsigned fl = flags[2 * (size_t)j]) { p->err = presync_panic_text(fl); return RSSYNC_E_NONFINITE; }
+        const double* c = &costs[(size_t)j * D];
+        int best = 0;  // std::min_element over (cost, delay) pairs, :89
+        for (int d = 1; d < D; ++d)
+            if (c[d] < c[best] || (c[d] == c[best] && delays[(size_t)d] < delays[(size_t)best])) best = d;
+        out_cost[j] = c[best];
+        out_delay[j] = delays[(size_t)best];
+        if (out_curves) std::memcpy(out_curves + (size_t)j * D, c, sizeof(double) * D);
+    }
+    return RSSYNC_OK;
+}
+
+// Re-time the pixel frames of [fb, fe) in place at `readout`: afterwards the problem holds what ingesting
+// them with lens.readout = readout would have produced (tiles, orig / pos, frame table).
+int rssync_set_readout(rssync_problem* p, double readout, int64_t fb, int64_t fe) {
+    RS_NVTX_RANGE();
+    if (!p) return RSSYNC_E_INVALID;
+    if (int rc = check_readouts(p, &readout, 1, "set-readout")) return rc;
+    std::vector<FrameDesc> sel;
+    for (auto it = p->frames.lower_bound(fb); it != p->frames.end() && it->first < fe; ++it) sel.push_back(it->second);
+    if (int rc = require_retime(p, sel, "set-readout")) return rc;
+    if (sel.empty()) return RSSYNC_OK;
+    const int F = (int)sel.size();
+    CUDA_TRY(p, cudaSetDevice(p->device));
+    if (int rc = wait_arena_copies(p)) return rc;  // a replication still reading the arena, the staging block
+    if (int rc = flush(p)) return rc;              // uploads and ingests in flight land first
+    p->version++;
+    std::vector<int32_t> dst((size_t)F);
+    for (int f = 0; f < F; ++f) dst[(size_t)f] = sel[(size_t)f].off;
+    const std::vector<rs::PixelFrame> rec = retime_records(p, sel, dst);
+    CUDA_TRY(p, p->d_rt_frames.reserve((size_t)F));
+    CUDA_TRY(p, p->d_rt_ext.reserve((size_t)F * 4));
+    if (int rc = h2d(p, p->d_rt_frames.ptr, rec.data(), sizeof(rs::PixelFrame) * F)) return rc;
+    rs::launch_retime_frames(p->d_rt_frames.ptr, F, p->d_rays.ptr, p->d_orig.ptr, p->d_rowq.ptr, readout,
+                             p->d_rays.ptr, p->d_orig.ptr, p->d_pos.ptr, p->d_rt_ext.ptr, p->stream);
+    CUDA_TRY(p, cudaGetLastError());
+    std::vector<double> ext((size_t)F * 4);
+    if (int rc = d2h(p, ext.data(), p->d_rt_ext.ptr, ext.size() * sizeof(double))) return rc;
+    CUDA_TRY(p, cudaStreamSynchronize(p->stream));
+    if (const int line = rs::checked_assert_line()) {
+        p->err = "device-side assertion failed at engine.cu:" + std::to_string(line);
+        return RSSYNC_E_CUDA;
+    }
+    for (int f = 0; f < F; ++f) {
+        FrameDesc& fd = p->frames.at(sel[(size_t)f].id);
+        retimed_bounds(rec[(size_t)f], &ext[(size_t)f * 4], readout, fd.ts_lo, fd.ts_hi);
+    }
+    return RSSYNC_OK;
+}
+
 int rssync_sync(rssync_problem* p, double initial, int64_t fb, int64_t fe, double center,
                 double radius, double* out_cost, double* out_delay) {
     RS_NVTX_RANGE();
@@ -2922,6 +3162,7 @@ int rssync_adopt_state(rssync_problem* p, const rssync_frame_desc* frames, size_
     p->version++;
     p->pending.clear();
     p->gyro_dirty = false;
+    p->retime.clear();  // an adopted arena comes without row fractions
     // the same table as last time (a caller replicating fresh data of an unchanged frame set): keep the map
     bool same = p->frames.size() == n_frames;
     if (same) {

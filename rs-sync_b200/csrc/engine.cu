@@ -1650,7 +1650,7 @@ __device__ __forceinline__ void ingest_sort_and_store(const PixelFrame& f, const
 __global__ void __launch_bounds__(kIngestThreads)
 ingest_pixels_kernel(const PixelFrame* __restrict__ frames, const double* __restrict__ pa,
                      const double* __restrict__ pb, LensDev L, double rows, double* __restrict__ rays,
-                     int32_t* __restrict__ orig, int32_t* __restrict__ pos) {
+                     int32_t* __restrict__ orig, int32_t* __restrict__ pos, double2* __restrict__ rowq) {
     __shared__ double s_ts[kMaxRaysPerFrame];  // ts_a of point i (sort key)
     __shared__ int s_idx[kMaxRaysPerFrame];    // permutation being sorted
     __shared__ double s_val[7][kMaxRaysPerFrame];  // ts_b, ra.xyz, rb.xyz of point i
@@ -1663,8 +1663,10 @@ ingest_pixels_kernel(const PixelFrame* __restrict__ frames, const double* __rest
             double ua, va, ub, vb;
             undistort_point(L, ax, ay, ua, va);
             undistort_point(L, bx, by, ub, vb);
-            s_ts[i] = f.ts_a + L.ro * (ay / rows);  // :144
-            s_val[0][i] = f.ts_b + L.ro * (by / rows);  // :145
+            const double qa = ay / rows, qb = by / rows;
+            rowq[f.off + i] = make_double2(qa, qb);  // kept for re-timing (retime_frames_kernel)
+            s_ts[i] = f.ts_a + L.ro * qa;  // :144
+            s_val[0][i] = f.ts_b + L.ro * qb;  // :145
             const double na = sqrt(ua * ua + va * va + 1.0), nb = sqrt(ub * ub + vb * vb + 1.0);
             s_val[1][i] = ua / na; s_val[2][i] = va / na; s_val[3][i] = 1.0 / na;  // :153
             s_val[4][i] = ub / nb; s_val[5][i] = vb / nb; s_val[6][i] = 1.0 / nb;  // :154
@@ -1673,6 +1675,62 @@ ingest_pixels_kernel(const PixelFrame* __restrict__ frames, const double* __rest
         }
     }
     __syncthreads();
+    ingest_sort_and_store(f, s_ts, s_idx, s_val, rays, orig, pos);
+}
+
+// Rolling-shutter re-timing of frames ingested from pixels: the rays stay, the timestamps are
+// recomputed at readout `ro` from the row fractions ingest_pixels_kernel kept (rowq[off + i] = {y_a,
+// y_b} / rows of caller ray i), with its expression, and the frame is sorted and stored again.
+// f.src: the frame's offset in the source arena, f.off: in the destination arena (the same arena is
+// allowed: the block holds the whole frame in shared memory before it writes).  ext (optional): per
+// frame the smallest / largest q_a and q_b, from which the host derives the frame's timestamp bounds.
+__global__ void __launch_bounds__(kIngestThreads)
+retime_frames_kernel(const PixelFrame* __restrict__ frames, const double* src_rays, const int32_t* src_orig,
+                     const double2* __restrict__ rowq, double ro, double* rays, int32_t* orig, int32_t* pos,
+                     double4* __restrict__ ext) {
+    __shared__ double s_ts[kMaxRaysPerFrame];
+    __shared__ int s_idx[kMaxRaysPerFrame];
+    __shared__ double s_val[7][kMaxRaysPerFrame];
+    __shared__ double s_ext[kIngestThreads / 32][4];
+    const PixelFrame f = frames[blockIdx.x];
+    RS_ASSERT(f.n >= 0 && f.n <= kMaxRaysPerFrame && f.src >= 0);
+    const double inf = __longlong_as_double(0x7ff0000000000000LL);
+    double qa_lo = inf, qa_hi = -inf, qb_lo = inf, qb_hi = -inf;
+    for (int j = threadIdx.x; j < kMaxRaysPerFrame; j += kIngestThreads) {
+        s_idx[j] = j;
+        if (j >= f.n) s_ts[j] = inf;  // padding sorts last (a slot >= n is never a caller index)
+    }
+    for (int j = threadIdx.x; j < f.n; j += kIngestThreads) {  // stored slot j holds caller ray i
+        const int i = src_orig[f.src + j];
+        RS_ASSERT(i >= 0 && i < f.n);
+        const double* t = src_rays + ((size_t)f.src + (j & ~31)) * 8 + (j & 31);
+        const double2 q = rowq[f.src + i];
+        s_ts[i] = f.ts_a + ro * q.x;      // ingest_pixels_kernel's (core_testcode.cpp:144)
+        s_val[0][i] = f.ts_b + ro * q.y;  // (:145)
+#pragma unroll
+        for (int c = 1; c < 7; ++c) s_val[c][i] = t[32 * (c + 1)];
+        qa_lo = fmin(qa_lo, q.x); qa_hi = fmax(qa_hi, q.x);
+        qb_lo = fmin(qb_lo, q.y); qb_hi = fmax(qb_hi, q.y);
+    }
+    if (ext) {
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            qa_lo = fmin(qa_lo, __shfl_xor_sync(FULL, qa_lo, o)); qa_hi = fmax(qa_hi, __shfl_xor_sync(FULL, qa_hi, o));
+            qb_lo = fmin(qb_lo, __shfl_xor_sync(FULL, qb_lo, o)); qb_hi = fmax(qb_hi, __shfl_xor_sync(FULL, qb_hi, o));
+        }
+        if ((threadIdx.x & 31) == 0) {
+            double* e = s_ext[threadIdx.x >> 5];
+            e[0] = qa_lo; e[1] = qa_hi; e[2] = qb_lo; e[3] = qb_hi;
+        }
+    }
+    __syncthreads();  // the whole frame is staged: from here on the block may overwrite its source
+    if (ext && threadIdx.x == 0) {
+        for (int w = 1; w < kIngestThreads / 32; ++w) {
+            qa_lo = fmin(qa_lo, s_ext[w][0]); qa_hi = fmax(qa_hi, s_ext[w][1]);
+            qb_lo = fmin(qb_lo, s_ext[w][2]); qb_hi = fmax(qb_hi, s_ext[w][3]);
+        }
+        ext[blockIdx.x] = make_double4(qa_lo, qa_hi, qb_lo, qb_hi);
+    }
     ingest_sort_and_store(f, s_ts, s_idx, s_val, rays, orig, pos);
 }
 
@@ -2313,10 +2371,22 @@ void launch_probe_guess(const DeviceData& dd, FrameDesc fd, double delay, int it
 
 void launch_ingest_pixels(const PixelFrame* d_frames, int n_frames, const double* d_points_a,
                           const double* d_points_b, LensDev lens, double image_rows, double* d_rays,
-                          int32_t* d_orig, int32_t* d_pos, cudaStream_t st) {
+                          int32_t* d_orig, int32_t* d_pos, double* d_rowq, cudaStream_t st) {
     if (n_frames <= 0) return;
     ingest_pixels_kernel<<<n_frames, kIngestThreads, 0, st>>>(d_frames, d_points_a, d_points_b, lens,
-                                                               image_rows, d_rays, d_orig, d_pos);
+                                                               image_rows, d_rays, d_orig, d_pos,
+                                                               reinterpret_cast<double2*>(d_rowq));
+    g_launches += 1;
+}
+
+void launch_retime_frames(const PixelFrame* d_frames, int n_frames, const double* d_src_rays,
+                          const int32_t* d_src_orig, const double* d_rowq, double readout, double* d_rays,
+                          int32_t* d_orig, int32_t* d_pos, double* d_ext, cudaStream_t st) {
+    if (n_frames <= 0) return;
+    retime_frames_kernel<<<n_frames, kIngestThreads, 0, st>>>(d_frames, d_src_rays, d_src_orig,
+                                                               reinterpret_cast<const double2*>(d_rowq), readout,
+                                                               d_rays, d_orig, d_pos,
+                                                               reinterpret_cast<double4*>(d_ext));
     g_launches += 1;
 }
 

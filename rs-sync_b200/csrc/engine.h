@@ -146,9 +146,20 @@ struct PixelFrame {
 // One block per frame: undistort both points of every pair (lens_undistort_point, :63-95),
 // rolling-shutter timestamps (:144-145), unit rays (:153-154), sort by ts_a (ties keep the caller's
 // order) and write the frame's tiles and orig / pos planes straight into the device arena.
+// d_rowq: the row-fraction plane, 2 doubles per arena ray; ray i of a frame (caller's order) gets
+// {y_a / image_rows, y_b / image_rows}, the factors of the readout in the timestamps.
 void launch_ingest_pixels(const PixelFrame* d_frames, int n_frames, const double* d_points_a,
                           const double* d_points_b, LensDev lens, double image_rows, double* d_rays,
-                          int32_t* d_orig, int32_t* d_pos, cudaStream_t st);
+                          int32_t* d_orig, int32_t* d_pos, double* d_rowq, cudaStream_t st);
+// Re-time frames ingested from pixels at another readout: one block per frame reads the frame's tiles
+// and orig plane at PixelFrame::src of (d_src_rays, d_src_orig) and its row fractions d_rowq[2 (src +
+// i) ..], recomputes ts = frame_ts + readout * q (ingest_pixels_kernel's expression; PixelFrame::ts_a /
+// ts_b are the frame timestamps), sorts by (ts_a, caller index) and writes tiles and orig / pos at
+// PixelFrame::off of (d_rays, d_orig, d_pos) -- which may be the source arena itself.  d_ext (4 doubles
+// per frame, or null): min q_a, max q_a, min q_b, max q_b of the frame (+inf, -inf for no rays).
+void launch_retime_frames(const PixelFrame* d_frames, int n_frames, const double* d_src_rays,
+                          const int32_t* d_src_orig, const double* d_rowq, double readout, double* d_rays,
+                          int32_t* d_orig, int32_t* d_pos, double* d_ext, cudaStream_t st);
 
 // SetTrackResult for a batch of frames with the sort + transpose on the device: the callers' buffers
 // (ts_a, ts_b: n doubles; rays_a, rays_b: n x 3 doubles, concatenated over frames) are staged as they

@@ -2269,13 +2269,10 @@ void launch_presync_reduce(const double* d_framecost, int F, int D, double* d_co
 void launch_presync_grid(const DeviceData& dd, const FrameDesc* d_frames, int F, int max_n,
                          const double* d_delays, int D, uint64_t seed, uint64_t stream,
                          uint64_t call_no, uint64_t idx_base, double* d_framecost, double* d_costs,
-                         unsigned* d_flags, cudaStream_t st, cudaEvent_t ev_begin, cudaEvent_t ev_end,
-                         const uint64_t* d_frame_call_no, const int* d_win_begin, int n_windows,
-                         int max_chunk, bool simplified) {
-    if (ev_begin && F > 0 && D > 0) cudaEventRecord(ev_begin, st);
+                         unsigned* d_flags, cudaStream_t st, int max_chunk, bool simplified,
+                         const uint64_t* d_frame_call_no, const int* d_win_begin, int n_windows) {
     launch_presync_tasks(dd, d_frames, F, max_n, d_delays, D, seed, stream, call_no, idx_base, d_framecost, F,
                          d_flags, st, d_frame_call_no, max_chunk, simplified);
-    if (ev_end && F > 0 && D > 0) cudaEventRecord(ev_end, st);
     launch_presync_reduce(d_framecost, F, D, d_costs, st, d_win_begin, n_windows);
 }
 

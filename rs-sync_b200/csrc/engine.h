@@ -40,13 +40,12 @@ enum : unsigned { kFlagP = 1u, kFlagM = 2u, kFlagR = 4u, kFlagRho = 8u };
 void launch_presync_grid(const DeviceData& dd, const FrameDesc* d_frames, int F, int max_n,
                          const double* d_delays, int D, uint64_t seed, uint64_t stream,
                          uint64_t call_no, uint64_t idx_base, double* d_framecost, double* d_costs,
-                         unsigned* d_flags, cudaStream_t st, cudaEvent_t ev_begin = nullptr,
-                         cudaEvent_t ev_end = nullptr,
+                         unsigned* d_flags, cudaStream_t st, int max_chunk, bool simplified,
                          // several windows in one grid: the F frames are the windows' frames
                          // concatenated, frame f belongs to the call d_frame_call_no[f], window w
                          // covers frames [d_win_begin[w], d_win_begin[w+1]); d_costs is W x D
                          const uint64_t* d_frame_call_no = nullptr, const int* d_win_begin = nullptr,
-                         int n_windows = 0, int max_chunk = 0, bool simplified = false);
+                         int n_windows = 0);
 
 // How many consecutive delays of the (host copy of the) delay list one work unit of the grid kernel
 // may hold so that the spline window of any frame whose timestamps span at most frame_span_s seconds

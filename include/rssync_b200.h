@@ -47,8 +47,9 @@ int rssync_create(rssync_problem** out);
  * the other devices receive the finished device state (ray arena, spline records) by ncclBroadcast
  * over NVLink when a compute call finds them stale.  PreSync / DebugPreSync / rssync_presync_grid
  * shard the delay grid by offset range (one ncclAllGather of the curve slices per call),
- * rssync_sync_batch* / rssync_presync_windows shard by syncpoint and rssync_orientation_search* by
- * variant (results assembled on the host, where the solver's control loop produces them); every
+ * rssync_sync_batch* / rssync_presync_windows shard by syncpoint, rssync_orientation_search* and
+ * rssync_rotation_search by variant (results assembled on the host, where the solver's control loop
+ * produces them); every
  * result is bit-identical to the single-device one.  A single rssync_sync call runs on devices[0].
  * NCCL (libnccl.so.2) is loaded at run time, only by this call and only when n_devices > 1.
  * Leaves devices[0] the calling thread's current device. */
@@ -179,6 +180,18 @@ int rssync_last_sync_trace(const rssync_problem* p, double* delays, double* step
  * (csrc/spec_trig.h).  Differs from one sequential recurrence with libm by rounding only. */
 int rssync_integrate_gyro(const double* timestamps_s, const double* gyro_xyz, size_t count,
                           const char* orientation, double* quats_out);
+/* rssync_integrate_gyro with the axis mapping given as a 3x3 row-major matrix M (NULL = identity):
+ * w = M g per sample, then the same blocked integration.  Arithmetic of w (part of the contract):
+ * w_c = sum over the j with M[c][j] != 0 of M[c][j] g_j -- terms with a zero coefficient are omitted,
+ * the first kept term is the product, the others are added left to right, without contraction --
+ * and w_c = +0.0 when row c is zero; then a_c = w_c dt.  A gyro_orientation string is the signed
+ * permutation matrix with M[i][src] = +-1 for its character i, and under this rule it gives the string's
+ * bits exactly (signs of zeros and a NaN or inf on an axis it does not read included):
+ * rssync_integrate_gyro(s) == rssync_integrate_gyro_matrix(matrix of s).  Any finite matrix is
+ * accepted (a rotation is the usual case; a diagonal models a gyro gain error); a non-finite entry
+ * gives RSSYNC_E_INVALID.  Host code; the searches run the same arithmetic on the device. */
+int rssync_integrate_gyro_matrix(const double* timestamps_s, const double* gyro_xyz, size_t count,
+                                 const double* matrix, double* quats_out);
 /* The orientation search the reference keeps commented out in core_testcode.cpp:184-233 (README.md:
  * 47-48, guess_orient): for each of n_orient gyro_orientation strings, integrate the raw gyro,
  * ingest it through the variable-rate SetGyroQuaternions (timestamps truncated to integer
@@ -199,6 +212,21 @@ int rssync_orientation_search_ex(rssync_problem* p, const double* timestamps_s, 
                                  double initial_delay, int64_t frame_begin, int64_t frame_end,
                                  double search_step, double search_radius, const uint64_t* call_nos,
                                  double* out_cost, double* out_delay);
+/* The orientation search over n_rot arbitrary axis mappings (n_rot x 9, 3x3 row-major each) in place
+ * of the strings: a search over camera mount rotations (a camera tilted against the gyro that logs it).
+ * Result i equals rssync_integrate_gyro_matrix(matrices + 9 i) -> rssync_set_gyro_var (timestamps
+ * truncated to integer microseconds) -> rssync_presync keyed by call_nos[i] (NULL: the counter, which
+ * advances by n_rot).  out_curves (n_rot x D or NULL): row i = that PreSync's cost over
+ * rssync_presync_delays(initial_delay, search_step, search_radius).  The problem is left holding the
+ * last variant's gyro.  A non-finite matrix entry gives RSSYNC_E_INVALID ("rotation-search: matrix <i>
+ * has a non-finite entry") before anything is done: the counter and the gyro are left as they were.
+ * matrices == NULL with n_rot > 0: RSSYNC_E_INVALID.  Otherwise it behaves as rssync_orientation_search_ex,
+ * errors and multi-device sharding by variant included. */
+int rssync_rotation_search(rssync_problem* p, const double* timestamps_s, const double* gyro_xyz,
+                           size_t count, const double* matrices, int n_rot, double initial_delay,
+                           int64_t frame_begin, int64_t frame_end, double search_step,
+                           double search_radius, const uint64_t* call_nos, double* out_cost,
+                           double* out_delay, double* out_curves);
 
 /* Rolling-shutter readout search: PreSync(initial_delay, frame_begin, frame_end, search_step, search_radius)
  * at each of n_readouts candidate readouts (seconds, as rssync_lens.readout), without re-ingesting.  Every

@@ -1867,7 +1867,7 @@ __global__ void spline_finish_kernel(const double* __restrict__ y, const double*
 }
 
 // ------------------------------------------------------------------------------------------
-// K8: the gyro ingest on the device, for n_var orientation variants at once.
+// K8: the gyro ingest on the device, for n_var gyro axis mappings (3x3 matrices, gyro_scan.h) at once.
 //
 //  * gyro_local / gyro_prefix / gyro_apply: optdata_fill_gyro (core_testcode.cpp:37-53) as a blocked
 //    scan.  q_i = normalise(d_i (x) q_{i-1}) is not associative once every step normalises, so the
@@ -1887,8 +1887,7 @@ __global__ void spline_finish_kernel(const double* __restrict__ y, const double*
 //    components run side by side, which is what the orientation search needs; a single long track is
 //    faster on the host (SetGyroQuaternions' fixed-rate form keeps using it).
 struct OrientDev {
-    int src[3];
-    double sgn[3];
+    double m[9];  // the variant's gyro axis mapping, 3x3 row-major (gyro_scan.h)
 };
 __global__ void gyro_local_kernel(const double* __restrict__ ts, const double* __restrict__ gyro, int n,
                                   const OrientDev* __restrict__ orients, int n_var, double* __restrict__ local) {
@@ -1902,7 +1901,7 @@ __global__ void gyro_local_kernel(const double* __restrict__ ts, const double* _
     const int i1 = min(n, (b + 1) * (int)kGyroScanBlock);
     for (int i = b * (int)kGyroScanBlock; i < i1; ++i) {
         double d[4], q[4];
-        gyro_increment(ts, gyro, (size_t)i, o.src, o.sgn, d);
+        gyro_increment(ts, gyro, (size_t)i, o.m, d);
         quat_mul_normalise(d, prev, q);
         prev[0] = q[0]; prev[1] = q[1]; prev[2] = q[2]; prev[3] = q[3];
         double2* dst = reinterpret_cast<double2*>(out + (size_t)i * 4);
@@ -2425,13 +2424,11 @@ void launch_spline_finish(const double* d_quats, const double* d_rhs, const doub
     g_launches += 1;
 }
 
-void launch_gyro_integrate(const double* d_ts, const double* d_gyro, int n, const int* h_src, const double* h_sgn,
-                           int n_var, void* d_orients, double* d_quats, double* d_prefix, cudaStream_t st) {
+void launch_gyro_integrate(const double* d_ts, const double* d_gyro, int n, const double* h_matrices, int n_var,
+                           void* d_orients, double* d_quats, double* d_prefix, cudaStream_t st) {
     if (n <= 0 || n_var <= 0) return;
-    std::vector<OrientDev> o((size_t)n_var);
-    for (int v = 0; v < n_var; ++v)
-        for (int c = 0; c < 3; ++c) { o[(size_t)v].src[c] = h_src[3 * v + c]; o[(size_t)v].sgn[c] = h_sgn[3 * v + c]; }
-    cudaMemcpyAsync(d_orients, o.data(), sizeof(OrientDev) * (size_t)n_var, cudaMemcpyHostToDevice, st);  // pageable: staged before return
+    static_assert(sizeof(OrientDev) == 9 * sizeof(double), "OrientDev is one 3x3 matrix");
+    cudaMemcpyAsync(d_orients, h_matrices, sizeof(OrientDev) * (size_t)n_var, cudaMemcpyHostToDevice, st);  // pageable: staged before return
     const int nb = (n + (int)kGyroScanBlock - 1) / (int)kGyroScanBlock;
     gyro_local_kernel<<<(nb * n_var + 31) / 32, 32, 0, st>>>(d_ts, d_gyro, n, static_cast<const OrientDev*>(d_orients), n_var, d_quats);
     gyro_prefix_kernel<<<(n_var + 31) / 32, 32, 0, st>>>(d_quats, n, n_var, d_prefix);

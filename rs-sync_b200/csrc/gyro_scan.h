@@ -11,13 +11,30 @@ namespace rs {
 
 constexpr size_t kGyroScanBlock = 512;  // samples per block of the blocked recurrence
 
-// d_0 = identity; src / sgn: the gyro_orientation mapping (source axis and sign per output axis)
-RS_TRIG_HD void gyro_increment(const double* ts, const double* gyro, size_t i, const int src[3],
-                               const double sgn[3], double d[4]) {
+// The gyro axis mapping is a 3x3 row-major matrix m: the angular velocity in the integration's frame
+// is w = m g.  Its arithmetic (part of the contract, DESIGN.md section 3.8): w_c sums m[3c+j] g_j over
+// the j with m[3c+j] != 0 only; the first kept term is the product, the others are added to it left to
+// right, without contraction; a row without a non-zero coefficient gives w_c = +0.0.  A signed
+// permutation matrix therefore gives w_c = (+-1 g_src) bit for bit, the sign of a zero and a NaN or inf
+// on an axis it does not read included.
+RS_TRIG_HD double gyro_map_row(const double* row, const double* g) {
+    double w = 0.0;
+    bool kept = false;
+    for (int j = 0; j < 3; ++j)
+        if (row[j] != 0.0) {
+            const double t = row[j] * g[j];
+            w = kept ? w + t : t;
+            kept = true;
+        }
+    return w;
+}
+
+// d_0 = identity; d_i = quat_from_aa((m g_i) (t_i - t_{i-1}))
+RS_TRIG_HD void gyro_increment(const double* ts, const double* gyro, size_t i, const double m[9], double d[4]) {
     if (i == 0) { d[0] = 1.0; d[1] = 0.0; d[2] = 0.0; d[3] = 0.0; return; }
     const double dt = ts[i] - ts[i - 1];
-    const double a0 = sgn[0] * gyro[3 * i + src[0]] * dt, a1 = sgn[1] * gyro[3 * i + src[1]] * dt,
-                 a2 = sgn[2] * gyro[3 * i + src[2]] * dt;
+    const double* g = gyro + 3 * i;
+    const double a0 = gyro_map_row(m, g) * dt, a1 = gyro_map_row(m + 3, g) * dt, a2 = gyro_map_row(m + 6, g) * dt;
     const double th2 = (a0 * a0 + a1 * a1) + a2 * a2;
     if (th2 > 0.) {
         const double th = trig_detail::sqrt_(th2), half = th * 0.5, k = spec_sin(half) / th;

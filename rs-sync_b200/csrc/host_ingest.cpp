@@ -121,26 +121,21 @@ void build_spline_system(const double* quats, size_t n, double* rhs, double* dia
     }
 }
 
-bool parse_orientation(const char* orient, int src[3], double sgn[3]) {
-    src[0] = 0; src[1] = 1; src[2] = 2;
-    sgn[0] = sgn[1] = sgn[2] = 1.0;
+bool parse_orientation(const char* orient, double m[9]) {
+    for (int k = 0; k < 9; ++k) m[k] = (k % 4 == 0) ? 1.0 : 0.0;
     if (!orient) return true;
     for (int i = 0; i < 3; ++i) {
         const char ch = orient[i];
         const char lo = (char)(ch | 0x20);
         if (lo < 'x' || lo > 'z') return false;
-        src[i] = lo - 'x';
-        sgn[i] = (ch == lo) ? -1.0 : 1.0;
+        m[3 * i + 0] = m[3 * i + 1] = m[3 * i + 2] = 0.0;
+        m[3 * i + (lo - 'x')] = (ch == lo) ? -1.0 : 1.0;
     }
     return orient[3] == 0;
 }
 
-bool integrate_gyro(const double* ts, const double* gyro, size_t count, const char* orient,
-                    double* out) {
-    int src[3];
-    double sgn[3];
-    if (!parse_orientation(orient, src, sgn)) return false;
-    if (count == 0) return true;
+void integrate_gyro(const double* ts, const double* gyro, size_t count, const double m[9], double* out) {
+    if (count == 0) return;
     // The contract's order of operations (the device kernels of engine.cu follow the same one, see
     // gyro_local_kernel): the recurrence runs inside blocks of kGyroScanBlock samples, each from the
     // identity; the blocks' last values are chained into per-block prefixes; every sample is its
@@ -153,7 +148,7 @@ bool integrate_gyro(const double* ts, const double* gyro, size_t count, const ch
         const double* prev = ident;
         for (size_t i = b * B; i < std::min(count, (b + 1) * B); ++i) {
             double d[4];
-            gyro_increment(ts, gyro, i, src, sgn, d);
+            gyro_increment(ts, gyro, i, m, d);
             quat_mul_normalise(d, prev, &local[4 * i]);
             prev = &local[4 * i];
         }
@@ -162,7 +157,6 @@ bool integrate_gyro(const double* ts, const double* gyro, size_t count, const ch
     for (size_t b = 0; b < nb; ++b)
         quat_mul_normalise(&local[4 * (std::min(count, (b + 1) * B) - 1)], &prefix[4 * b], &prefix[4 * (b + 1)]);
     for (size_t i = 0; i < count; ++i) quat_mul_normalise(&local[4 * i], &prefix[4 * (i / B)], out + 4 * i);
-    return true;
 }
 
 // SyncProblemPrivate::SetGyroQuaternions(const int64_t*, const double*, size_t),

@@ -113,6 +113,36 @@ int rssync_set_track_pixels_device(rssync_problem* p, size_t n_frames, const int
                                    const double* frame_ts_b, const double* points_a,
                                    const double* points_b, const rssync_lens* lens,
                                    double image_rows, void* stream);
+/* SetTrackResult for n_frames frames whose rays the caller computed (any camera model), with the
+ * rolling-shutter timestamps formed here from per-ray row fractions.  Ray k of frame i gets
+ * ts_a = frame_ts_a[i] + readout * frac_a[k] (ts_b alike): one multiply and one add, not contracted,
+ * the expression of the pixels forms with the caller's fraction in place of y / image_rows.  The fraction
+ * is usually y / image_rows; any finite value is accepted (x / width for a sensor read along columns).
+ * counts / frames and the per-ray buffers use rssync_set_track_batch's layouts: frac_a / frac_b 1 double
+ * per ray, rays_a / rays_b 3, concatenated in `frames` order.
+ * Afterwards the problem holds, byte for byte, what rssync_set_track_batch with those timestamps gives
+ * (frame table, arena tiles, orig / pos) and every later call returns what it would return on that
+ * problem.  The frames also keep their row fractions and frame timestamps, so rssync_readout_search and
+ * rssync_set_readout accept them, alone or beside pixel-ingested frames; a frame that a rays form or an
+ * adoption overwrites later loses them.  A frame id given more than once: the last occurrence wins.
+ * Everything is checked before anything is applied: a null argument, a count above 512 or a non-finite
+ * readout: RSSYNC_E_INVALID; then non-finite frame timestamps (as rssync_set_track_pixels); then, frame
+ * by frame, the first frame holding a non-finite value fails with rssync_set_track_batch's code and
+ * message for rays_a, rays_b, ts_a, ts_b in that order, where a non-finite fraction, or a timestamp that
+ * overflows, counts as a non-finite ts. */
+int rssync_set_track_row_fractions(rssync_problem* p, size_t n_frames, const int64_t* frames,
+                                   const size_t* counts, const double* frame_ts_a, const double* frame_ts_b,
+                                   const double* frac_a, const double* frac_b,
+                                   const double* rays_a, const double* rays_b, double readout);
+/* The same with frac_a / frac_b / rays_a / rays_b in device memory of the problem's (primary) device;
+ * frames, counts and the frame timestamps stay on the host.  Same ordering / borrow contract as
+ * rssync_set_track_batch_device; a per-ray buffer that is not device (or managed) memory of the
+ * problem's device: RSSYNC_E_INVALID.  Results are bit-identical to the host form. */
+int rssync_set_track_row_fractions_device(rssync_problem* p, size_t n_frames, const int64_t* frames,
+                                          const size_t* counts, const double* frame_ts_a,
+                                          const double* frame_ts_b, const double* frac_a,
+                                          const double* frac_b, const double* rays_a, const double* rays_b,
+                                          double readout, void* stream);
 /* PreSync(initial_delay, frame_begin, frame_end, search_step, search_radius) -> {cost, delay}
  *                                                                  rssync.h:19-21 */
 int rssync_presync(rssync_problem* p, double initial_delay, int64_t frame_begin, int64_t frame_end,
@@ -230,11 +260,12 @@ int rssync_rotation_search(rssync_problem* p, const double* timestamps_s, const 
 
 /* Rolling-shutter readout search: PreSync(initial_delay, frame_begin, frame_end, search_step, search_radius)
  * at each of n_readouts candidate readouts (seconds, as rssync_lens.readout), without re-ingesting.  Every
- * frame in [frame_begin, frame_end) must have been ingested by rssync_set_track_pixels(_device) and not
- * been overwritten by a rays form or adopted since (else RSSYNC_E_STATE naming the frame): those keep
- * y / image_rows of every ray on the device and their frame timestamps on the host.  Result j equals,
- * bit for bit, rssync_presync on a problem that ingested the same pixels, lens, image rows and frame
- * timestamps with lens.readout = readouts[j], keyed by RNG call number call_nos[j] (NULL: consecutive
+ * frame in [frame_begin, frame_end) must have been ingested by rssync_set_track_pixels(_device) or
+ * rssync_set_track_row_fractions(_device) and not been overwritten by a rays form or adopted since (else
+ * RSSYNC_E_STATE naming the frame): those keep the row fraction of every ray (y / image_rows, or the
+ * caller's) on the device and their frame timestamps on the host.  Result j equals, bit for bit,
+ * rssync_presync on a problem that ingested the same input (pixels, lens and image rows, or rays and row
+ * fractions) and frame timestamps with readout = readouts[j], keyed by RNG call number call_nos[j] (NULL: consecutive
  * values of the problem's counter, which then advances by n_readouts); out_curves (n_readouts x D, or
  * NULL) row j is that call's cost over rssync_presync_delays(initial_delay, search_step, search_radius).
  * The problem's arena, frame table and gyro are left as they are.  A non-finite readout or n_readouts < 0:
@@ -244,10 +275,10 @@ int rssync_rotation_search(rssync_problem* p, const double* timestamps_s, const 
 int rssync_readout_search(rssync_problem* p, const double* readouts, int n_readouts, double initial_delay,
                           int64_t frame_begin, int64_t frame_end, double search_step, double search_radius,
                           const uint64_t* call_nos, double* out_cost, double* out_delay, double* out_curves);
-/* Apply a readout: re-time the pixel-ingested frames of [frame_begin, frame_end) in place, so that the
- * problem holds, byte for byte, what ingesting them with lens.readout = readout gives (arena tiles, orig /
- * pos, frame table) and every later call returns what it would return on that problem.  Frames ingested
- * later use the lens of their own call.  Errors as rssync_readout_search's. */
+/* Apply a readout: re-time the frames of [frame_begin, frame_end), ingested from pixels or row fractions,
+ * in place, so that the problem holds, byte for byte, what ingesting them with readout = readout gives
+ * (arena tiles, orig / pos, frame table) and every later call returns what it would return on that
+ * problem.  Frames ingested later use the readout of their own call.  Errors as rssync_readout_search's. */
 int rssync_set_readout(rssync_problem* p, double readout, int64_t frame_begin, int64_t frame_end);
 
 /* Pinned RNG of the randomised translation estimator (replaces the reference's

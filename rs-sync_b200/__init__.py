@@ -42,6 +42,7 @@ C_ABI_SYMBOLS = [
     "rssync_set_loss_mode", "rssync_probe_spec_trig",
     "rssync_set_track_batch_device", "rssync_set_track_pixels_device",
     "rssync_readout_search", "rssync_set_readout", "rssync_integrate_gyro_matrix", "rssync_rotation_search",
+    "rssync_set_track_row_fractions", "rssync_set_track_row_fractions_device",
 ]
 # Itanium-ABI symbols of the C++ drop-in face (same set the reference's librssync_core exports)
 CXX_ABI_SYMBOLS = [
@@ -128,6 +129,11 @@ def load_library():
     L.rssync_set_track_batch_device.argtypes = [P, C.c_size_t, c_i64_p, C.POINTER(C.c_size_t), P, P, P, P, P]
     L.rssync_set_track_pixels_device.argtypes = [P, C.c_size_t, c_i64_p, C.POINTER(C.c_size_t), c_double_p,
                                                  c_double_p, P, P, C.POINTER(Lens), C.c_double, P]
+    L.rssync_set_track_row_fractions.argtypes = [P, C.c_size_t, c_i64_p, C.POINTER(C.c_size_t), c_double_p,
+                                                 c_double_p, c_double_p, c_double_p, c_double_p, c_double_p,
+                                                 C.c_double]
+    L.rssync_set_track_row_fractions_device.argtypes = [P, C.c_size_t, c_i64_p, C.POINTER(C.c_size_t), c_double_p,
+                                                        c_double_p, P, P, P, P, C.c_double, P]
     L.rssync_presync.argtypes = [P, C.c_double, C.c_int64, C.c_int64, C.c_double, C.c_double, c_double_p, c_double_p]
     L.rssync_sync.argtypes = [P, C.c_double, C.c_int64, C.c_int64, C.c_double, C.c_double, c_double_p, c_double_p]
     L.rssync_debug_presync.argtypes = [P, C.c_double, C.c_int64, C.c_int64, C.c_double, c_double_p, c_double_p, C.c_int]
@@ -509,6 +515,26 @@ class SyncProblem:
         pa, pb = _f64(points_a), _f64(points_b)
         self._check(self.L.rssync_set_track_pixels(*args, _dp(pa), _dp(pb), C.byref(lens_c), float(image_rows)))
 
+    def set_track_row_fractions(self, frames, counts, frame_ts_a, frame_ts_b, frac_a, frac_b, rays_a, rays_b,
+                                readout):
+        """set_track_batch for rays the caller computed with its own camera model, with the timestamps
+        formed here: ts = frame_ts + readout * frac per ray (frac usually y / image_rows).  The frames keep
+        their row fractions, so readout_search / set_readout accept them.  frac_a / frac_b (1 value per
+        ray) and rays_a / rays_b (3 per ray) may all be torch CUDA tensors (as in set_track_batch);
+        frames, counts and frame_ts_a / frame_ts_b stay on the host."""
+        fr = np.ascontiguousarray(frames, dtype=np.int64)
+        cn = np.ascontiguousarray(counts, dtype=np.uint64)
+        ta, tb = _f64(frame_ts_a), _f64(frame_ts_b)
+        args = (self.h, fr.shape[0], fr.ctypes.data_as(c_i64_p), cn.ctypes.data_as(C.POINTER(C.c_size_t)), _dp(ta),
+                _dp(tb))
+        if _cuda_tensors(frac_a, frac_b, rays_a, rays_b):
+            n = int(cn.sum())
+            ptrs, stream = _device_ptrs((frac_a, frac_b, rays_a, rays_b), (n, n, 3 * n, 3 * n))
+            self._check(self.L.rssync_set_track_row_fractions_device(*args, *ptrs, float(readout), stream))
+            return
+        a = [_f64(x) for x in (frac_a, frac_b, rays_a, rays_b)]
+        self._check(self.L.rssync_set_track_row_fractions(*args, *[_dp(x) for x in a], float(readout)))
+
     def load(self, w, bulk=False):
         """Feed a synth.Workload the way core_testcode feeds a video (core_testcode.cpp:257-268)."""
         self.SetGyroQuaternions(w.quats, w.quats.shape[0], w.gyro_rate, w.gyro_t0)
@@ -573,8 +599,8 @@ class SyncProblem:
 
     def readout_search(self, readouts, initial_delay, frame_begin, frame_end, search_step, search_radius,
                        call_nos=None, curves=False):
-        """PreSync at every candidate rolling-shutter readout (seconds) over frames ingested from pixels,
-        without re-ingesting them (rssync_readout_search).  Returns (costs, delays), plus the n x D cost
+        """PreSync at every candidate rolling-shutter readout (seconds) over frames ingested from pixels
+        or row fractions, without re-ingesting them (rssync_readout_search).  Returns (costs, delays), plus the n x D cost
         curves over presync_delays(...) when curves=True.  call_nos: explicit RNG call number per readout
         (the problem's counter is then left alone)."""
         r = _f64(readouts).ravel()
@@ -596,8 +622,8 @@ class SyncProblem:
         return (costs, delays, cv) if curves else (costs, delays)
 
     def set_readout(self, readout, frame_begin, frame_end):
-        """Re-time the pixel-ingested frames of [frame_begin, frame_end) at `readout` (seconds) in place,
-        as if they had been ingested with lens.readout = readout (rssync_set_readout)."""
+        """Re-time the frames of [frame_begin, frame_end), ingested from pixels or row fractions, at
+        `readout` (seconds) in place, as if they had been ingested with that readout (rssync_set_readout)."""
         self._check(self.L.rssync_set_readout(self.h, float(readout), int(frame_begin), int(frame_end)))
 
     def device_count(self):

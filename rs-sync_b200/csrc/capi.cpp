@@ -2506,6 +2506,180 @@ int rssync_set_track_pixels_device(rssync_problem* p, size_t n_frames, const int
     return end_device_ingest(p);
 }
 
+}  // extern "C"
+
+namespace {
+
+const char* const kMsgRowFractionsNull = "set-track-row-fractions: null argument";
+
+// the row-fractions forms' counts and readout
+int check_row_fraction_args(rssync_problem* p, size_t n_frames, const size_t* counts, double readout,
+                            std::vector<size_t>& at) {
+    if (int rc = frame_offsets(p, n_frames, counts, at)) return rc;
+    if (!std::isfinite(readout)) {
+        p->err = "set-track-row-fractions: non-finite readout";
+        return RSSYNC_E_INVALID;
+    }
+    return RSSYNC_OK;
+}
+
+// The row-fractions forms once every frame has passed its checks: place the last occurrence of each frame
+// id (an ingest block per occurrence would write the same arena range twice), fill its ingest record
+// (rec[0..k)), keep its frame timestamps for re-timing, and make room for the arena and the row-fraction
+// plane.  lo / hi: each frame's timestamp bounds.
+int place_row_fraction_frames(rssync_problem* p, size_t n_frames, const int64_t* frames, const size_t* counts,
+                              const std::vector<size_t>& at, const double* frame_ts_a, const double* frame_ts_b,
+                              const std::vector<double>& lo, const std::vector<double>& hi, rs::PixelFrame* rec,
+                              size_t& k) {
+    std::vector<char> last(n_frames, 0);
+    {
+        std::unordered_set<int64_t> seen;
+        for (size_t i = n_frames; i-- > 0;) last[i] = seen.insert(frames[i]).second;
+    }
+    p->version++;
+    k = 0;
+    for (size_t i = 0; i < n_frames; ++i) {
+        if (!last[i]) continue;
+        FrameDesc* fd = nullptr;
+        if (int rc = place_track(p, frames[i], counts[i], &fd, /*host_mirror=*/false)) return rc;
+        fd->ts_lo = lo[i];
+        fd->ts_hi = hi[i];
+        rec[k++] = rs::PixelFrame{fd->off, fd->n, (int64_t)at[i], frame_ts_a[i], frame_ts_b[i]};
+        p->retime[frames[i]] = {frame_ts_a[i], frame_ts_b[i]};
+    }
+    if (int rc = reserve_device_arena(p)) return rc;
+    return reserve_rowq(p);
+}
+
+}  // namespace
+
+extern "C" {
+
+// SetTrackResult with the rolling-shutter timestamps formed from the caller's row fractions.  Like
+// rssync_set_track_pixels: one pass on the worker pool checks every frame while it copies it into the
+// pinned staging block and takes its timestamp bounds, then one upload and one ingest launch.  Staging
+// block, in doubles: [records: 4 per frame][frac_a n][frac_b n][rays_a 3n][rays_b 3n], the part after the
+// records in ingest_rays_kernel's layout.
+int rssync_set_track_row_fractions(rssync_problem* p, size_t n_frames, const int64_t* frames, const size_t* counts,
+                                   const double* frame_ts_a, const double* frame_ts_b, const double* frac_a,
+                                   const double* frac_b, const double* rays_a, const double* rays_b,
+                                   double readout) {
+    RS_NVTX_RANGE();
+    if (!p) return RSSYNC_E_INVALID;
+    if (n_frames == 0) return RSSYNC_OK;
+    if (!frames || !counts || !frame_ts_a || !frame_ts_b || !frac_a || !frac_b || !rays_a || !rays_b ||
+        n_frames > (size_t)INT32_MAX) {
+        p->err = kMsgRowFractionsNull;
+        return RSSYNC_E_INVALID;
+    }
+    std::vector<size_t> at;
+    if (int rc = check_row_fraction_args(p, n_frames, counts, readout, at)) return rc;
+    const size_t total = at[n_frames];
+    if (int rc = check_frame_ts(p, n_frames, frame_ts_a, frame_ts_b)) return rc;
+    CUDA_TRY(p, cudaSetDevice(p->device));
+    if (int rc = wait_arena_copies(p)) return rc;  // an earlier call's staging block is free again
+    // frames set one by one before this call are older than it: their upload goes first
+    if (!p->pending.empty()) {
+        if (int rc = flush(p)) return rc;
+    } else if (int rc = wait_in_flight(p)) {
+        return rc;
+    }
+    const size_t block = 4 * n_frames + 8 * total;
+    CUDA_TRY(p, p->h_stage.reserve(block + 1));
+    double* h_fa = p->h_stage.ptr + 4 * n_frames;
+    double* h_fb = h_fa + total;
+    double* h_ra = h_fb + total;
+    double* h_rb = h_ra + 3 * total;
+    std::vector<int> bad(n_frames, 0);  // 1 + the first buffer (kRaysA .. kTsB) holding a non-finite value
+    std::vector<double> lo(n_frames, 0.0), hi(n_frames, 0.0);
+    parallel_frames(n_frames, [&](size_t i, size_t) {
+        const size_t a0 = at[i], n = counts[i];
+        const bool ok_ra = copy_checked(h_ra + 3 * a0, rays_a + 3 * a0, 3 * n, nullptr, nullptr);
+        const bool ok_rb = copy_checked(h_rb + 3 * a0, rays_b + 3 * a0, 3 * n, nullptr, nullptr);
+        const double fa = frame_ts_a[i], fb = frame_ts_b[i];
+        bool ok_ta = true, ok_tb = true;
+        double l = 0.0, h = 0.0;
+        for (size_t k = 0; k < n; ++k) {
+            const double qa = frac_a[a0 + k], qb = frac_b[a0 + k];
+            h_fa[a0 + k] = qa;
+            h_fb[a0 + k] = qb;
+            // ingest_rays_kernel's expression (host code is built without contraction); a non-finite q
+            // gives a non-finite timestamp, since the readout is finite
+            const double ta = fa + readout * qa, tb = fb + readout * qb;
+            ok_ta = ok_ta && std::isfinite(ta);
+            ok_tb = ok_tb && std::isfinite(tb);
+            if (k == 0) l = h = ta;
+            l = ta < l ? ta : l;
+            h = ta > h ? ta : h;
+            l = tb < l ? tb : l;
+            h = tb > h ? tb : h;
+        }
+        lo[i] = l;
+        hi[i] = h;
+        // rssync_set_track_batch's order of checks (core_private.cpp:199-202)
+        bad[i] = !ok_ra ? 1 + kRaysA : !ok_rb ? 1 + kRaysB : !ok_ta ? 1 + kTsA : !ok_tb ? 1 + kTsB : 0;
+    });
+    for (size_t i = 0; i < n_frames; ++i)
+        if (bad[i]) {
+            p->err = kMsgNonFinite[bad[i] - 1];
+            return RSSYNC_E_NONFINITE;
+        }
+    rs::PixelFrame* rec = reinterpret_cast<rs::PixelFrame*>(p->h_stage.ptr);
+    size_t k = 0;
+    if (int rc = place_row_fraction_frames(p, n_frames, frames, counts, at, frame_ts_a, frame_ts_b, lo, hi, rec, k))
+        return rc;
+    CUDA_TRY(p, p->d_stage.reserve(block + 1));
+    if (int rc = h2d(p, p->d_stage.ptr, p->h_stage.ptr, block * sizeof(double))) return rc;
+    const double* d_fa = p->d_stage.ptr + 4 * n_frames;
+    rs::launch_ingest_row_fractions(reinterpret_cast<const rs::PixelFrame*>(p->d_stage.ptr), (int)k, d_fa,
+                                    d_fa + total, d_fa + 2 * total, d_fa + 5 * total, readout, p->d_rays.ptr,
+                                    p->d_orig.ptr, p->d_pos.ptr, p->d_rowq.ptr, p->stream);
+    return end_device_ingest(p);
+}
+
+// rssync_set_track_row_fractions with the per-ray buffers in device memory: the check, the timestamp
+// bounds and the copy into the staging buffer run on the device (stage_tracks_kernel); as in the host
+// form, everything is checked before anything is placed.
+int rssync_set_track_row_fractions_device(rssync_problem* p, size_t n_frames, const int64_t* frames,
+                                          const size_t* counts, const double* frame_ts_a, const double* frame_ts_b,
+                                          const double* frac_a, const double* frac_b, const double* rays_a,
+                                          const double* rays_b, double readout, void* stream) {
+    RS_NVTX_RANGE();
+    if (!p) return RSSYNC_E_INVALID;
+    if (n_frames == 0) return RSSYNC_OK;
+    if (!frames || !counts || !frame_ts_a || !frame_ts_b || n_frames > (size_t)INT32_MAX) {
+        p->err = kMsgRowFractionsNull;
+        return RSSYNC_E_INVALID;
+    }
+    std::vector<size_t> at;
+    if (int rc = check_row_fraction_args(p, n_frames, counts, readout, at)) return rc;
+    const size_t total = at[n_frames];
+    if (int rc = check_device_buffers(p, {frac_a, frac_b, rays_a, rays_b}, total)) return rc;
+    if (int rc = check_frame_ts(p, n_frames, frame_ts_a, frame_ts_b)) return rc;
+    DeviceStaging s;
+    if (int rc = begin_device_staging(p, at, 8 * total, frame_ts_a, frame_ts_b, stream, s)) return rc;
+    rs::launch_stage_row_fractions(s.d_at, s.d_fts, (int)n_frames, (int64_t)total, rays_a, rays_b, frac_a, frac_b,
+                                   readout, s.d_data, s.d_info, p->stream);
+    if (int rc = read_stage_info(p, n_frames, s)) return rc;
+    std::vector<double> lo(n_frames), hi(n_frames);
+    for (size_t i = 0; i < n_frames; ++i) {
+        if (s.h_info[i].bad) {
+            p->err = kMsgNonFinite[__builtin_ctz(s.h_info[i].bad)];
+            return RSSYNC_E_NONFINITE;
+        }
+        lo[i] = s.h_info[i].lo;
+        hi[i] = s.h_info[i].hi;
+    }
+    size_t k = 0;
+    if (int rc = place_row_fraction_frames(p, n_frames, frames, counts, at, frame_ts_a, frame_ts_b, lo, hi, s.h_rec, k))
+        return rc;
+    if (int rc = h2d(p, s.d_rec, s.h_rec, k * sizeof(rs::PixelFrame))) return rc;
+    rs::launch_ingest_row_fractions(s.d_rec, (int)k, s.d_data, s.d_data + total, s.d_data + 2 * total,
+                                    s.d_data + 5 * total, readout, p->d_rays.ptr, p->d_orig.ptr, p->d_pos.ptr,
+                                    p->d_rowq.ptr, p->stream);
+    return end_device_ingest(p);
+}
+
 int rssync_set_kernel_timing(rssync_problem* p, int enabled) {
     if (!p) return RSSYNC_E_INVALID;
     if (enabled && !p->ev0) {
@@ -2862,13 +3036,13 @@ int check_readouts(rssync_problem* p, const double* readouts, int n, const char*
     return RSSYNC_OK;
 }
 
-// every frame of `sel` can be re-timed: it was ingested from pixels and not overwritten since
+// every frame of `sel` can be re-timed: it was ingested from pixels or row fractions and not overwritten since
 int require_retime(rssync_problem* p, const std::vector<FrameDesc>& sel, const char* who) {
     for (const FrameDesc& fd : sel)
         if (!p->retime.count(fd.id)) {
             p->err = std::string(who) + ": frame " + std::to_string(fd.id) +
-                     " has no row fractions to re-time (it was not ingested from pixels, or was overwritten or"
-                     " adopted since)";
+                     " has no row fractions to re-time (it was not ingested by a pixels or row-fractions form,"
+                     " or was overwritten or adopted since)";
             return RSSYNC_E_STATE;
         }
     return RSSYNC_OK;

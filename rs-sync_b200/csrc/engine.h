@@ -167,6 +167,13 @@ void launch_retime_frames(const PixelFrame* d_frames, int n_frames, const double
 void launch_ingest_rays(const PixelFrame* d_frames, int n_frames, const double* d_ts_a,
                         const double* d_ts_b, const double* d_rays_a, const double* d_rays_b,
                         double* d_rays, int32_t* d_orig, int32_t* d_pos, cudaStream_t st);
+// The same with row fractions in place of the timestamps (d_frac_a / d_frac_b: 1 double per ray): ray i
+// gets ts = PixelFrame::ts_a + readout * frac_a[i] (ts_b alike), ingest_pixels_kernel's expression, and
+// d_rowq its {frac_a, frac_b} as launch_ingest_pixels writes them.
+void launch_ingest_row_fractions(const PixelFrame* d_frames, int n_frames, const double* d_frac_a,
+                                 const double* d_frac_b, const double* d_rays_a, const double* d_rays_b,
+                                 double readout, double* d_rays, int32_t* d_orig, int32_t* d_pos, double* d_rowq,
+                                 cudaStream_t st);
 
 // ---- track buffers the caller holds in device memory (rssync_set_track_*_device) ---------------
 // What the check-and-stage kernel reports per frame; the host reads these back and places the frames.
@@ -189,6 +196,13 @@ void launch_stage_rays(const int64_t* d_at, int n_frames, int64_t total, const d
 void launch_stage_points(const int64_t* d_at, const double* d_frame_ts, int n_frames, int64_t total,
                          const double* points_a, const double* points_b, double readout, double rows,
                          double* d_stage, StageInfo* d_info, cudaStream_t st);
+// Row-fractions form: src = {rays_a, rays_b, frac_a, frac_b} (3, 3, 1, 1 doubles per ray); d_stage holds
+// frac_a, frac_b, rays_a, rays_b (the rays form's layout, fractions in the ts slots); bit 2 / 3 is also
+// set when frame_ts + readout * frac is not finite; lo / hi over those timestamps.
+void launch_stage_row_fractions(const int64_t* d_at, const double* d_frame_ts, int n_frames, int64_t total,
+                                const double* rays_a, const double* rays_b, const double* frac_a,
+                                const double* frac_b, double readout, double* d_stage, StageInfo* d_info,
+                                cudaStream_t st);
 
 // ---- stage probes (tests only) ---------------------------------------------------------------
 void launch_probe_problem_matrix(const DeviceData& dd, FrameDesc fd, double delay, double* d_P,

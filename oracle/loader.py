@@ -83,7 +83,9 @@ def lib():
     L.orc_problem_matrix.argtypes = [C.c_void_p, C.c_int64, C.c_double, c_double_p]
     L.orc_guess_motion.argtypes = [C.c_void_p, C.c_int64, C.c_double, C.c_int, C.c_uint64, C.c_uint64,
                                    C.c_uint64, c_double_p, c_double_p]
-    L.orc_loss3.argtypes = [C.c_void_p, C.c_int64, C.c_double, c_double_p, C.c_double, c_double_p]
+    L.orc_estimator_trace.argtypes = [C.c_void_p, C.c_int64, C.c_double, C.c_int, C.c_uint64, C.c_uint64,
+                                      C.c_uint64, c_double_p, c_double_p, C.POINTER(C.c_int)]
+    L.orc_loss3.argtypes =[C.c_void_p, C.c_int64, C.c_double, c_double_p, C.c_double, c_double_p]
     L.orc_loss5.argtypes = [C.c_void_p, C.c_int64, C.c_double, c_double_p, C.c_double, c_double_p, c_double_p]
     L.orc_lbfgs.argtypes = [C.c_void_p, C.c_int64, C.c_double, c_double_p, C.c_double, c_double_p,
                             C.POINTER(C.c_int), C.POINTER(C.c_int)]
@@ -256,6 +258,16 @@ class OracleProblem:
         k = C.c_double()
         self._check(self.L.orc_guess_motion(self.h, frame, delay, iters, stream, call_no, offset_idx, _dp(m), C.byref(k)))
         return m, k.value
+
+    def estimator_trace(self, frame, delay, iters, stream, call_no, offset_idx):
+        """guess_motion with every hypothesis kept -> (hypotheses (iters, 3), exact quartiles (iters,),
+        index of the winner: the first strict minimum)"""
+        v = np.empty((iters, 3))
+        q = np.empty(iters)
+        best = C.c_int()
+        self._check(self.L.orc_estimator_trace(self.h, frame, delay, iters, stream, call_no, offset_idx, _dp(v),
+                                               _dp(q), C.byref(best)))
+        return v, q, best.value
 
     def loss3(self, frame, delay, m, k):
         m = np.ascontiguousarray(m, dtype=np.float64)

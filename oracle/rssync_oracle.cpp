@@ -826,6 +826,42 @@ int orc_guess_motion(void* h, int64_t frame, double delay, int iters, uint64_t s
                          : clamp_k(1.0 / norm_PM(P.data(), f.n, f.order.data(), m) * 1e2);
     return OK;
 }
+// guess_motion's spec-mode loop with every hypothesis kept: v_out[3 t..3 t + 2] the hypothesis of
+// iteration t, q_out[t] its exact quartile r2[n/4], *best the index of the first strict minimum (the
+// one guess_motion returns).  Lets the tests check what a frame built to tie actually ties.
+int orc_estimator_trace(void* h, int64_t frame, double delay, int iters, uint64_t stream,
+                        uint64_t call_no, uint64_t offset_idx, double* v_out, double* q_out, int* best) {
+    Oracle& o = *(Oracle*)h;
+    auto it = o.frames.find(frame);
+    if (it == o.frames.end()) { o.err = "no such frame"; return E_INVALID; }
+    const Frame& f = it->second;
+    const int n = f.n;
+    std::vector<double> P((size_t)n * 3), nP((size_t)n * 3), r2(n);
+    problem_matrix(o, f, delay, P.data());
+    const uint64_t key = rng_task_key(o.seed, stream, call_no, offset_idx, frame);
+    for (int i = 0; i < n; ++i) safe_normalize3(&P[3 * i], &nP[3 * i]);
+    double least = std::numeric_limits<double>::infinity();
+    *best = 0;
+    for (int t = 0; t < iters; ++t) {
+        uint32_t a = rng_index(key, t, 0, n);
+        uint32_t b, k = 1;
+        do { b = rng_index(key, t, k++, n); } while (b == a);
+        const double* pa = &P[3 * a];
+        const double* pb = &P[3 * b];
+        double c[3] = {hyp_cross_term(pa[1], pb[2], pa[2] * pb[1]), hyp_cross_term(pa[2], pb[0], pa[0] * pb[2]),
+                       hyp_cross_term(pa[0], pb[1], pa[1] * pb[0])};
+        double* v = v_out + 3 * t;
+        safe_normalize3(c, v);
+        for (int i = 0; i < n; ++i) {
+            double r = dot3(&nP[3 * i], v);
+            r2[i] = r * r;
+        }
+        std::nth_element(r2.begin(), r2.begin() + n / 4, r2.end());
+        q_out[t] = r2[n / 4];
+        if (q_out[t] < least) { least = q_out[t]; *best = t; }
+    }
+    return OK;
+}
 int orc_loss3(void* h, int64_t frame, double delay, const double* m, double k, double* out) {
     Oracle& o = *(Oracle*)h;
     auto it = o.frames.find(frame);

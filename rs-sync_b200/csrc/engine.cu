@@ -555,8 +555,11 @@ __device__ __forceinline__ unsigned warp_select32(const float (&s)[SLOTS], int k
 // The tournament's inputs: the frame's rows, row-normalised, in fp32, in registers -- lane l holds
 // the three components of its SLOTS rays.  Any accuracy the margin covers will do, so the norm is
 // taken with rsqrt.approx (rel. error <= 2^-22.4).  Rows that safe_normalize would leave unscaled
-// (|row| < 1e-12, also out of fp32 range) and non-finite rows poison `fin`: returns false, and the
-// task goes to the exact estimator.  Rows past the frame's last ray (zero rows) become +0 keys.
+// (|row| < 1e-12, also out of fp32 range) and non-finite rows poison `fin`.  fp32(1e-24) is above
+// 1e-24, and |row|^2 just below 1e-24 rounds to it: hence <=, so that every row safe_normalize leaves
+// unscaled is caught (a few just above 1e-12 are too, harmlessly): returns false, and the
+// task goes to the exact estimator (which of the two it was is only worked out there, on the cold
+// path: warp_ransac).  Rows past the frame's last ray (zero rows) become +0 keys.
 template <int SLOTS>
 __device__ __forceinline__ bool load_normalised_rows32(const double* __restrict__ sP, int n, int lane,
                                                        float (&nx)[SLOTS], float (&ny)[SLOTS],
@@ -571,7 +574,7 @@ __device__ __forceinline__ bool load_normalised_rows32(const double* __restrict_
         float rs;
         asm("rsqrt.approx.f32 %0, %1;" : "=f"(rs) : "f"(n2));
         if (i >= n) rs = 0.f;
-        else if (n2 < 1e-24f) rs = __uint_as_float(0x7fc00000u);
+        else if (n2 <= 1e-24f) rs = __uint_as_float(0x7fc00000u);
         nx[s] = (float)r0 * rs;
         ny[s] = (float)r1 * rs;
         nz[s] = (float)r2 * rs;
@@ -580,8 +583,9 @@ __device__ __forceinline__ bool load_normalised_rows32(const double* __restrict_
     return __all_sync(FULL, (__float_as_uint(fin) & 0x7f800000u) != 0x7f800000u);
 }
 
-// Result of the fast path: the winner is certified / it is not (run the exact estimator) / the rows
-// themselves are not finite (exact estimator, and pre_sync's "non-finite numbers in P" condition).
+// Result of the fast path: the winner is certified / it is not (run the exact estimator) / a row is
+// not finite or too small to normalise in fp32 (exact estimator; pre_sync's "non-finite numbers in P"
+// condition only if a row component really is non-finite).
 // kFastRetry: the run started from a prior threshold that turned out too tight (see `prior`): run again
 // without one.
 enum FastStatus { kFastOk = 0, kFastUndecided = 1, kFastRowsNotFinite = 2, kFastRetry = 3 };
@@ -744,8 +748,10 @@ __device__ __forceinline__ FastStatus warp_ransac_fast(const DeviceData& dd, con
     return kFastOk;
 }
 
-// Phases B + C of an estimator task.  Returns kFlagP when the rows are not all finite.  prior / tau_out:
-// see warp_ransac_fast (*tau_out = 0 when the winner did not come out of the fast path).
+// Phases B + C of an estimator task.  Returns kFlagP when the fp32 tournament could not take the rows (a
+// row not finite, or too small to normalise): a hint only, the caller's cold path decides whether
+// pre_sync's "non-finite numbers in P" condition holds (presync_diagnose).  prior / tau_out: see
+// warp_ransac_fast (*tau_out = 0 when the winner did not come out of the fast path).
 template <int SLOTS>
 __device__ __forceinline__ unsigned warp_ransac(const DeviceData& dd, const FrameDesc& fd,
                                                 const WarpSmem& w, int iters, uint64_t key, int lane,
@@ -1050,14 +1056,19 @@ __device__ __forceinline__ double warp_norm_PM(const double* sP, int NP, int nsl
     return sqrt(warp_sum(ss));
 }
 
-// which of pre_sync's panic conditions (core_private.cpp:76-83) a task with a non-finite cost hit;
-// pm: P.M of the warp's rays (the loss phase leaves it in the first plane of the rows)
-__device__ __noinline__ unsigned presync_diagnose(const double* pm, int nslots, int lane, double scale,
+// which of pre_sync's panic conditions (core_private.cpp:76-83) a task hit; pm: the warp's rows, with
+// P.M of each ray (simplified mode: the row's norm) in place of the first component (the loss phase
+// leaves it there).  A non-finite row component makes P.M non-finite, and P.M of finite rows with the M
+// the estimator draws from them (finite) is finite, so P.M and the other two planes tell whether a row
+// is not finite (a row merely too small for the fp32 tournament is not)
+__device__ __noinline__ unsigned presync_diagnose(const double* pm, int NP, int nslots, int lane, double scale,
                                                   double m0, double m1, double m2, const double* tab) {
     unsigned bad = 0;
     if (!(is_finite(m0) && is_finite(m1) && is_finite(m2))) bad |= kFlagM;
     for (int s = 0; s < nslots; ++s) {
-        const double r = pm[s * 32 + lane] * scale;
+        const int i = s * 32 + lane;
+        if (!(is_finite(pm[i]) && is_finite(pm[NP + i]) && is_finite(pm[2 * NP + i]))) bad |= kFlagP;
+        const double r = pm[i] * scale;
         if (!is_finite(r)) bad |= kFlagR;
         if (!is_finite(log1p_nonneg(r * r, tab))) bad |= kFlagRho;
     }
@@ -1355,10 +1366,10 @@ presync_kernel(DeviceData dd, const FrameDesc* __restrict__ frames, int F,
         const double cost = sqrt(warp_sum(acc));
         if (lane == 0) framecost[(size_t)di * cost_stride + fi] = cost;
         // the panic conditions of :76-83: non-finite values propagate into the cost, so the stage
-        // that produced them is only looked for when the cost (or a row) is not finite
+        // that produced them is only looked for when the cost is not finite or the estimator could not
+        // take the rows (bad: non-finite rows, or rows too small for fp32, which are no panic)
         if (bad || !is_finite(cost)) {
-            if (simplified && !is_finite(ss)) bad |= kFlagP;  // no estimator to notice non-finite rows
-            bad |= presync_diagnose(w.P, (fd.n + 31) >> 5, lane, scale, M[0], M[1], M[2], tab);
+            bad = presync_diagnose(w.P, NP, (fd.n + 31) >> 5, lane, scale, M[0], M[1], M[2], tab);
             bad = __reduce_or_sync(FULL, bad);
             if (bad && lane == 0) atomicOr(flags, bad);
         }

@@ -86,7 +86,13 @@ typedef struct rssync_lens {
  * seconds (cur_ts / 1000, next_ts / 1000).  Per pair: lens_undistort_point (:63-95) on both points,
  * ts = frame_ts + readout * (y / image_rows) (:144-145), unit rays (x', y', 1) / |.| (:147-154).
  * Equivalent to computing those on the host and calling rssync_set_track for each frame, up to
- * the rounding of tan / cos (CUDA's instead of libm's, <= 2 ulp). */
+ * the rounding of tan / cos (CUDA's instead of libm's, <= 2 ulp).
+ * Rejected before anything is applied: a lens with a non-finite field, fx or fy = 0, or k1..k4 so
+ * large that a bound of |theta (1 + k1 theta^2 + .. + k4 theta^8)| or of its derivative over
+ * [0, pi/2] overflows, and a non-finite or non-positive image_rows (RSSYNC_E_INVALID, "bad lens profile
+ * or image height"); a non-finite frame timestamp, and a point that is not finite or whose
+ * (x - cx) / fx, (y - cy) / fy or their squared norm is not (RSSYNC_E_NONFINITE, reported as the
+ * ray buffer of its side: "non-finite numbers in rays_a" for points_a).  Either would give NaN rays. */
 int rssync_set_track_pixels(rssync_problem* p, size_t n_frames, const int64_t* frames,
                             const size_t* counts, const double* frame_ts_a, const double* frame_ts_b,
                             const double* points_a, const double* points_b, const rssync_lens* lens,

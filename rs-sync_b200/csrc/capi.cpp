@@ -2220,11 +2220,34 @@ int frame_offsets(rssync_problem* p, size_t n_frames, const size_t* counts, std:
     return RSSYNC_OK;
 }
 
+// Upper bounds of |theta (1 + k1 theta^2 + .. + k4 theta^8)| and of its derivative over [0, pi/2], where
+// undistort_point (engine.cu) keeps its Newton iterates: while both are finite, so are the iterates (a
+// derivative of exactly 0 aside).  Twice the bounds are checked, headroom for the roundings of both sides.
+bool lens_polynomial_bounded(const rssync_lens& l) {
+    const double h = 1.5707963267948966, h2 = h * h;
+    const double a1 = std::fabs(l.k1), a2 = std::fabs(l.k2), a3 = std::fabs(l.k3), a4 = std::fabs(l.k4);
+    const double f = h * (1.0 + h2 * (a1 + h2 * (a2 + h2 * (a3 + h2 * a4))));
+    const double df = 1.0 + h2 * (3.0 * a1 + h2 * (5.0 * a2 + h2 * (7.0 * a3 + h2 * 9.0 * a4)));
+    return std::isfinite(2.0 * f) && std::isfinite(2.0 * df);
+}
+
+// n points (x, y) are finite, and so are undistort_point's x_ = (px - cx) / fx, y_ and theta_^2 = x_^2 + y_^2
+// (engine.cu): a finite pixel far enough out for the focal length is not, and would give a NaN ray
+bool points_ok(const double* pts, size_t n, const rssync_lens& l) {
+    if (!all_finite(pts, 2 * n)) return false;
+    for (size_t k = 0; k < n; ++k) {
+        const double x_ = (pts[2 * k] - l.cx) / l.fx, y_ = (pts[2 * k + 1] - l.cy) / l.fy;
+        if (!std::isfinite(x_ * x_ + y_ * y_)) return false;
+    }
+    return true;
+}
+
 // the pixels forms' lens profile, image height and counts
 int check_pixel_args(rssync_problem* p, size_t n_frames, const size_t* counts, const rssync_lens* lens,
                      double image_rows, std::vector<size_t>& at) {
     const double lv[9] = {lens->readout, lens->fx, lens->fy, lens->cx, lens->cy, lens->k1, lens->k2, lens->k3, lens->k4};
-    if (!all_finite(lv, 9) || !(image_rows > 0) || !std::isfinite(image_rows) || lens->fx == 0 || lens->fy == 0) {
+    if (!all_finite(lv, 9) || !(image_rows > 0) || !std::isfinite(image_rows) || lens->fx == 0 || lens->fy == 0 ||
+        !lens_polynomial_bounded(*lens)) {
         p->err = "set-track-pixels: bad lens profile or image height";
         return RSSYNC_E_INVALID;
     }
@@ -2417,8 +2440,8 @@ int rssync_set_track_pixels(rssync_problem* p, size_t n_frames, const int64_t* f
         const double* a = points_a + 2 * at[i];
         const double* b = points_b + 2 * at[i];
         const size_t n = counts[i];
-        if (!all_finite(a, 2 * n)) { bad[i] = 1; return; }
-        if (!all_finite(b, 2 * n)) { bad[i] = 2; return; }
+        if (!points_ok(a, n, *lens)) { bad[i] = 1; return; }
+        if (!points_ok(b, n, *lens)) { bad[i] = 2; return; }
         std::memcpy(p->h_pix.ptr + 2 * at[i], a, 2 * n * sizeof(double));
         std::memcpy(p->h_pix.ptr + 2 * total + 2 * at[i], b, 2 * n * sizeof(double));
         double l = 0.0, h = 0.0;
@@ -2480,8 +2503,9 @@ int rssync_set_track_pixels_device(rssync_problem* p, size_t n_frames, const int
     if (int rc = check_frame_ts(p, n_frames, frame_ts_a, frame_ts_b)) return rc;
     DeviceStaging s;
     if (int rc = begin_device_staging(p, at, 4 * total, frame_ts_a, frame_ts_b, stream, s)) return rc;
-    rs::launch_stage_points(s.d_at, s.d_fts, (int)n_frames, (int64_t)total, points_a, points_b, lens->readout,
-                            image_rows, s.d_data, s.d_info, p->stream);
+    const rs::LensDev L{lens->readout, lens->fx, lens->fy, lens->cx, lens->cy, lens->k1, lens->k2, lens->k3, lens->k4};
+    rs::launch_stage_points(s.d_at, s.d_fts, (int)n_frames, (int64_t)total, points_a, points_b, L, image_rows,
+                            s.d_data, s.d_info, p->stream);
     if (int rc = read_stage_info(p, n_frames, s)) return rc;
     for (size_t i = 0; i < n_frames; ++i)
         if (s.h_info[i].bad) {
@@ -2500,7 +2524,6 @@ int rssync_set_track_pixels_device(rssync_problem* p, size_t n_frames, const int
     if (int rc = reserve_device_arena(p)) return rc;
     if (int rc = reserve_rowq(p)) return rc;
     if (int rc = h2d(p, s.d_rec, s.h_rec, n_frames * sizeof(rs::PixelFrame))) return rc;
-    rs::LensDev L{lens->readout, lens->fx, lens->fy, lens->cx, lens->cy, lens->k1, lens->k2, lens->k3, lens->k4};
     rs::launch_ingest_pixels(s.d_rec, (int)n_frames, s.d_data, s.d_data + 2 * total, L, image_rows, p->d_rays.ptr,
                              p->d_orig.ptr, p->d_pos.ptr, p->d_rowq.ptr, p->stream);
     return end_device_ingest(p);

@@ -1797,6 +1797,7 @@ struct StageArgs {
     const double* frame_ts;  // pixels and row-fractions forms: ts_a, ts_b per frame
     double ro, rows;
     StageInfo* info;
+    double fx, fy, cx, cy;  // pixels form: the lens's normalisation (undistort_point)
 };
 enum class StageMode { kRays, kPoints, kRowFractions };
 template <StageMode M>
@@ -1827,6 +1828,12 @@ __global__ void __launch_bounds__(kStageThreads) stage_tracks_kernel(StageArgs a
                 // non-finite one
                 const double t = kPixels ? fts + a.ro * (v / a.rows) : kRowFractions ? fts + a.ro * v : v;
                 if (kRowFractions && !isfinite(t)) bad |= 1u << b;
+                // a finite point whose x_, y_ or theta_^2 in undistort_point overflows: its ray would be
+                // NaN (the x of the point is the element before, read by the neighbouring lane)
+                if (kPixels) {
+                    const double x_ = (s[base + j - 1] - a.cx) / a.fx, y_ = (v - a.cy) / a.fy;
+                    if (!isfinite(x_ * x_ + y_ * y_)) bad |= 1u << b;
+                }
                 lo = t < lo ? t : lo;
                 hi = t > hi ? t : hi;
             }
@@ -2459,11 +2466,11 @@ void launch_stage_row_fractions(const int64_t* d_at, const double* d_frame_ts, i
 }
 
 void launch_stage_points(const int64_t* d_at, const double* d_frame_ts, int n_frames, int64_t total,
-                         const double* points_a, const double* points_b, double readout, double rows,
+                         const double* points_a, const double* points_b, const LensDev& lens, double rows,
                          double* d_stage, StageInfo* d_info, cudaStream_t st) {
     if (n_frames <= 0) return;
     StageArgs a{d_at, total, {points_a, points_b, nullptr, nullptr}, {d_stage, d_stage + 2 * total, nullptr, nullptr},
-                d_frame_ts, readout, rows, d_info};
+                d_frame_ts, lens.ro, rows, d_info, lens.fx, lens.fy, lens.cx, lens.cy};
     stage_tracks_kernel<StageMode::kPoints><<<n_frames, kStageThreads, 0, st>>>(a);
     g_launches += 1;
 }

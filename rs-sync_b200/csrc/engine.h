@@ -191,10 +191,11 @@ void launch_stage_rays(const int64_t* d_at, int n_frames, int64_t total, const d
                        const double* rays_b, const double* ts_a, const double* ts_b, double* d_stage,
                        StageInfo* d_info, cudaStream_t st);
 // Pixels form: src = {points_a, points_b} (2 doubles per point); d_stage holds points_a, points_b;
-// lo / hi over frame_ts + readout * (y / rows), the expression ingest_pixels_kernel uses.
-// d_frame_ts: ts_a, ts_b of each frame (2 per frame).
+// lo / hi over frame_ts + lens.ro * (y / rows), the expression ingest_pixels_kernel uses.  Bit b is
+// also set when a point's (p - c) / f or its squared norm is not finite (undistort_point's x_, y_,
+// theta_).  d_frame_ts: ts_a, ts_b of each frame (2 per frame).
 void launch_stage_points(const int64_t* d_at, const double* d_frame_ts, int n_frames, int64_t total,
-                         const double* points_a, const double* points_b, double readout, double rows,
+                         const double* points_a, const double* points_b, const LensDev& lens, double rows,
                          double* d_stage, StageInfo* d_info, cudaStream_t st);
 // Row-fractions form: src = {rays_a, rays_b, frac_a, frac_b} (3, 3, 1, 1 doubles per ray); d_stage holds
 // frac_a, frac_b, rays_a, rays_b (the rays form's layout, fractions in the ts slots); bit 2 / 3 is also

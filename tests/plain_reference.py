@@ -188,7 +188,7 @@ def safe_normalize(v):
 class Estimate:
     """opt_guess_translational_motion (core_private.cpp:34-59) with every hypothesis kept"""
 
-    def __init__(self, P, key, iters):
+    def __init__(self, P, key, iters, row_err=0.0):
         n = P.shape[0]
         self.pairs = draws(key, iters, n)
         a = np.array([p[0] for p in self.pairs])
@@ -208,8 +208,10 @@ class Estimate:
         self.near = [t for t in range(iters)
                      if self.quartile[t] - qb <= TIE_REL * qb or self.quartile[t] <= TIE_FLOOR]
         row_norm = np.sqrt(np.sum(P * P, axis=1))
-        self.dM = np.minimum(2.0, E * (1.0 + (row_norm[a] + row_norm[b]).astype(np.float64)
-                                       / np.maximum(self.raw_norm.astype(np.float64), 1e-300)))
+        row_err = np.broadcast_to(np.asarray(row_err, dtype=np.float64), (n,))
+        raw = np.maximum(self.raw_norm.astype(np.float64), 1e-300)
+        self.dM = np.minimum(2.0, E * (1.0 + (row_norm[a] + row_norm[b]).astype(np.float64) / raw)
+                             + (row_err[a] + row_err[b]) / raw)
 
     def distinct_near(self):
         """near-tie members with distinct hypotheses (index of the first of each)"""
@@ -246,19 +248,22 @@ def _sqrt_bound(S, dS):
     return dS / den if den > 0 else np.sqrt(dS)
 
 
-def presync_cost(P, M=None, dM=0.0, simplified=False):
+def presync_cost(P, M=None, dM=0.0, simplified=False, row_err=0.0):
     """per-frame body of pre_sync (core_private.cpp:75-85): k = clamp(1e2 / ||P M||),
     r = P M k / |M|, cost = sqrt(sum sqrt(log1p(r^2))).  Simplified mode (include/rssync_b200.h):
-    the residual of a ray is its row's norm.  -> (cost, bound, k, bound of k)"""
+    the residual of a ray is its row's norm.  row_err: an absolute error of each row (per row or one
+    for all) on top of the rows' own rounding, e.g. from rays that are themselves approximations.
+    -> (cost, bound, k, bound of k)"""
     n = P.shape[0]
     rn = np.sqrt(np.sum(P * P, axis=1))
+    row_err = np.broadcast_to(np.asarray(row_err, dtype=np.float64), (n,))
     if simplified:
         v = rn
-        d = np.full(n, E)
+        d = E + row_err
         scale_div = LD(1)
     else:
         v = P @ M
-        d = E + rn.astype(np.float64) * dM
+        d = E + row_err + rn.astype(np.float64) * dM
         scale_div = np.sqrt(np.sum(M * M))
     N = np.sqrt(np.sum(v * v))
     with np.errstate(divide="ignore"):
@@ -276,14 +281,14 @@ def presync_cost(P, M=None, dM=0.0, simplified=False):
     return float(cost), _sqrt_bound(float(S), dS) + EPS * float(cost), kf, dk + E * kf
 
 
-def presync_cell(P, key=None, simplified=False, iters=20):
+def presync_cell(P, key=None, simplified=False, iters=20, row_err=0.0):
     """one (delay, frame) cell of the PreSync grid: the frame's cost for every near-tie hypothesis
-    of the estimator -> list of (cost, bound)"""
+    of the estimator -> list of (cost, bound).  row_err: as in presync_cost"""
     if simplified:
-        c, b, _, _ = presync_cost(P, simplified=True)
+        c, b, _, _ = presync_cost(P, simplified=True, row_err=row_err)
         return [(c, b)]
-    est = Estimate(P, key, iters)
-    return [presync_cost(P, est.hyp[t], float(est.dM[t]))[:2] for t in est.distinct_near()]
+    est = Estimate(P, key, iters, row_err)
+    return [presync_cost(P, est.hyp[t], float(est.dM[t]), row_err=row_err)[:2] for t in est.distinct_near()]
 
 
 def cell_ratio(got, cands):

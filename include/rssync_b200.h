@@ -48,8 +48,8 @@ int rssync_create(rssync_problem** out);
  * over NVLink when a compute call finds them stale.  PreSync / DebugPreSync / rssync_presync_grid
  * shard the delay grid by offset range (one ncclAllGather of the curve slices per call),
  * rssync_sync_batch* / rssync_presync_windows shard by syncpoint, rssync_orientation_search* and
- * rssync_rotation_search by variant (results assembled on the host, where the solver's control loop
- * produces them); every
+ * rssync_rotation_search by variant, rssync_readout_search by readout (results assembled on the host,
+ * where the solver's control loop produces them); every
  * result is bit-identical to the single-device one.  A single rssync_sync call runs on devices[0].
  * NCCL (libnccl.so.2) is loaded at run time, only by this call and only when n_devices > 1.
  * Leaves devices[0] the calling thread's current device. */
@@ -276,15 +276,20 @@ int rssync_rotation_search(rssync_problem* p, const double* timestamps_s, const 
  * NULL) row j is that call's cost over rssync_presync_delays(initial_delay, search_step, search_radius).
  * The problem's arena, frame table and gyro are left as they are.  A non-finite readout or n_readouts < 0:
  * RSSYNC_E_INVALID; n_readouts == 0: nothing done.  Otherwise rssync_presync's errors.  A multi-device
- * problem runs the whole search on devices[0]: the row fractions live there only, and sharding the
- * readouts would mean replicating them and widening rssync_device_state_t, which this version does not. */
+ * problem (n_readouts > 1) shards the readouts: every check runs on devices[0] first, then each device
+ * runs a contiguous share of them on its own scratch arena.  The row fractions (the plane and the
+ * re-timing table) reach the other devices by one grouped ncclBroadcast, sent only by a search that
+ * finds their copy stale (after an ingest, an overwrite, arena growth or an adoption).  Results, errors,
+ * the counter and the grid statistics equal the single-device search's. */
 int rssync_readout_search(rssync_problem* p, const double* readouts, int n_readouts, double initial_delay,
                           int64_t frame_begin, int64_t frame_end, double search_step, double search_radius,
                           const uint64_t* call_nos, double* out_cost, double* out_delay, double* out_curves);
 /* Apply a readout: re-time the frames of [frame_begin, frame_end), ingested from pixels or row fractions,
  * in place, so that the problem holds, byte for byte, what ingesting them with readout = readout gives
  * (arena tiles, orig / pos, frame table) and every later call returns what it would return on that
- * problem.  Frames ingested later use the readout of their own call.  Errors as rssync_readout_search's. */
+ * problem.  Frames ingested later use the readout of their own call.  Errors as rssync_readout_search's.
+ * A multi-device problem re-times on devices[0]; the other devices receive the arena at the next compute
+ * call, as after any Set* call. */
 int rssync_set_readout(rssync_problem* p, double readout, int64_t frame_begin, int64_t frame_end);
 
 /* Pinned RNG of the randomised translation estimator (replaces the reference's
@@ -352,7 +357,8 @@ int rssync_get_stats(const rssync_problem* p, rssync_stats* out);
  * other process) to hold a copy: it registers the frame table and sizes and allocates the buffers,
  * whose pointers rssync_device_state then returns for the caller to fill by whatever transport
  * it has (ncclBroadcast over NVLink in bench.py; rssync_create_multi does the same internally).
- * Results of the adopting problem equal the source's bit for bit. */
+ * Results of the adopting problem equal the source's bit for bit.  An adopted state comes without row
+ * fractions: rssync_readout_search / rssync_set_readout need them too (rssync_adopt_row_fractions). */
 typedef struct rssync_frame_desc {
     int64_t id;
     int32_t off, n;
@@ -371,6 +377,28 @@ int rssync_device_state(rssync_problem* p, rssync_device_state_t* out);
 int rssync_adopt_state(rssync_problem* p, const rssync_frame_desc* frames, size_t n_frames,
                        size_t arena_rays, size_t gyro_samples, double sample_rate,
                        double first_timestamp);
+
+/* The row fractions of an adopted state, so that the adopting problem can run rssync_readout_search and
+ * rssync_set_readout too.  The same three steps as above:
+ * rssync_retime_table (host only): the frames that hold row fractions, ascending id, with their frame
+ *   timestamps; returns their number, fills at most cap.
+ * rssync_row_fraction_plane: flushes like rssync_device_state, then *plane = the row-fraction plane
+ *   (2 doubles per arena ray, indexed by arena offset like the arena; *n_doubles = 2 * arena_rays),
+ *   NULL / 0 when no frame holds row fractions.
+ * rssync_adopt_row_fractions: on a problem whose state came from rssync_adopt_state with no Set* call
+ *   since (else RSSYNC_E_STATE), registers the table and allocates the plane.  An id not in the adopted
+ *   frame table, an id given twice, a non-finite timestamp or frames == NULL with n > 0:
+ *   RSSYNC_E_INVALID, the problem unchanged.  The caller then fills the plane through
+ *   rssync_row_fraction_plane and announces the stream that writes it with
+ *   rssync_expect_chunk(p, 0, arena_rays, stream): the re-timing waits for it.  A later
+ *   rssync_adopt_state, or a rays form overwriting a frame, drops the frame's row fractions. */
+typedef struct rssync_retime_desc {
+    int64_t id;
+    double frame_ts_a, frame_ts_b;
+} rssync_retime_desc;
+int rssync_retime_table(const rssync_problem* p, rssync_retime_desc* out, size_t cap);
+int rssync_row_fraction_plane(rssync_problem* p, double** plane, size_t* n_doubles);
+int rssync_adopt_row_fractions(rssync_problem* p, const rssync_retime_desc* frames, size_t n);
 
 /* Pipelined form of the same, for a source that has just taken a bulk SetTrackResult whose chunks are
  * still on their way to its device.  rssync_device_state_pipelined returns the pointers WITHOUT

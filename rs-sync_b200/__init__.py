@@ -43,6 +43,7 @@ C_ABI_SYMBOLS = [
     "rssync_set_track_batch_device", "rssync_set_track_pixels_device",
     "rssync_readout_search", "rssync_set_readout", "rssync_integrate_gyro_matrix", "rssync_rotation_search",
     "rssync_set_track_row_fractions", "rssync_set_track_row_fractions_device",
+    "rssync_retime_table", "rssync_row_fraction_plane", "rssync_adopt_row_fractions",
 ]
 # Itanium-ABI symbols of the C++ drop-in face (same set the reference's librssync_core exports)
 CXX_ABI_SYMBOLS = [
@@ -71,6 +72,14 @@ class DeviceState(C.Structure):
     _fields_ = [("rays", C.c_void_p), ("orig", C.c_void_p), ("pos", C.c_void_p), ("spline_records", C.c_void_p),
                 ("arena_rays", C.c_size_t), ("gyro_samples", C.c_size_t), ("sample_rate", C.c_double),
                 ("first_timestamp", C.c_double)]
+
+
+class RetimeDesc(C.Structure):
+    """rssync_retime_desc: a frame that holds row fractions, and its two frame timestamps"""
+    _fields_ = [("id", C.c_int64), ("frame_ts_a", C.c_double), ("frame_ts_b", C.c_double)]
+
+
+RETIME_DTYPE = np.dtype([("id", "<i8"), ("frame_ts_a", "<f8"), ("frame_ts_b", "<f8")])
 
 
 class Lens(C.Structure):
@@ -103,6 +112,9 @@ def load_library():
     L.rssync_frame_table.argtypes = [P, C.POINTER(FrameDesc), C.c_size_t]
     L.rssync_device_state.argtypes = [P, C.POINTER(DeviceState)]
     L.rssync_adopt_state.argtypes = [P, C.POINTER(FrameDesc), C.c_size_t, C.c_size_t, C.c_size_t, C.c_double, C.c_double]
+    L.rssync_retime_table.argtypes = [P, C.POINTER(RetimeDesc), C.c_size_t]
+    L.rssync_row_fraction_plane.argtypes = [P, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t)]
+    L.rssync_adopt_row_fractions.argtypes = [P, C.POINTER(RetimeDesc), C.c_size_t]
     L.rssync_device_state_pipelined.argtypes = [P, C.POINTER(DeviceState), C.POINTER(C.c_size_t), C.POINTER(C.c_size_t),
                                                 C.c_size_t, C.POINTER(C.c_size_t)]
     L.rssync_stream_wait_chunk.argtypes = [P, C.c_int, C.c_void_p]
@@ -684,6 +696,27 @@ class SyncProblem:
         self._check(self.L.rssync_adopt_state(self.h, ft.ctypes.data_as(C.POINTER(FrameDesc)), ft.shape[0],
                                               int(arena_rays), int(gyro_samples), float(sample_rate),
                                               float(first_timestamp)))
+
+    def retime_table(self):
+        """frames that hold row fractions (ascending id) as a numpy structured array (id, frame_ts_a,
+        frame_ts_b)"""
+        n = self.L.rssync_retime_table(self.h, None, 0)
+        arr = (RetimeDesc * max(n, 1))()
+        self.L.rssync_retime_table(self.h, arr, n)
+        return np.frombuffer(bytes(arr), dtype=RETIME_DTYPE, count=n).copy()
+
+    def row_fraction_plane(self):
+        """flush, then (device pointer, bytes) of the row-fraction plane (2 doubles per arena ray);
+        (0, 0) when no frame holds row fractions"""
+        ptr, n = C.c_void_p(), C.c_size_t(0)
+        self._check(self.L.rssync_row_fraction_plane(self.h, C.byref(ptr), C.byref(n)))
+        return (ptr.value or 0, n.value * 8)
+
+    def adopt_row_fractions(self, table):
+        """after adopt_state: register another problem's retime_table() and allocate the plane (fill it
+        through row_fraction_plane(), then expect_chunk(0, arena_rays, stream) for the writing stream)"""
+        t = np.ascontiguousarray(table, dtype=RETIME_DTYPE)
+        self._check(self.L.rssync_adopt_row_fractions(self.h, t.ctypes.data_as(C.POINTER(RetimeDesc)), t.shape[0]))
 
     def set_kernel_timing(self, enabled=True):
         self._check(self.L.rssync_set_kernel_timing(self.h, 1 if enabled else 0))

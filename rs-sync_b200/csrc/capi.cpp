@@ -320,6 +320,11 @@ struct rssync_problem {
     // frame of an adopted state, has no entry.  d_rowq is allocated by the first pixels ingest.
     std::unordered_map<int64_t, std::pair<double, double>> retime;
     DevBuf<double> d_rowq;
+    // A multi-device problem sends `retime` and d_rowq to its replicas only for a readout search:
+    // rowq_version counts the changes of either (and moves of the plane), rowq_synced is the one a replica
+    // holds.  adopted_version: the `version` rssync_adopt_state left, which rssync_adopt_row_fractions
+    // requires to be current (no input set since).
+    uint64_t rowq_version = 0, rowq_synced = 0, adopted_version = ~0ull;
     // re-timing scratch: the readout search's arena of the selected frames, and the frames' row extremes
     // (4 doubles per frame)
     DevBuf<double> d_rt_rays, d_rt_ext;
@@ -1497,6 +1502,7 @@ int rssync_create_multi(const int* devices, int n_devices, rssync_problem** out)
         r->is_replica = true;
         r->owns_stream = true;
         r->synced_version = ~0ull;
+        r->rowq_synced = ~0ull;
         p->replicas.push_back(r);
     }
     p->comms.assign((size_t)n_devices, nullptr);
@@ -1808,6 +1814,7 @@ int place_track(rssync_problem* p, int64_t frame, size_t count, FrameDesc** fd_o
     }
     if (it == p->frames.end()) it = p->frames.emplace_hint(pos, frame, FrameDesc{});
     if (!p->retime.empty()) p->retime.erase(frame);  // the pixels forms enter it again after placing
+    p->rowq_version++;
     FrameDesc& fd = it->second;  // map nodes are stable: fill_track completes ts_lo / ts_hi
     fd = FrameDesc{frame, (int32_t)off, (int32_t)count, 0.0, 0.0};
     p->total_rays += count;
@@ -2354,6 +2361,67 @@ int end_device_ingest(rssync_problem* p) {
 // The row-fraction plane of the pixels forms, as large as the device arena (contents kept)
 int reserve_rowq(rssync_problem* p) {
     CUDA_TRY(p, p->d_rowq.grow(2 * std::max<size_t>(p->d_orig.cap, 1), 2 * p->dev_used, p->stream));
+    p->rowq_version++;
+    return RSSYNC_OK;
+}
+
+// A plane that covers the whole device arena: frames a rays form appended since the last row fractions
+// have grown the arena but not the plane (their rays have no row fractions; the bytes only have to exist)
+int rowq_cover_arena(rssync_problem* p) {
+    if (2 * p->dev_used <= p->d_rowq.cap) return RSSYNC_OK;
+    if (int rc = wait_reader(p)) return rc;  // a replication still reading the old plane
+    return reserve_rowq(p);
+}
+
+// The row fractions to every replica whose copy is stale: the re-timing table on the host, the plane
+// (2 doubles per arena ray) as ONE grouped ncclBroadcast of [0, 2 dev_used) doubles on the replication
+// streams, behind the arena's replication (multi_replicate, called first), announced to each replica as
+// an arena range in flight so that its re-timing waits for it.  Only the readout search reads them.
+int multi_replicate_row_fractions(rssync_problem* p) {
+    RS_NVTX_RANGE();
+    bool stale = false;
+    for (const rssync_problem* r : p->replicas) stale = stale || r->rowq_synced != p->rowq_version;
+    if (!stale) return RSSYNC_OK;
+    const bool plane = !p->retime.empty();
+    if (plane)
+        if (int rc = rowq_cover_arena(p)) return rc;
+    const size_t rays = p->dev_used;
+    DeviceGuard guard;
+    for (rssync_problem* r : p->replicas) {
+        cudaSetDevice(r->device);
+        r->retime = p->retime;
+        cudaError_t e = cudaStreamSynchronize(r->stream);  // no earlier search still reads the old plane
+        if (e == cudaSuccess && r->repl_stream) e = cudaStreamSynchronize(r->repl_stream);
+        if (e == cudaSuccess && plane) e = r->d_rowq.reserve(2 * std::max<size_t>(rays, 1));
+        if (e == cudaSuccess && !r->repl_stream) e = cudaStreamCreateWithFlags(&r->repl_stream, cudaStreamNonBlocking);
+        if (e != cudaSuccess) {
+            p->err = std::string("CUDA error on device ") + std::to_string(r->device) + ": " + cudaGetErrorString(e);
+            return RSSYNC_E_CUDA;
+        }
+    }
+    if (plane && rays) {
+        cudaSetDevice(p->device);
+        if (!p->repl_stream) CUDA_TRY(p, cudaStreamCreateWithFlags(&p->repl_stream, cudaStreamNonBlocking));
+        if (int rc = rssync_stream_wait_chunk(p, -1, p->repl_stream)) return rc;  // the plane as the ingests left it
+        const rs::Nccl* nc = rs::Nccl::get();
+        NCCL_TRY(p, nc->GroupStart());
+        for (int i = 0; i < n_ranks(p); ++i) {
+            rssync_problem* q = rank_problem(p, i);
+            cudaSetDevice(q->device);
+            NCCL_TRY(p, nc->Broadcast(q->d_rowq.ptr, q->d_rowq.ptr, 2 * rays * sizeof(double), rs::Nccl::kChar, 0,
+                                      p->comms[(size_t)i], q->repl_stream));
+        }
+        NCCL_TRY(p, nc->GroupEnd());
+        p->nccl_calls += 1;
+        p->broadcast_bytes += 2 * rays * sizeof(double);
+        for (rssync_problem* r : p->replicas)
+            if (int rc = rssync_expect_chunk(r, 0, rays, r->repl_stream)) {
+                p->err = r->err;
+                return rc;
+            }
+        if (int rc = rssync_note_reader(p, p->repl_stream)) return rc;  // the next ingest waits for this send
+    }
+    for (rssync_problem* r : p->replicas) r->rowq_synced = p->rowq_version;
     return RSSYNC_OK;
 }
 
@@ -3101,7 +3169,8 @@ extern "C" {
 // PreSync at n_readouts rolling-shutter readouts without re-ingesting: the selected frames are re-timed
 // into a scratch arena (retime_frames_kernel) and the loss grid runs on it, per readout, back to back on
 // the problem's stream; one read-back at the end.  The problem's own arena, frame table and gyro are
-// not touched.  Runs on the primary device of a multi-device problem.
+// not touched.  A multi-device problem shards the readouts over its devices, as the orientation search
+// does its variants.
 int rssync_readout_search(rssync_problem* p, const double* readouts, int n_readouts, double initial,
                           int64_t fb, int64_t fe, double step, double radius, const uint64_t* call_nos,
                           double* out_cost, double* out_delay, double* out_curves) {
@@ -3123,6 +3192,23 @@ int rssync_readout_search(rssync_problem* p, const double* readouts, int n_reado
     if (int rc = check_grid_size(p, F, D)) return rc;
     const std::vector<uint64_t> calls = call_numbers(p, call_nos, n);
     if (!call_nos) p->call_no += (uint64_t)n;
+    if (is_multi(p) && n > 1) {
+        // readouts are independent: shard them, explicit call numbers.  Every device re-times into its
+        // own scratch arena and leaves its inputs alone, so no replica is stale afterwards.  Rank order
+        // is readout order: of several failing readouts, the first one's error is reported.
+        if (int rc = multi_replicate(p)) return rc;
+        if (int rc = multi_replicate_row_fractions(p)) return rc;
+        const int rc = multi_for_each_shard(p, n, false, [&](rssync_problem* q, int lo, int cnt) {
+            return rssync_readout_search(q, readouts + lo, cnt, initial, fb, fe, step, radius, calls.data() + lo,
+                                         out_cost + lo, out_delay + lo, out_curves ? out_curves + (size_t)lo * D : nullptr);
+        });
+        if (F > 0 && (rc == RSSYNC_OK || rc == RSSYNC_E_NONFINITE)) {  // the statistics of the last readout's grid
+            const rssync_problem* last = rank_problem(p, n_ranks(p) - 1);
+            p->grid_tasks = last->grid_tasks;
+            p->grid_exact_tasks = last->grid_exact_tasks;
+        }
+        return rc;
+    }
     CUDA_TRY(p, cudaSetDevice(p->device));
     if (int rc = flush(p)) return rc;  // pending gyro and tracks; ordered behind ingests in flight
     std::vector<double> costs((size_t)n * D, 0.0);  // no frames: the reference sums over none
@@ -3392,7 +3478,8 @@ int rssync_adopt_state(rssync_problem* p, const rssync_frame_desc* frames, size_
     p->version++;
     p->pending.clear();
     p->gyro_dirty = false;
-    p->retime.clear();  // an adopted arena comes without row fractions
+    p->retime.clear();  // an adopted arena comes without row fractions (rssync_adopt_row_fractions adds them)
+    p->rowq_version++;
     // the same table as last time (a caller replicating fresh data of an unchanged frame set): keep the map
     bool same = p->frames.size() == n_frames;
     if (same) {
@@ -3428,6 +3515,66 @@ int rssync_adopt_state(rssync_problem* p, const rssync_frame_desc* frames, size_
     CUDA_TRY(p, p->d_pos.reserve(std::max<size_t>(arena_rays, 1)));
     CUDA_TRY(p, p->d_rec.reserve(std::max<size_t>(gyro_samples, 1) * 16));
     // the pinned host mirror belongs to frames set one by one; an adopted arena has none
+    p->adopted_version = p->version;
+    return RSSYNC_OK;
+}
+
+int rssync_retime_table(const rssync_problem* p, rssync_retime_desc* out, size_t cap) {
+    if (!p) return 0;
+    std::vector<int64_t> ids;
+    ids.reserve(p->retime.size());
+    for (const auto& kv : p->retime) ids.push_back(kv.first);
+    std::sort(ids.begin(), ids.end());
+    for (size_t i = 0; out && i < ids.size() && i < cap; ++i) {
+        const std::pair<double, double>& ts = p->retime.at(ids[i]);
+        out[i] = rssync_retime_desc{ids[i], ts.first, ts.second};
+    }
+    return (int)ids.size();
+}
+
+int rssync_row_fraction_plane(rssync_problem* p, double** plane, size_t* n_doubles) {
+    RS_NVTX_RANGE();
+    if (!p || !plane || !n_doubles) return RSSYNC_E_INVALID;
+    *plane = nullptr;
+    *n_doubles = 0;
+    if (int rc = flush(p)) return rc;
+    CUDA_TRY(p, cudaStreamSynchronize(p->stream));
+    if (p->retime.empty()) return RSSYNC_OK;
+    if (int rc = rowq_cover_arena(p)) return rc;
+    *plane = p->d_rowq.ptr;
+    *n_doubles = 2 * p->dev_used;
+    return RSSYNC_OK;
+}
+
+int rssync_adopt_row_fractions(rssync_problem* p, const rssync_retime_desc* frames, size_t n) {
+    RS_NVTX_RANGE();
+    if (!p) return RSSYNC_E_INVALID;
+    if (p->adopted_version != p->version) {
+        p->err = "adopt-row-fractions: the problem's state must come from rssync_adopt_state, with no input set since";
+        return RSSYNC_E_STATE;
+    }
+    if (n && !frames) { p->err = "adopt-row-fractions: null argument"; return RSSYNC_E_INVALID; }
+    std::unordered_map<int64_t, std::pair<double, double>> table;
+    table.reserve(n);
+    for (size_t i = 0; i < n; ++i) {
+        const rssync_retime_desc& f = frames[i];
+        const std::string which = "adopt-row-fractions: frame " + std::to_string(f.id);
+        if (!p->frames.count(f.id)) { p->err = which + " is not in the adopted frame table"; return RSSYNC_E_INVALID; }
+        if (!std::isfinite(f.frame_ts_a) || !std::isfinite(f.frame_ts_b)) {
+            p->err = which + " has a non-finite frame timestamp";
+            return RSSYNC_E_INVALID;
+        }
+        if (!table.emplace(f.id, std::make_pair(f.frame_ts_a, f.frame_ts_b)).second) {
+            p->err = which + " is given more than once";
+            return RSSYNC_E_INVALID;
+        }
+    }
+    CUDA_TRY(p, cudaSetDevice(p->device));
+    if (int rc = wait_reader(p)) return rc;
+    CUDA_TRY(p, cudaStreamSynchronize(p->stream));  // no re-timing still reads the plane
+    if (n) CUDA_TRY(p, p->d_rowq.reserve(2 * std::max<size_t>(p->dev_used, 1)));
+    p->retime.swap(table);
+    p->rowq_version++;
     return RSSYNC_OK;
 }
 

@@ -6,6 +6,8 @@ units sharded, one small gather per call (SURVEY.md §8(e)).
   single-GPU curve bit for bit.
 * Sync: syncpoint i goes to rank i % world; each rank advances its syncpoints side by side on its
   own device (in independent lanes); (cost, delay) pairs are gathered at the end.
+* The orientation / rotation and readout searches: variant or readout k on rank k % world, RNG call
+  number call_no_base + k, results gathered at the end.
 
 The functions only need a `torch.distributed` process group (NCCL on GPUs, gloo in the CPU tests)
 and a problem object with the SyncProblem methods, so the logic is testable without a GPU.
@@ -26,7 +28,9 @@ def _gather_rows(local, sizes, group_size, device, dist):
     The rows are born on the host (the engine's C ABI returns host arrays), NCCL moves device
     memory: one copy each way around the collective."""
     import torch
-    local = np.ascontiguousarray(local, dtype=np.float64).reshape(local.shape[0], -1)
+    local = np.ascontiguousarray(local, dtype=np.float64)
+    if local.ndim == 1:
+        local = local.reshape(-1, 1)
     cols = local.shape[1]
     m = max(max(sizes), 1)
     buf = torch.zeros((m, cols), dtype=torch.float64, device=device)
@@ -133,6 +137,30 @@ def orientation_search_sharded(problem, search_fn, orientations, *, seed, call_n
     outc[order] = both[:, 0]
     outd[order] = both[:, 1]
     return outc, outd
+
+
+def readout_search_sharded(problem, readouts, initial_delay, frame_begin, frame_end, search_step, search_radius, *,
+                           call_no_base=0, rank=0, world=1, device="cpu", curves=False):
+    """The rolling-shutter readout search (problem.readout_search) with readout k on rank k % world and
+    RNG call number call_no_base + k, so the gathered result equals one problem's readout_search whose
+    call counter starts at call_no_base.  Every rank needs the frames' row fractions (ingested there, or
+    replicate_state + replicate_row_fractions).  Every rank returns (costs, delays), plus the n x D cost
+    curves when curves=True."""
+    r = np.ascontiguousarray(readouts, dtype=np.float64).ravel()
+    n = r.shape[0]
+    mine = np.arange(rank, n, world)
+    out = problem.readout_search(r[mine], initial_delay, frame_begin, frame_end, search_step, search_radius,
+                                 call_nos=call_no_base + mine.astype(np.uint64), curves=curves)
+    if world == 1:
+        return out
+    import torch.distributed as dist
+    rows = np.column_stack([out[0], out[1]] + ([out[2]] if curves else []))
+    both = _gather_rows(rows, [len(range(q, n, world)) for q in range(world)], world, device, dist)
+    # rank q contributed readouts q, q+world, ...: undo the round-robin
+    order = np.concatenate([np.arange(q, n, world) for q in range(world)])
+    res = np.empty_like(both)
+    res[order] = both
+    return (res[:, 0], res[:, 1], res[:, 2:]) if curves else (res[:, 0], res[:, 1])
 
 
 class _DevicePtr:
@@ -280,3 +308,47 @@ def replicate_state(problem, *, rank, world, device, src=0, groups=2):
                 problem.expect_chunk(lo, hi, handle)
         if rank == src:
             problem.note_reader(handle)  # the next Set* call waits for these sends
+
+
+def replicate_row_fractions(problem, *, rank, world, device, src=0):
+    """The row fractions of rank `src`'s frames (retime_table and the row-fraction plane) to every other
+    rank, so that readout_search and set_readout run there too.  Call it after replicate_state, whose
+    adoption drops them.  The table travels like the frame table (host bytes, one broadcast), the plane
+    as one broadcast on the replication's side stream straight into the receivers' allocations, which
+    are told that the plane is in flight (expect_chunk): their re-timing waits for it."""
+    import torch
+    import torch.distributed as dist
+    if world == 1:
+        return
+    rt_dtype = np.dtype([("id", "<i8"), ("frame_ts_a", "<f8"), ("frame_ts_b", "<f8")])
+    if rank == src:
+        raw = problem.retime_table().tobytes()
+        head = torch.tensor([len(raw) // rt_dtype.itemsize], dtype=torch.int64, device=device)
+    else:
+        head = torch.empty(1, dtype=torch.int64, device=device)
+    dist.broadcast(head, src)
+    nf = int(head.item())
+    if nf:
+        if rank == src:
+            tab = torch.from_numpy(np.frombuffer(raw, dtype=np.uint8).copy()).to(device)
+        else:
+            tab = torch.empty(nf * rt_dtype.itemsize, dtype=torch.uint8, device=device)
+        dist.broadcast(tab, src)
+    if rank != src:
+        problem.adopt_row_fractions(np.frombuffer(tab.cpu().numpy().tobytes(), dtype=rt_dtype) if nf
+                                    else np.empty(0, dtype=rt_dtype))
+    if not nf:
+        return
+    ptr, nbytes = problem.row_fraction_plane()
+    plane = torch.as_tensor(_DevicePtr(ptr, nbytes), device="cuda")
+    didx = torch.device(device).index or 0
+    side = _side_streams.get(didx)
+    if side is None:
+        side = _side_streams[didx] = torch.cuda.Stream(device=device)
+    side.wait_stream(torch.cuda.current_stream())
+    with torch.cuda.stream(side):
+        dist.broadcast(plane, src, async_op=True).wait()  # the side stream follows the collective's stream
+        if rank == src:
+            problem.note_reader(side.cuda_stream)  # the next Set* call waits for this send
+        else:
+            problem.expect_chunk(0, nbytes // 16, side.cuda_stream)

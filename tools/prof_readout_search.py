@@ -16,7 +16,20 @@ flushed between calls.  The search's (cost, delay) pairs are checked bit for bit
 the same RNG call numbers.  Needs a CUDA GPU and fails without one.  Prints the results as JSON; with
 --out DIR also writes them to DIR/prof_readout_search.json.
 
-    python tools/prof_readout_search.py [--out DIR] [--reps 10]
+With --devices 0,1,2,3 it times instead the same search on one problem spread over those devices
+(rssync_create_multi, readouts sharded by device) against the problem on the first device alone:
+
+  * one_device: readout_search on the single-device problem;
+  * multi_repeat: readout_search on the multi-device problem whose replicas already hold the row fractions;
+  * multi_first: the same right after a re-ingest of the same pixels (in place), once a PreSync grid has
+    sent the arena on: the search sends the row-fraction plane first (one grouped broadcast).
+
+The three alternate; medians over --reps.  Results (curves included) are checked bit for bit against the
+single-device search, the bytes and collectives of the plane's broadcast are read from the problem's
+statistics, and the card's name, power limit and max SM clock are read for every device used.  Written to
+DIR/prof_readout_search_<G>gpu.json with --out.
+
+    python tools/prof_readout_search.py [--out DIR] [--reps 10] [--devices 0,1,2,3]
 """
 import argparse
 import importlib
@@ -34,18 +47,103 @@ sys.path.insert(0, ROOT)
 HBM_TBS = 7.7  # HGX B200 data sheet, one GPU
 
 
-def gpu_info():
+def gpu_info(device=0):
     import torch
-    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
-                       capture_output=True, text=True)
-    return {"torch_name": torch.cuda.get_device_name(0),
+    q = subprocess.run(["nvidia-smi", "-i", str(device), "--query-gpu=name,power.limit,clocks.max.sm",
+                        "--format=csv,noheader"], capture_output=True, text=True)
+    return {"torch_name": torch.cuda.get_device_name(device),
             "nvidia_smi": q.stdout.strip().splitlines()[0] if q.returncode == 0 and q.stdout.strip() else None}
+
+
+def multi_main(args, pkg, synth, w, devices):
+    """the readout search on a multi-device problem against the same problem on devices[0]"""
+    import torch
+    F, N = w.n_frames, w.n_rays
+    counts = np.full(F, N)
+    ta, tb = w.frame_ids / w.fps, (w.frame_ids + 1) / w.fps
+    pa, pb = w.px_a.reshape(-1), w.px_b.reshape(-1)
+    fb, fe = int(w.frame_ids[0]), int(w.frame_ids[-1]) + 1
+    initial, step, radius = 0.0, w.presync_step, w.presync_radius
+    delays = pkg.presync_delays(initial, step, radius)
+    readouts = np.linspace(0.0, 0.02, 11)
+    calls = np.arange(len(readouts), dtype=np.uint64) + 50
+    lens = (float(synth.READOUT),) + tuple(synth.LENS[1:])
+
+    def make(devs):
+        p = pkg.SyncProblem(seed=100, devices=devs)
+        p.SetGyroQuaternions(w.quats, w.quats.shape[0], w.gyro_rate, w.gyro_t0)
+        p.set_track_pixels(w.frame_ids, counts, ta, tb, pa, pb, lens, synth.HEIGHT)
+        return p
+
+    one, many = make([devices[0]]), make(devices)
+    assert many.device_count() == len(devices)
+    many.presync_grid(fb, fe, delays[:8], call_no=1)  # the arena goes out here, not inside the timed search
+
+    def sync_all():
+        for d in devices:
+            torch.cuda.synchronize(d)
+
+    def search(p):
+        return p.readout_search(readouts, initial, fb, fe, step, radius, call_nos=calls, curves=True)
+
+    def first():
+        many.set_track_pixels(w.frame_ids, counts, ta, tb, pa, pb, lens, synth.HEIGHT)  # in place: the plane is stale
+        many.presync_grid(fb, fe, delays[:8], call_no=1)
+        sync_all()
+        s0 = many.stats()
+        t0 = time.perf_counter()
+        out = search(many)
+        sync_all()
+        ms = (time.perf_counter() - t0) * 1e3
+        s1 = many.stats()
+        return out, ms, (s1["broadcast_bytes"] - s0["broadcast_bytes"], s1["nccl_calls"] - s0["nccl_calls"])
+
+    def timed(p):
+        sync_all()
+        t0 = time.perf_counter()
+        out = search(p)
+        sync_all()
+        return out, (time.perf_counter() - t0) * 1e3
+
+    t = {"one_device": [], "multi_repeat": [], "multi_first": []}
+    want, same, plane = None, True, None
+    for i in range(args.reps + 1):
+        want, ms1 = timed(one)
+        got_first, msf, plane = first()
+        got, msr = timed(many)
+        same = same and all(np.array_equal(a, b) for a, b in zip(want, got)) and \
+            all(np.array_equal(a, b) for a, b in zip(want, got_first))
+        if i >= 1:  # the first round warms every shape up
+            t["one_device"].append(ms1)
+            t["multi_first"].append(msf)
+            t["multi_repeat"].append(msr)
+    arena = many.device_state()["arena_rays"]
+    G = len(devices)
+    out = {"gpus": [gpu_info(d) for d in devices], "devices": list(devices),
+           "shape": {"frames": F, "pixel_pairs_per_frame": N, "readouts": len(readouts), "delays": int(delays.size),
+                     "arena_rays": int(arena)},
+           "results_bit_identical": bool(same),
+           "plane_broadcast": {"bytes": int(plane[0]), "collectives": int(plane[1]),
+                               "expected_bytes": 16 * int(arena) if G > 1 else 0},
+           "rounds": -(-len(readouts) // G),
+           "ms_median": {k: float(np.median(v)) for k, v in t.items()},
+           "ms_p10_p90": {k: [float(np.percentile(v, 10)), float(np.percentile(v, 90))] for k, v in t.items()},
+           "reps": args.reps}
+    out["speedup_repeat_vs_one_device"] = out["ms_median"]["one_device"] / out["ms_median"]["multi_repeat"]
+    out["plane_cost_ms"] = out["ms_median"]["multi_first"] - out["ms_median"]["multi_repeat"]
+    if args.out:
+        os.makedirs(args.out, exist_ok=True)
+        with open(os.path.join(args.out, f"prof_readout_search_{G}gpu.json"), "w") as f:
+            json.dump(out, f, indent=1)
+    print(json.dumps(out, indent=1))
 
 
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", default=None, help="directory for prof_readout_search.json (default: print only)")
     ap.add_argument("--reps", type=int, default=10)
+    ap.add_argument("--devices", default=None,
+                    help="comma-separated CUDA devices: time the search on one problem spread over them")
     args = ap.parse_args()
     import torch
     if not torch.cuda.is_available():
@@ -53,6 +151,11 @@ def main():
     pkg = importlib.import_module("rs-sync_b200")
     synth = importlib.import_module("rs-sync_b200.synth")
     w = synth.make_workload("C2", procs=min(16, os.cpu_count() or 1))
+    if args.devices:
+        devices = [int(d) for d in args.devices.split(",")]
+        if len(devices) > torch.cuda.device_count():
+            raise SystemExit(f"prof_readout_search: {len(devices)} devices asked, {torch.cuda.device_count()} present")
+        return multi_main(args, pkg, synth, w, devices)
     F, N = w.n_frames, w.n_rays
     counts = np.full(F, N)
     ta, tb = w.frame_ids / w.fps, (w.frame_ids + 1) / w.fps

@@ -48,7 +48,8 @@ int rssync_create(rssync_problem** out);
  * over NVLink when a compute call finds them stale.  PreSync / DebugPreSync / rssync_presync_grid
  * shard the delay grid by offset range (one ncclAllGather of the curve slices per call),
  * rssync_sync_batch* / rssync_presync_windows shard by syncpoint, rssync_orientation_search* and
- * rssync_rotation_search by variant, rssync_readout_search by readout (results assembled on the host,
+ * rssync_rotation_search(_windows) by variant, rssync_readout_search(_windows) by readout (results
+ * assembled on the host,
  * where the solver's control loop produces them); every
  * result is bit-identical to the single-device one.  A single rssync_sync call runs on devices[0].
  * NCCL (libnccl.so.2) is loaded at run time, only by this call and only when n_devices > 1.
@@ -263,6 +264,30 @@ int rssync_rotation_search(rssync_problem* p, const double* timestamps_s, const 
                            int64_t frame_begin, int64_t frame_end, double search_step,
                            double search_radius, const uint64_t* call_nos, double* out_cost,
                            double* out_delay, double* out_curves);
+/* rssync_rotation_search over n_windows frame windows [frame_begin[w], frame_end[w]) at once, each with
+ * its own delay argmin.  Entry [j][w] (j W + w, W = n_windows) of out_cost / out_delay (n_rot x W) equals,
+ * bit for bit, rssync_integrate_gyro_matrix(matrices + 9 j) -> rssync_set_gyro_var -> rssync_presync(
+ * initial_delay, frame_begin[w], frame_end[w], search_step, search_radius) keyed by call_nos[j W + w]
+ * (NULL: consecutive values of the counter in that order, which advances by n_rot W).  out_curves
+ * (n_rot x W x D, or NULL): row [j][w] is that call's cost over rssync_presync_delays(...); the delay grid
+ * is shared by all windows, so a clip whose delay drifts needs a radius that covers the drift.  Windows
+ * may overlap or be empty (cost 0 at every delay, as rssync_presync on no frames).  Score a candidate by
+ * the sum of its row, out_cost[j W + 0 .. W): each window sees about one delay, and the sum averages the
+ * windows' tracking noise.  Per variant, one integration and one loss grid over all windows run.  For the
+ * 48 gyro_orientation strings, pass the matrices of the strings (rssync_integrate_gyro_matrix's "matrix
+ * of s", Python's orientation_matrix(s)): they integrate to the strings' bits exactly.  Errors: negative
+ * counts, n_rot W above INT32_MAX, or a null window buffer (with n_rot, W > 0): RSSYNC_E_INVALID before
+ * anything is done; n_rot == 0 or W == 0: nothing done; then rssync_rotation_search's errors, checked over
+ * the windows in order.  A non-finite value found on the device fails the first such variant in order,
+ * with the message of its grid's flags over all its windows (the first failing window's message when its
+ * windows fail alike, as a non-finite gyro or ray makes them).  The problem is left holding the last
+ * variant's gyro, the grid statistics are those of the last variant's grid, and a multi-device problem
+ * shards by variant as rssync_rotation_search does. */
+int rssync_rotation_search_windows(rssync_problem* p, const double* timestamps_s, const double* gyro_xyz,
+                                   size_t count, const double* matrices, int n_rot, int n_windows,
+                                   const int64_t* frame_begin, const int64_t* frame_end, double initial_delay,
+                                   double search_step, double search_radius, const uint64_t* call_nos,
+                                   double* out_cost, double* out_delay, double* out_curves);
 
 /* Rolling-shutter readout search: PreSync(initial_delay, frame_begin, frame_end, search_step, search_radius)
  * at each of n_readouts candidate readouts (seconds, as rssync_lens.readout), without re-ingesting.  Every
@@ -284,6 +309,25 @@ int rssync_rotation_search(rssync_problem* p, const double* timestamps_s, const 
 int rssync_readout_search(rssync_problem* p, const double* readouts, int n_readouts, double initial_delay,
                           int64_t frame_begin, int64_t frame_end, double search_step, double search_radius,
                           const uint64_t* call_nos, double* out_cost, double* out_delay, double* out_curves);
+/* rssync_readout_search over n_windows frame windows [frame_begin[w], frame_end[w]) at once, each with its
+ * own delay argmin.  Entry [j][w] (j W + w, W = n_windows) of out_cost / out_delay (n_readouts x W) equals,
+ * bit for bit, rssync_presync(initial_delay, frame_begin[w], frame_end[w], search_step, search_radius) on
+ * a problem that ingested the same input with readout = readouts[j], keyed by call_nos[j W + w] (NULL:
+ * consecutive values of the counter in that order, which advances by n_readouts W).  out_curves
+ * (n_readouts x W x D, or NULL) as in rssync_rotation_search_windows; the delay grid is shared by all
+ * windows.  Windows may overlap or be empty.  Score a readout by the sum of its row.  Per readout, the
+ * union of the windows' frames is re-timed once and one loss grid over all windows runs.  Errors:
+ * negative counts, n_readouts W above INT32_MAX, a null buffer or a non-finite readout: RSSYNC_E_INVALID;
+ * a frame without row fractions: RSSYNC_E_STATE naming the first such frame in window order; both before
+ * anything is done.  n_readouts == 0 or W == 0: nothing done.  A non-finite value found on the device
+ * fails the first such readout in order, with the message of its grid's flags over all its windows (as
+ * in rssync_rotation_search_windows).  The arena, frame table and gyro are left as they are, the grid
+ * statistics are those of the last readout's grid, and a multi-device problem shards by readout as
+ * rssync_readout_search does. */
+int rssync_readout_search_windows(rssync_problem* p, const double* readouts, int n_readouts, int n_windows,
+                                  const int64_t* frame_begin, const int64_t* frame_end, double initial_delay,
+                                  double search_step, double search_radius, const uint64_t* call_nos,
+                                  double* out_cost, double* out_delay, double* out_curves);
 /* Apply a readout: re-time the frames of [frame_begin, frame_end), ingested from pixels or row fractions,
  * in place, so that the problem holds, byte for byte, what ingesting them with readout = readout gives
  * (arena tiles, orig / pos, frame table) and every later call returns what it would return on that

@@ -44,6 +44,7 @@ C_ABI_SYMBOLS = [
     "rssync_readout_search", "rssync_set_readout", "rssync_integrate_gyro_matrix", "rssync_rotation_search",
     "rssync_set_track_row_fractions", "rssync_set_track_row_fractions_device",
     "rssync_retime_table", "rssync_row_fraction_plane", "rssync_adopt_row_fractions",
+    "rssync_readout_search_windows", "rssync_rotation_search_windows",
 ]
 # Itanium-ABI symbols of the C++ drop-in face (same set the reference's librssync_core exports)
 CXX_ABI_SYMBOLS = [
@@ -195,6 +196,12 @@ def load_library():
     L.rssync_rotation_search.argtypes = [P, c_double_p, c_double_p, C.c_size_t, c_double_p, C.c_int, C.c_double,
                                          C.c_int64, C.c_int64, C.c_double, C.c_double, C.POINTER(C.c_uint64),
                                          c_double_p, c_double_p, c_double_p]
+    L.rssync_readout_search_windows.argtypes = [P, c_double_p, C.c_int, C.c_int, c_i64_p, c_i64_p, C.c_double,
+                                                C.c_double, C.c_double, C.POINTER(C.c_uint64), c_double_p,
+                                                c_double_p, c_double_p]
+    L.rssync_rotation_search_windows.argtypes = [P, c_double_p, c_double_p, C.c_size_t, c_double_p, C.c_int, C.c_int,
+                                                 c_i64_p, c_i64_p, C.c_double, C.c_double, C.c_double,
+                                                 C.POINTER(C.c_uint64), c_double_p, c_double_p, c_double_p]
     _lib = L
     return L
 
@@ -631,6 +638,67 @@ class SyncProblem:
         self._check(self.L.rssync_readout_search(self.h, _dp(r), n, initial_delay, frame_begin, frame_end,
                                                  search_step, search_radius, cn, _dp(costs), _dp(delays),
                                                  _dp(cv) if curves else None))
+        return (costs, delays, cv) if curves else (costs, delays)
+
+    def _windowed_args(self, n, frame_begin, frame_end, initial_delay, search_step, search_radius, call_nos,
+                       curves):
+        """the window arrays, call numbers and output buffers of the windowed searches"""
+        fb = np.ascontiguousarray(frame_begin, dtype=np.int64).ravel()
+        fe = np.ascontiguousarray(frame_end, dtype=np.int64).ravel()
+        if fb.shape != fe.shape:
+            raise ValueError(f"{fb.shape[0]} window starts but {fe.shape[0]} window ends")
+        W = fb.shape[0]
+        cn = None
+        if call_nos is not None:
+            cn_arr = np.ascontiguousarray(call_nos, dtype=np.uint64).ravel()
+            if cn_arr.shape[0] != n * W:
+                raise ValueError(f"{n} candidates x {W} windows but {cn_arr.shape[0]} call numbers")
+            cn = cn_arr
+        costs, delays = np.empty((n, W)), np.empty((n, W))
+        cv = None
+        if curves:
+            D = self.L.rssync_presync_delays(initial_delay, search_step, search_radius, None, 0)
+            cv = np.empty((n, W, max(D, 0)))
+        return fb, fe, cn, costs, delays, cv
+
+    def readout_search_windows(self, readouts, initial_delay, frame_begin, frame_end, search_step, search_radius,
+                               call_nos=None, curves=False):
+        """readout_search over W frame windows [frame_begin[w], frame_end[w]) at once
+        (rssync_readout_search_windows).  Returns (costs, delays) of shape (n, W), plus the (n, W, D) cost
+        curves when curves=True; entry [j, w] is PreSync over window w at readout j, keyed by call number
+        call_nos[j * W + w] (None: the next n * W values of the problem's counter).  Score the readouts by
+        the sum over windows: estimate_readout(readouts, costs.sum(axis=1))."""
+        r = _f64(readouts).ravel()
+        n = r.shape[0]
+        fb, fe, cn, costs, delays, cv = self._windowed_args(n, frame_begin, frame_end, initial_delay, search_step,
+                                                            search_radius, call_nos, curves)
+        self._check(self.L.rssync_readout_search_windows(
+            self.h, _dp(r), n, fb.shape[0], fb.ctypes.data_as(c_i64_p), fe.ctypes.data_as(c_i64_p), initial_delay,
+            search_step, search_radius, None if cn is None else cn.ctypes.data_as(C.POINTER(C.c_uint64)),
+            _dp(costs), _dp(delays), _dp(cv) if curves else None))
+        return (costs, delays, cv) if curves else (costs, delays)
+
+    def rotation_search_windows(self, timestamps_s, gyro_xyz, rotations, initial_delay, frame_begin, frame_end,
+                                search_step, search_radius, call_nos=None, curves=False):
+        """rotation_search over W frame windows [frame_begin[w], frame_end[w]) at once
+        (rssync_rotation_search_windows); shapes and call numbers as in readout_search_windows.  Score the
+        rotations by the sum over windows: estimate_angle(angles, costs.sum(axis=1)).  For gyro_orientation
+        strings, pass [orientation_matrix(s) for s in strings]."""
+        ts = _f64(timestamps_s)
+        g = _f64(gyro_xyz)
+        m = _f64(rotations)
+        if m.size == 0:
+            m = m.reshape(0, 3, 3)
+        if m.ndim != 3 or m.shape[1:] != (3, 3):
+            raise ValueError(f"rotations must be a list of 3x3 matrices or an (n, 3, 3) array, got shape {m.shape}")
+        n = m.shape[0]
+        fb, fe, cn, costs, delays, cv = self._windowed_args(n, frame_begin, frame_end, initial_delay, search_step,
+                                                            search_radius, call_nos, curves)
+        self._check(self.L.rssync_rotation_search_windows(
+            self.h, _dp(ts), _dp(g), ts.shape[0], _dp(m), n, fb.shape[0], fb.ctypes.data_as(c_i64_p),
+            fe.ctypes.data_as(c_i64_p), initial_delay, search_step, search_radius,
+            None if cn is None else cn.ctypes.data_as(C.POINTER(C.c_uint64)), _dp(costs), _dp(delays),
+            _dp(cv) if curves else None))
         return (costs, delays, cv) if curves else (costs, delays)
 
     def set_readout(self, readout, frame_begin, frame_end):

@@ -18,6 +18,7 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <unordered_map>
 #include <unordered_set>
 #include <utility>
 #include <vector>
@@ -2911,6 +2912,87 @@ int rssync_integrate_gyro_matrix(const double* timestamps_s, const double* gyro_
 
 namespace {
 
+// The frame windows of a windowed search (W >= 1): every window's frames, concatenated in window order
+// (a frame in several windows appears once per window), the window starts into that list, and the
+// largest frame.  All windows are checked, in window order, before anything runs; `check` (optional)
+// is a search's own check of a window's frames.
+struct SearchWindows {
+    std::vector<FrameDesc> frames;
+    std::vector<int> begin;  // W + 1 offsets into frames
+    int max_n = 0;
+
+    int select(rssync_problem* p, int W, const int64_t* fb, const int64_t* fe,
+               const std::function<int(const std::vector<FrameDesc>&)>& check = nullptr) {
+        frames.clear();
+        begin.assign(1, 0);
+        std::vector<FrameDesc> sel;
+        for (int w = 0; w < W; ++w) {
+            int mn = 0;
+            if (int rc = select_frames(p, fb[w], fe[w], sel, mn, "pre-sync")) return rc;
+            if (check)
+                if (int rc = check(sel)) return rc;
+            max_n = std::max(max_n, mn);
+            frames.insert(frames.end(), sel.begin(), sel.end());
+            begin.push_back((int)frames.size());
+        }
+        return RSSYNC_OK;
+    }
+    int F() const { return (int)frames.size(); }
+    int W() const { return (int)begin.size() - 1; }
+
+    // the RNG call number of every listed frame for candidate j: calls[j W + its window]
+    std::vector<uint64_t> frame_calls(const std::vector<uint64_t>& calls, int n) const {
+        std::vector<uint64_t> fc((size_t)n * F());
+        for (int j = 0; j < n; ++j)
+            for (int w = 0; w < W(); ++w)
+                for (int f = begin[(size_t)w]; f < begin[(size_t)w + 1]; ++f)
+                    fc[(size_t)j * F() + f] = calls[(size_t)j * W() + w];
+        return fc;
+    }
+};
+
+// Checks shared by the windowed searches: counts and window buffers.  `who` names the search.
+int check_search_counts(rssync_problem* p, int n, int W, const int64_t* fb, const int64_t* fe, const char* who) {
+    if (n < 0 || W < 0) { p->err = std::string(who) + ": negative candidate or window count"; return RSSYNC_E_INVALID; }
+    if ((long long)n * W > INT32_MAX) { p->err = std::string(who) + ": too many candidate windows"; return RSSYNC_E_INVALID; }
+    if (n > 0 && W > 0 && (!fb || !fe)) { p->err = std::string(who) + ": null window buffer"; return RSSYNC_E_INVALID; }
+    return RSSYNC_OK;
+}
+
+// For candidate grids with more than one window: the per-frame call numbers of all n candidates and the
+// window starts, on the device (rssync_presync_windows' arrays).  One window needs neither.
+int stage_windows(rssync_problem* p, const SearchWindows& win, const std::vector<uint64_t>& calls, int n) {
+    if (win.W() == 1 || win.F() == 0) return RSSYNC_OK;
+    const std::vector<uint64_t> fcall = win.frame_calls(calls, n);
+    CUDA_TRY(p, p->d_frame_call.reserve(fcall.size()));
+    CUDA_TRY(p, p->d_win_begin.reserve(win.begin.size()));
+    if (int rc = h2d(p, p->d_frame_call.ptr, fcall.data(), sizeof(uint64_t) * fcall.size())) return rc;
+    return h2d(p, p->d_win_begin.ptr, win.begin.data(), sizeof(int) * win.begin.size());
+}
+
+// candidate j's grid over the windows: one window is a plain grid, several are rssync_presync_windows'
+// multi-window grid with the per-frame call numbers staged by stage_windows
+void launch_candidate_grid(rssync_problem* p, const rs::DeviceData& dd, const SearchWindows& win, int j,
+                           const FrameDesc* d_frames, const double* d_delays, int D, uint64_t call, int max_chunk,
+                           cudaStream_t st) {
+    const int F = win.F(), W = win.W();
+    rs::launch_presync_grid(dd, d_frames, F, win.max_n, d_delays, D, p->seed, rs::kStreamPreSync, call, 0,
+                            p->d_framecost.ptr, p->d_costs.ptr + (size_t)j * W * D, p->d_flags.ptr + 2 * (size_t)j, st,
+                            max_chunk, p->simplified, W > 1 ? p->d_frame_call.ptr + (size_t)j * F : nullptr,
+                            W > 1 ? p->d_win_begin.ptr : nullptr, W);
+}
+
+// candidate j's W results from the curves (n x W x D)
+void candidate_results(int j, int W, const std::vector<double>& costs, const std::vector<double>& delays,
+                       double* out_cost, double* out_delay, double* out_curves) {
+    const int D = (int)delays.size();
+    for (int w = 0; w < W; ++w) {
+        const size_t r = (size_t)j * W + w;
+        curve_argmin(&costs[r * D], delays.data(), D, &out_cost[r], &out_delay[r]);
+        if (out_curves) std::memcpy(out_curves + r * D, &costs[r * D], sizeof(double) * D);
+    }
+}
+
 // The axis mappings of a gyro-variant search: gyro_orientation strings (the orientation search) or 3x3
 // row-major matrices (the rotation search).  The search turns either into matrices at the same step.
 struct GyroVariants {
@@ -2938,32 +3020,36 @@ struct GyroVariants {
 
 // The orientation search of core_testcode.cpp:184-233, for any axis mappings: for every variant,
 // integrate the raw gyro (optdata_fill_gyro, :37-53) under its mapping, ingest it through the
-// variable-rate SetGyroQuaternions and run PreSync over the frame range.  out_curves (n x D or null):
-// every variant's cost curve.
+// variable-rate SetGyroQuaternions and run PreSync over each of the W frame windows [fb[w], fe[w]) -- one
+// loss grid per variant over all windows.  Results are n x W, variant-major; out_curves (n x W x D or
+// null): every variant's cost curve per window.
 int gyro_variant_search(rssync_problem* p, const double* timestamps_s, const double* gyro_xyz, size_t count,
-                        const GyroVariants& variants, int n_orient, double initial_delay, int64_t fb, int64_t fe,
-                        double step, double radius, const uint64_t* call_nos, double* out_cost, double* out_delay,
-                        double* out_curves) {
+                        const GyroVariants& variants, int n_orient, double initial_delay, int W, const int64_t* fb,
+                        const int64_t* fe, double step, double radius, const uint64_t* call_nos, double* out_cost,
+                        double* out_delay, double* out_curves) {
     if (!p || n_orient < 0) return RSSYNC_E_INVALID;
-    if (n_orient == 0) return RSSYNC_OK;
+    if (int rc = check_search_counts(p, n_orient, W, fb, fe, "rotation-search")) return rc;
+    if (n_orient == 0 || W == 0) return RSSYNC_OK;
     if (!timestamps_s || !gyro_xyz || (!variants.strings && !variants.matrices) || !out_cost || !out_delay)
         return RSSYNC_E_INVALID;
+    const int nw = n_orient * W;
     if (is_multi(p) && n_orient > 1) {
         // variants are independent: shard them.  Every device sets its own gyro per variant, so the
         // replicas' inputs are stale afterwards; the primary takes the LAST share, which leaves it
         // holding the last variant's gyro as the single-device search does.
         if (int rc = multi_replicate(p)) return rc;
-        const std::vector<uint64_t> callno = call_numbers(p, call_nos, n_orient);
-        // curve rows per variant (a window the shards reject leaves no curves to place)
+        const std::vector<uint64_t> callno = call_numbers(p, call_nos, nw);
+        // curve rows per variant and window (a window the shards reject leaves no curves to place)
         const size_t D = out_curves && step > 0 && std::isfinite(initial_delay) && std::isfinite(radius)
                              ? (size_t)std::max(0, rssync_presync_delays(initial_delay, step, radius, nullptr, 0))
                              : 0;
         const int rc = multi_for_each_shard(p, n_orient, true, [&](rssync_problem* q, int lo, int cnt) {
-            return gyro_variant_search(q, timestamps_s, gyro_xyz, count, variants.from(lo), cnt, initial_delay, fb,
-                                       fe, step, radius, callno.data() + lo, out_cost + lo, out_delay + lo,
-                                       out_curves ? out_curves + (size_t)lo * D : nullptr);
+            const size_t r = (size_t)lo * W;
+            return gyro_variant_search(q, timestamps_s, gyro_xyz, count, variants.from(lo), cnt, initial_delay, W,
+                                       fb, fe, step, radius, callno.data() + r, out_cost + r, out_delay + r,
+                                       out_curves ? out_curves + r * D : nullptr);
         });
-        if (!call_nos) p->call_no += (uint64_t)n_orient;
+        if (!call_nos) p->call_no += (uint64_t)nw;
         for (rssync_problem* r : p->replicas) r->synced_version = ~0ull;
         return rc;
     }
@@ -2988,12 +3074,11 @@ int gyro_variant_search(rssync_problem* p, const double* timestamps_s, const dou
     std::vector<double> delays;
     if (int rc = presync_delay_grid(p, initial_delay, step, radius, delays)) return rc;
     const int D = (int)delays.size();
-    std::vector<FrameDesc> sel;
-    int max_n = 0;
-    if (int rc = select_frames(p, fb, fe, sel, max_n, "pre-sync")) return rc;
-    const int F = (int)sel.size();
+    SearchWindows win;
+    if (int rc = win.select(p, W, fb, fe)) return rc;
+    const int F = win.F();
     if (int rc = check_grid_size(p, F, D)) return rc;
-    const std::vector<uint64_t> calls = call_numbers(p, call_nos, n_orient);
+    const std::vector<uint64_t> calls = call_numbers(p, call_nos, nw);
     join_gyro(p);
     if (int rc = flush(p)) return rc;  // the tracks, and whatever gyro was pending
     cudaSetDevice(p->device);
@@ -3018,9 +3103,10 @@ int gyro_variant_search(rssync_problem* p, const double* timestamps_s, const dou
     CUDA_TRY(p, cudaMemcpyAsync(p->d_var_in.ptr + n, gyro_xyz, 3 * n * sizeof(double), cudaMemcpyHostToDevice, st));
     CUDA_TRY(p, cudaMemsetAsync(p->d_var_flags.ptr, 0, (size_t)n_orient * sizeof(unsigned), st));
     p->h2d += n * (sizeof(int64_t) + 4 * sizeof(double));
-    if (int rc = stage_grid(p, sel.data(), sel.size(), F, delays.data(), D, n_orient)) return rc;
+    if (int rc = stage_grid(p, win.frames.data(), win.frames.size(), F, delays.data(), D, nw)) return rc;
+    if (int rc = stage_windows(p, win, calls, n_orient)) return rc;
     if (int rc = upload_elimination(p, nq, st)) return rc;
-    const int max_chunk = grid_max_chunk(sel.data(), F, delays.data(), D, plan.sample_rate, max_n);
+    const int max_chunk = grid_max_chunk(win.frames.data(), F, delays.data(), D, plan.sample_rate, win.max_n);
     rs::DeviceData dd = p->device_data();
     dd.nq = (int)nq;
     dd.q0 = plan.first_timestamp;
@@ -3038,10 +3124,8 @@ int gyro_variant_search(rssync_problem* p, const double* timestamps_s, const dou
                                      p->d_elim.ptr + 2 * nq, (int)nq, rec, st);
             if (F > 0) {
                 dd.rec = rec;
-                rs::launch_presync_grid(dd, p->d_frames.ptr, F, max_n, p->d_delays.ptr, D, p->seed, rs::kStreamPreSync,
-                                        calls[(size_t)(k0 + v)], 0, p->d_framecost.ptr,
-                                        p->d_costs.ptr + (size_t)(k0 + v) * D, p->d_flags.ptr + 2 * (size_t)(k0 + v), st,
-                                        max_chunk, p->simplified);
+                launch_candidate_grid(p, dd, win, k0 + v, p->d_frames.ptr, p->d_delays.ptr, D,
+                                      calls[(size_t)(k0 + v) * W], max_chunk, st);
             }
         }
         CUDA_TRY(p, cudaGetLastError());
@@ -3051,7 +3135,7 @@ int gyro_variant_search(rssync_problem* p, const double* timestamps_s, const dou
                                         cudaMemcpyDeviceToDevice, st));
         }
     }
-    std::vector<double> costs((size_t)n_orient * D, 0.0);
+    std::vector<double> costs((size_t)nw * D, 0.0);
     std::vector<unsigned> resampled((size_t)n_orient, 0u), flags((size_t)n_orient * 2, 0u);
     if (F > 0)
         if (int rc = d2h(p, costs.data(), p->d_costs.ptr, costs.size() * sizeof(double))) return rc;
@@ -3063,13 +3147,12 @@ int gyro_variant_search(rssync_problem* p, const double* timestamps_s, const dou
     p->q0 = plan.first_timestamp;
     p->nq = nq;
     p->gyro_dirty = false;
-    if (!call_nos) p->call_no += (uint64_t)n_orient;
+    if (!call_nos) p->call_no += (uint64_t)nw;
     p->grid_tasks = (uint64_t)F * (uint64_t)D;
     for (int k = 0; k < n_orient; ++k) {
         if (resampled[(size_t)k]) { p->err = "set-gyro-quaternions: non-finite sample after interpolation"; return RSSYNC_E_NONFINITE; }
         if (const unsigned fl = flags[2 * (size_t)k]) { p->err = presync_panic_text(fl); return RSSYNC_E_NONFINITE; }
-        curve_argmin(&costs[(size_t)k * D], delays.data(), D, &out_cost[k], &out_delay[k]);
-        if (out_curves) std::memcpy(out_curves + (size_t)k * D, &costs[(size_t)k * D], sizeof(double) * D);
+        candidate_results(k, W, costs, delays, out_cost, out_delay, out_curves);
     }
     return RSSYNC_OK;
 }
@@ -3094,17 +3177,21 @@ int rssync_orientation_search_ex(rssync_problem* p, const double* timestamps_s, 
                                  const uint64_t* call_nos, double* out_cost, double* out_delay) {
     RS_NVTX_RANGE();
     return gyro_variant_search(p, timestamps_s, gyro_xyz, count, GyroVariants{orientations, nullptr}, n_orient,
-                               initial_delay, fb, fe, step, radius, call_nos, out_cost, out_delay, nullptr);
+                               initial_delay, 1, &fb, &fe, step, radius, call_nos, out_cost, out_delay, nullptr);
 }
 
-// The same search over arbitrary 3x3 gyro axis mappings, e.g. candidate camera mount rotations
-int rssync_rotation_search(rssync_problem* p, const double* timestamps_s, const double* gyro_xyz, size_t count,
-                           const double* matrices, int n_rot, double initial_delay, int64_t fb, int64_t fe,
-                           double step, double radius, const uint64_t* call_nos, double* out_cost,
-                           double* out_delay, double* out_curves) {
-    RS_NVTX_RANGE();
+}  // extern "C"
+
+namespace {
+
+// The rotation search over W windows (W = 1: rssync_rotation_search)
+int rotation_search_impl(rssync_problem* p, const double* timestamps_s, const double* gyro_xyz, size_t count,
+                         const double* matrices, int n_rot, int W, const int64_t* fb, const int64_t* fe,
+                         double initial_delay, double step, double radius, const uint64_t* call_nos,
+                         double* out_cost, double* out_delay, double* out_curves) {
     if (!p || n_rot < 0) return RSSYNC_E_INVALID;
-    if (n_rot == 0) return RSSYNC_OK;
+    if (int rc = check_search_counts(p, n_rot, W, fb, fe, "rotation-search")) return rc;
+    if (n_rot == 0 || W == 0) return RSSYNC_OK;
     if (!matrices) return RSSYNC_E_INVALID;
     for (int i = 0; i < n_rot; ++i)
         if (!all_finite(matrices + (size_t)i * 9, 9)) {
@@ -3112,7 +3199,31 @@ int rssync_rotation_search(rssync_problem* p, const double* timestamps_s, const 
             return RSSYNC_E_INVALID;
         }
     return gyro_variant_search(p, timestamps_s, gyro_xyz, count, GyroVariants{nullptr, matrices}, n_rot,
-                               initial_delay, fb, fe, step, radius, call_nos, out_cost, out_delay, out_curves);
+                               initial_delay, W, fb, fe, step, radius, call_nos, out_cost, out_delay, out_curves);
+}
+
+}  // namespace
+
+extern "C" {
+
+// The same search over arbitrary 3x3 gyro axis mappings, e.g. candidate camera mount rotations
+int rssync_rotation_search(rssync_problem* p, const double* timestamps_s, const double* gyro_xyz, size_t count,
+                           const double* matrices, int n_rot, double initial_delay, int64_t fb, int64_t fe,
+                           double step, double radius, const uint64_t* call_nos, double* out_cost,
+                           double* out_delay, double* out_curves) {
+    RS_NVTX_RANGE();
+    return rotation_search_impl(p, timestamps_s, gyro_xyz, count, matrices, n_rot, 1, &fb, &fe, initial_delay, step,
+                                radius, call_nos, out_cost, out_delay, out_curves);
+}
+
+int rssync_rotation_search_windows(rssync_problem* p, const double* timestamps_s, const double* gyro_xyz,
+                                   size_t count, const double* matrices, int n_rot, int n_windows,
+                                   const int64_t* fb, const int64_t* fe, double initial_delay, double step,
+                                   double radius, const uint64_t* call_nos, double* out_cost, double* out_delay,
+                                   double* out_curves) {
+    RS_NVTX_RANGE();
+    return rotation_search_impl(p, timestamps_s, gyro_xyz, count, matrices, n_rot, n_windows, fb, fe, initial_delay,
+                                step, radius, call_nos, out_cost, out_delay, out_curves);
 }
 
 }  // extern "C"
@@ -3162,36 +3273,32 @@ void retimed_bounds(const rs::PixelFrame& f, const double* e, double r, double& 
     hi = std::max(std::max(a0, a1), std::max(b0, b1));
 }
 
-}  // namespace
-
-extern "C" {
-
-// PreSync at n_readouts rolling-shutter readouts without re-ingesting: the selected frames are re-timed
-// into a scratch arena (retime_frames_kernel) and the loss grid runs on it, per readout, back to back on
-// the problem's stream; one read-back at the end.  The problem's own arena, frame table and gyro are
-// not touched.  A multi-device problem shards the readouts over its devices, as the orientation search
-// does its variants.
-int rssync_readout_search(rssync_problem* p, const double* readouts, int n_readouts, double initial,
-                          int64_t fb, int64_t fe, double step, double radius, const uint64_t* call_nos,
-                          double* out_cost, double* out_delay, double* out_curves) {
-    RS_NVTX_RANGE();
+// PreSync at n rolling-shutter readouts over W frame windows without re-ingesting: the union of the
+// windows' frames is re-timed into a scratch arena (retime_frames_kernel) and one loss grid over all
+// windows runs on it, per readout, back to back on the problem's stream; one read-back at the end.  The
+// problem's own arena, frame table and gyro are not touched.  A multi-device problem shards the readouts
+// over its devices, as the orientation search does its variants.
+int readout_search_impl(rssync_problem* p, const double* readouts, int n, int W, const int64_t* fb,
+                        const int64_t* fe, double initial, double step, double radius, const uint64_t* call_nos,
+                        double* out_cost, double* out_delay, double* out_curves) {
     if (!p) return RSSYNC_E_INVALID;
-    if (n_readouts < 0) { p->err = "readout-search: negative readout count"; return RSSYNC_E_INVALID; }
-    if (n_readouts == 0) return RSSYNC_OK;
+    if (int rc = check_search_counts(p, n, W, fb, fe, "readout-search")) return rc;
+    if (n == 0 || W == 0) return RSSYNC_OK;
     if (!readouts || !out_cost || !out_delay) { p->err = "readout-search: null buffer"; return RSSYNC_E_INVALID; }
-    if (int rc = check_readouts(p, readouts, n_readouts, "readout-search")) return rc;
+    if (int rc = check_readouts(p, readouts, n, "readout-search")) return rc;
     if (int rc = require_gyro(p, "pre-sync")) return rc;
     std::vector<double> delays;
     if (int rc = presync_delay_grid(p, initial, step, radius, delays)) return rc;
     const int D = (int)delays.size();
-    std::vector<FrameDesc> sel;
-    int max_n = 0;
-    if (int rc = select_frames(p, fb, fe, sel, max_n, "pre-sync")) return rc;
-    if (int rc = require_retime(p, sel, "readout-search")) return rc;
-    const int F = (int)sel.size(), n = n_readouts;
+    SearchWindows win;
+    if (int rc = win.select(p, W, fb, fe, [p](const std::vector<FrameDesc>& sel) {
+            return require_retime(p, sel, "readout-search");
+        }))
+        return rc;
+    const int F = win.F(), nw = n * W;
     if (int rc = check_grid_size(p, F, D)) return rc;
-    const std::vector<uint64_t> calls = call_numbers(p, call_nos, n);
-    if (!call_nos) p->call_no += (uint64_t)n;
+    const std::vector<uint64_t> calls = call_numbers(p, call_nos, nw);
+    if (!call_nos) p->call_no += (uint64_t)nw;
     if (is_multi(p) && n > 1) {
         // readouts are independent: shard them, explicit call numbers.  Every device re-times into its
         // own scratch arena and leaves its inputs alone, so no replica is stale afterwards.  Rank order
@@ -3199,8 +3306,9 @@ int rssync_readout_search(rssync_problem* p, const double* readouts, int n_reado
         if (int rc = multi_replicate(p)) return rc;
         if (int rc = multi_replicate_row_fractions(p)) return rc;
         const int rc = multi_for_each_shard(p, n, false, [&](rssync_problem* q, int lo, int cnt) {
-            return rssync_readout_search(q, readouts + lo, cnt, initial, fb, fe, step, radius, calls.data() + lo,
-                                         out_cost + lo, out_delay + lo, out_curves ? out_curves + (size_t)lo * D : nullptr);
+            const size_t r = (size_t)lo * W;
+            return readout_search_impl(q, readouts + lo, cnt, W, fb, fe, initial, step, radius, calls.data() + r,
+                                       out_cost + r, out_delay + r, out_curves ? out_curves + r * D : nullptr);
         });
         if (F > 0 && (rc == RSSYNC_OK || rc == RSSYNC_E_NONFINITE)) {  // the statistics of the last readout's grid
             const rssync_problem* last = rank_problem(p, n_ranks(p) - 1);
@@ -3211,29 +3319,41 @@ int rssync_readout_search(rssync_problem* p, const double* readouts, int n_reado
     }
     CUDA_TRY(p, cudaSetDevice(p->device));
     if (int rc = flush(p)) return rc;  // pending gyro and tracks; ordered behind ingests in flight
-    std::vector<double> costs((size_t)n * D, 0.0);  // no frames: the reference sums over none
+    std::vector<double> costs((size_t)nw * D, 0.0);  // no frames: the reference sums over none
     std::vector<unsigned> flags((size_t)n * 2, 0u);
     if (F > 0) {
         cudaStream_t st = p->stream;
-        // the scratch arena holds the selected frames back to back
-        std::vector<int32_t> dst((size_t)F);
+        // the scratch arena holds the union of the windows' frames back to back; uidx[f]: listed frame f's
+        // place in the union
+        std::vector<FrameDesc> sel;
+        std::vector<int> uidx((size_t)F);
+        {
+            std::unordered_map<int64_t, int> at;
+            for (int f = 0; f < F; ++f) {
+                const auto ins = at.emplace(win.frames[(size_t)f].id, (int)sel.size());
+                if (ins.second) sel.push_back(win.frames[(size_t)f]);
+                uidx[(size_t)f] = ins.first->second;
+            }
+        }
+        const int U = (int)sel.size();
+        std::vector<int32_t> dst((size_t)U);
         size_t rays = 0;
-        for (int f = 0; f < F; ++f) {
-            dst[(size_t)f] = (int32_t)rays;
-            rays += (size_t)(sel[(size_t)f].n + 31) / 32 * 32;
+        for (int u = 0; u < U; ++u) {
+            dst[(size_t)u] = (int32_t)rays;
+            rays += (size_t)(sel[(size_t)u].n + 31) / 32 * 32;
         }
         const std::vector<rs::PixelFrame> rec = retime_records(p, sel, dst);
         CUDA_TRY(p, p->d_rt_rays.reserve(rays * 8));
         CUDA_TRY(p, p->d_rt_orig.reserve(rays));
         CUDA_TRY(p, p->d_rt_pos.reserve(rays));
-        CUDA_TRY(p, p->d_pixframes.reserve((size_t)F));
-        CUDA_TRY(p, p->d_rt_ext.reserve((size_t)F * 4));
-        if (int rc = h2d(p, p->d_pixframes.ptr, rec.data(), sizeof(rs::PixelFrame) * F)) return rc;
+        CUDA_TRY(p, p->d_pixframes.reserve((size_t)U));
+        CUDA_TRY(p, p->d_rt_ext.reserve((size_t)U * 4));
+        if (int rc = h2d(p, p->d_pixframes.ptr, rec.data(), sizeof(rs::PixelFrame) * U)) return rc;
         // the first readout's re-time also reports each frame's row extremes, from which the host takes
         // every readout's frame bounds (the frame tables and the grids' staging windows)
-        rs::launch_retime_frames(p->d_pixframes.ptr, F, p->d_rays.ptr, p->d_orig.ptr, p->d_rowq.ptr, readouts[0],
+        rs::launch_retime_frames(p->d_pixframes.ptr, U, p->d_rays.ptr, p->d_orig.ptr, p->d_rowq.ptr, readouts[0],
                                  p->d_rt_rays.ptr, p->d_rt_orig.ptr, p->d_rt_pos.ptr, p->d_rt_ext.ptr, st);
-        std::vector<double> ext((size_t)F * 4);
+        std::vector<double> ext((size_t)U * 4);
         if (int rc = d2h(p, ext.data(), p->d_rt_ext.ptr, ext.size() * sizeof(double))) return rc;
         if (int rc = finish_stream(p, st)) return rc;
         std::vector<FrameDesc> tables((size_t)n * F);
@@ -3241,24 +3361,24 @@ int rssync_readout_search(rssync_problem* p, const double* readouts, int n_reado
         for (int j = 0; j < n; ++j) {
             FrameDesc* table = &tables[(size_t)j * F];
             for (int f = 0; f < F; ++f) {
-                table[f] = FrameDesc{sel[(size_t)f].id, dst[(size_t)f], sel[(size_t)f].n, 0.0, 0.0};
-                retimed_bounds(rec[(size_t)f], &ext[(size_t)f * 4], readouts[j], table[f].ts_lo, table[f].ts_hi);
+                const size_t u = (size_t)uidx[(size_t)f];
+                table[f] = FrameDesc{sel[u].id, dst[u], sel[u].n, 0.0, 0.0};
+                retimed_bounds(rec[u], &ext[u * 4], readouts[j], table[f].ts_lo, table[f].ts_hi);
             }
-            max_chunk[(size_t)j] = grid_max_chunk(table, F, delays.data(), D, p->sr, max_n);
+            max_chunk[(size_t)j] = grid_max_chunk(table, F, delays.data(), D, p->sr, win.max_n);
         }
-        if (int rc = stage_grid(p, tables.data(), tables.size(), F, delays.data(), D, n)) return rc;
+        if (int rc = stage_grid(p, tables.data(), tables.size(), F, delays.data(), D, nw)) return rc;
+        if (int rc = stage_windows(p, win, calls, n)) return rc;
         rs::DeviceData dd = p->device_data();
         dd.rays = p->d_rt_rays.ptr;
         dd.orig = p->d_rt_orig.ptr;
         dd.pos = p->d_rt_pos.ptr;
         for (int j = 0; j < n; ++j) {
             if (j > 0)
-                rs::launch_retime_frames(p->d_pixframes.ptr, F, p->d_rays.ptr, p->d_orig.ptr, p->d_rowq.ptr, readouts[j],
+                rs::launch_retime_frames(p->d_pixframes.ptr, U, p->d_rays.ptr, p->d_orig.ptr, p->d_rowq.ptr, readouts[j],
                                          p->d_rt_rays.ptr, p->d_rt_orig.ptr, p->d_rt_pos.ptr, nullptr, st);
-            rs::launch_presync_grid(dd, p->d_frames.ptr + (size_t)j * F, F, max_n, p->d_delays.ptr, D, p->seed,
-                                    rs::kStreamPreSync, calls[(size_t)j], 0, p->d_framecost.ptr,
-                                    p->d_costs.ptr + (size_t)j * D, p->d_flags.ptr + 2 * (size_t)j, st,
-                                    max_chunk[(size_t)j], p->simplified);
+            launch_candidate_grid(p, dd, win, j, p->d_frames.ptr + (size_t)j * F, p->d_delays.ptr, D,
+                                  calls[(size_t)j * W], max_chunk[(size_t)j], st);
         }
         if (int rc = d2h(p, costs.data(), p->d_costs.ptr, costs.size() * sizeof(double))) return rc;
         if (int rc = d2h(p, flags.data(), p->d_flags.ptr, flags.size() * sizeof(unsigned))) return rc;
@@ -3268,11 +3388,31 @@ int rssync_readout_search(rssync_problem* p, const double* readouts, int n_reado
     }
     for (int j = 0; j < n; ++j) {
         if (const unsigned fl = flags[2 * (size_t)j]) { p->err = presync_panic_text(fl); return RSSYNC_E_NONFINITE; }
-        const double* c = &costs[(size_t)j * D];
-        curve_argmin(c, delays.data(), D, &out_cost[j], &out_delay[j]);
-        if (out_curves) std::memcpy(out_curves + (size_t)j * D, c, sizeof(double) * D);
+        candidate_results(j, W, costs, delays, out_cost, out_delay, out_curves);
     }
     return RSSYNC_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int rssync_readout_search(rssync_problem* p, const double* readouts, int n_readouts, double initial,
+                          int64_t fb, int64_t fe, double step, double radius, const uint64_t* call_nos,
+                          double* out_cost, double* out_delay, double* out_curves) {
+    RS_NVTX_RANGE();
+    if (p && n_readouts < 0) { p->err = "readout-search: negative readout count"; return RSSYNC_E_INVALID; }
+    return readout_search_impl(p, readouts, n_readouts, 1, &fb, &fe, initial, step, radius, call_nos, out_cost,
+                               out_delay, out_curves);
+}
+
+int rssync_readout_search_windows(rssync_problem* p, const double* readouts, int n_readouts, int n_windows,
+                                  const int64_t* fb, const int64_t* fe, double initial, double step, double radius,
+                                  const uint64_t* call_nos, double* out_cost, double* out_delay,
+                                  double* out_curves) {
+    RS_NVTX_RANGE();
+    return readout_search_impl(p, readouts, n_readouts, n_windows, fb, fe, initial, step, radius, call_nos, out_cost,
+                               out_delay, out_curves);
 }
 
 // Re-time the pixel frames of [fb, fe) in place at `readout`: afterwards the problem holds what ingesting

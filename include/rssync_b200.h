@@ -120,6 +120,64 @@ int rssync_set_track_pixels_device(rssync_problem* p, size_t n_frames, const int
                                    const double* frame_ts_b, const double* points_a,
                                    const double* points_b, const rssync_lens* lens,
                                    double image_rows, void* stream);
+/* Parameters of rssync_track_frames_device (NULL there = the defaults shown). */
+typedef struct rssync_track_params {
+    int levels;     /* pyramid levels, 1..6 (default 3) */
+    int window;     /* odd window side in pixels, 5..63 (default 21) */
+    int max_iters;  /* LK iterations per level, 1..100 (default 30) */
+    double epsilon; /* stop when |delta| < epsilon px (default 0.01) */
+    double min_eig; /* lost when the minimum eigenvalue of G / window^2 < this (default 1e-4) */
+} rssync_track_params;
+/* Track points between decoded frames on the device, then ingest the pairs (the first half of
+ * track_frames, core_testcode.cpp:97-162, with sparse pyramidal Lucas-Kanade in place of dense flow).
+ * images: n_frames + 1 8-bit luma planes in device (or managed) memory of the problem's (primary)
+ * device, `height` rows of `pitch` bytes each (pitch >= width), planes back to back: row y of image j
+ * starts at images + (j * height + y) * pitch (an NV12 Y plane as decoded, a strided uint8 tensor).
+ * Frame i (id frames[i]) pairs image i (timestamp image_ts[i], seconds) with image i + 1
+ * (image_ts[i + 1]); points (device, sum(counts) x 2 doubles, x then y, frames concatenated) are its query
+ * points on image i.  A clip goes in batches that overlap by one image.
+ * Every point is tracked from image i to image i + 1.  The kept points then give exactly, byte for byte,
+ * what rssync_set_track_pixels_device gives with points_a = the kept query points, points_b = their
+ * tracked positions, counts = the kept counts (a frame may keep 0), frame_ts_a / frame_ts_b =
+ * image_ts[i] / image_ts[i + 1] and image_rows = height: frame table, arena, row fractions and re-timing
+ * table, so rssync_readout_search(_windows) and rssync_set_readout accept the frames.  The call counter
+ * and the gyro are untouched.
+ * A point is lost (status 0, not ingested) when it starts or ends outside [0, width - 1] x [0, height - 1],
+ * when the minimum-eigenvalue test fails at any level, or when an update is not finite.  tracked_out
+ * (sum(counts) x 2) and status_out (sum(counts) bytes), device memory or NULL, receive every point's
+ * position and status; a point lost before its last level has ended gets NaN.
+ * Algorithm (float32 throughout, evaluated in the order written; a sum over a window: lane k of a warp
+ * adds the pixels t = k, k + 32, ... of the row-major window in that order, then the 32 partials are
+ * combined by the butterfly xor 16, 8, 4, 2, 1):
+ *  - Pyramid: level 0 is the plane as given.  Level l + 1 has size ((w + 1) / 2, (h + 1) / 2); its pixel
+ *    (X, Y) is the [1 4 6 4 1] / 16 blur of level l at (2X, 2Y) with BORDER_REFLECT_101: per row
+ *    r = (s[-2] + s[2]) + 4 (s[-1] + s[1]) + 6 s[0], then the same over the rows r, times 1/256
+ *    (cv2.pyrDown of float32 input).  Images are processed in chunks whose pyramids fit 256 MiB of
+ *    scratch (at least 2 images): max(2, floor(2^26 / floats of levels 1..levels-1 of one image)); each
+ *    image's pyramid is built once; the chunks change no result.
+ *  - A level is read at integer (x, y) clamped to the level (the nearest edge pixel), and at sub-pixel
+ *    (x0 + ax, y0 + ay), x0 = floor: (1 - ay)((1 - ax) I00 + ax I01) + ay((1 - ax) I10 + ax I11).
+ *  - LK (Bouguet), coarse to fine, guess g = 0 at level levels - 1, g = 2 (g + v) going down a level.
+ *    At level l the query point is p = (float)q * 2^-l.  Side a: the (window + 2)^2 samples A at p + (dx, dy),
+ *    |dx|, |dy| <= window / 2 + 1; gradients over the window: Ix = (3 (A[-1][+1] - A[-1][-1]) +
+ *    10 (A[0][+1] - A[0][-1]) + 3 (A[+1][+1] - A[+1][-1])) / 32, Iy alike with rows and columns swapped;
+ *    G = [sum Ix^2, sum Ix Iy; ., sum Iy^2].  Lost unless ((gxx + gyy) - sqrt((gxx - gyy)^2 +
+ *    4 gxy^2)) / (2 window^2) >= min_eig.  Then, from v = 0, up to max_iters times: b = sum (A - B) [Ix, Iy]
+ *    with B the side-b samples at p + g + v + (dx, dy), delta = G^-1 b = ((gyy bx - gxy by) / det,
+ *    (gxx by - gxy bx) / det), det = gxx gyy - gxy^2; lost if delta is not finite; v += delta; stop when
+ *    |delta|^2 < epsilon^2.  The tracked position is q + (double)(g + v) of level 0.
+ * Checked before anything is applied: RSSYNC_E_INVALID for images / points (or a non-NULL output) that are
+ * not device memory of the problem's device, pitch < width, width or height below window * 2^(levels - 1),
+ * params out of range, a count above 512, and the lens / image-height checks of the pixels forms;
+ * RSSYNC_E_NONFINITE for a non-finite image_ts (reported as the pixels forms report frame timestamps, with
+ * image_ts[0..n_frames) the a side) and a non-finite query point ("non-finite numbers in rays_a").
+ * Ordering and borrowing as in the other _device forms: reads are ordered after `stream`, and the library
+ * has finished with images and points when the call returns.  A multi-device problem ingests on its
+ * primary; the replicas receive the arena at the next compute call. */
+int rssync_track_frames_device(rssync_problem* p, size_t n_frames, const int64_t* frames, const size_t* counts,
+                               const double* image_ts, const double* points, const uint8_t* images, size_t pitch,
+                               int width, int height, const rssync_lens* lens, const rssync_track_params* params,
+                               double* tracked_out, uint8_t* status_out, void* stream);
 /* SetTrackResult for n_frames frames whose rays the caller computed (any camera model), with the
  * rolling-shutter timestamps formed here from per-ray row fractions.  Ray k of frame i gets
  * ts_a = frame_ts_a[i] + readout * frac_a[k] (ts_b alike): one multiply and one add, not contracted,

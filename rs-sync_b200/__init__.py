@@ -44,7 +44,7 @@ C_ABI_SYMBOLS = [
     "rssync_readout_search", "rssync_set_readout", "rssync_integrate_gyro_matrix", "rssync_rotation_search",
     "rssync_set_track_row_fractions", "rssync_set_track_row_fractions_device",
     "rssync_retime_table", "rssync_row_fraction_plane", "rssync_adopt_row_fractions",
-    "rssync_readout_search_windows", "rssync_rotation_search_windows",
+    "rssync_readout_search_windows", "rssync_rotation_search_windows", "rssync_track_frames_device",
 ]
 # Itanium-ABI symbols of the C++ drop-in face (same set the reference's librssync_core exports)
 CXX_ABI_SYMBOLS = [
@@ -86,6 +86,29 @@ RETIME_DTYPE = np.dtype([("id", "<i8"), ("frame_ts_a", "<f8"), ("frame_ts_b", "<
 class Lens(C.Structure):
     """rssync_lens: readout_s fx fy cx cy k1 k2 k3 k4 (one line of the reference's lens file)"""
     _fields_ = [(n, C.c_double) for n in ("readout", "fx", "fy", "cx", "cy", "k1", "k2", "k3", "k4")]
+
+
+class TrackParams(C.Structure):
+    """rssync_track_params: the pyramidal Lucas-Kanade tracker's settings (track_frames)"""
+    _fields_ = [("levels", C.c_int), ("window", C.c_int), ("max_iters", C.c_int), ("epsilon", C.c_double),
+                ("min_eig", C.c_double)]
+
+    def __init__(self, levels=3, window=21, max_iters=30, epsilon=0.01, min_eig=1e-4):
+        super().__init__(levels, window, max_iters, epsilon, min_eig)
+
+
+def grid_points(width, height, step):
+    """The query grid of the reference's front end: every `step` pixels in x and y, as an (n, 2) float64 array,
+    x fastest.  Origin (this engine's choice; the reference's exact offsets are not known here): the grid is
+    centred, its first point at ((width - 1 - step * (nx - 1)) / 2, likewise in y) with nx = (width - 1) // step
+    + 1 points per row, so the margins to both edges are equal."""
+    if step <= 0 or width < 1 or height < 1:
+        raise ValueError("grid_points: width, height and step must be positive")
+    nx, ny = (int(width) - 1) // int(step) + 1, (int(height) - 1) // int(step) + 1
+    x0, y0 = (width - 1 - step * (nx - 1)) / 2.0, (height - 1 - step * (ny - 1)) / 2.0
+    gy, gx = np.meshgrid(y0 + step * np.arange(ny, dtype=np.float64), x0 + step * np.arange(nx, dtype=np.float64),
+                         indexing="ij")
+    return np.ascontiguousarray(np.stack([gx.ravel(), gy.ravel()], axis=-1))
 
 
 class RsSyncError(RuntimeError):
@@ -147,6 +170,9 @@ def load_library():
                                                  C.c_double]
     L.rssync_set_track_row_fractions_device.argtypes = [P, C.c_size_t, c_i64_p, C.POINTER(C.c_size_t), c_double_p,
                                                         c_double_p, P, P, P, P, C.c_double, P]
+    L.rssync_track_frames_device.argtypes = [P, C.c_size_t, c_i64_p, C.POINTER(C.c_size_t), c_double_p, P, P,
+                                             C.c_size_t, C.c_int, C.c_int, C.POINTER(Lens), C.POINTER(TrackParams),
+                                             P, P, P]
     L.rssync_presync.argtypes = [P, C.c_double, C.c_int64, C.c_int64, C.c_double, C.c_double, c_double_p, c_double_p]
     L.rssync_sync.argtypes = [P, C.c_double, C.c_int64, C.c_int64, C.c_double, C.c_double, c_double_p, c_double_p]
     L.rssync_debug_presync.argtypes = [P, C.c_double, C.c_int64, C.c_int64, C.c_double, c_double_p, c_double_p, C.c_int]
@@ -553,6 +579,43 @@ class SyncProblem:
             return
         a = [_f64(x) for x in (frac_a, frac_b, rays_a, rays_b)]
         self._check(self.L.rssync_set_track_row_fractions(*args, *[_dp(x) for x in a], float(readout)))
+
+    def track_frames(self, frames, counts, image_ts, points, images, lens, params=None):
+        """Track points between decoded frames on the device and ingest the kept pairs
+        (rssync_track_frames_device).  images: CUDA uint8 tensor (n_frames + 1, H, W) whose last dimension is
+        contiguous (row pitch = stride(1)); frame i pairs images[i] (image_ts[i]) with images[i + 1];
+        points: CUDA float64 tensor (sum(counts), 2), the query points on image i, frames concatenated.
+        frames, counts and image_ts stay on the host; params: TrackParams or None (the defaults).  Ordered
+        after the current stream of the tensors' device.  Returns (tracked, status): CUDA tensors
+        (sum(counts), 2) float64 and (sum(counts),) uint8, every point's tracked position and status
+        (1 = kept and ingested)."""
+        import torch
+        fr = np.ascontiguousarray(frames, dtype=np.int64)
+        cn = np.ascontiguousarray(counts, dtype=np.uint64)
+        ts = _f64(image_ts)
+        n = int(cn.sum())
+        if not (getattr(images, "is_cuda", False) and getattr(points, "is_cuda", False)):
+            raise TypeError("track_frames: images and points must be CUDA tensors")
+        if images.dtype != torch.uint8 or images.dim() != 3 or images.stride(2) != 1:
+            raise ValueError("track_frames: images must be a uint8 tensor (n_frames + 1, H, W) with contiguous rows")
+        if images.shape[0] != fr.shape[0] + 1 or ts.shape[0] != fr.shape[0] + 1:
+            raise ValueError(f"track_frames: {fr.shape[0]} frames need {fr.shape[0] + 1} images and image timestamps, "
+                             f"got {images.shape[0]} and {ts.shape[0]}")
+        if images.shape[0] > 1 and images.stride(0) != images.shape[1] * images.stride(1):
+            raise ValueError("track_frames: the planes must lie back to back (stride(0) = H * stride(1))")
+        dev = images.device
+        (pp,), stream = _device_ptrs((points,), (2 * n,))
+        if points.device != dev:
+            raise ValueError(f"track_frames: images on {dev}, points on {points.device}")
+        tracked = torch.empty((n, 2), dtype=torch.float64, device=dev)
+        status = torch.empty((n,), dtype=torch.uint8, device=dev)
+        lens_c = lens if isinstance(lens, Lens) else Lens(*[float(x) for x in lens])
+        prm = None if params is None else C.byref(params)
+        self._check(self.L.rssync_track_frames_device(
+            self.h, fr.shape[0], fr.ctypes.data_as(c_i64_p), cn.ctypes.data_as(C.POINTER(C.c_size_t)), _dp(ts), pp,
+            C.c_void_p(images.data_ptr()), images.stride(1), images.shape[2], images.shape[1], C.byref(lens_c), prm,
+            C.c_void_p(tracked.data_ptr() if n else None), C.c_void_p(status.data_ptr() if n else None), stream))
+        return tracked, status
 
     def load(self, w, bulk=False):
         """Feed a synth.Workload the way core_testcode feeds a video (core_testcode.cpp:257-268)."""

@@ -330,6 +330,14 @@ struct rssync_problem {
     // (4 doubles per frame)
     DevBuf<double> d_rt_rays, d_rt_ext;
     DevBuf<int32_t> d_rt_orig, d_rt_pos;
+    // rssync_track_frames_device: image pyramids, the compacted pairs and the tracked positions when the
+    // caller takes none (6 doubles per point), the kept offsets, the statuses, the non-finite-query flag
+    DevBuf<float> d_trk_pyr;
+    DevBuf<double> d_trk_pts;
+    DevBuf<int64_t> d_trk_at;
+    DevBuf<uint8_t> d_trk_status;
+    DevBuf<unsigned> d_trk_flag;
+    PinBuf<unsigned> h_trk_flag;
 
     std::vector<std::pair<double, int32_t>> sort_scratch;
     std::vector<double> trace_delay, trace_step;
@@ -1572,6 +1580,8 @@ void rssync_destroy(rssync_problem* p) {
     p->d_var_rec.release(); p->d_var_prefix.release(); p->d_elim.release();
     p->d_var_orients.release(); p->d_var_flags.release();
     p->d_rowq.release(); p->d_rt_rays.release(); p->d_rt_ext.release(); p->d_rt_orig.release(); p->d_rt_pos.release();
+    p->d_trk_pyr.release(); p->d_trk_pts.release(); p->d_trk_at.release(); p->d_trk_status.release();
+    p->d_trk_flag.release(); p->h_trk_flag.release();
     if (p->owns_stream && p->stream) { cudaStreamSynchronize(p->stream); cudaStreamDestroy(p->stream); }
     for (SyncLane& L : p->lanes) L.release();
     if (p->ev_sync_ready) cudaEventDestroy(p->ev_sync_ready);
@@ -2553,6 +2563,82 @@ int rssync_set_track_pixels(rssync_problem* p, size_t n_frames, const int64_t* f
     return RSSYNC_OK;
 }
 
+}  // extern "C"
+
+namespace {
+
+// Points that kernels on the problem's stream write during the call, with their frame offsets
+// (rssync_track_frames_device): `queue` enqueues the writers and the copies back of what the host needs,
+// and returns the offsets (device, n_frames + 1) for the stage kernel; `verdict`, after the round trip,
+// sets the host offsets or fails the call before anything is placed.
+struct DevicePointSource {
+    std::function<const int64_t*(const DeviceStaging&)> queue;
+    std::function<int(const DeviceStaging&, std::vector<size_t>&)> verdict;
+};
+
+// The body of rssync_set_track_pixels_device once its host checks have passed: the check, the timestamp
+// bounds and the copy into the staging buffer on the device (stage_tracks_kernel), the per-frame verdicts
+// back in the one round trip, then placement and ingest.  at: the frames' offsets in points_a / points_b;
+// the staging buffer holds at[n_frames] points per side.  src (or null): the points are written on the
+// device first, at offsets only known after the round trip (at then becomes those offsets).
+int ingest_pixels_device(rssync_problem* p, size_t n_frames, const int64_t* frames, std::vector<size_t>& at,
+                         const double* frame_ts_a, const double* frame_ts_b, const double* points_a,
+                         const double* points_b, const rssync_lens* lens, double image_rows, void* stream,
+                         const DevicePointSource* src = nullptr) {
+    const size_t total = at[n_frames];
+    DeviceStaging s;
+    if (int rc = begin_device_staging(p, at, 4 * total, frame_ts_a, frame_ts_b, stream, s)) return rc;
+    const int64_t* d_at = src ? src->queue(s) : s.d_at;
+    if (!d_at) return RSSYNC_E_CUDA;  // (p->err set by queue)
+    const rs::LensDev L{lens->readout, lens->fx, lens->fy, lens->cx, lens->cy, lens->k1, lens->k2, lens->k3, lens->k4};
+    rs::launch_stage_points(d_at, s.d_fts, (int)n_frames, (int64_t)total, points_a, points_b, L, image_rows,
+                            s.d_data, s.d_info, p->stream);
+    if (int rc = read_stage_info(p, n_frames, s)) return rc;
+    if (src)
+        if (int rc = src->verdict(s, at)) return rc;
+    for (size_t i = 0; i < n_frames; ++i)
+        if (s.h_info[i].bad) {
+            p->err = kMsgNonFinite[(s.h_info[i].bad & 1u) ? kRaysA : kRaysB];
+            return RSSYNC_E_NONFINITE;
+        }
+    p->version++;
+    for (size_t i = 0; i < n_frames; ++i) {
+        FrameDesc* fd = nullptr;
+        if (int rc = place_track(p, frames[i], at[i + 1] - at[i], &fd, /*host_mirror=*/false)) return rc;
+        fd->ts_lo = s.h_info[i].lo;
+        fd->ts_hi = s.h_info[i].hi;
+        s.h_rec[i] = rs::PixelFrame{fd->off, fd->n, (int64_t)at[i], frame_ts_a[i], frame_ts_b[i]};
+    }
+    for (size_t i = 0; i < n_frames; ++i) p->retime[frames[i]] = {frame_ts_a[i], frame_ts_b[i]};
+    if (int rc = reserve_device_arena(p)) return rc;
+    if (int rc = reserve_rowq(p)) return rc;
+    if (int rc = h2d(p, s.d_rec, s.h_rec, n_frames * sizeof(rs::PixelFrame))) return rc;
+    rs::launch_ingest_pixels(s.d_rec, (int)n_frames, s.d_data, s.d_data + 2 * total, L, image_rows, p->d_rays.ptr,
+                             p->d_orig.ptr, p->d_pos.ptr, p->d_rowq.ptr, p->stream);
+    return end_device_ingest(p);
+}
+
+// The buffers of rssync_track_frames_device: device (or managed) memory of the problem's device, as
+// check_device_buffers requires of per-ray buffers
+int check_device_pointer(rssync_problem* p, const void* b, const char* what) {
+    cudaPointerAttributes attr{};
+    const cudaError_t e = b ? cudaPointerGetAttributes(&attr, b) : cudaErrorInvalidValue;
+    if (e != cudaSuccess) cudaGetLastError();  // (clears the error)
+    if (e != cudaSuccess || (attr.type != cudaMemoryTypeDevice && attr.type != cudaMemoryTypeManaged) ||
+        attr.device != p->device) {
+        p->err = std::string("track-frames: ") + what + " is not device memory of the problem's device";
+        return RSSYNC_E_INVALID;
+    }
+    return RSSYNC_OK;
+}
+
+// the tracker's scratch budget: the pyramids of as many images as fit are alive at once
+constexpr size_t kTrackScratchBytes = size_t(256) << 20;
+
+}  // namespace
+
+extern "C" {
+
 // rssync_set_track_pixels with the points in device memory: the check, the timestamp bounds and the
 // copy into the staging buffer run on the device (stage_tracks_kernel).  As in the host form,
 // everything is checked before anything is placed.
@@ -2570,32 +2656,88 @@ int rssync_set_track_pixels_device(rssync_problem* p, size_t n_frames, const int
     const size_t total = at[n_frames];
     if (int rc = check_device_buffers(p, {points_a, points_b}, total)) return rc;
     if (int rc = check_frame_ts(p, n_frames, frame_ts_a, frame_ts_b)) return rc;
-    DeviceStaging s;
-    if (int rc = begin_device_staging(p, at, 4 * total, frame_ts_a, frame_ts_b, stream, s)) return rc;
-    const rs::LensDev L{lens->readout, lens->fx, lens->fy, lens->cx, lens->cy, lens->k1, lens->k2, lens->k3, lens->k4};
-    rs::launch_stage_points(s.d_at, s.d_fts, (int)n_frames, (int64_t)total, points_a, points_b, L, image_rows,
-                            s.d_data, s.d_info, p->stream);
-    if (int rc = read_stage_info(p, n_frames, s)) return rc;
-    for (size_t i = 0; i < n_frames; ++i)
-        if (s.h_info[i].bad) {
-            p->err = kMsgNonFinite[(s.h_info[i].bad & 1u) ? kRaysA : kRaysB];
-            return RSSYNC_E_NONFINITE;
-        }
-    p->version++;
-    for (size_t i = 0; i < n_frames; ++i) {
-        FrameDesc* fd = nullptr;
-        if (int rc = place_track(p, frames[i], counts[i], &fd, /*host_mirror=*/false)) return rc;
-        fd->ts_lo = s.h_info[i].lo;
-        fd->ts_hi = s.h_info[i].hi;
-        s.h_rec[i] = rs::PixelFrame{fd->off, fd->n, (int64_t)at[i], frame_ts_a[i], frame_ts_b[i]};
+    return ingest_pixels_device(p, n_frames, frames, at, frame_ts_a, frame_ts_b, points_a, points_b, lens, image_rows,
+                                stream);
+}
+
+// Sparse pyramidal Lucas-Kanade from image i to image i + 1 of the caller's luma planes, then the kept
+// pairs through rssync_set_track_pixels_device's ingest (ingest_pixels_device), compacted on the device.
+int rssync_track_frames_device(rssync_problem* p, size_t n_frames, const int64_t* frames, const size_t* counts,
+                               const double* image_ts, const double* points, const uint8_t* images, size_t pitch,
+                               int width, int height, const rssync_lens* lens, const rssync_track_params* params,
+                               double* tracked_out, uint8_t* status_out, void* stream) {
+    RS_NVTX_RANGE();
+    if (!p) return RSSYNC_E_INVALID;
+    if (n_frames == 0) return RSSYNC_OK;
+    if (!frames || !counts || !image_ts || !lens || n_frames > (size_t)INT32_MAX - 1) return RSSYNC_E_INVALID;
+    const rssync_track_params tp = params ? *params : rssync_track_params{3, 21, 30, 0.01, 1e-4};
+    if (tp.levels < 1 || tp.levels > 6 || tp.window < 5 || tp.window > 63 || tp.window % 2 == 0 || tp.max_iters < 1 ||
+        tp.max_iters > 100 || !(tp.epsilon >= 0.0) || !std::isfinite(tp.epsilon) || !(tp.min_eig >= 0.0) ||
+        !std::isfinite(tp.min_eig)) {
+        p->err = "track-frames: parameters out of range";
+        return RSSYNC_E_INVALID;
     }
-    for (size_t i = 0; i < n_frames; ++i) p->retime[frames[i]] = {frame_ts_a[i], frame_ts_b[i]};
-    if (int rc = reserve_device_arena(p)) return rc;
-    if (int rc = reserve_rowq(p)) return rc;
-    if (int rc = h2d(p, s.d_rec, s.h_rec, n_frames * sizeof(rs::PixelFrame))) return rc;
-    rs::launch_ingest_pixels(s.d_rec, (int)n_frames, s.d_data, s.d_data + 2 * total, L, image_rows, p->d_rays.ptr,
-                             p->d_orig.ptr, p->d_pos.ptr, p->d_rowq.ptr, p->stream);
-    return end_device_ingest(p);
+    const int64_t min_side = (int64_t)tp.window << (tp.levels - 1);
+    if (width < min_side || height < min_side || pitch < (size_t)width) {
+        p->err = "track-frames: image smaller than window * 2^(levels - 1), or pitch below width";
+        return RSSYNC_E_INVALID;
+    }
+    std::vector<size_t> at;
+    if (int rc = check_pixel_args(p, n_frames, counts, lens, (double)height, at)) return rc;
+    const size_t total = at[n_frames];
+    if (int rc = check_device_pointer(p, images, "images")) return rc;
+    if (total)
+        if (int rc = check_device_pointer(p, points, "points")) return rc;
+    for (void* out : {(void*)tracked_out, (void*)status_out})
+        if (out && total)
+            if (int rc = check_device_pointer(p, out, "an output buffer")) return rc;
+    if (int rc = check_frame_ts(p, n_frames, image_ts, image_ts + 1)) return rc;
+
+    const size_t per_image = rs::track_pyramid_floats(width, height, tp.levels);
+    const size_t n_images = n_frames + 1;
+    const size_t slots = per_image ? std::min(n_images, std::max<size_t>(2, kTrackScratchBytes / (4 * per_image)))
+                                   : n_images;
+    CUDA_TRY(p, cudaSetDevice(p->device));
+    CUDA_TRY(p, p->d_trk_pyr.reserve(std::max<size_t>(1, slots * per_image)));
+    CUDA_TRY(p, p->d_trk_pts.reserve(6 * total + 1));  // compacted a, b (4 per point), tracked (2 per point)
+    CUDA_TRY(p, p->d_trk_at.reserve(n_frames + 1));
+    CUDA_TRY(p, p->d_trk_status.reserve(total + 1));
+    CUDA_TRY(p, p->d_trk_flag.reserve(1));
+    CUDA_TRY(p, p->h_trk_flag.reserve(1));
+    double* d_a = p->d_trk_pts.ptr;
+    double* d_b = d_a + 2 * total;
+    double* d_tracked = tracked_out ? tracked_out : d_b + 2 * total;
+    uint8_t* d_status = status_out ? status_out : p->d_trk_status.ptr;
+    int64_t* d_kept_at = p->d_trk_at.ptr;
+    std::vector<int64_t> q_at(at.begin(), at.end());
+    const rs::TrackImages im{images, (int64_t)pitch, width, height, tp.levels, tp.window, tp.max_iters,
+                             (float)tp.epsilon, (float)tp.min_eig};
+    DevicePointSource src;
+    // s.d_at holds the query offsets (begin_device_staging); s.h_at receives the kept ones
+    src.queue = [&](const DeviceStaging& s) -> const int64_t* {
+        const cudaError_t e = cudaMemsetAsync(p->d_trk_flag.ptr, 0, sizeof(unsigned), p->stream);
+        if (e != cudaSuccess) {
+            p->err = std::string("CUDA error: ") + cudaGetErrorString(e);
+            return nullptr;
+        }
+        rs::launch_track_frames(im, (int)n_frames, q_at.data(), s.d_at, points, p->d_trk_pyr.ptr, (int)slots,
+                                d_tracked, d_status, p->d_trk_flag.ptr, p->stream);
+        rs::launch_track_compact(s.d_at, (int)n_frames, points, d_tracked, d_status, d_a, d_b, d_kept_at, p->stream);
+        if (d2h(p, s.h_at, d_kept_at, (n_frames + 1) * sizeof(int64_t)) ||
+            d2h(p, p->h_trk_flag.ptr, p->d_trk_flag.ptr, sizeof(unsigned)))
+            return nullptr;
+        return d_kept_at;
+    };
+    src.verdict = [&](const DeviceStaging& s, std::vector<size_t>& kept) {
+        if (*p->h_trk_flag.ptr) {
+            p->err = kMsgNonFinite[kRaysA];
+            return (int)RSSYNC_E_NONFINITE;
+        }
+        for (size_t i = 0; i <= n_frames; ++i) kept[i] = (size_t)s.h_at[i];
+        return (int)RSSYNC_OK;
+    };
+    return ingest_pixels_device(p, n_frames, frames, at, image_ts, image_ts + 1, d_a, d_b, lens, (double)height,
+                                stream, &src);
 }
 
 }  // extern "C"

@@ -1868,6 +1868,230 @@ __global__ void __launch_bounds__(kStageThreads) stage_tracks_kernel(StageArgs a
 }
 
 // ------------------------------------------------------------------------------------------
+// Sparse pyramidal Lucas-Kanade (rssync_track_frames_device; the arithmetic contract is stated in
+// include/rssync_b200.h).  The build uses -fmad=false, so every float32 expression below is evaluated
+// in the order written.
+struct TrackPyr {
+    TrackImages im;
+    float* lvl[kTrackMaxLevels];  // levels 1..: row y of slot s at lvl[l] + (s * h[l] + y) * w[l]
+    int w[kTrackMaxLevels], h[kTrackMaxLevels];
+    int slots;
+};
+
+__device__ __forceinline__ int reflect101(int i, int n) {
+    i = i < 0 ? -i : i;
+    i = i >= n ? 2 * (n - 1) - i : i;
+    return min(max(i, 0), n - 1);  // (only tile cells no output reads fall outside after the reflection)
+}
+
+// level l of image j (slot j % slots above level 0) at integer (x, y), clamped to the level's edge
+__device__ __forceinline__ float track_px(const TrackPyr& P, int l, int j, int x, int y) {
+    x = min(max(x, 0), P.w[l] - 1);
+    y = min(max(y, 0), P.h[l] - 1);
+    if (l == 0) return (float)__ldg(P.im.img0 + ((int64_t)j * P.im.h0 + y) * P.im.pitch0 + x);
+    return __ldg(P.lvl[l] + ((int64_t)(j % P.slots) * P.h[l] + y) * P.w[l] + x);
+}
+
+__device__ __forceinline__ float track_bilinear(const TrackPyr& P, int l, int j, int x, int y, float ax, float ay) {
+    const float i00 = track_px(P, l, j, x, y), i01 = track_px(P, l, j, x + 1, y);
+    const float i10 = track_px(P, l, j, x, y + 1), i11 = track_px(P, l, j, x + 1, y + 1);
+    return (1.f - ay) * ((1.f - ax) * i00 + ax * i01) + ay * ((1.f - ax) * i10 + ax * i11);
+}
+
+// One launch per level: level l -> l + 1 of images [j0, j0 + gridDim.z).  A block's 32 x 8 outputs read a
+// (2*8 + 3) x (2*32 + 3) tile of level l (BORDER_REFLECT_101), blur its rows into shared memory, then
+// its columns: h = (s[-2] + s[2]) + 4 (s[-1] + s[1]) + 6 s[0] per row, the same over h per column, times
+// 1/256.
+constexpr int kPyrTX = 32, kPyrTY = 8;
+__global__ void __launch_bounds__(kPyrTX * kPyrTY) track_pyramid_kernel(TrackPyr P, int l, int j0) {
+    constexpr int TH = 2 * kPyrTY + 3, TW = 2 * kPyrTX + 3;
+    __shared__ float s_in[TH][TW];
+    __shared__ float s_h[TH][kPyrTX];
+    const int j = j0 + blockIdx.z;
+    const int w = P.w[l], h = P.h[l];
+    const int X0 = blockIdx.x * kPyrTX, Y0 = blockIdx.y * kPyrTY;
+    for (int k = threadIdx.x; k < TH * TW; k += kPyrTX * kPyrTY) {
+        const int r = k / TW, c = k % TW;
+        s_in[r][c] = track_px(P, l, j, reflect101(2 * X0 - 2 + c, w), reflect101(2 * Y0 - 2 + r, h));
+    }
+    __syncthreads();
+    for (int k = threadIdx.x; k < TH * kPyrTX; k += kPyrTX * kPyrTY) {
+        const int r = k / kPyrTX, c = k % kPyrTX;
+        const float* s = &s_in[r][2 * c];
+        s_h[r][c] = ((s[0] + s[4]) + 4.f * (s[1] + s[3])) + 6.f * s[2];
+    }
+    __syncthreads();
+    const int tx = threadIdx.x % kPyrTX, ty = threadIdx.x / kPyrTX;
+    const int X = X0 + tx, Y = Y0 + ty;
+    if (X < P.w[l + 1] && Y < P.h[l + 1]) {
+        const int r = 2 * ty;
+        const float v = ((s_h[r][tx] + s_h[r + 4][tx]) + 4.f * (s_h[r + 1][tx] + s_h[r + 3][tx])) + 6.f * s_h[r + 2][tx];
+        P.lvl[l + 1][((int64_t)(j % P.slots) * P.h[l + 1] + Y) * P.w[l + 1] + X] = v * (1.f / 256.f);
+    }
+}
+
+// sum over the 32 lanes: xor butterfly 16, 8, 4, 2, 1 (every lane ends with the same bits)
+__device__ __forceinline__ float track_warp_sum(float v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(FULL, v, o);
+    return v;
+}
+
+// One warp per query point, all levels.  Per warp in shared memory: the side-a patch, (window + 2)^2
+// bilinear samples, and its Scharr gradients over the window.
+constexpr int kLkWarps = 4;
+__global__ void __launch_bounds__(kLkWarps * 32) track_lk_kernel(TrackPyr P, const int64_t* __restrict__ q_at,
+                                                                int f0, int f1, const double* __restrict__ pts,
+                                                                double* __restrict__ tracked,
+                                                                uint8_t* __restrict__ status, unsigned* flag) {
+    extern __shared__ float s_lk[];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int win = P.im.window, r = win / 2, pw = win + 2, nw = win * win;
+    float* sA = s_lk + (size_t)warp * (pw * pw + 2 * nw);
+    float* sIx = sA + pw * pw;
+    float* sIy = sIx + nw;
+    const int64_t k = q_at[f0] + (int64_t)blockIdx.x * kLkWarps + warp;
+    if (k >= q_at[f1]) return;
+    int lo = f0, hi = f1 - 1;  // the frame holding point k: the last f with q_at[f] <= k
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (q_at[mid] <= k) lo = mid; else hi = mid - 1;
+    }
+    const int ja = lo, jb = lo + 1;
+    const double qx = pts[2 * k], qy = pts[2 * k + 1];
+    const bool finite = isfinite(qx) && isfinite(qy);
+    if (!finite && lane == 0) atomicOr(flag, 1u);
+    bool ok = finite && qx >= 0.0 && qx <= P.w[0] - 1 && qy >= 0.0 && qy <= P.h[0] - 1;
+    const float px0 = (float)qx, py0 = (float)qy;
+    const float eps2 = P.im.epsilon * P.im.epsilon, area = (float)nw;
+    float gx = 0.f, gy = 0.f, vx = 0.f, vy = 0.f;
+    for (int l = P.im.levels - 1; ok && l >= 0; --l) {
+        const float s = ldexpf(1.f, -l);
+        const float ax = px0 * s, ay = py0 * s;
+        const float fx = floorf(ax), fy = floorf(ay);
+        const float wx = ax - fx, wy = ay - fy;
+        const int ix = (int)fx, iy = (int)fy;
+        __syncwarp();  // the previous level's readers of sA are done
+        for (int t = lane; t < pw * pw; t += 32)
+            sA[t] = track_bilinear(P, l, ja, ix + t % pw - r - 1, iy + t / pw - r - 1, wx, wy);
+        __syncwarp();
+        float gxx = 0.f, gxy = 0.f, gyy = 0.f;
+        for (int t = lane; t < nw; t += 32) {
+            const float* c = sA + (t / win + 1) * pw + (t % win + 1);
+            const float dx = ((3.f * (c[-pw + 1] - c[-pw - 1]) + 10.f * (c[1] - c[-1])) + 3.f * (c[pw + 1] - c[pw - 1])) *
+                             (1.f / 32.f);
+            const float dy = ((3.f * (c[pw - 1] - c[-pw - 1]) + 10.f * (c[pw] - c[-pw])) + 3.f * (c[pw + 1] - c[-pw + 1])) *
+                             (1.f / 32.f);
+            sIx[t] = dx;
+            sIy[t] = dy;
+            gxx += dx * dx;
+            gxy += dx * dy;
+            gyy += dy * dy;
+        }
+        gxx = track_warp_sum(gxx);
+        gxy = track_warp_sum(gxy);
+        gyy = track_warp_sum(gyy);
+        const float d = gxx - gyy;
+        const float min_eig = ((gxx + gyy) - sqrtf(d * d + 4.f * (gxy * gxy))) / (2.f * area);
+        if (!(min_eig >= P.im.min_eig)) { ok = false; break; }
+        const float det = gxx * gyy - gxy * gxy;
+        __syncwarp();
+        // side b positions far outside the level read its edge pixels only: clamp them there first so the
+        // integer conversion stays in range
+        const float lim_lo = -2.f * pw, lim_x = (float)(P.w[l] + 2 * pw), lim_y = (float)(P.h[l] + 2 * pw);
+        for (int it = 0; it < P.im.max_iters; ++it) {
+            const float bxp = ax + gx + vx, byp = ay + gy + vy;
+            const float bfx = floorf(bxp), bfy = floorf(byp);
+            const float bwx = bxp - bfx, bwy = byp - bfy;
+            const int bix = (int)fminf(fmaxf(bfx, lim_lo), lim_x), biy = (int)fminf(fmaxf(bfy, lim_lo), lim_y);
+            float bx = 0.f, by = 0.f;
+            for (int t = lane; t < nw; t += 32) {
+                const int tx = t % win, ty = t / win;
+                const float B = track_bilinear(P, l, jb, bix + tx - r, biy + ty - r, bwx, bwy);
+                const float diff = sA[(ty + 1) * pw + tx + 1] - B;
+                bx += diff * sIx[t];
+                by += diff * sIy[t];
+            }
+            bx = track_warp_sum(bx);
+            by = track_warp_sum(by);
+            const float ex = (gyy * bx - gxy * by) / det, ey = (gxx * by - gxy * bx) / det;
+            if (!isfinite(ex) || !isfinite(ey)) { ok = false; break; }
+            vx += ex;
+            vy += ey;
+            if (ex * ex + ey * ey < eps2) break;
+        }
+        if (!ok) break;
+        if (l > 0) {
+            gx = 2.f * (gx + vx);
+            gy = 2.f * (gy + vy);
+            vx = vy = 0.f;
+        }
+    }
+    if (lane == 0) {
+        double tx = __longlong_as_double(0x7ff8000000000000LL), ty = tx;  // NaN: lost before the last level ended
+        if (ok) {
+            tx = qx + (double)(gx + vx);
+            ty = qy + (double)(gy + vy);
+            ok = tx >= 0.0 && tx <= P.w[0] - 1 && ty >= 0.0 && ty <= P.h[0] - 1;
+        }
+        tracked[2 * k] = tx;
+        tracked[2 * k + 1] = ty;
+        status[k] = ok ? 1 : 0;
+    }
+}
+
+// One block: kept count per frame (warp per frame), prefix sum (warp 0), then every warp writes its
+// frames' kept pairs in query order.
+constexpr int kCompactThreads = 1024;
+__global__ void __launch_bounds__(kCompactThreads) track_compact_kernel(const int64_t* __restrict__ q_at, int n,
+                                                                       const double* __restrict__ pts,
+                                                                       const double* __restrict__ tracked,
+                                                                       const uint8_t* __restrict__ status,
+                                                                       double* __restrict__ out_a,
+                                                                       double* __restrict__ out_b, int64_t* kept_at) {
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    constexpr int W = kCompactThreads / 32;
+    for (int f = warp; f < n; f += W) {
+        int64_t c = 0;
+        for (int64_t k = q_at[f] + lane; k - lane < q_at[f + 1]; k += 32)
+            c += __popc(__ballot_sync(FULL, k < q_at[f + 1] && status[k] != 0));
+        if (lane == 0) kept_at[f + 1] = c;
+    }
+    __syncthreads();
+    if (warp == 0) {
+        int64_t carry = 0;
+        if (lane == 0) kept_at[0] = 0;
+        for (int base = 0; base < n; base += 32) {
+            int64_t v = base + lane < n ? kept_at[base + lane + 1] : 0;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const int64_t u = __shfl_up_sync(FULL, v, o);
+                if (lane >= o) v += u;
+            }
+            v += carry;
+            if (base + lane < n) kept_at[base + lane + 1] = v;
+            carry = __shfl_sync(FULL, v, 31);
+        }
+    }
+    __syncthreads();
+    for (int f = warp; f < n; f += W) {
+        int64_t o = kept_at[f];
+        for (int64_t k = q_at[f] + lane; k - lane < q_at[f + 1]; k += 32) {
+            const bool keep = k < q_at[f + 1] && status[k] != 0;
+            const unsigned m = __ballot_sync(FULL, keep);
+            if (keep) {
+                const int64_t d = o + __popc(m & ((1u << lane) - 1u));
+                out_a[2 * d] = pts[2 * k];
+                out_a[2 * d + 1] = pts[2 * k + 1];
+                out_b[2 * d] = tracked[2 * k];
+                out_b[2 * d + 1] = tracked[2 * k + 1];
+            }
+            o += __popc(m);
+        }
+    }
+}
+
+// ------------------------------------------------------------------------------------------
 // K7:the parallel half of ndspline::make (ndspline.cpp:13-19 / minispline.cpp:34-44).  The host
 // eliminates the tridiagonal system (two sequential sweeps, host_ingest.cpp) and sends what is left
 // of it -- rhs and diag, 5 doubles per sample instead of the 16 of a finished record -- with the
@@ -2472,6 +2696,71 @@ void launch_stage_points(const int64_t* d_at, const double* d_frame_ts, int n_fr
     StageArgs a{d_at, total, {points_a, points_b, nullptr, nullptr}, {d_stage, d_stage + 2 * total, nullptr, nullptr},
                 d_frame_ts, lens.ro, rows, d_info, lens.fx, lens.fy, lens.cx, lens.cy};
     stage_tracks_kernel<StageMode::kPoints><<<n_frames, kStageThreads, 0, st>>>(a);
+    g_launches += 1;
+}
+
+namespace {
+TrackPyr track_pyr(const TrackImages& im, float* d_pyr, int slots) {
+    TrackPyr P{};
+    P.im = im;
+    P.slots = slots;
+    P.w[0] = im.w0;
+    P.h[0] = im.h0;
+    size_t at = 0;
+    for (int l = 1; l < im.levels; ++l) {
+        P.w[l] = (P.w[l - 1] + 1) / 2;
+        P.h[l] = (P.h[l - 1] + 1) / 2;
+        P.lvl[l] = d_pyr + at;
+        at += (size_t)slots * P.w[l] * P.h[l];
+    }
+    return P;
+}
+}  // namespace
+
+size_t track_pyramid_floats(int w0, int h0, int levels) {
+    size_t n = 0;
+    for (int l = 1, w = w0, h = h0; l < levels; ++l) {
+        w = (w + 1) / 2;
+        h = (h + 1) / 2;
+        n += (size_t)w * h;
+    }
+    return n;
+}
+
+void launch_track_frames(const TrackImages& im, int n_frames, const int64_t* h_q_at, const int64_t* d_q_at,
+                         const double* d_points, float* d_pyr, int slots, double* d_tracked, uint8_t* d_status,
+                         unsigned* d_flag, cudaStream_t st) {
+    if (n_frames <= 0) return;
+    const TrackPyr P = track_pyr(im, d_pyr, slots);
+    const int pw = im.window + 2;
+    const size_t smem = (size_t)kLkWarps * (pw * pw + 2 * im.window * im.window) * sizeof(float);
+    allow_smem(track_lk_kernel, smem);
+    // chunk: build the pyramids of images [built, e), then track frames [f0, e - 1); image f0 is the
+    // last one of the previous chunk, still in its slot
+    for (int f0 = 0, built = 0; f0 < n_frames;) {
+        const int e = std::min(n_frames + 1, f0 + slots);
+        for (int l = 0; l + 1 < im.levels && e > built; ++l) {
+            const dim3 grid((P.w[l + 1] + kPyrTX - 1) / kPyrTX, (P.h[l + 1] + kPyrTY - 1) / kPyrTY, e - built);
+            track_pyramid_kernel<<<grid, kPyrTX * kPyrTY, 0, st>>>(P, l, built);
+            g_launches += 1;
+        }
+        const int64_t pts = h_q_at[e - 1] - h_q_at[f0];
+        if (pts > 0) {
+            track_lk_kernel<<<(unsigned)((pts + kLkWarps - 1) / kLkWarps), kLkWarps * 32, smem, st>>>(
+                P, d_q_at, f0, e - 1, d_points, d_tracked, d_status, d_flag);
+            g_launches += 1;
+        }
+        built = e;
+        f0 = e - 1;
+    }
+}
+
+void launch_track_compact(const int64_t* d_q_at, int n_frames, const double* d_points, const double* d_tracked,
+                          const uint8_t* d_status, double* d_out_a, double* d_out_b, int64_t* d_kept_at,
+                          cudaStream_t st) {
+    if (n_frames <= 0) return;
+    track_compact_kernel<<<1, kCompactThreads, 0, st>>>(d_q_at, n_frames, d_points, d_tracked, d_status, d_out_a,
+                                                        d_out_b, d_kept_at);
     g_launches += 1;
 }
 

@@ -205,6 +205,32 @@ void launch_stage_row_fractions(const int64_t* d_at, const double* d_frame_ts, i
                                 const double* frac_b, double readout, double* d_stage, StageInfo* d_info,
                                 cudaStream_t st);
 
+// ---- sparse pyramidal Lucas-Kanade between decoded frames (rssync_track_frames_device) -----------
+// The arithmetic is the contract stated at rssync_track_frames_device in include/rssync_b200.h.
+constexpr int kTrackMaxLevels = 6;
+struct TrackImages {
+    const uint8_t* img0;  // n_frames + 1 luma planes: row y of image j at img0 + (j * h0 + y) * pitch0
+    int64_t pitch0;
+    int w0, h0;
+    int levels, window, max_iters;
+    float epsilon, min_eig;
+};
+// floats of one image's pyramid levels 1 .. levels - 1
+size_t track_pyramid_floats(int w0, int h0, int levels);
+// Tracks every query point of frame i (d_points[2 d_q_at[i] ..], host copy h_q_at) from image i to
+// image i + 1, for i in [0, n_frames).  The pyramids of `slots` (>= 2) images live in d_pyr at once
+// (slots * track_pyramid_floats floats): the images are processed in chunks, image j in slot j % slots,
+// each pyramid built once.  Per point: d_tracked (2 doubles) and d_status (1 = kept); *d_flag gets bit 0
+// when a query point is not finite.
+void launch_track_frames(const TrackImages& im, int n_frames, const int64_t* h_q_at, const int64_t* d_q_at,
+                         const double* d_points, float* d_pyr, int slots, double* d_tracked, uint8_t* d_status,
+                         unsigned* d_flag, cudaStream_t st);
+// The kept pairs, frame by frame in the query order: d_out_a / d_out_b at the kept offsets d_kept_at
+// (n_frames + 1, written here), the layout launch_stage_points reads.
+void launch_track_compact(const int64_t* d_q_at, int n_frames, const double* d_points, const double* d_tracked,
+                          const uint8_t* d_status, double* d_out_a, double* d_out_b, int64_t* d_kept_at,
+                          cudaStream_t st);
+
 // ---- stage probes (tests only) ---------------------------------------------------------------
 void launch_probe_problem_matrix(const DeviceData& dd, FrameDesc fd, double delay, double* d_P,
                                  cudaStream_t st);

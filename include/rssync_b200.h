@@ -178,6 +178,56 @@ int rssync_track_frames_device(rssync_problem* p, size_t n_frames, const int64_t
                                const double* image_ts, const double* points, const uint8_t* images, size_t pitch,
                                int width, int height, const rssync_lens* lens, const rssync_track_params* params,
                                double* tracked_out, uint8_t* status_out, void* stream);
+/* Options of rssync_track_frames_ex_device (NULL there = the defaults shown). */
+typedef struct rssync_track_options {
+    int cell;          /* selection cell side in px, 16..128 (default 128) */
+    int block;         /* structure-tensor window side, 3, 5 or 7 (default 5) */
+    double quality;    /* keep a cell's pick only if score >= quality * image max, (0, 1] (default 0.01) */
+    int max_points;    /* per frame when selecting, 1..512 (default 512) */
+    double fb_max;     /* forward-backward threshold in px, >= 0; 0 = no backward pass (default 1.0) */
+} rssync_track_options;
+/* rssync_track_frames_device with two more steps: the query points may be chosen on the device, and
+ * every point kept forward may be tracked back and rejected when it does not return.
+ * points and counts both non-NULL: the caller's query points, as in rssync_track_frames_device.  Both
+ * NULL: the points of frame i are selected on image i (below).  Only one NULL: RSSYNC_E_INVALID.
+ * Outputs, each may be NULL, hold sum(counts) points, frames concatenated (in selection mode size the
+ * device buffers for n_frames * max_points): points_out (device, 2 doubles per point: the query points),
+ * counts_out (host, n_frames), tracked_out (device, 2 doubles), status_out (device, 1 byte) and fb_out
+ * (device, 1 double).  counts_out comes back in the ingest's one round trip.
+ * Status: 0 lost (as in rssync_track_frames_device), 1 kept and ingested, 2 tracked forward but rejected
+ * by the backward check (tracked_out holds the forward position).  fb_out: the forward-backward distance
+ * of each point the backward pass kept, NaN for every other point.
+ * The kept points (status 1) give exactly what rssync_set_track_pixels_device gives on them, as stated at
+ * rssync_track_frames_device; a frame whose points are all lost or rejected is ingested with 0 rays.
+ * With the caller's points and fb_max = 0 the call equals rssync_track_frames_device.
+ * Selection (float32, evaluated in the order written, no contraction; I = (float)plane[y][x]; reads
+ * outside the image use BORDER_REFLECT_101, though no candidate's score or its neighbours' reach one):
+ *  - Gradients (3 x 3 Sobel): dx = (((I[y-1][x+1] - I[y-1][x-1]) + 2 (I[y][x+1] - I[y][x-1])) +
+ *    (I[y+1][x+1] - I[y+1][x-1])) * s, dy the same with rows and columns swapped,
+ *    s = (float)(1.0 / (4 block 255)).
+ *  - Sxx, Sxy, Syy: block x block sums of dx dx, dx dy, dy dy, each row summed left to right first, then
+ *    the row sums top to bottom.  Score: (a + c) - sqrt((a - c)^2 + b^2), a = 0.5 Sxx, c = 0.5 Syy,
+ *    b = Sxy (cv2.cornerMinEigenVal(img, block, 3)).
+ *  - Candidate: x in [m, w - 1 - m], y in [m, h - 1 - m] with m = block / 2 + 2, score > 0, and score >=
+ *    each of its 8 neighbours' scores.
+ *  - Cells: cell x cell squares from (0, 0), the last row and column may be partial.  A cell's pick is
+ *    its candidate of greatest score, a tie going to the smallest y w + x.  This cell rule stands in for
+ *    cv2.goodFeaturesToTrack's greedy minDistance, which is sequential.
+ *  - Threshold: M is the greatest pick score of the image; a pick is kept iff score >= (float)quality M.
+ *    When more than max_points picks are kept, those with the greatest score stay, a tie going to the
+ *    smaller cell index (row-major).
+ *  - The points: the kept picks in ascending row-major cell order, ((double)x, (double)y).
+ * Forward-backward (fb_max > 0): for a point q kept forward at t, the tracker above runs from image i + 1
+ * to image i with query t, giving u (or losing the point); fb = sqrt((u.x - q.x)^2 + (u.y - q.y)^2) in
+ * double; status 2 when u is lost or !(fb <= fb_max), else 1.  fb_max = 0 skips the backward pass.
+ * Checked before anything is applied, besides the checks of rssync_track_frames_device: RSSYNC_E_INVALID
+ * for an option out of range, in selection mode width or height below 2 (block / 2 + 2) + 1 or more than
+ * 65536 cells per image, and outputs that are neither NULL nor device memory of the problem's device. */
+int rssync_track_frames_ex_device(rssync_problem* p, size_t n_frames, const int64_t* frames, const size_t* counts,
+                                  const double* image_ts, const double* points, const uint8_t* images, size_t pitch,
+                                  int width, int height, const rssync_lens* lens, const rssync_track_params* params,
+                                  const rssync_track_options* options, double* points_out, size_t* counts_out,
+                                  double* tracked_out, uint8_t* status_out, double* fb_out, void* stream);
 /* SetTrackResult for n_frames frames whose rays the caller computed (any camera model), with the
  * rolling-shutter timestamps formed here from per-ray row fractions.  Ray k of frame i gets
  * ts_a = frame_ts_a[i] + readout * frac_a[k] (ts_b alike): one multiply and one add, not contracted,

@@ -10,6 +10,7 @@ The directory name contains a hyphen, so import it with
 """
 from __future__ import annotations
 
+import collections
 import ctypes as C
 import os
 
@@ -45,6 +46,7 @@ C_ABI_SYMBOLS = [
     "rssync_set_track_row_fractions", "rssync_set_track_row_fractions_device",
     "rssync_retime_table", "rssync_row_fraction_plane", "rssync_adopt_row_fractions",
     "rssync_readout_search_windows", "rssync_rotation_search_windows", "rssync_track_frames_device",
+    "rssync_track_frames_ex_device",
 ]
 # Itanium-ABI symbols of the C++ drop-in face (same set the reference's librssync_core exports)
 CXX_ABI_SYMBOLS = [
@@ -95,6 +97,18 @@ class TrackParams(C.Structure):
 
     def __init__(self, levels=3, window=21, max_iters=30, epsilon=0.01, min_eig=1e-4):
         super().__init__(levels, window, max_iters, epsilon, min_eig)
+
+
+class TrackOptions(C.Structure):
+    """rssync_track_options: point selection and the forward-backward check (track_frames_ex)"""
+    _fields_ = [("cell", C.c_int), ("block", C.c_int), ("quality", C.c_double), ("max_points", C.c_int),
+                ("fb_max", C.c_double)]
+
+    def __init__(self, cell=128, block=5, quality=0.01, max_points=512, fb_max=1.0):
+        super().__init__(cell, block, quality, max_points, fb_max)
+
+
+TrackResult = collections.namedtuple("TrackResult", "points counts tracked status fb_error")
 
 
 def grid_points(width, height, step):
@@ -173,6 +187,10 @@ def load_library():
     L.rssync_track_frames_device.argtypes = [P, C.c_size_t, c_i64_p, C.POINTER(C.c_size_t), c_double_p, P, P,
                                              C.c_size_t, C.c_int, C.c_int, C.POINTER(Lens), C.POINTER(TrackParams),
                                              P, P, P]
+    L.rssync_track_frames_ex_device.argtypes = [P, C.c_size_t, c_i64_p, C.POINTER(C.c_size_t), c_double_p, P, P,
+                                                C.c_size_t, C.c_int, C.c_int, C.POINTER(Lens),
+                                                C.POINTER(TrackParams), C.POINTER(TrackOptions), P,
+                                                C.POINTER(C.c_size_t), P, P, P, P]
     L.rssync_presync.argtypes = [P, C.c_double, C.c_int64, C.c_int64, C.c_double, C.c_double, c_double_p, c_double_p]
     L.rssync_sync.argtypes = [P, C.c_double, C.c_int64, C.c_int64, C.c_double, C.c_double, c_double_p, c_double_p]
     L.rssync_debug_presync.argtypes = [P, C.c_double, C.c_int64, C.c_int64, C.c_double, c_double_p, c_double_p, C.c_int]
@@ -616,6 +634,61 @@ class SyncProblem:
             C.c_void_p(images.data_ptr()), images.stride(1), images.shape[2], images.shape[1], C.byref(lens_c), prm,
             C.c_void_p(tracked.data_ptr() if n else None), C.c_void_p(status.data_ptr() if n else None), stream))
         return tracked, status
+
+    def track_frames_ex(self, frames, image_ts, images, lens, params=None, options=None, points=None, counts=None):
+        """track_frames with the query points selected on the device (points and counts None) and the
+        forward-backward check (rssync_track_frames_ex_device).  images, frames, image_ts, lens and params as in
+        track_frames; options: TrackOptions or None (the defaults: 128-px cells, block 5, quality 0.01, 512
+        points per frame, fb_max 1 px).  Returns TrackResult(points, counts, tracked, status, fb_error): the
+        query points, tracked positions (CUDA float64 (n, 2)), statuses (CUDA uint8 (n,): 0 lost, 1 kept and
+        ingested, 2 rejected by the backward check) and forward-backward distances (CUDA float64 (n,), NaN
+        where the backward pass did not keep the point or did not run), n = sum(counts); counts: numpy."""
+        import torch
+        fr = np.ascontiguousarray(frames, dtype=np.int64)
+        ts = _f64(image_ts)
+        if (points is None) != (counts is None):
+            raise ValueError("track_frames_ex: give both points and counts, or neither (selection)")
+        if not getattr(images, "is_cuda", False):
+            raise TypeError("track_frames_ex: images must be a CUDA tensor")
+        if images.dtype != torch.uint8 or images.dim() != 3 or images.stride(2) != 1:
+            raise ValueError("track_frames_ex: images must be a uint8 tensor (n_frames + 1, H, W) with contiguous rows")
+        if images.shape[0] != fr.shape[0] + 1 or ts.shape[0] != fr.shape[0] + 1:
+            raise ValueError(f"track_frames_ex: {fr.shape[0]} frames need {fr.shape[0] + 1} images and image "
+                             f"timestamps, got {images.shape[0]} and {ts.shape[0]}")
+        if images.shape[0] > 1 and images.stride(0) != images.shape[1] * images.stride(1):
+            raise ValueError("track_frames_ex: the planes must lie back to back (stride(0) = H * stride(1))")
+        dev = images.device
+        opt = TrackOptions() if options is None else options
+        if points is None:
+            cn, pp, cap = None, None, fr.shape[0] * max(int(opt.max_points), 0)
+            stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        else:
+            cn = np.ascontiguousarray(counts, dtype=np.uint64)
+            cap = int(cn.sum())
+            if not getattr(points, "is_cuda", False):
+                raise TypeError("track_frames_ex: points must be a CUDA tensor")
+            if points.device != dev:
+                raise ValueError(f"track_frames_ex: images on {dev}, points on {points.device}")
+            (pp,), stream = _device_ptrs((points,), (2 * cap,))
+        pts_out = torch.empty((cap, 2), dtype=torch.float64, device=dev)
+        tracked = torch.empty((cap, 2), dtype=torch.float64, device=dev)
+        status = torch.empty((cap,), dtype=torch.uint8, device=dev)
+        fb = torch.empty((cap,), dtype=torch.float64, device=dev)
+        counts_out = np.zeros(fr.shape[0], dtype=np.uint64)
+        lens_c = lens if isinstance(lens, Lens) else Lens(*[float(x) for x in lens])
+        prm = None if params is None else C.byref(params)
+
+        def ptr(t):
+            return C.c_void_p(t.data_ptr() if cap else None)
+
+        self._check(self.L.rssync_track_frames_ex_device(
+            self.h, fr.shape[0], fr.ctypes.data_as(c_i64_p),
+            None if cn is None else cn.ctypes.data_as(C.POINTER(C.c_size_t)), _dp(ts), pp,
+            C.c_void_p(images.data_ptr()), images.stride(1), images.shape[2], images.shape[1], C.byref(lens_c), prm,
+            C.byref(opt), ptr(pts_out), counts_out.ctypes.data_as(C.POINTER(C.c_size_t)), ptr(tracked), ptr(status),
+            ptr(fb), stream))
+        n = int(counts_out.sum())
+        return TrackResult(pts_out[:n], counts_out.astype(np.int64), tracked[:n], status[:n], fb[:n])
 
     def load(self, w, bulk=False):
         """Feed a synth.Workload the way core_testcode feeds a video (core_testcode.cpp:257-268)."""

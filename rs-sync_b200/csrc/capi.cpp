@@ -338,6 +338,12 @@ struct rssync_problem {
     DevBuf<uint8_t> d_trk_status;
     DevBuf<unsigned> d_trk_flag;
     PinBuf<unsigned> h_trk_flag;
+    // rssync_track_frames_ex_device's selection: cell keys, picks and pick counts of a chunk; the
+    // selected offsets read back
+    DevBuf<unsigned long long> d_trk_keys;
+    DevBuf<uint32_t> d_trk_picks;
+    DevBuf<int32_t> d_trk_count;
+    PinBuf<int64_t> h_trk_qat;
 
     std::vector<std::pair<double, int32_t>> sort_scratch;
     std::vector<double> trace_delay, trace_step;
@@ -1582,6 +1588,7 @@ void rssync_destroy(rssync_problem* p) {
     p->d_rowq.release(); p->d_rt_rays.release(); p->d_rt_ext.release(); p->d_rt_orig.release(); p->d_rt_pos.release();
     p->d_trk_pyr.release(); p->d_trk_pts.release(); p->d_trk_at.release(); p->d_trk_status.release();
     p->d_trk_flag.release(); p->h_trk_flag.release();
+    p->d_trk_keys.release(); p->d_trk_picks.release(); p->d_trk_count.release(); p->h_trk_qat.release();
     if (p->owns_stream && p->stream) { cudaStreamSynchronize(p->stream); cudaStreamDestroy(p->stream); }
     for (SyncLane& L : p->lanes) L.release();
     if (p->ev_sync_ready) cudaEventDestroy(p->ev_sync_ready);
@@ -2635,6 +2642,145 @@ int check_device_pointer(rssync_problem* p, const void* b, const char* what) {
 // the tracker's scratch budget: the pyramids of as many images as fit are alive at once
 constexpr size_t kTrackScratchBytes = size_t(256) << 20;
 
+// the outputs of rssync_track_frames_ex_device (each may be null)
+struct TrackOutputs {
+    double* points;
+    size_t* counts;
+    double* tracked;
+    uint8_t* status;
+    double* fb;
+};
+
+// The body of both tracking entry points once their null checks have passed.  opt null: the plain form
+// (caller's points, no backward pass, no options checked).
+int track_frames(rssync_problem* p, size_t n_frames, const int64_t* frames, const size_t* counts,
+                 const double* image_ts, const double* points, const uint8_t* images, size_t pitch, int width,
+                 int height, const rssync_lens* lens, const rssync_track_params* params,
+                 const rssync_track_options* opt, const TrackOutputs& out, void* stream) {
+    const rssync_track_params tp = params ? *params : rssync_track_params{3, 21, 30, 0.01, 1e-4};
+    if (tp.levels < 1 || tp.levels > 6 || tp.window < 5 || tp.window > 63 || tp.window % 2 == 0 || tp.max_iters < 1 ||
+        tp.max_iters > 100 || !(tp.epsilon >= 0.0) || !std::isfinite(tp.epsilon) || !(tp.min_eig >= 0.0) ||
+        !std::isfinite(tp.min_eig)) {
+        p->err = "track-frames: parameters out of range";
+        return RSSYNC_E_INVALID;
+    }
+    const bool select = opt && !points;
+    if (opt && (opt->cell < 16 || opt->cell > 128 || (opt->block != 3 && opt->block != 5 && opt->block != 7) ||
+                !(opt->quality > 0.0 && opt->quality <= 1.0) || opt->max_points < 1 ||
+                opt->max_points > rs::kMaxRaysPerFrame || !(opt->fb_max >= 0.0))) {
+        p->err = "track-frames: options out of range";
+        return RSSYNC_E_INVALID;
+    }
+    const int64_t min_side = (int64_t)tp.window << (tp.levels - 1);
+    if (width < min_side || height < min_side || pitch < (size_t)width) {
+        p->err = "track-frames: image smaller than window * 2^(levels - 1), or pitch below width";
+        return RSSYNC_E_INVALID;
+    }
+    rs::TrackSelect sel{};
+    if (select) {
+        sel.cell = opt->cell;
+        sel.block = opt->block;
+        sel.max_points = opt->max_points;
+        sel.quality = (float)opt->quality;
+        sel.cells_x = (width + opt->cell - 1) / opt->cell;
+        sel.cells_y = (height + opt->cell - 1) / opt->cell;
+        const int min_sel = 2 * (opt->block / 2 + 2) + 1;
+        if (width < min_sel || height < min_sel) {
+            p->err = "track-frames: image smaller than 2 * (block / 2 + 2) + 1 for the selection";
+            return RSSYNC_E_INVALID;
+        }
+        if ((int64_t)sel.cells_x * sel.cells_y > 65536) {
+            p->err = "track-frames: more than 65536 selection cells per image";
+            return RSSYNC_E_INVALID;
+        }
+    }
+    // selection: every frame is sized for max_points points until the device has chosen them
+    const std::vector<size_t> bound(select ? n_frames : 0, select ? (size_t)opt->max_points : 0);
+    std::vector<size_t> at;
+    if (int rc = check_pixel_args(p, n_frames, select ? bound.data() : counts, lens, (double)height, at)) return rc;
+    const size_t total = at[n_frames];
+    if (int rc = check_device_pointer(p, images, "images")) return rc;
+    if (total && !select)
+        if (int rc = check_device_pointer(p, points, "points")) return rc;
+    for (void* o : {(void*)out.points, (void*)out.tracked, (void*)out.status, (void*)out.fb})
+        if (o && total)
+            if (int rc = check_device_pointer(p, o, "an output buffer")) return rc;
+    if (int rc = check_frame_ts(p, n_frames, image_ts, image_ts + 1)) return rc;
+
+    const size_t per_image = rs::track_pyramid_floats(width, height, tp.levels);
+    const size_t n_images = n_frames + 1;
+    size_t slots = per_image ? std::min(n_images, std::max<size_t>(2, kTrackScratchBytes / (4 * per_image)))
+                             : n_images;
+    const size_t n_cells = (size_t)sel.cells_x * sel.cells_y;
+    if (select) {  // the selection's scratch per image counts against the same budget
+        const size_t bytes = 4 * per_image + 8 * n_cells + 4 * (size_t)sel.max_points + 4;
+        slots = std::min({n_images, std::max<size_t>(2, kTrackScratchBytes / bytes), size_t(65536)});
+    }
+    const double fb_max = opt ? opt->fb_max : 0.0;
+    CUDA_TRY(p, cudaSetDevice(p->device));
+    CUDA_TRY(p, p->d_trk_pyr.reserve(std::max<size_t>(1, slots * per_image)));
+    // compacted a, b (4 per point), tracked (2 per point), selected points (2 per point)
+    CUDA_TRY(p, p->d_trk_pts.reserve((select ? 8 : 6) * total + 1));
+    CUDA_TRY(p, p->d_trk_at.reserve(n_frames + 1));
+    CUDA_TRY(p, p->d_trk_status.reserve(total + 1));
+    CUDA_TRY(p, p->d_trk_flag.reserve(1));
+    CUDA_TRY(p, p->h_trk_flag.reserve(1));
+    if (select) {
+        CUDA_TRY(p, p->d_trk_keys.reserve(slots * n_cells));
+        CUDA_TRY(p, p->d_trk_picks.reserve(slots * sel.max_points));
+        CUDA_TRY(p, p->d_trk_count.reserve(slots));
+        CUDA_TRY(p, p->h_trk_qat.reserve(n_frames + 1));
+        sel.d_keys = p->d_trk_keys.ptr;
+        sel.d_picks = p->d_trk_picks.ptr;
+        sel.d_count = p->d_trk_count.ptr;
+    }
+    double* d_a = p->d_trk_pts.ptr;
+    double* d_b = d_a + 2 * total;
+    double* d_tracked = out.tracked ? out.tracked : d_b + 2 * total;
+    double* d_points = select ? (out.points ? out.points : d_b + 4 * total) : const_cast<double*>(points);
+    uint8_t* d_status = out.status ? out.status : p->d_trk_status.ptr;
+    int64_t* d_kept_at = p->d_trk_at.ptr;
+    std::vector<int64_t> q_at(at.begin(), at.end());
+    const rs::TrackImages im{images, (int64_t)pitch, width, height, tp.levels, tp.window, tp.max_iters,
+                             (float)tp.epsilon, (float)tp.min_eig};
+    const rs::TrackExtra ex{select ? &sel : nullptr, fb_max, out.fb};
+    DevicePointSource src;
+    // s.d_at holds the query offsets (begin_device_staging; in selection mode the bound, overwritten on
+    // the device by the selected offsets); s.h_at receives the kept ones
+    src.queue = [&](const DeviceStaging& s) -> const int64_t* {
+        cudaError_t e = cudaMemsetAsync(p->d_trk_flag.ptr, 0, sizeof(unsigned), p->stream);
+        if (e == cudaSuccess && out.fb && total) e = cudaMemsetAsync(out.fb, 0xff, total * sizeof(double), p->stream);
+        if (e == cudaSuccess && out.points && total && !select)
+            e = cudaMemcpyAsync(out.points, points, 2 * total * sizeof(double), cudaMemcpyDeviceToDevice, p->stream);
+        if (e != cudaSuccess) {
+            p->err = std::string("CUDA error: ") + cudaGetErrorString(e);
+            return nullptr;
+        }
+        rs::launch_track_frames(im, (int)n_frames, select ? nullptr : q_at.data(), s.d_at, d_points, p->d_trk_pyr.ptr,
+                                (int)slots, d_tracked, d_status, p->d_trk_flag.ptr, ex, p->stream);
+        rs::launch_track_compact(s.d_at, (int)n_frames, d_points, d_tracked, d_status, d_a, d_b, d_kept_at,
+                                 p->stream);
+        if (d2h(p, s.h_at, d_kept_at, (n_frames + 1) * sizeof(int64_t)) ||
+            d2h(p, p->h_trk_flag.ptr, p->d_trk_flag.ptr, sizeof(unsigned)) ||
+            (select && d2h(p, p->h_trk_qat.ptr, s.d_at, (n_frames + 1) * sizeof(int64_t))))
+            return nullptr;
+        return d_kept_at;
+    };
+    src.verdict = [&](const DeviceStaging& s, std::vector<size_t>& kept) {
+        if (*p->h_trk_flag.ptr) {
+            p->err = kMsgNonFinite[kRaysA];
+            return (int)RSSYNC_E_NONFINITE;
+        }
+        if (out.counts)
+            for (size_t i = 0; i < n_frames; ++i)
+                out.counts[i] = select ? (size_t)(p->h_trk_qat.ptr[i + 1] - p->h_trk_qat.ptr[i]) : counts[i];
+        for (size_t i = 0; i <= n_frames; ++i) kept[i] = (size_t)s.h_at[i];
+        return (int)RSSYNC_OK;
+    };
+    return ingest_pixels_device(p, n_frames, frames, at, image_ts, image_ts + 1, d_a, d_b, lens, (double)height,
+                                stream, &src);
+}
+
 }  // namespace
 
 extern "C" {
@@ -2670,74 +2816,28 @@ int rssync_track_frames_device(rssync_problem* p, size_t n_frames, const int64_t
     if (!p) return RSSYNC_E_INVALID;
     if (n_frames == 0) return RSSYNC_OK;
     if (!frames || !counts || !image_ts || !lens || n_frames > (size_t)INT32_MAX - 1) return RSSYNC_E_INVALID;
-    const rssync_track_params tp = params ? *params : rssync_track_params{3, 21, 30, 0.01, 1e-4};
-    if (tp.levels < 1 || tp.levels > 6 || tp.window < 5 || tp.window > 63 || tp.window % 2 == 0 || tp.max_iters < 1 ||
-        tp.max_iters > 100 || !(tp.epsilon >= 0.0) || !std::isfinite(tp.epsilon) || !(tp.min_eig >= 0.0) ||
-        !std::isfinite(tp.min_eig)) {
-        p->err = "track-frames: parameters out of range";
-        return RSSYNC_E_INVALID;
-    }
-    const int64_t min_side = (int64_t)tp.window << (tp.levels - 1);
-    if (width < min_side || height < min_side || pitch < (size_t)width) {
-        p->err = "track-frames: image smaller than window * 2^(levels - 1), or pitch below width";
-        return RSSYNC_E_INVALID;
-    }
-    std::vector<size_t> at;
-    if (int rc = check_pixel_args(p, n_frames, counts, lens, (double)height, at)) return rc;
-    const size_t total = at[n_frames];
-    if (int rc = check_device_pointer(p, images, "images")) return rc;
-    if (total)
-        if (int rc = check_device_pointer(p, points, "points")) return rc;
-    for (void* out : {(void*)tracked_out, (void*)status_out})
-        if (out && total)
-            if (int rc = check_device_pointer(p, out, "an output buffer")) return rc;
-    if (int rc = check_frame_ts(p, n_frames, image_ts, image_ts + 1)) return rc;
+    return track_frames(p, n_frames, frames, counts, image_ts, points, images, pitch, width, height, lens, params,
+                        nullptr, TrackOutputs{nullptr, nullptr, tracked_out, status_out, nullptr}, stream);
+}
 
-    const size_t per_image = rs::track_pyramid_floats(width, height, tp.levels);
-    const size_t n_images = n_frames + 1;
-    const size_t slots = per_image ? std::min(n_images, std::max<size_t>(2, kTrackScratchBytes / (4 * per_image)))
-                                   : n_images;
-    CUDA_TRY(p, cudaSetDevice(p->device));
-    CUDA_TRY(p, p->d_trk_pyr.reserve(std::max<size_t>(1, slots * per_image)));
-    CUDA_TRY(p, p->d_trk_pts.reserve(6 * total + 1));  // compacted a, b (4 per point), tracked (2 per point)
-    CUDA_TRY(p, p->d_trk_at.reserve(n_frames + 1));
-    CUDA_TRY(p, p->d_trk_status.reserve(total + 1));
-    CUDA_TRY(p, p->d_trk_flag.reserve(1));
-    CUDA_TRY(p, p->h_trk_flag.reserve(1));
-    double* d_a = p->d_trk_pts.ptr;
-    double* d_b = d_a + 2 * total;
-    double* d_tracked = tracked_out ? tracked_out : d_b + 2 * total;
-    uint8_t* d_status = status_out ? status_out : p->d_trk_status.ptr;
-    int64_t* d_kept_at = p->d_trk_at.ptr;
-    std::vector<int64_t> q_at(at.begin(), at.end());
-    const rs::TrackImages im{images, (int64_t)pitch, width, height, tp.levels, tp.window, tp.max_iters,
-                             (float)tp.epsilon, (float)tp.min_eig};
-    DevicePointSource src;
-    // s.d_at holds the query offsets (begin_device_staging); s.h_at receives the kept ones
-    src.queue = [&](const DeviceStaging& s) -> const int64_t* {
-        const cudaError_t e = cudaMemsetAsync(p->d_trk_flag.ptr, 0, sizeof(unsigned), p->stream);
-        if (e != cudaSuccess) {
-            p->err = std::string("CUDA error: ") + cudaGetErrorString(e);
-            return nullptr;
-        }
-        rs::launch_track_frames(im, (int)n_frames, q_at.data(), s.d_at, points, p->d_trk_pyr.ptr, (int)slots,
-                                d_tracked, d_status, p->d_trk_flag.ptr, p->stream);
-        rs::launch_track_compact(s.d_at, (int)n_frames, points, d_tracked, d_status, d_a, d_b, d_kept_at, p->stream);
-        if (d2h(p, s.h_at, d_kept_at, (n_frames + 1) * sizeof(int64_t)) ||
-            d2h(p, p->h_trk_flag.ptr, p->d_trk_flag.ptr, sizeof(unsigned)))
-            return nullptr;
-        return d_kept_at;
-    };
-    src.verdict = [&](const DeviceStaging& s, std::vector<size_t>& kept) {
-        if (*p->h_trk_flag.ptr) {
-            p->err = kMsgNonFinite[kRaysA];
-            return (int)RSSYNC_E_NONFINITE;
-        }
-        for (size_t i = 0; i <= n_frames; ++i) kept[i] = (size_t)s.h_at[i];
-        return (int)RSSYNC_OK;
-    };
-    return ingest_pixels_device(p, n_frames, frames, at, image_ts, image_ts + 1, d_a, d_b, lens, (double)height,
-                                stream, &src);
+// rssync_track_frames_device with the points selected on the device (points and counts NULL) and the
+// forward-backward check
+int rssync_track_frames_ex_device(rssync_problem* p, size_t n_frames, const int64_t* frames, const size_t* counts,
+                                  const double* image_ts, const double* points, const uint8_t* images, size_t pitch,
+                                  int width, int height, const rssync_lens* lens, const rssync_track_params* params,
+                                  const rssync_track_options* options, double* points_out, size_t* counts_out,
+                                  double* tracked_out, uint8_t* status_out, double* fb_out, void* stream) {
+    RS_NVTX_RANGE();
+    if (!p) return RSSYNC_E_INVALID;
+    if (n_frames == 0) return RSSYNC_OK;
+    if (!frames || !image_ts || !lens || n_frames > (size_t)INT32_MAX - 1) return RSSYNC_E_INVALID;
+    if (!points != !counts) {
+        p->err = "track-frames: points and counts must both be given or both be NULL";
+        return RSSYNC_E_INVALID;
+    }
+    const rssync_track_options opt = options ? *options : rssync_track_options{128, 5, 0.01, 512, 1.0};
+    return track_frames(p, n_frames, frames, counts, image_ts, points, images, pitch, width, height, lens, params,
+                        &opt, TrackOutputs{points_out, counts_out, tracked_out, status_out, fb_out}, stream);
 }
 
 }  // extern "C"

@@ -1939,11 +1939,18 @@ __device__ __forceinline__ float track_warp_sum(float v) {
 
 // One warp per query point, all levels.  Per warp in shared memory: the side-a patch, (window + 2)^2
 // bilinear samples, and its Scharr gradients over the window.
+// kBack: the backward pass of the forward-backward check.  Only points with status 1 take part; the
+// query is the forward result tracked[k] on image i + 1 (side a), side b is image i; the result u gives
+// fb = |u - pts[k]| (double) in fb_out[k] when u is kept (lost: fb_out[k] keeps the NaN it was filled
+// with), and the status becomes 2 unless u is kept and fb <= fb_max.
+// The forward instantiation writes neither fb_out nor reads fb_max.
 constexpr int kLkWarps = 4;
+template <bool kBack>
 __global__ void __launch_bounds__(kLkWarps * 32) track_lk_kernel(TrackPyr P, const int64_t* __restrict__ q_at,
                                                                 int f0, int f1, const double* __restrict__ pts,
                                                                 double* __restrict__ tracked,
-                                                                uint8_t* __restrict__ status, unsigned* flag) {
+                                                                uint8_t* __restrict__ status, unsigned* flag,
+                                                                double fb_max, double* __restrict__ fb_out) {
     extern __shared__ float s_lk[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int win = P.im.window, r = win / 2, pw = win + 2, nw = win * win;
@@ -1957,10 +1964,11 @@ __global__ void __launch_bounds__(kLkWarps * 32) track_lk_kernel(TrackPyr P, con
         const int mid = (lo + hi + 1) >> 1;
         if (q_at[mid] <= k) lo = mid; else hi = mid - 1;
     }
-    const int ja = lo, jb = lo + 1;
-    const double qx = pts[2 * k], qy = pts[2 * k + 1];
+    const int ja = kBack ? lo + 1 : lo, jb = kBack ? lo : lo + 1;
+    if (kBack && status[k] != 1) return;
+    const double qx = kBack ? tracked[2 * k] : pts[2 * k], qy = kBack ? tracked[2 * k + 1] : pts[2 * k + 1];
     const bool finite = isfinite(qx) && isfinite(qy);
-    if (!finite && lane == 0) atomicOr(flag, 1u);
+    if (!kBack && !finite && lane == 0) atomicOr(flag, 1u);
     bool ok = finite && qx >= 0.0 && qx <= P.w[0] - 1 && qy >= 0.0 && qy <= P.h[0] - 1;
     const float px0 = (float)qx, py0 = (float)qy;
     const float eps2 = P.im.epsilon * P.im.epsilon, area = (float)nw;
@@ -2034,9 +2042,16 @@ __global__ void __launch_bounds__(kLkWarps * 32) track_lk_kernel(TrackPyr P, con
             ty = qy + (double)(gy + vy);
             ok = tx >= 0.0 && tx <= P.w[0] - 1 && ty >= 0.0 && ty <= P.h[0] - 1;
         }
-        tracked[2 * k] = tx;
-        tracked[2 * k + 1] = ty;
-        status[k] = ok ? 1 : 0;
+        if constexpr (kBack) {
+            const double ex = tx - pts[2 * k], ey = ty - pts[2 * k + 1];
+            const double fb = sqrt(ex * ex + ey * ey);
+            if (ok && fb_out) fb_out[k] = fb;  // (the caller filled fb_out with NaN)
+            status[k] = ok && fb <= fb_max ? 1 : 2;
+        } else {
+            tracked[2 * k] = tx;
+            tracked[2 * k + 1] = ty;
+            status[k] = ok ? 1 : 0;
+        }
     }
 }
 
@@ -2054,7 +2069,7 @@ __global__ void __launch_bounds__(kCompactThreads) track_compact_kernel(const in
     for (int f = warp; f < n; f += W) {
         int64_t c = 0;
         for (int64_t k = q_at[f] + lane; k - lane < q_at[f + 1]; k += 32)
-            c += __popc(__ballot_sync(FULL, k < q_at[f + 1] && status[k] != 0));
+            c += __popc(__ballot_sync(FULL, k < q_at[f + 1] && status[k] == 1));
         if (lane == 0) kept_at[f + 1] = c;
     }
     __syncthreads();
@@ -2077,7 +2092,7 @@ __global__ void __launch_bounds__(kCompactThreads) track_compact_kernel(const in
     for (int f = warp; f < n; f += W) {
         int64_t o = kept_at[f];
         for (int64_t k = q_at[f] + lane; k - lane < q_at[f + 1]; k += 32) {
-            const bool keep = k < q_at[f + 1] && status[k] != 0;
+            const bool keep = k < q_at[f + 1] && status[k] == 1;
             const unsigned m = __ballot_sync(FULL, keep);
             if (keep) {
                 const int64_t d = o + __popc(m & ((1u << lane) - 1u));
@@ -2087,6 +2102,218 @@ __global__ void __launch_bounds__(kCompactThreads) track_compact_kernel(const in
                 out_b[2 * d + 1] = tracked[2 * k + 1];
             }
             o += __popc(m);
+        }
+    }
+}
+
+// ------------------------------------------------------------------------------------------
+// Point selection (rssync_track_frames_ex_device; the contract is stated in include/rssync_b200.h):
+// the minimum eigenvalue of the structure tensor (cv2.cornerMinEigenVal), its 3 x 3 local maxima, the
+// best of each cell, then a threshold and a top-max_points cut per image.  float32 in the order written
+// (-fmad=false), so the scores equal a numpy float32 restatement bit for bit.
+constexpr int kSelThreads = 256, kSelStrip = 32, kPickThreads = 1024;
+
+// One block per (cell, image).  Shared memory: the cell's pixels with a halo of block / 2 + 2, the
+// scores of the cell and a 1-pixel ring, and, per strip of kSelStrip score rows, the Sobel gradients
+// and the row sums of their products.  The halo keeps every pixel a candidate's or its neighbours'
+// scores read inside the image, so reads outside it (clamped here) reach no used score.  Writes the
+// cell's best candidate as the key (score bits << 32) | ~(y * w + x): the greater key is the greater
+// score, then the smaller index; 0 = no candidate.
+__global__ void __launch_bounds__(kSelThreads) select_cells_kernel(TrackImages im, TrackSelect S, int j0) {
+    extern __shared__ float s_sel[];
+    const int C = S.cell, B = S.block, r = B / 2, hal = r + 2;
+    const int PW = C + 2 * hal, SW = C + 2, GW = SW + 2 * r, GR = kSelStrip + 2 * r;
+    float* sS = s_sel;           // SW x SW scores: row sy, column sx <-> (X0 - 1 + sx, Y0 - 1 + sy)
+    float* sDx = sS + SW * SW;   // GR x GW gradients of a strip
+    float* sDy = sDx + GR * GW;
+    float* sHxx = sDy + GR * GW;  // GR x SW row sums of a strip
+    float* sHxy = sHxx + GR * SW;
+    float* sHyy = sHxy + GR * SW;
+    uint8_t* sP = reinterpret_cast<uint8_t*>(sHyy + GR * SW);  // PW x PW pixels from (X0 - hal, Y0 - hal)
+    const int w = im.w0, h = im.h0;
+    const int X0 = (blockIdx.x % S.cells_x) * C, Y0 = (blockIdx.x / S.cells_x) * C;
+    const uint8_t* img = im.img0 + (int64_t)(j0 + blockIdx.y) * h * im.pitch0;
+    for (int t = threadIdx.x; t < PW * PW; t += kSelThreads) {
+        const int y = min(max(Y0 - hal + t / PW, 0), h - 1), x = min(max(X0 - hal + t % PW, 0), w - 1);
+        sP[t] = __ldg(img + (int64_t)y * im.pitch0 + x);
+    }
+    const float sc = (float)(1.0 / (4.0 * B * 255.0));
+    __syncthreads();
+    for (int s0 = 0; s0 < SW; s0 += kSelStrip) {
+        const int nr = min(kSelStrip, SW - s0), gr = nr + 2 * r;
+        // gradient row t, column u <-> (X0 - 1 - r + u, Y0 - 1 - r + s0 + t), pixel row s0 + t + 1, column u + 1
+        for (int t = threadIdx.x; t < gr * GW; t += kSelThreads) {
+            const uint8_t* c = sP + (s0 + t / GW + 1) * PW + t % GW + 1;
+            const float i00 = c[-PW - 1], i01 = c[-PW], i02 = c[-PW + 1], i10 = c[-1], i12 = c[1];
+            const float i20 = c[PW - 1], i21 = c[PW], i22 = c[PW + 1];
+            sDx[t] = (((i02 - i00) + 2.f * (i12 - i10)) + (i22 - i20)) * sc;
+            sDy[t] = (((i20 - i00) + 2.f * (i21 - i01)) + (i22 - i02)) * sc;
+        }
+        __syncthreads();
+        // row sums: column v <-> x = X0 - 1 + v adds gradient columns v .. v + 2r, left to right
+        for (int t = threadIdx.x; t < gr * SW; t += kSelThreads) {
+            const float* dx = sDx + (t / SW) * GW + t % SW;
+            const float* dy = sDy + (t / SW) * GW + t % SW;
+            float xx = dx[0] * dx[0], xy = dx[0] * dy[0], yy = dy[0] * dy[0];
+            for (int i = 1; i < B; ++i) {
+                xx += dx[i] * dx[i];
+                xy += dx[i] * dy[i];
+                yy += dy[i] * dy[i];
+            }
+            sHxx[t] = xx;
+            sHxy[t] = xy;
+            sHyy[t] = yy;
+        }
+        __syncthreads();
+        // score row s0 + t adds row sums t .. t + 2r, top to bottom
+        for (int t = threadIdx.x; t < nr * SW; t += kSelThreads) {
+            float xx = sHxx[t], xy = sHxy[t], yy = sHyy[t];
+            for (int i = 1; i < B; ++i) {
+                xx += sHxx[t + i * SW];
+                xy += sHxy[t + i * SW];
+                yy += sHyy[t + i * SW];
+            }
+            const float a = 0.5f * xx, c = 0.5f * yy, d = a - c;
+            sS[s0 * SW + t] = (a + c) - sqrtf(d * d + xy * xy);
+        }
+        __syncthreads();
+    }
+    const int m = hal;
+    unsigned long long best = 0;
+    for (int t = threadIdx.x; t < C * C; t += kSelThreads) {
+        const int x = X0 + t % C, y = Y0 + t / C;
+        if (x < m || x > w - 1 - m || y < m || y > h - 1 - m) continue;
+        const float* c = sS + (t / C + 1) * SW + t % C + 1;
+        const float v = c[0];
+        if (v > 0.f && v >= c[-SW - 1] && v >= c[-SW] && v >= c[-SW + 1] && v >= c[-1] && v >= c[1] &&
+            v >= c[SW - 1] && v >= c[SW] && v >= c[SW + 1]) {
+            const unsigned long long key = ((unsigned long long)__float_as_uint(v) << 32) |
+                                           (unsigned)~((unsigned)y * (unsigned)w + (unsigned)x);
+            best = key > best ? key : best;
+        }
+    }
+    __shared__ unsigned long long s_best[kSelThreads / 32];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const unsigned long long u = __shfl_xor_sync(FULL, best, o);
+        best = u > best ? u : best;
+    }
+    if ((threadIdx.x & 31) == 0) s_best[threadIdx.x >> 5] = best;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        for (int i = 1; i < kSelThreads / 32; ++i) best = s_best[i] > best ? s_best[i] : best;
+        S.d_keys[(size_t)blockIdx.y * S.cells_x * S.cells_y + blockIdx.x] = best;
+    }
+}
+
+__device__ __forceinline__ unsigned block_reduce_max_sum(unsigned v, bool is_max, unsigned* s_red) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const unsigned u = __shfl_xor_sync(FULL, v, o);
+        v = is_max ? max(v, u) : v + u;
+    }
+    __syncthreads();  // (s_red's previous readers are done)
+    if ((threadIdx.x & 31) == 0) s_red[threadIdx.x >> 5] = v;
+    __syncthreads();
+    v = s_red[0];
+    for (int i = 1; i < (int)(blockDim.x >> 5); ++i) v = is_max ? max(v, s_red[i]) : v + s_red[i];
+    return v;
+}
+
+// One block per image of a chunk: M (the greatest pick score), the threshold (float)quality * M, and,
+// when more than max_points picks pass it, the max_points-th greatest selection key (score bits << 32) |
+// ~cell by an MSB radix select (8 passes of 8 bits; the keys are distinct).  Then the kept picks in
+// ascending cell order: their pixel indices to d_picks[image * max_points ..], their number to d_count.
+__global__ void __launch_bounds__(kPickThreads) select_points_kernel(TrackSelect S) {
+    __shared__ unsigned s_red[kPickThreads / 32];
+    __shared__ unsigned s_hist[256];
+    __shared__ unsigned long long s_cut;
+    __shared__ unsigned s_need;
+    const int nc = S.cells_x * S.cells_y, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const unsigned long long* keys = S.d_keys + (size_t)blockIdx.x * nc;
+    unsigned mx = 0;
+    for (int c = threadIdx.x; c < nc; c += kPickThreads) mx = max(mx, (unsigned)(keys[c] >> 32));
+    mx = block_reduce_max_sum(mx, true, s_red);
+    const float thr = S.quality * __uint_as_float(mx);
+    auto kept = [&](unsigned long long key) { return key != 0 && __uint_as_float((unsigned)(key >> 32)) >= thr; };
+    unsigned n = 0;
+    for (int c = threadIdx.x; c < nc; c += kPickThreads) n += kept(keys[c]) ? 1u : 0u;
+    n = block_reduce_max_sum(n, false, s_red);
+    unsigned long long cut = 0;  // keep a pick whose selection key is >= cut
+    if (n > (unsigned)S.max_points) {
+        if (threadIdx.x == 0) {
+            s_cut = 0;
+            s_need = S.max_points;
+        }
+        for (int shift = 56; shift >= 0; shift -= 8) {
+            for (int i = threadIdx.x; i < 256; i += kPickThreads) s_hist[i] = 0;
+            __syncthreads();
+            const unsigned long long hi = shift == 56 ? 0ull : ~0ull << (shift + 8), pre = s_cut & hi;
+            for (int c = threadIdx.x; c < nc; c += kPickThreads) {
+                const unsigned long long key = keys[c];
+                const unsigned long long sk = (key & 0xffffffff00000000ull) | (unsigned)~(unsigned)c;
+                if (kept(key) && (sk & hi) == pre) atomicAdd(&s_hist[(sk >> shift) & 255], 1u);
+            }
+            __syncthreads();
+            if (threadIdx.x == 0) {
+                unsigned need = s_need;
+                int d = 255;
+                for (; d > 0 && s_hist[d] < need; --d) need -= s_hist[d];
+                s_need = need;
+                s_cut |= (unsigned long long)d << shift;
+            }
+            __syncthreads();
+        }
+        cut = s_cut;
+    }
+    unsigned base = 0;
+    for (int c0 = 0; c0 < nc; c0 += kPickThreads) {
+        const int c = c0 + threadIdx.x;
+        const unsigned long long key = c < nc ? keys[c] : 0ull;
+        const bool keep = kept(key) && ((key & 0xffffffff00000000ull) | (unsigned)~(unsigned)c) >= cut;
+        const unsigned bal = __ballot_sync(FULL, keep);
+        __syncthreads();  // (s_red's previous readers are done)
+        if (lane == 0) s_red[warp] = __popc(bal);
+        __syncthreads();
+        unsigned off = base, tot = 0;
+        for (int i = 0; i < kPickThreads / 32; ++i) {
+            off += i < warp ? s_red[i] : 0u;
+            tot += s_red[i];
+        }
+        if (keep) S.d_picks[(size_t)blockIdx.x * S.max_points + off + __popc(bal & ((1u << lane) - 1u))] = ~(unsigned)key;
+        base += tot;
+    }
+    if (threadIdx.x == 0) S.d_count[blockIdx.x] = (int32_t)base;
+}
+
+// One block: the prefix of the picks of frames [f0, f1) from q_at[f0] (q_at[0] = 0) into q_at, then
+// every frame's picks as points ((double)x, (double)y) at their offsets.
+__global__ void __launch_bounds__(kPickThreads) select_prefix_kernel(TrackSelect S, int64_t* q_at, int f0, int f1,
+                                                                     int w, double* __restrict__ pts) {
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, n = f1 - f0;
+    constexpr int W = kPickThreads / 32;
+    if (warp == 0) {
+        int64_t carry = f0 == 0 ? 0 : q_at[f0];
+        if (f0 == 0 && lane == 0) q_at[0] = 0;
+        for (int base = 0; base < n; base += 32) {
+            int64_t v = base + lane < n ? S.d_count[base + lane] : 0;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const int64_t u = __shfl_up_sync(FULL, v, o);
+                if (lane >= o) v += u;
+            }
+            v += carry;
+            if (base + lane < n) q_at[f0 + base + lane + 1] = v;
+            carry = __shfl_sync(FULL, v, 31);
+        }
+    }
+    __syncthreads();
+    for (int i = warp; i < n; i += W) {
+        const int64_t o = q_at[f0 + i];
+        for (int k = lane; k < S.d_count[i]; k += 32) {
+            const unsigned idx = S.d_picks[(size_t)i * S.max_points + k];
+            pts[2 * (o + k)] = (double)(idx % (unsigned)w);
+            pts[2 * (o + k) + 1] = (double)(idx / (unsigned)w);
         }
     }
 }
@@ -2727,14 +2954,24 @@ size_t track_pyramid_floats(int w0, int h0, int levels) {
     return n;
 }
 
-void launch_track_frames(const TrackImages& im, int n_frames, const int64_t* h_q_at, const int64_t* d_q_at,
-                         const double* d_points, float* d_pyr, int slots, double* d_tracked, uint8_t* d_status,
-                         unsigned* d_flag, cudaStream_t st) {
+size_t track_select_smem(int cell, int block) {
+    const int r = block / 2, PW = cell + 2 * (r + 2), SW = cell + 2, GW = SW + 2 * r, GR = kSelStrip + 2 * r;
+    return ((size_t)SW * SW + 2 * (size_t)GR * GW + 3 * (size_t)GR * SW) * sizeof(float) + (size_t)PW * PW;
+}
+
+void launch_track_frames(const TrackImages& im, int n_frames, const int64_t* h_q_at, int64_t* d_q_at,
+                         double* d_points, float* d_pyr, int slots, double* d_tracked, uint8_t* d_status,
+                         unsigned* d_flag, const TrackExtra& ex, cudaStream_t st) {
     if (n_frames <= 0) return;
     const TrackPyr P = track_pyr(im, d_pyr, slots);
     const int pw = im.window + 2;
     const size_t smem = (size_t)kLkWarps * (pw * pw + 2 * im.window * im.window) * sizeof(float);
-    allow_smem(track_lk_kernel, smem);
+    allow_smem(track_lk_kernel<false>, smem);
+    const bool back = ex.fb_max > 0.0;
+    if (back) allow_smem(track_lk_kernel<true>, smem);
+    const TrackSelect* S = ex.sel;
+    const size_t sel_smem = S ? track_select_smem(S->cell, S->block) : 0;
+    if (S) allow_smem(select_cells_kernel, sel_smem);
     // chunk: build the pyramids of images [built, e), then track frames [f0, e - 1); image f0 is the
     // last one of the previous chunk, still in its slot
     for (int f0 = 0, built = 0; f0 < n_frames;) {
@@ -2744,11 +2981,26 @@ void launch_track_frames(const TrackImages& im, int n_frames, const int64_t* h_q
             track_pyramid_kernel<<<grid, kPyrTX * kPyrTY, 0, st>>>(P, l, built);
             g_launches += 1;
         }
-        const int64_t pts = h_q_at[e - 1] - h_q_at[f0];
+        // selection on the chunk's side-a images f0 .. e - 2; the tracker's grid then covers the bound
+        // max_points per frame and its warps past q_at[e - 1] return at once
+        const int nf = e - 1 - f0;
+        if (S) {
+            select_cells_kernel<<<dim3(S->cells_x * S->cells_y, nf), kSelThreads, sel_smem, st>>>(im, *S, f0);
+            select_points_kernel<<<nf, kPickThreads, 0, st>>>(*S);
+            select_prefix_kernel<<<1, kPickThreads, 0, st>>>(*S, d_q_at, f0, e - 1, im.w0, d_points);
+            g_launches += 3;
+        }
+        const int64_t pts = S ? (int64_t)nf * S->max_points : h_q_at[e - 1] - h_q_at[f0];
         if (pts > 0) {
-            track_lk_kernel<<<(unsigned)((pts + kLkWarps - 1) / kLkWarps), kLkWarps * 32, smem, st>>>(
-                P, d_q_at, f0, e - 1, d_points, d_tracked, d_status, d_flag);
+            const unsigned blocks = (unsigned)((pts + kLkWarps - 1) / kLkWarps);
+            track_lk_kernel<false><<<blocks, kLkWarps * 32, smem, st>>>(P, d_q_at, f0, e - 1, d_points, d_tracked,
+                                                                       d_status, d_flag, 0.0, nullptr);
             g_launches += 1;
+            if (back) {
+                track_lk_kernel<true><<<blocks, kLkWarps * 32, smem, st>>>(P, d_q_at, f0, e - 1, d_points, d_tracked,
+                                                                          d_status, d_flag, ex.fb_max, ex.d_fb);
+                g_launches += 1;
+            }
         }
         built = e;
         f0 = e - 1;

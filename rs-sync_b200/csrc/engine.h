@@ -217,19 +217,43 @@ struct TrackImages {
 };
 // floats of one image's pyramid levels 1 .. levels - 1
 size_t track_pyramid_floats(int w0, int h0, int levels);
-// Tracks every query point of frame i (d_points[2 d_q_at[i] ..], host copy h_q_at) from image i to
-// image i + 1, for i in [0, n_frames).  The pyramids of `slots` (>= 2) images live in d_pyr at once
-// (slots * track_pyramid_floats floats): the images are processed in chunks, image j in slot j % slots,
-// each pyramid built once.  Per point: d_tracked (2 doubles) and d_status (1 = kept); *d_flag gets bit 0
-// when a query point is not finite.
-void launch_track_frames(const TrackImages& im, int n_frames, const int64_t* h_q_at, const int64_t* d_q_at,
-                         const double* d_points, float* d_pyr, int slots, double* d_tracked, uint8_t* d_status,
-                         unsigned* d_flag, cudaStream_t st);
 // The kept pairs, frame by frame in the query order: d_out_a / d_out_b at the kept offsets d_kept_at
 // (n_frames + 1, written here), the layout launch_stage_points reads.
 void launch_track_compact(const int64_t* d_q_at, int n_frames, const double* d_points, const double* d_tracked,
                           const uint8_t* d_status, double* d_out_a, double* d_out_b, int64_t* d_kept_at,
                           cudaStream_t st);
+
+// ---- point selection and the forward-backward check (rssync_track_frames_ex_device) -------------
+// The selection contract is stated at rssync_track_frames_ex_device in include/rssync_b200.h.
+struct TrackSelect {
+    int cell, block, max_points;
+    float quality;
+    int cells_x, cells_y;  // cells per row and column of an image
+    unsigned long long* d_keys;  // scratch: one key per (cell, image) of a chunk, slots * cells_x * cells_y
+    uint32_t* d_picks;           // scratch: per frame of a chunk, max_points pixel indices y * w + x
+    int32_t* d_count;            // scratch: per frame of a chunk, the number of picks
+};
+// Options of launch_track_frames beyond forward tracking.  sel null: the query points are the
+// caller's (h_q_at known); otherwise the points of frame i are selected on image i into d_points (which
+// holds n_frames * max_points points) and d_q_at (written here, from d_q_at[0] = 0).  fb_max > 0: every
+// point kept forward is tracked back, its distance written to d_fb and its status set to 2 when the
+// backward pass loses it or the distance exceeds fb_max.
+struct TrackExtra {
+    const TrackSelect* sel;
+    double fb_max;
+    double* d_fb;
+};
+// Shared memory of one select_cells_kernel block
+size_t track_select_smem(int cell, int block);
+// Tracks every query point of frame i (d_points[2 d_q_at[i] ..], host copy h_q_at) from image i to
+// image i + 1, for i in [0, n_frames).  The pyramids of `slots` (>= 2) images live in d_pyr at once
+// (slots * track_pyramid_floats floats): the images are processed in chunks, image j in slot j % slots,
+// each pyramid built once.  Per point: d_tracked (2 doubles) and d_status (1 = kept); *d_flag gets bit 0
+// when a query point is not finite.  ex: selection and the backward pass (TrackExtra); with ex.sel null
+// and ex.fb_max 0 the launches are the forward tracker's alone.
+void launch_track_frames(const TrackImages& im, int n_frames, const int64_t* h_q_at, int64_t* d_q_at,
+                         double* d_points, float* d_pyr, int slots, double* d_tracked, uint8_t* d_status,
+                         unsigned* d_flag, const TrackExtra& ex, cudaStream_t st);
 
 // ---- stage probes (tests only) ---------------------------------------------------------------
 void launch_probe_problem_matrix(const DeviceData& dd, FrameDesc fd, double delay, double* d_P,

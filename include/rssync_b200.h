@@ -228,6 +228,29 @@ int rssync_track_frames_ex_device(rssync_problem* p, size_t n_frames, const int6
                                   int width, int height, const rssync_lens* lens, const rssync_track_params* params,
                                   const rssync_track_options* options, double* points_out, size_t* counts_out,
                                   double* tracked_out, uint8_t* status_out, double* fb_out, void* stream);
+/* rssync_track_frames_ex_device on 16-bit luma planes (P010 / P016, 10- or 12-bit decoder output).
+ * images: n_frames + 1 planes of uint16_t samples, `height` rows of `pitch` BYTES each, row y of image j at
+ * (const uint8_t*)images + (j * height + y) * pitch.  The one difference from rssync_track_frames_ex_device:
+ * the level-0 intensity is I = (float)v * 2^-shift, v the 16-bit sample, in place of (float)plane[y][x]
+ * (pyramid, bilinear reads, LK and selection).  shift 0..8: 8 for P010 / P016 (sample in the most
+ * significant bits), 2 for 10-bit and 4 for 12-bit samples in the least significant bits; with the right
+ * shift intensities span [0, 256), so min_eig, quality and the Sobel scale keep their 8-bit meaning.  Every
+ * other word of the contract above stands as written: statuses, outputs, the ingest identity with
+ * rssync_set_track_pixels_device, ordering and borrowing, multi-device behaviour.
+ * Identities: v < 2^16 is exact in float32 and the scaling by a power of two is exact, so for an 8-bit
+ * plane P and any shift, the 16-bit plane v = P << shift gives byte for byte what
+ * rssync_track_frames_ex_device gives on P (every output, frame table, arena, row fractions and re-timing
+ * table); likewise a P010 plane (x << 6, shift 8) gives what the LSB-aligned plane x gives with shift 2.
+ * There is no 16-bit form of rssync_track_frames_device: with the caller's points and fb_max = 0 this call
+ * equals it.
+ * Checked before anything is applied, besides the checks of rssync_track_frames_ex_device: RSSYNC_E_INVALID
+ * for shift outside 0..8, images not 2-byte aligned, and an odd pitch or pitch < 2 width. */
+int rssync_track_frames16_device(rssync_problem* p, size_t n_frames, const int64_t* frames, const size_t* counts,
+                                 const double* image_ts, const double* points, const uint16_t* images,
+                                 size_t pitch /* bytes */, int width, int height, int shift,
+                                 const rssync_lens* lens, const rssync_track_params* params,
+                                 const rssync_track_options* options, double* points_out, size_t* counts_out,
+                                 double* tracked_out, uint8_t* status_out, double* fb_out, void* stream);
 /* SetTrackResult for n_frames frames whose rays the caller computed (any camera model), with the
  * rolling-shutter timestamps formed here from per-ray row fractions.  Ray k of frame i gets
  * ts_a = frame_ts_a[i] + readout * frac_a[k] (ts_b alike): one multiply and one add, not contracted,

@@ -46,7 +46,7 @@ C_ABI_SYMBOLS = [
     "rssync_set_track_row_fractions", "rssync_set_track_row_fractions_device",
     "rssync_retime_table", "rssync_row_fraction_plane", "rssync_adopt_row_fractions",
     "rssync_readout_search_windows", "rssync_rotation_search_windows", "rssync_track_frames_device",
-    "rssync_track_frames_ex_device",
+    "rssync_track_frames_ex_device", "rssync_track_frames16_device",
 ]
 # Itanium-ABI symbols of the C++ drop-in face (same set the reference's librssync_core exports)
 CXX_ABI_SYMBOLS = [
@@ -191,6 +191,10 @@ def load_library():
                                                 C.c_size_t, C.c_int, C.c_int, C.POINTER(Lens),
                                                 C.POINTER(TrackParams), C.POINTER(TrackOptions), P,
                                                 C.POINTER(C.c_size_t), P, P, P, P]
+    L.rssync_track_frames16_device.argtypes = [P, C.c_size_t, c_i64_p, C.POINTER(C.c_size_t), c_double_p, P, P,
+                                               C.c_size_t, C.c_int, C.c_int, C.c_int, C.POINTER(Lens),
+                                               C.POINTER(TrackParams), C.POINTER(TrackOptions), P,
+                                               C.POINTER(C.c_size_t), P, P, P, P]
     L.rssync_presync.argtypes = [P, C.c_double, C.c_int64, C.c_int64, C.c_double, C.c_double, c_double_p, c_double_p]
     L.rssync_sync.argtypes = [P, C.c_double, C.c_int64, C.c_int64, C.c_double, C.c_double, c_double_p, c_double_p]
     L.rssync_debug_presync.argtypes = [P, C.c_double, C.c_int64, C.c_int64, C.c_double, c_double_p, c_double_p, C.c_int]
@@ -635,14 +639,18 @@ class SyncProblem:
             C.c_void_p(tracked.data_ptr() if n else None), C.c_void_p(status.data_ptr() if n else None), stream))
         return tracked, status
 
-    def track_frames_ex(self, frames, image_ts, images, lens, params=None, options=None, points=None, counts=None):
+    def track_frames_ex(self, frames, image_ts, images, lens, params=None, options=None, points=None, counts=None,
+                        shift=None):
         """track_frames with the query points selected on the device (points and counts None) and the
         forward-backward check (rssync_track_frames_ex_device).  images, frames, image_ts, lens and params as in
         track_frames; options: TrackOptions or None (the defaults: 128-px cells, block 5, quality 0.01, 512
         points per frame, fb_max 1 px).  Returns TrackResult(points, counts, tracked, status, fb_error): the
         query points, tracked positions (CUDA float64 (n, 2)), statuses (CUDA uint8 (n,): 0 lost, 1 kept and
         ingested, 2 rejected by the backward check) and forward-backward distances (CUDA float64 (n,), NaN
-        where the backward pass did not keep the point or did not run), n = sum(counts); counts: numpy."""
+        where the backward pass did not keep the point or did not run), n = sum(counts); counts: numpy.
+        16-bit planes (rssync_track_frames16_device): a torch.uint16 tensor with shift, the intensity being
+        sample * 2^-shift: 8 for P010 / P016, 2 for 10-bit and 4 for 12-bit samples in the low bits.  shift
+        is required for uint16 and must be None for uint8."""
         import torch
         fr = np.ascontiguousarray(frames, dtype=np.int64)
         ts = _f64(image_ts)
@@ -650,8 +658,15 @@ class SyncProblem:
             raise ValueError("track_frames_ex: give both points and counts, or neither (selection)")
         if not getattr(images, "is_cuda", False):
             raise TypeError("track_frames_ex: images must be a CUDA tensor")
-        if images.dtype != torch.uint8 or images.dim() != 3 or images.stride(2) != 1:
-            raise ValueError("track_frames_ex: images must be a uint8 tensor (n_frames + 1, H, W) with contiguous rows")
+        wide = images.dtype == torch.uint16
+        if not (wide or images.dtype == torch.uint8) or images.dim() != 3 or images.stride(2) != 1:
+            raise ValueError("track_frames_ex: images must be a uint8 or uint16 tensor (n_frames + 1, H, W) with "
+                             "contiguous rows")
+        if wide and shift is None:
+            raise ValueError("track_frames_ex: uint16 images need a shift (8 for P010 / P016, 2 for 10-bit and 4 "
+                             "for 12-bit samples in the low bits)")
+        if not wide and shift is not None:
+            raise ValueError("track_frames_ex: shift applies to uint16 images only")
         if images.shape[0] != fr.shape[0] + 1 or ts.shape[0] != fr.shape[0] + 1:
             raise ValueError(f"track_frames_ex: {fr.shape[0]} frames need {fr.shape[0] + 1} images and image "
                              f"timestamps, got {images.shape[0]} and {ts.shape[0]}")
@@ -681,12 +696,16 @@ class SyncProblem:
         def ptr(t):
             return C.c_void_p(t.data_ptr() if cap else None)
 
-        self._check(self.L.rssync_track_frames_ex_device(
-            self.h, fr.shape[0], fr.ctypes.data_as(c_i64_p),
-            None if cn is None else cn.ctypes.data_as(C.POINTER(C.c_size_t)), _dp(ts), pp,
-            C.c_void_p(images.data_ptr()), images.stride(1), images.shape[2], images.shape[1], C.byref(lens_c), prm,
-            C.byref(opt), ptr(pts_out), counts_out.ctypes.data_as(C.POINTER(C.c_size_t)), ptr(tracked), ptr(status),
-            ptr(fb), stream))
+        head = (self.h, fr.shape[0], fr.ctypes.data_as(c_i64_p),
+                None if cn is None else cn.ctypes.data_as(C.POINTER(C.c_size_t)), _dp(ts), pp,
+                C.c_void_p(images.data_ptr()), images.stride(1) * images.element_size(), images.shape[2],
+                images.shape[1])
+        tail = (C.byref(lens_c), prm, C.byref(opt), ptr(pts_out), counts_out.ctypes.data_as(C.POINTER(C.c_size_t)),
+                ptr(tracked), ptr(status), ptr(fb), stream)
+        if wide:
+            self._check(self.L.rssync_track_frames16_device(*head, int(shift), *tail))
+        else:
+            self._check(self.L.rssync_track_frames_ex_device(*head, *tail))
         n = int(counts_out.sum())
         return TrackResult(pts_out[:n], counts_out.astype(np.int64), tracked[:n], status[:n], fb[:n])
 

@@ -2651,12 +2651,14 @@ struct TrackOutputs {
     double* fb;
 };
 
-// The body of both tracking entry points once their null checks have passed.  opt null: the plain form
-// (caller's points, no backward pass, no options checked).
+// The body of the tracking entry points once their null checks have passed.  opt null: the plain form
+// (caller's points, no backward pass, no options checked).  sample: bytes per sample of the planes, 1
+// (uint8) or 2 (uint16, level 0 = v * 2^-shift).
 int track_frames(rssync_problem* p, size_t n_frames, const int64_t* frames, const size_t* counts,
-                 const double* image_ts, const double* points, const uint8_t* images, size_t pitch, int width,
+                 const double* image_ts, const double* points, const void* images, size_t pitch, int width,
                  int height, const rssync_lens* lens, const rssync_track_params* params,
-                 const rssync_track_options* opt, const TrackOutputs& out, void* stream) {
+                 const rssync_track_options* opt, const TrackOutputs& out, void* stream, int sample = 1,
+                 int shift = 0) {
     const rssync_track_params tp = params ? *params : rssync_track_params{3, 21, 30, 0.01, 1e-4};
     if (tp.levels < 1 || tp.levels > 6 || tp.window < 5 || tp.window > 63 || tp.window % 2 == 0 || tp.max_iters < 1 ||
         tp.max_iters > 100 || !(tp.epsilon >= 0.0) || !std::isfinite(tp.epsilon) || !(tp.min_eig >= 0.0) ||
@@ -2675,6 +2677,16 @@ int track_frames(rssync_problem* p, size_t n_frames, const int64_t* frames, cons
     if (width < min_side || height < min_side || pitch < (size_t)width) {
         p->err = "track-frames: image smaller than window * 2^(levels - 1), or pitch below width";
         return RSSYNC_E_INVALID;
+    }
+    if (sample == 2) {
+        if (shift < 0 || shift > 8) {
+            p->err = "track-frames: shift outside 0..8";
+            return RSSYNC_E_INVALID;
+        }
+        if (reinterpret_cast<uintptr_t>(images) % 2 || pitch % 2 || pitch < 2 * (size_t)width) {
+            p->err = "track-frames: 16-bit images need a 2-byte aligned address and an even pitch >= 2 * width bytes";
+            return RSSYNC_E_INVALID;
+        }
     }
     rs::TrackSelect sel{};
     if (select) {
@@ -2741,8 +2753,9 @@ int track_frames(rssync_problem* p, size_t n_frames, const int64_t* frames, cons
     uint8_t* d_status = out.status ? out.status : p->d_trk_status.ptr;
     int64_t* d_kept_at = p->d_trk_at.ptr;
     std::vector<int64_t> q_at(at.begin(), at.end());
-    const rs::TrackImages im{images, (int64_t)pitch, width, height, tp.levels, tp.window, tp.max_iters,
-                             (float)tp.epsilon, (float)tp.min_eig};
+    const rs::TrackImages im{static_cast<const uint8_t*>(images), (int64_t)pitch, width, height, tp.levels,
+                             tp.window, tp.max_iters, (float)tp.epsilon, (float)tp.min_eig, (uint8_t)sample,
+                             (uint8_t)shift};
     const rs::TrackExtra ex{select ? &sel : nullptr, fb_max, out.fb};
     DevicePointSource src;
     // s.d_at holds the query offsets (begin_device_staging; in selection mode the bound, overwritten on
@@ -2779,6 +2792,25 @@ int track_frames(rssync_problem* p, size_t n_frames, const int64_t* frames, cons
     };
     return ingest_pixels_device(p, n_frames, frames, at, image_ts, image_ts + 1, d_a, d_b, lens, (double)height,
                                 stream, &src);
+}
+
+// The ex entry points (rssync_track_frames_ex_device, rssync_track_frames16_device): their null checks and
+// default options, then track_frames
+int track_frames_ex(rssync_problem* p, size_t n_frames, const int64_t* frames, const size_t* counts,
+                    const double* image_ts, const double* points, const void* images, size_t pitch, int width,
+                    int height, const rssync_lens* lens, const rssync_track_params* params,
+                    const rssync_track_options* options, const TrackOutputs& out, void* stream, int sample,
+                    int shift) {
+    if (!p) return RSSYNC_E_INVALID;
+    if (n_frames == 0) return RSSYNC_OK;
+    if (!frames || !image_ts || !lens || n_frames > (size_t)INT32_MAX - 1) return RSSYNC_E_INVALID;
+    if (!points != !counts) {
+        p->err = "track-frames: points and counts must both be given or both be NULL";
+        return RSSYNC_E_INVALID;
+    }
+    const rssync_track_options opt = options ? *options : rssync_track_options{128, 5, 0.01, 512, 1.0};
+    return track_frames(p, n_frames, frames, counts, image_ts, points, images, pitch, width, height, lens, params,
+                        &opt, out, stream, sample, shift);
 }
 
 }  // namespace
@@ -2828,16 +2860,22 @@ int rssync_track_frames_ex_device(rssync_problem* p, size_t n_frames, const int6
                                   const rssync_track_options* options, double* points_out, size_t* counts_out,
                                   double* tracked_out, uint8_t* status_out, double* fb_out, void* stream) {
     RS_NVTX_RANGE();
-    if (!p) return RSSYNC_E_INVALID;
-    if (n_frames == 0) return RSSYNC_OK;
-    if (!frames || !image_ts || !lens || n_frames > (size_t)INT32_MAX - 1) return RSSYNC_E_INVALID;
-    if (!points != !counts) {
-        p->err = "track-frames: points and counts must both be given or both be NULL";
-        return RSSYNC_E_INVALID;
-    }
-    const rssync_track_options opt = options ? *options : rssync_track_options{128, 5, 0.01, 512, 1.0};
-    return track_frames(p, n_frames, frames, counts, image_ts, points, images, pitch, width, height, lens, params,
-                        &opt, TrackOutputs{points_out, counts_out, tracked_out, status_out, fb_out}, stream);
+    return track_frames_ex(p, n_frames, frames, counts, image_ts, points, images, pitch, width, height, lens, params,
+                           options, TrackOutputs{points_out, counts_out, tracked_out, status_out, fb_out}, stream, 1,
+                           0);
+}
+
+// rssync_track_frames_ex_device on 16-bit planes: level 0 is (float)v * 2^-shift
+int rssync_track_frames16_device(rssync_problem* p, size_t n_frames, const int64_t* frames, const size_t* counts,
+                                 const double* image_ts, const double* points, const uint16_t* images, size_t pitch,
+                                 int width, int height, int shift, const rssync_lens* lens,
+                                 const rssync_track_params* params, const rssync_track_options* options,
+                                 double* points_out, size_t* counts_out, double* tracked_out, uint8_t* status_out,
+                                 double* fb_out, void* stream) {
+    RS_NVTX_RANGE();
+    return track_frames_ex(p, n_frames, frames, counts, image_ts, points, images, pitch, width, height, lens, params,
+                           options, TrackOutputs{points_out, counts_out, tracked_out, status_out, fb_out}, stream, 2,
+                           shift);
 }
 
 }  // extern "C"

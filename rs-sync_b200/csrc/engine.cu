@@ -1876,6 +1876,7 @@ struct TrackPyr {
     float* lvl[kTrackMaxLevels];  // levels 1..: row y of slot s at lvl[l] + (s * h[l] + y) * w[l]
     int w[kTrackMaxLevels], h[kTrackMaxLevels];
     int slots;
+    float scale;  // 2^-im.shift (a kernel parameter, so the 16-bit reads take it from the constant bank)
 };
 
 __device__ __forceinline__ int reflect101(int i, int n) {
@@ -1884,17 +1885,30 @@ __device__ __forceinline__ int reflect101(int i, int n) {
     return min(max(i, 0), n - 1);  // (only tile cells no output reads fall outside after the reflection)
 }
 
+// The level-0 intensity of a sample: (float)v, and for 16-bit samples (float)v * scale, scale = 2^-shift;
+// both are exact (v < 2^16), so v = P << shift gives the 8-bit plane P's intensities bit for bit.
+template <typename T>
+__device__ __forceinline__ float track_level0(T v, float scale) {
+    if constexpr (sizeof(T) == 1) return (float)v;
+    else return (float)v * scale;
+}
+
 // level l of image j (slot j % slots above level 0) at integer (x, y), clamped to the level's edge
+template <typename T>
 __device__ __forceinline__ float track_px(const TrackPyr& P, int l, int j, int x, int y) {
     x = min(max(x, 0), P.w[l] - 1);
     y = min(max(y, 0), P.h[l] - 1);
-    if (l == 0) return (float)__ldg(P.im.img0 + ((int64_t)j * P.im.h0 + y) * P.im.pitch0 + x);
+    if (l == 0) {
+        const T* row = reinterpret_cast<const T*>(P.im.img0 + ((int64_t)j * P.im.h0 + y) * P.im.pitch0);
+        return track_level0<T>(__ldg(row + x), P.scale);
+    }
     return __ldg(P.lvl[l] + ((int64_t)(j % P.slots) * P.h[l] + y) * P.w[l] + x);
 }
 
+template <typename T>
 __device__ __forceinline__ float track_bilinear(const TrackPyr& P, int l, int j, int x, int y, float ax, float ay) {
-    const float i00 = track_px(P, l, j, x, y), i01 = track_px(P, l, j, x + 1, y);
-    const float i10 = track_px(P, l, j, x, y + 1), i11 = track_px(P, l, j, x + 1, y + 1);
+    const float i00 = track_px<T>(P, l, j, x, y), i01 = track_px<T>(P, l, j, x + 1, y);
+    const float i10 = track_px<T>(P, l, j, x, y + 1), i11 = track_px<T>(P, l, j, x + 1, y + 1);
     return (1.f - ay) * ((1.f - ax) * i00 + ax * i01) + ay * ((1.f - ax) * i10 + ax * i11);
 }
 
@@ -1902,7 +1916,9 @@ __device__ __forceinline__ float track_bilinear(const TrackPyr& P, int l, int j,
 // (2*8 + 3) x (2*32 + 3) tile of level l (BORDER_REFLECT_101), blur its rows into shared memory, then
 // its columns: h = (s[-2] + s[2]) + 4 (s[-1] + s[1]) + 6 s[0] per row, the same over h per column, times
 // 1/256.
+// T: the type of the level-0 samples (uint8_t or uint16_t).
 constexpr int kPyrTX = 32, kPyrTY = 8;
+template <typename T>
 __global__ void __launch_bounds__(kPyrTX * kPyrTY) track_pyramid_kernel(TrackPyr P, int l, int j0) {
     constexpr int TH = 2 * kPyrTY + 3, TW = 2 * kPyrTX + 3;
     __shared__ float s_in[TH][TW];
@@ -1912,7 +1928,7 @@ __global__ void __launch_bounds__(kPyrTX * kPyrTY) track_pyramid_kernel(TrackPyr
     const int X0 = blockIdx.x * kPyrTX, Y0 = blockIdx.y * kPyrTY;
     for (int k = threadIdx.x; k < TH * TW; k += kPyrTX * kPyrTY) {
         const int r = k / TW, c = k % TW;
-        s_in[r][c] = track_px(P, l, j, reflect101(2 * X0 - 2 + c, w), reflect101(2 * Y0 - 2 + r, h));
+        s_in[r][c] = track_px<T>(P, l, j, reflect101(2 * X0 - 2 + c, w), reflect101(2 * Y0 - 2 + r, h));
     }
     __syncthreads();
     for (int k = threadIdx.x; k < TH * kPyrTX; k += kPyrTX * kPyrTY) {
@@ -1945,12 +1961,15 @@ __device__ __forceinline__ float track_warp_sum(float v) {
 // with), and the status becomes 2 unless u is kept and fb <= fb_max.
 // The forward instantiation writes neither fb_out nor reads fb_max.
 constexpr int kLkWarps = 4;
-template <bool kBack>
-__global__ void __launch_bounds__(kLkWarps * 32) track_lk_kernel(TrackPyr P, const int64_t* __restrict__ q_at,
-                                                                int f0, int f1, const double* __restrict__ pts,
-                                                                double* __restrict__ tracked,
-                                                                uint8_t* __restrict__ status, unsigned* flag,
-                                                                double fb_max, double* __restrict__ fb_out) {
+// Minimum blocks per SM in the launch bounds: 0 (none) for 8-bit samples; 7 (at most 72 registers) for
+// 16-bit samples, which ptxas otherwise fits in 64 registers with a spill.
+template <typename T>
+constexpr int kLkMinBlocks = sizeof(T) == 1 ? 0 : 7;
+template <typename T, bool kBack>
+__global__ void __launch_bounds__(kLkWarps * 32, kLkMinBlocks<T>)
+    track_lk_kernel(TrackPyr P, const int64_t* __restrict__ q_at, int f0, int f1, const double* __restrict__ pts,
+                    double* __restrict__ tracked, uint8_t* __restrict__ status, unsigned* flag, double fb_max,
+                    double* __restrict__ fb_out) {
     extern __shared__ float s_lk[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int win = P.im.window, r = win / 2, pw = win + 2, nw = win * win;
@@ -1981,7 +2000,7 @@ __global__ void __launch_bounds__(kLkWarps * 32) track_lk_kernel(TrackPyr P, con
         const int ix = (int)fx, iy = (int)fy;
         __syncwarp();  // the previous level's readers of sA are done
         for (int t = lane; t < pw * pw; t += 32)
-            sA[t] = track_bilinear(P, l, ja, ix + t % pw - r - 1, iy + t / pw - r - 1, wx, wy);
+            sA[t] = track_bilinear<T>(P, l, ja, ix + t % pw - r - 1, iy + t / pw - r - 1, wx, wy);
         __syncwarp();
         float gxx = 0.f, gxy = 0.f, gyy = 0.f;
         for (int t = lane; t < nw; t += 32) {
@@ -2015,7 +2034,7 @@ __global__ void __launch_bounds__(kLkWarps * 32) track_lk_kernel(TrackPyr P, con
             float bx = 0.f, by = 0.f;
             for (int t = lane; t < nw; t += 32) {
                 const int tx = t % win, ty = t / win;
-                const float B = track_bilinear(P, l, jb, bix + tx - r, biy + ty - r, bwx, bwy);
+                const float B = track_bilinear<T>(P, l, jb, bix + tx - r, biy + ty - r, bwx, bwy);
                 const float diff = sA[(ty + 1) * pw + tx + 1] - B;
                 bx += diff * sIx[t];
                 by += diff * sIy[t];
@@ -2118,7 +2137,9 @@ constexpr int kSelThreads = 256, kSelStrip = 32, kPickThreads = 1024;
 // and the row sums of their products.  The halo keeps every pixel a candidate's or its neighbours'
 // scores read inside the image, so reads outside it (clamped here) reach no used score.  Writes the
 // cell's best candidate as the key (score bits << 32) | ~(y * w + x): the greater key is the greater
-// score, then the smaller index; 0 = no candidate.
+// score, then the smaller index; 0 = no candidate.  The pixels are staged as the plane's samples (T) and
+// converted by track_level0 where the Sobel stencil reads them.
+template <typename T>
 __global__ void __launch_bounds__(kSelThreads) select_cells_kernel(TrackImages im, TrackSelect S, int j0) {
     extern __shared__ float s_sel[];
     const int C = S.cell, B = S.block, r = B / 2, hal = r + 2;
@@ -2129,23 +2150,25 @@ __global__ void __launch_bounds__(kSelThreads) select_cells_kernel(TrackImages i
     float* sHxx = sDy + GR * GW;  // GR x SW row sums of a strip
     float* sHxy = sHxx + GR * SW;
     float* sHyy = sHxy + GR * SW;
-    uint8_t* sP = reinterpret_cast<uint8_t*>(sHyy + GR * SW);  // PW x PW pixels from (X0 - hal, Y0 - hal)
+    T* sP = reinterpret_cast<T*>(sHyy + GR * SW);  // PW x PW samples from (X0 - hal, Y0 - hal)
     const int w = im.w0, h = im.h0;
     const int X0 = (blockIdx.x % S.cells_x) * C, Y0 = (blockIdx.x / S.cells_x) * C;
     const uint8_t* img = im.img0 + (int64_t)(j0 + blockIdx.y) * h * im.pitch0;
     for (int t = threadIdx.x; t < PW * PW; t += kSelThreads) {
         const int y = min(max(Y0 - hal + t / PW, 0), h - 1), x = min(max(X0 - hal + t % PW, 0), w - 1);
-        sP[t] = __ldg(img + (int64_t)y * im.pitch0 + x);
+        sP[t] = __ldg(reinterpret_cast<const T*>(img + (int64_t)y * im.pitch0) + x);
     }
-    const float sc = (float)(1.0 / (4.0 * B * 255.0));
+    const float sc = (float)(1.0 / (4.0 * B * 255.0)), scale = ldexpf(1.f, -im.shift);
     __syncthreads();
     for (int s0 = 0; s0 < SW; s0 += kSelStrip) {
         const int nr = min(kSelStrip, SW - s0), gr = nr + 2 * r;
         // gradient row t, column u <-> (X0 - 1 - r + u, Y0 - 1 - r + s0 + t), pixel row s0 + t + 1, column u + 1
         for (int t = threadIdx.x; t < gr * GW; t += kSelThreads) {
-            const uint8_t* c = sP + (s0 + t / GW + 1) * PW + t % GW + 1;
-            const float i00 = c[-PW - 1], i01 = c[-PW], i02 = c[-PW + 1], i10 = c[-1], i12 = c[1];
-            const float i20 = c[PW - 1], i21 = c[PW], i22 = c[PW + 1];
+            const T* c = sP + (s0 + t / GW + 1) * PW + t % GW + 1;
+            const float i00 = track_level0<T>(c[-PW - 1], scale), i01 = track_level0<T>(c[-PW], scale);
+            const float i02 = track_level0<T>(c[-PW + 1], scale), i10 = track_level0<T>(c[-1], scale);
+            const float i12 = track_level0<T>(c[1], scale), i20 = track_level0<T>(c[PW - 1], scale);
+            const float i21 = track_level0<T>(c[PW], scale), i22 = track_level0<T>(c[PW + 1], scale);
             sDx[t] = (((i02 - i00) + 2.f * (i12 - i10)) + (i22 - i20)) * sc;
             sDy[t] = (((i20 - i00) + 2.f * (i21 - i01)) + (i22 - i02)) * sc;
         }
@@ -2931,6 +2954,7 @@ TrackPyr track_pyr(const TrackImages& im, float* d_pyr, int slots) {
     TrackPyr P{};
     P.im = im;
     P.slots = slots;
+    P.scale = std::ldexp(1.f, -im.shift);
     P.w[0] = im.w0;
     P.h[0] = im.h0;
     size_t at = 0;
@@ -2954,38 +2978,39 @@ size_t track_pyramid_floats(int w0, int h0, int levels) {
     return n;
 }
 
-size_t track_select_smem(int cell, int block) {
+size_t track_select_smem(int cell, int block, int sample) {
     const int r = block / 2, PW = cell + 2 * (r + 2), SW = cell + 2, GW = SW + 2 * r, GR = kSelStrip + 2 * r;
-    return ((size_t)SW * SW + 2 * (size_t)GR * GW + 3 * (size_t)GR * SW) * sizeof(float) + (size_t)PW * PW;
+    return ((size_t)SW * SW + 2 * (size_t)GR * GW + 3 * (size_t)GR * SW) * sizeof(float) + (size_t)PW * PW * sample;
 }
 
-void launch_track_frames(const TrackImages& im, int n_frames, const int64_t* h_q_at, int64_t* d_q_at,
-                         double* d_points, float* d_pyr, int slots, double* d_tracked, uint8_t* d_status,
-                         unsigned* d_flag, const TrackExtra& ex, cudaStream_t st) {
-    if (n_frames <= 0) return;
+namespace {
+template <typename T>
+void launch_track_frames_t(const TrackImages& im, int n_frames, const int64_t* h_q_at, int64_t* d_q_at,
+                           double* d_points, float* d_pyr, int slots, double* d_tracked, uint8_t* d_status,
+                           unsigned* d_flag, const TrackExtra& ex, cudaStream_t st) {
     const TrackPyr P = track_pyr(im, d_pyr, slots);
     const int pw = im.window + 2;
     const size_t smem = (size_t)kLkWarps * (pw * pw + 2 * im.window * im.window) * sizeof(float);
-    allow_smem(track_lk_kernel<false>, smem);
+    allow_smem(track_lk_kernel<T, false>, smem);
     const bool back = ex.fb_max > 0.0;
-    if (back) allow_smem(track_lk_kernel<true>, smem);
+    if (back) allow_smem(track_lk_kernel<T, true>, smem);
     const TrackSelect* S = ex.sel;
-    const size_t sel_smem = S ? track_select_smem(S->cell, S->block) : 0;
-    if (S) allow_smem(select_cells_kernel, sel_smem);
+    const size_t sel_smem = S ? track_select_smem(S->cell, S->block, (int)sizeof(T)) : 0;
+    if (S) allow_smem(select_cells_kernel<T>, sel_smem);
     // chunk: build the pyramids of images [built, e), then track frames [f0, e - 1); image f0 is the
     // last one of the previous chunk, still in its slot
     for (int f0 = 0, built = 0; f0 < n_frames;) {
         const int e = std::min(n_frames + 1, f0 + slots);
         for (int l = 0; l + 1 < im.levels && e > built; ++l) {
             const dim3 grid((P.w[l + 1] + kPyrTX - 1) / kPyrTX, (P.h[l + 1] + kPyrTY - 1) / kPyrTY, e - built);
-            track_pyramid_kernel<<<grid, kPyrTX * kPyrTY, 0, st>>>(P, l, built);
+            track_pyramid_kernel<T><<<grid, kPyrTX * kPyrTY, 0, st>>>(P, l, built);
             g_launches += 1;
         }
         // selection on the chunk's side-a images f0 .. e - 2; the tracker's grid then covers the bound
         // max_points per frame and its warps past q_at[e - 1] return at once
         const int nf = e - 1 - f0;
         if (S) {
-            select_cells_kernel<<<dim3(S->cells_x * S->cells_y, nf), kSelThreads, sel_smem, st>>>(im, *S, f0);
+            select_cells_kernel<T><<<dim3(S->cells_x * S->cells_y, nf), kSelThreads, sel_smem, st>>>(im, *S, f0);
             select_points_kernel<<<nf, kPickThreads, 0, st>>>(*S);
             select_prefix_kernel<<<1, kPickThreads, 0, st>>>(*S, d_q_at, f0, e - 1, im.w0, d_points);
             g_launches += 3;
@@ -2993,18 +3018,32 @@ void launch_track_frames(const TrackImages& im, int n_frames, const int64_t* h_q
         const int64_t pts = S ? (int64_t)nf * S->max_points : h_q_at[e - 1] - h_q_at[f0];
         if (pts > 0) {
             const unsigned blocks = (unsigned)((pts + kLkWarps - 1) / kLkWarps);
-            track_lk_kernel<false><<<blocks, kLkWarps * 32, smem, st>>>(P, d_q_at, f0, e - 1, d_points, d_tracked,
-                                                                       d_status, d_flag, 0.0, nullptr);
+            track_lk_kernel<T, false><<<blocks, kLkWarps * 32, smem, st>>>(P, d_q_at, f0, e - 1, d_points, d_tracked,
+                                                                          d_status, d_flag, 0.0, nullptr);
             g_launches += 1;
             if (back) {
-                track_lk_kernel<true><<<blocks, kLkWarps * 32, smem, st>>>(P, d_q_at, f0, e - 1, d_points, d_tracked,
-                                                                          d_status, d_flag, ex.fb_max, ex.d_fb);
+                track_lk_kernel<T, true><<<blocks, kLkWarps * 32, smem, st>>>(P, d_q_at, f0, e - 1, d_points,
+                                                                             d_tracked, d_status, d_flag, ex.fb_max,
+                                                                             ex.d_fb);
                 g_launches += 1;
             }
         }
         built = e;
         f0 = e - 1;
     }
+}
+}  // namespace
+
+void launch_track_frames(const TrackImages& im, int n_frames, const int64_t* h_q_at, int64_t* d_q_at,
+                         double* d_points, float* d_pyr, int slots, double* d_tracked, uint8_t* d_status,
+                         unsigned* d_flag, const TrackExtra& ex, cudaStream_t st) {
+    if (n_frames <= 0) return;
+    if (im.sample == 2)
+        launch_track_frames_t<uint16_t>(im, n_frames, h_q_at, d_q_at, d_points, d_pyr, slots, d_tracked, d_status,
+                                        d_flag, ex, st);
+    else
+        launch_track_frames_t<uint8_t>(im, n_frames, h_q_at, d_q_at, d_points, d_pyr, slots, d_tracked, d_status,
+                                       d_flag, ex, st);
 }
 
 void launch_track_compact(const int64_t* d_q_at, int n_frames, const double* d_points, const double* d_tracked,

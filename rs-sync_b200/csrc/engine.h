@@ -209,11 +209,13 @@ void launch_stage_row_fractions(const int64_t* d_at, const double* d_frame_ts, i
 // The arithmetic is the contract stated at rssync_track_frames_device in include/rssync_b200.h.
 constexpr int kTrackMaxLevels = 6;
 struct TrackImages {
-    const uint8_t* img0;  // n_frames + 1 luma planes: row y of image j at img0 + (j * h0 + y) * pitch0
+    const uint8_t* img0;  // n_frames + 1 luma planes: row y of image j at img0 + (j * h0 + y) * pitch0 bytes
     int64_t pitch0;
     int w0, h0;
     int levels, window, max_iters;
     float epsilon, min_eig;
+    uint8_t sample;  // bytes per sample: 1 (uint8_t, level 0 = (float)v) or 2 (uint16_t)
+    uint8_t shift;   // 16-bit samples: level 0 = (float)v * 2^-shift, shift 0..8
 };
 // floats of one image's pyramid levels 1 .. levels - 1
 size_t track_pyramid_floats(int w0, int h0, int levels);
@@ -243,14 +245,14 @@ struct TrackExtra {
     double fb_max;
     double* d_fb;
 };
-// Shared memory of one select_cells_kernel block
-size_t track_select_smem(int cell, int block);
+// Shared memory of one select_cells_kernel block staging `sample`-byte pixels
+size_t track_select_smem(int cell, int block, int sample);
 // Tracks every query point of frame i (d_points[2 d_q_at[i] ..], host copy h_q_at) from image i to
 // image i + 1, for i in [0, n_frames).  The pyramids of `slots` (>= 2) images live in d_pyr at once
 // (slots * track_pyramid_floats floats): the images are processed in chunks, image j in slot j % slots,
 // each pyramid built once.  Per point: d_tracked (2 doubles) and d_status (1 = kept); *d_flag gets bit 0
 // when a query point is not finite.  ex: selection and the backward pass (TrackExtra); with ex.sel null
-// and ex.fb_max 0 the launches are the forward tracker's alone.
+// and ex.fb_max 0 the launches are the forward tracker's alone.  im.sample picks the kernels' pixel type.
 void launch_track_frames(const TrackImages& im, int n_frames, const int64_t* h_q_at, int64_t* d_q_at,
                          double* d_points, float* d_pyr, int slots, double* d_tracked, uint8_t* d_status,
                          unsigned* d_flag, const TrackExtra& ex, cudaStream_t st);

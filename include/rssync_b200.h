@@ -251,6 +251,49 @@ int rssync_track_frames16_device(rssync_problem* p, size_t n_frames, const int64
                                  const rssync_lens* lens, const rssync_track_params* params,
                                  const rssync_track_options* options, double* points_out, size_t* counts_out,
                                  double* tracked_out, uint8_t* status_out, double* fb_out, void* stream);
+/* The caller's mask of rssync_track_frames_masked_device: row y of image j's mask at
+ * mask + j * image_stride + y * pitch bytes. */
+typedef struct rssync_track_mask {
+    const uint8_t* mask;  /* device memory of the problem's device; nonzero = a point may lie here */
+    size_t pitch;         /* bytes per mask row, >= width */
+    size_t image_stride;  /* bytes from image j's mask to image j + 1's; 0 = one mask for all n_frames + 1 images */
+    int margin;           /* px, 0..63 */
+} rssync_track_mask;
+/* rssync_track_frames_ex_device (sample_bytes 1, shift 0) or rssync_track_frames16_device (sample_bytes 2,
+ * shift 0..8) that keeps points out of the regions the caller's mask excludes: burned-in overlays, parts of
+ * the rig in view, independently moving objects.  images, pitch (bytes) and every other argument as there.
+ *  - Eligibility: pixel (x, y) of image j is eligible iff every mask pixel (x', y') of image j with
+ *    |x' - x| <= margin and |y' - y| <= margin that lies inside the image is nonzero; pixels outside the
+ *    image count as usable (cv2.erode of (mask != 0) by a (2 margin + 1)^2 square, default border).  A
+ *    position (x, y) in double is looked up at its nearest pixel (floor(x + 0.5), floor(y + 0.5)).  The
+ *    margin keeps the level-0 structure-tensor block and LK window of a point off the excluded region (the
+ *    side-a patch is window / 2 + 1 px); it is not scaled per pyramid level.
+ *  - Selection: a candidate must also be eligible on image i; the rest of the selection contract applies to
+ *    eligible candidates only (a cell's pick, the maximum M behind the quality threshold, the max_points
+ *    cut), and a cell without an eligible candidate has no pick.
+ *  - Status 3 (masked): a point gets status 3 exactly where the unmasked forward tracker gives status 1 and
+ *    its query point is not eligible on image i or its tracked position is not eligible on image i + 1.
+ *    tracked_out holds the forward position; a status-3 point takes no part in the backward pass, its fb_out
+ *    is NaN, and it is not ingested.
+ * Identities: mask == NULL gives byte for byte what rssync_track_frames_ex_device (sample_bytes 1) or
+ * rssync_track_frames16_device (sample_bytes 2) gives: every output, frame table, arena, row fractions and
+ * re-timing table; so does a mask that is nonzero everywhere, for any margin.  On the caller's points,
+ * tracked_out equals the unmasked call's and the statuses differ only as 1 -> 3.  The kept points (status 1)
+ * give exactly what rssync_set_track_pixels_device gives on them, as stated at rssync_track_frames_device.
+ * A shared mask is eroded once per call; per-image masks are eroded with the pyramids, and their planes
+ * (width * height bytes per image) count against the 256 MiB of chunk scratch; the chunks change no result.
+ * Multi-device problems: the mask lies on the primary, which ingests, as for the other tracking forms.
+ * Checked before anything is applied, besides the checks of rssync_track_frames_ex_device /
+ * rssync_track_frames16_device: RSSYNC_E_INVALID for sample_bytes other than 1 or 2, a nonzero shift with
+ * sample_bytes 1, a mask buffer that is not device memory of the problem's device, mask pitch < width, margin
+ * outside 0..63, and a nonzero image_stride below height * pitch. */
+int rssync_track_frames_masked_device(rssync_problem* p, size_t n_frames, const int64_t* frames,
+                                      const size_t* counts, const double* image_ts, const double* points,
+                                      const void* images, size_t pitch /* bytes */, int width, int height,
+                                      int sample_bytes /* 1 or 2 */, int shift, const rssync_track_mask* mask,
+                                      const rssync_lens* lens, const rssync_track_params* params,
+                                      const rssync_track_options* options, double* points_out, size_t* counts_out,
+                                      double* tracked_out, uint8_t* status_out, double* fb_out, void* stream);
 /* SetTrackResult for n_frames frames whose rays the caller computed (any camera model), with the
  * rolling-shutter timestamps formed here from per-ray row fractions.  Ray k of frame i gets
  * ts_a = frame_ts_a[i] + readout * frac_a[k] (ts_b alike): one multiply and one add, not contracted,

@@ -46,7 +46,7 @@ C_ABI_SYMBOLS = [
     "rssync_set_track_row_fractions", "rssync_set_track_row_fractions_device",
     "rssync_retime_table", "rssync_row_fraction_plane", "rssync_adopt_row_fractions",
     "rssync_readout_search_windows", "rssync_rotation_search_windows", "rssync_track_frames_device",
-    "rssync_track_frames_ex_device", "rssync_track_frames16_device",
+    "rssync_track_frames_ex_device", "rssync_track_frames16_device", "rssync_track_frames_masked_device",
 ]
 # Itanium-ABI symbols of the C++ drop-in face (same set the reference's librssync_core exports)
 CXX_ABI_SYMBOLS = [
@@ -108,7 +108,16 @@ class TrackOptions(C.Structure):
         super().__init__(cell, block, quality, max_points, fb_max)
 
 
+class TrackMask(C.Structure):
+    """rssync_track_mask: the caller's mask of track_frames_ex (mask=)"""
+    _fields_ = [("mask", C.c_void_p), ("pitch", C.c_size_t), ("image_stride", C.c_size_t), ("margin", C.c_int)]
+
+
 TrackResult = collections.namedtuple("TrackResult", "points counts tracked status fb_error")
+TrackResult.__doc__ = """The result of SyncProblem.track_frames_ex: query points, counts per frame, tracked positions,
+statuses and forward-backward distances.  Status: 0 lost, 1 kept and ingested, 2 rejected by the backward check,
+3 masked (kept by the forward tracker, but its query point or tracked position lies off the eligible region of the
+mask: not ingested, no backward pass, fb_error NaN)."""
 
 
 def grid_points(width, height, step):
@@ -195,6 +204,10 @@ def load_library():
                                                C.c_size_t, C.c_int, C.c_int, C.c_int, C.POINTER(Lens),
                                                C.POINTER(TrackParams), C.POINTER(TrackOptions), P,
                                                C.POINTER(C.c_size_t), P, P, P, P]
+    L.rssync_track_frames_masked_device.argtypes = [P, C.c_size_t, c_i64_p, C.POINTER(C.c_size_t), c_double_p, P,
+                                                    P, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_int,
+                                                    C.POINTER(TrackMask), C.POINTER(Lens), C.POINTER(TrackParams),
+                                                    C.POINTER(TrackOptions), P, C.POINTER(C.c_size_t), P, P, P, P]
     L.rssync_presync.argtypes = [P, C.c_double, C.c_int64, C.c_int64, C.c_double, C.c_double, c_double_p, c_double_p]
     L.rssync_sync.argtypes = [P, C.c_double, C.c_int64, C.c_int64, C.c_double, C.c_double, c_double_p, c_double_p]
     L.rssync_debug_presync.argtypes = [P, C.c_double, C.c_int64, C.c_int64, C.c_double, c_double_p, c_double_p, C.c_int]
@@ -640,17 +653,23 @@ class SyncProblem:
         return tracked, status
 
     def track_frames_ex(self, frames, image_ts, images, lens, params=None, options=None, points=None, counts=None,
-                        shift=None):
+                        shift=None, mask=None, mask_margin=None):
         """track_frames with the query points selected on the device (points and counts None) and the
         forward-backward check (rssync_track_frames_ex_device).  images, frames, image_ts, lens and params as in
         track_frames; options: TrackOptions or None (the defaults: 128-px cells, block 5, quality 0.01, 512
         points per frame, fb_max 1 px).  Returns TrackResult(points, counts, tracked, status, fb_error): the
         query points, tracked positions (CUDA float64 (n, 2)), statuses (CUDA uint8 (n,): 0 lost, 1 kept and
-        ingested, 2 rejected by the backward check) and forward-backward distances (CUDA float64 (n,), NaN
-        where the backward pass did not keep the point or did not run), n = sum(counts); counts: numpy.
+        ingested, 2 rejected by the backward check, 3 masked) and forward-backward distances (CUDA float64 (n,),
+        NaN where the backward pass did not keep the point or did not run), n = sum(counts); counts: numpy.
         16-bit planes (rssync_track_frames16_device): a torch.uint16 tensor with shift, the intensity being
         sample * 2^-shift: 8 for P010 / P016, 2 for 10-bit and 4 for 12-bit samples in the low bits.  shift
-        is required for uint16 and must be None for uint8."""
+        is required for uint16 and must be None for uint8.
+        mask (rssync_track_frames_masked_device): a CUDA bool or uint8 tensor on the images' device with
+        contiguous rows, nonzero where points may lie: (H, W) for one mask shared by every image, or
+        (n_frames + 1, H, W) for one per image (an expanded tensor, stride(0) = 0, is shared).  The mask is
+        eroded by mask_margin px (default params.window // 2 + 1, the level-0 LK patch): selection takes
+        eligible candidates only, and a tracked point whose start or end is not eligible gets status 3.  With
+        mask None the call is exactly the unmasked one."""
         import torch
         fr = np.ascontiguousarray(frames, dtype=np.int64)
         ts = _f64(image_ts)
@@ -702,12 +721,33 @@ class SyncProblem:
                 images.shape[1])
         tail = (C.byref(lens_c), prm, C.byref(opt), ptr(pts_out), counts_out.ctypes.data_as(C.POINTER(C.c_size_t)),
                 ptr(tracked), ptr(status), ptr(fb), stream)
-        if wide:
+        if mask is not None:
+            tm = self._track_mask(mask, images, params, mask_margin)
+            self._check(self.L.rssync_track_frames_masked_device(*head, 2 if wide else 1, int(shift or 0),
+                                                                 C.byref(tm), *tail))
+        elif mask_margin is not None:
+            raise ValueError("track_frames_ex: mask_margin needs a mask")
+        elif wide:
             self._check(self.L.rssync_track_frames16_device(*head, int(shift), *tail))
         else:
             self._check(self.L.rssync_track_frames_ex_device(*head, *tail))
         n = int(counts_out.sum())
         return TrackResult(pts_out[:n], counts_out.astype(np.int64), tracked[:n], status[:n], fb[:n])
+
+    @staticmethod
+    def _track_mask(mask, images, params, margin):
+        """track_frames_ex's mask tensor as an rssync_track_mask"""
+        import torch
+        if not getattr(mask, "is_cuda", False) or mask.device != images.device:
+            raise ValueError(f"track_frames_ex: the mask must be a CUDA tensor on the images' device {images.device}")
+        n, h, w = images.shape
+        if mask.dtype not in (torch.bool, torch.uint8) or mask.stride(-1) != 1 or \
+                tuple(mask.shape) not in ((h, w), (n, h, w)):
+            raise ValueError(f"track_frames_ex: the mask must be a bool or uint8 tensor ({h}, {w}) or ({n}, {h}, {w}) "
+                             f"with contiguous rows, got {mask.dtype} {tuple(mask.shape)}")
+        if margin is None:
+            margin = (TrackParams() if params is None else params).window // 2 + 1
+        return TrackMask(mask.data_ptr(), mask.stride(-2), mask.stride(0) if mask.dim() == 3 else 0, int(margin))
 
     def load(self, w, bulk=False):
         """Feed a synth.Workload the way core_testcode feeds a video (core_testcode.cpp:257-268)."""

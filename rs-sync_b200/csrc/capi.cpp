@@ -344,6 +344,8 @@ struct rssync_problem {
     DevBuf<uint32_t> d_trk_picks;
     DevBuf<int32_t> d_trk_count;
     PinBuf<int64_t> h_trk_qat;
+    // rssync_track_frames_masked_device: the eligibility planes (one, or one per pyramid slot)
+    DevBuf<uint8_t> d_trk_elig;
 
     std::vector<std::pair<double, int32_t>> sort_scratch;
     std::vector<double> trace_delay, trace_step;
@@ -2653,12 +2655,12 @@ struct TrackOutputs {
 
 // The body of the tracking entry points once their null checks have passed.  opt null: the plain form
 // (caller's points, no backward pass, no options checked).  sample: bytes per sample of the planes, 1
-// (uint8) or 2 (uint16, level 0 = v * 2^-shift).
+// (uint8) or 2 (uint16, level 0 = v * 2^-shift).  mask null: no mask.
 int track_frames(rssync_problem* p, size_t n_frames, const int64_t* frames, const size_t* counts,
                  const double* image_ts, const double* points, const void* images, size_t pitch, int width,
                  int height, const rssync_lens* lens, const rssync_track_params* params,
                  const rssync_track_options* opt, const TrackOutputs& out, void* stream, int sample = 1,
-                 int shift = 0) {
+                 int shift = 0, const rssync_track_mask* mask = nullptr) {
     const rssync_track_params tp = params ? *params : rssync_track_params{3, 21, 30, 0.01, 1e-4};
     if (tp.levels < 1 || tp.levels > 6 || tp.window < 5 || tp.window > 63 || tp.window % 2 == 0 || tp.max_iters < 1 ||
         tp.max_iters > 100 || !(tp.epsilon >= 0.0) || !std::isfinite(tp.epsilon) || !(tp.min_eig >= 0.0) ||
@@ -2717,17 +2719,32 @@ int track_frames(rssync_problem* p, size_t n_frames, const int64_t* frames, cons
     for (void* o : {(void*)out.points, (void*)out.tracked, (void*)out.status, (void*)out.fb})
         if (o && total)
             if (int rc = check_device_pointer(p, o, "an output buffer")) return rc;
+    if (mask) {
+        if (int rc = check_device_pointer(p, mask->mask, "mask")) return rc;
+        const char* bad = mask->pitch < (size_t)width ? "track-frames: mask pitch below width"
+                          : mask->margin < 0 || mask->margin > rs::kTrackMaxMargin
+                              ? "track-frames: mask margin outside 0..63"
+                          : mask->image_stride && mask->image_stride / mask->pitch < (size_t)height
+                              ? "track-frames: mask image_stride below height * pitch"
+                              : nullptr;
+        if (bad) {
+            p->err = bad;
+            return RSSYNC_E_INVALID;
+        }
+    }
     if (int rc = check_frame_ts(p, n_frames, image_ts, image_ts + 1)) return rc;
 
     const size_t per_image = rs::track_pyramid_floats(width, height, tp.levels);
     const size_t n_images = n_frames + 1;
-    size_t slots = per_image ? std::min(n_images, std::max<size_t>(2, kTrackScratchBytes / (4 * per_image)))
-                             : n_images;
+    const size_t plane = (size_t)width * height;
+    const bool mask_per_image = mask && mask->image_stride;
+    // bytes of one slot: its pyramid, the selection's scratch and a per-image mask's eligibility plane
     const size_t n_cells = (size_t)sel.cells_x * sel.cells_y;
-    if (select) {  // the selection's scratch per image counts against the same budget
-        const size_t bytes = 4 * per_image + 8 * n_cells + 4 * (size_t)sel.max_points + 4;
-        slots = std::min({n_images, std::max<size_t>(2, kTrackScratchBytes / bytes), size_t(65536)});
-    }
+    const size_t bytes = 4 * per_image + (select ? 8 * n_cells + 4 * (size_t)sel.max_points + 4 : 0) +
+                         (mask_per_image ? plane : 0);
+    size_t slots = bytes ? std::min(n_images, std::max<size_t>(2, kTrackScratchBytes / bytes)) : n_images;
+    if (select) slots = std::min(slots, size_t(65536));
+    if (mask_per_image) slots = std::min(slots, size_t(65535));  // (the erosion's grid.z)
     const double fb_max = opt ? opt->fb_max : 0.0;
     CUDA_TRY(p, cudaSetDevice(p->device));
     CUDA_TRY(p, p->d_trk_pyr.reserve(std::max<size_t>(1, slots * per_image)));
@@ -2746,6 +2763,12 @@ int track_frames(rssync_problem* p, size_t n_frames, const int64_t* frames, cons
         sel.d_picks = p->d_trk_picks.ptr;
         sel.d_count = p->d_trk_count.ptr;
     }
+    rs::TrackMask tm{};
+    if (mask) {
+        CUDA_TRY(p, p->d_trk_elig.reserve((mask_per_image ? slots : 1) * plane));
+        tm = rs::TrackMask{mask->mask, (int64_t)mask->pitch, (int64_t)mask->image_stride, mask->margin,
+                           p->d_trk_elig.ptr};
+    }
     double* d_a = p->d_trk_pts.ptr;
     double* d_b = d_a + 2 * total;
     double* d_tracked = out.tracked ? out.tracked : d_b + 2 * total;
@@ -2756,7 +2779,7 @@ int track_frames(rssync_problem* p, size_t n_frames, const int64_t* frames, cons
     const rs::TrackImages im{static_cast<const uint8_t*>(images), (int64_t)pitch, width, height, tp.levels,
                              tp.window, tp.max_iters, (float)tp.epsilon, (float)tp.min_eig, (uint8_t)sample,
                              (uint8_t)shift};
-    const rs::TrackExtra ex{select ? &sel : nullptr, fb_max, out.fb};
+    const rs::TrackExtra ex{select ? &sel : nullptr, fb_max, out.fb, mask ? &tm : nullptr};
     DevicePointSource src;
     // s.d_at holds the query offsets (begin_device_staging; in selection mode the bound, overwritten on
     // the device by the selected offsets); s.h_at receives the kept ones
@@ -2794,13 +2817,13 @@ int track_frames(rssync_problem* p, size_t n_frames, const int64_t* frames, cons
                                 stream, &src);
 }
 
-// The ex entry points (rssync_track_frames_ex_device, rssync_track_frames16_device): their null checks and
-// default options, then track_frames
+// The ex entry points (rssync_track_frames_ex_device, rssync_track_frames16_device,
+// rssync_track_frames_masked_device): their null checks and default options, then track_frames
 int track_frames_ex(rssync_problem* p, size_t n_frames, const int64_t* frames, const size_t* counts,
                     const double* image_ts, const double* points, const void* images, size_t pitch, int width,
                     int height, const rssync_lens* lens, const rssync_track_params* params,
                     const rssync_track_options* options, const TrackOutputs& out, void* stream, int sample,
-                    int shift) {
+                    int shift, const rssync_track_mask* mask = nullptr) {
     if (!p) return RSSYNC_E_INVALID;
     if (n_frames == 0) return RSSYNC_OK;
     if (!frames || !image_ts || !lens || n_frames > (size_t)INT32_MAX - 1) return RSSYNC_E_INVALID;
@@ -2810,7 +2833,7 @@ int track_frames_ex(rssync_problem* p, size_t n_frames, const int64_t* frames, c
     }
     const rssync_track_options opt = options ? *options : rssync_track_options{128, 5, 0.01, 512, 1.0};
     return track_frames(p, n_frames, frames, counts, image_ts, points, images, pitch, width, height, lens, params,
-                        &opt, out, stream, sample, shift);
+                        &opt, out, stream, sample, shift, mask);
 }
 
 }  // namespace
@@ -2876,6 +2899,26 @@ int rssync_track_frames16_device(rssync_problem* p, size_t n_frames, const int64
     return track_frames_ex(p, n_frames, frames, counts, image_ts, points, images, pitch, width, height, lens, params,
                            options, TrackOutputs{points_out, counts_out, tracked_out, status_out, fb_out}, stream, 2,
                            shift);
+}
+
+// rssync_track_frames_ex_device (sample_bytes 1) or rssync_track_frames16_device (sample_bytes 2) with the
+// caller's mask: selection takes eligible candidates only, and points kept forward off the eligible region get
+// status 3 and are not ingested
+int rssync_track_frames_masked_device(rssync_problem* p, size_t n_frames, const int64_t* frames, const size_t* counts,
+                                      const double* image_ts, const double* points, const void* images, size_t pitch,
+                                      int width, int height, int sample_bytes, int shift,
+                                      const rssync_track_mask* mask, const rssync_lens* lens,
+                                      const rssync_track_params* params, const rssync_track_options* options,
+                                      double* points_out, size_t* counts_out, double* tracked_out,
+                                      uint8_t* status_out, double* fb_out, void* stream) {
+    RS_NVTX_RANGE();
+    if (p && n_frames && (sample_bytes < 1 || sample_bytes > 2 || (sample_bytes == 1 && shift != 0))) {
+        p->err = "track-frames: sample_bytes must be 1 or 2, and shift 0 with 1-byte samples";
+        return RSSYNC_E_INVALID;
+    }
+    return track_frames_ex(p, n_frames, frames, counts, image_ts, points, images, pitch, width, height, lens, params,
+                           options, TrackOutputs{points_out, counts_out, tracked_out, status_out, fb_out}, stream,
+                           sample_bytes, shift, mask);
 }
 
 }  // extern "C"

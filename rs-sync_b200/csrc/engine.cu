@@ -1946,6 +1946,57 @@ __global__ void __launch_bounds__(kPyrTX * kPyrTY) track_pyramid_kernel(TrackPyr
     }
 }
 
+// Eligibility planes of the caller's mask (rssync_track_frames_masked_device): image j's byte of pixel
+// (x, y) at plane + (j % slots) * stride + y * w0 + x, 1 = eligible (stride 0: one plane for every image).
+// The unmasked kernels take it as their last parameter and never read it, so their other parameters keep
+// their offsets.
+struct TrackElig {
+    const uint8_t* plane;
+    int64_t stride;
+    int slots;
+};
+
+// whether the position (x, y) of image j is eligible, looked up at its nearest pixel (floor(x + 0.5),
+// floor(y + 0.5)); (x, y) lies in [0, w0 - 1] x [0, h0 - 1]
+__device__ __forceinline__ bool track_eligible(const TrackElig& E, int w0, int j, double x, double y) {
+    const int ix = (int)floor(x + 0.5), iy = (int)floor(y + 0.5);
+    return E.plane[(int64_t)(j % E.slots) * E.stride + (int64_t)iy * w0 + ix] != 0;
+}
+
+// Erosion of images [j0, j0 + gridDim.z) of the mask by a (2 m + 1)^2 square (cv2.erode of mask != 0, pixels
+// outside the image usable): a block's kErTX x kErTY outputs read a (kErTY + 2m) x (kErTX + 2m) tile, AND
+// its rows over 2m + 1 columns into shared memory, then the columns over 2m + 1 rows.
+constexpr int kErTX = 64, kErTY = 32;
+__global__ void __launch_bounds__(256) track_erode_kernel(TrackMask M, int w, int h, int j0, TrackElig E) {
+    constexpr int MH = kErTY + 2 * kTrackMaxMargin, MW = kErTX + 2 * kTrackMaxMargin;
+    __shared__ uint8_t s_in[MH][MW];
+    __shared__ uint8_t s_row[MH][kErTX];
+    const int m = M.margin, th = kErTY + 2 * m, tw = kErTX + 2 * m;
+    const int j = j0 + blockIdx.z;
+    const int X0 = blockIdx.x * kErTX - m, Y0 = blockIdx.y * kErTY - m;
+    const uint8_t* mask = M.mask + (int64_t)j * M.image_stride;
+    for (int k = threadIdx.x; k < th * tw; k += blockDim.x) {
+        const int r = k / tw, c = k % tw, x = X0 + c, y = Y0 + r;
+        s_in[r][c] = x < 0 || x >= w || y < 0 || y >= h || mask[(int64_t)y * M.pitch + x] != 0;
+    }
+    __syncthreads();
+    for (int k = threadIdx.x; k < th * kErTX; k += blockDim.x) {
+        const int r = k / kErTX, c = k % kErTX;
+        uint8_t v = 1;
+        for (int i = 0; i <= 2 * m; ++i) v &= s_in[r][c + i];
+        s_row[r][c] = v;
+    }
+    __syncthreads();
+    uint8_t* out = const_cast<uint8_t*>(E.plane) + (int64_t)(j % E.slots) * E.stride;
+    for (int k = threadIdx.x; k < kErTY * kErTX; k += blockDim.x) {
+        const int r = k / kErTX, c = k % kErTX, x = X0 + m + c, y = Y0 + m + r;
+        if (x >= w || y >= h) continue;
+        uint8_t v = 1;
+        for (int i = 0; i <= 2 * m; ++i) v &= s_row[r + i][c];
+        out[(int64_t)y * w + x] = v;
+    }
+}
+
 // sum over the 32 lanes: xor butterfly 16, 8, 4, 2, 1 (every lane ends with the same bits)
 __device__ __forceinline__ float track_warp_sum(float v) {
 #pragma unroll
@@ -1960,16 +2011,19 @@ __device__ __forceinline__ float track_warp_sum(float v) {
 // fb = |u - pts[k]| (double) in fb_out[k] when u is kept (lost: fb_out[k] keeps the NaN it was filled
 // with), and the status becomes 2 unless u is kept and fb <= fb_max.
 // The forward instantiation writes neither fb_out nor reads fb_max.
+// kMask (forward only): a point kept forward gets status 3 instead of 1 when its query position is not
+// eligible on image i or its tracked position is not eligible on image i + 1 (E).
 constexpr int kLkWarps = 4;
 // Minimum blocks per SM in the launch bounds: 0 (none) for 8-bit samples; 7 (at most 72 registers) for
 // 16-bit samples, which ptxas otherwise fits in 64 registers with a spill.
 template <typename T>
 constexpr int kLkMinBlocks = sizeof(T) == 1 ? 0 : 7;
-template <typename T, bool kBack>
+template <typename T, bool kBack, bool kMask = false>
 __global__ void __launch_bounds__(kLkWarps * 32, kLkMinBlocks<T>)
     track_lk_kernel(TrackPyr P, const int64_t* __restrict__ q_at, int f0, int f1, const double* __restrict__ pts,
                     double* __restrict__ tracked, uint8_t* __restrict__ status, unsigned* flag, double fb_max,
-                    double* __restrict__ fb_out) {
+                    double* __restrict__ fb_out, TrackElig E) {
+    static_assert(!(kBack && kMask), "the backward pass runs on status 1 only and takes no mask");
     extern __shared__ float s_lk[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int win = P.im.window, r = win / 2, pw = win + 2, nw = win * win;
@@ -2069,7 +2123,12 @@ __global__ void __launch_bounds__(kLkWarps * 32, kLkMinBlocks<T>)
         } else {
             tracked[2 * k] = tx;
             tracked[2 * k + 1] = ty;
-            status[k] = ok ? 1 : 0;
+            if constexpr (kMask)
+                status[k] = !ok ? 0
+                            : track_eligible(E, P.w[0], lo, qx, qy) && track_eligible(E, P.w[0], lo + 1, tx, ty) ? 1
+                                                                                                                : 3;
+            else
+                status[k] = ok ? 1 : 0;
         }
     }
 }
@@ -2138,9 +2197,9 @@ constexpr int kSelThreads = 256, kSelStrip = 32, kPickThreads = 1024;
 // scores read inside the image, so reads outside it (clamped here) reach no used score.  Writes the
 // cell's best candidate as the key (score bits << 32) | ~(y * w + x): the greater key is the greater
 // score, then the smaller index; 0 = no candidate.  The pixels are staged as the plane's samples (T) and
-// converted by track_level0 where the Sobel stencil reads them.
-template <typename T>
-__global__ void __launch_bounds__(kSelThreads) select_cells_kernel(TrackImages im, TrackSelect S, int j0) {
+// converted by track_level0 where the Sobel stencil reads them.  kMask: a candidate must also be eligible (E).
+template <typename T, bool kMask = false>
+__global__ void __launch_bounds__(kSelThreads) select_cells_kernel(TrackImages im, TrackSelect S, int j0, TrackElig E) {
     extern __shared__ float s_sel[];
     const int C = S.cell, B = S.block, r = B / 2, hal = r + 2;
     const int PW = C + 2 * hal, SW = C + 2, GW = SW + 2 * r, GR = kSelStrip + 2 * r;
@@ -2210,6 +2269,9 @@ __global__ void __launch_bounds__(kSelThreads) select_cells_kernel(TrackImages i
         const float v = c[0];
         if (v > 0.f && v >= c[-SW - 1] && v >= c[-SW] && v >= c[-SW + 1] && v >= c[-1] && v >= c[1] &&
             v >= c[SW - 1] && v >= c[SW] && v >= c[SW + 1]) {
+            // (read for the local maxima only: a load per pixel of the cell would stall this loop)
+            if constexpr (kMask)
+                if (!E.plane[(int64_t)((j0 + blockIdx.y) % E.slots) * E.stride + (int64_t)y * w + x]) continue;
             const unsigned long long key = ((unsigned long long)__float_as_uint(v) << 32) |
                                            (unsigned)~((unsigned)y * (unsigned)w + (unsigned)x);
             best = key > best ? key : best;
@@ -2991,12 +3053,24 @@ void launch_track_frames_t(const TrackImages& im, int n_frames, const int64_t* h
     const TrackPyr P = track_pyr(im, d_pyr, slots);
     const int pw = im.window + 2;
     const size_t smem = (size_t)kLkWarps * (pw * pw + 2 * im.window * im.window) * sizeof(float);
-    allow_smem(track_lk_kernel<T, false>, smem);
+    const TrackMask* M = ex.mask;
+    if (M) allow_smem(track_lk_kernel<T, false, true>, smem);
+    else allow_smem(track_lk_kernel<T, false>, smem);
     const bool back = ex.fb_max > 0.0;
     if (back) allow_smem(track_lk_kernel<T, true>, smem);
     const TrackSelect* S = ex.sel;
     const size_t sel_smem = S ? track_select_smem(S->cell, S->block, (int)sizeof(T)) : 0;
-    if (S) allow_smem(select_cells_kernel<T>, sel_smem);
+    if (S && M) allow_smem(select_cells_kernel<T, true>, sel_smem);
+    else if (S) allow_smem(select_cells_kernel<T>, sel_smem);
+    // a shared mask is eroded once, per-image masks with their pyramids
+    const bool per_image = M && M->image_stride != 0;
+    const TrackElig E{M ? M->d_elig : nullptr, per_image ? (int64_t)im.w0 * im.h0 : 0, per_image ? slots : 1};
+    auto erode = [&](int j0, int n) {
+        const dim3 grid((im.w0 + kErTX - 1) / kErTX, (im.h0 + kErTY - 1) / kErTY, n);
+        track_erode_kernel<<<grid, 256, 0, st>>>(*M, im.w0, im.h0, j0, E);
+        g_launches += 1;
+    };
+    if (M && !per_image) erode(0, 1);
     // chunk: build the pyramids of images [built, e), then track frames [f0, e - 1); image f0 is the
     // last one of the previous chunk, still in its slot
     for (int f0 = 0, built = 0; f0 < n_frames;) {
@@ -3006,11 +3080,14 @@ void launch_track_frames_t(const TrackImages& im, int n_frames, const int64_t* h
             track_pyramid_kernel<T><<<grid, kPyrTX * kPyrTY, 0, st>>>(P, l, built);
             g_launches += 1;
         }
+        if (per_image && e > built) erode(built, e - built);
         // selection on the chunk's side-a images f0 .. e - 2; the tracker's grid then covers the bound
         // max_points per frame and its warps past q_at[e - 1] return at once
         const int nf = e - 1 - f0;
         if (S) {
-            select_cells_kernel<T><<<dim3(S->cells_x * S->cells_y, nf), kSelThreads, sel_smem, st>>>(im, *S, f0);
+            const dim3 grid(S->cells_x * S->cells_y, nf);
+            if (M) select_cells_kernel<T, true><<<grid, kSelThreads, sel_smem, st>>>(im, *S, f0, E);
+            else select_cells_kernel<T><<<grid, kSelThreads, sel_smem, st>>>(im, *S, f0, E);
             select_points_kernel<<<nf, kPickThreads, 0, st>>>(*S);
             select_prefix_kernel<<<1, kPickThreads, 0, st>>>(*S, d_q_at, f0, e - 1, im.w0, d_points);
             g_launches += 3;
@@ -3018,13 +3095,18 @@ void launch_track_frames_t(const TrackImages& im, int n_frames, const int64_t* h
         const int64_t pts = S ? (int64_t)nf * S->max_points : h_q_at[e - 1] - h_q_at[f0];
         if (pts > 0) {
             const unsigned blocks = (unsigned)((pts + kLkWarps - 1) / kLkWarps);
-            track_lk_kernel<T, false><<<blocks, kLkWarps * 32, smem, st>>>(P, d_q_at, f0, e - 1, d_points, d_tracked,
-                                                                          d_status, d_flag, 0.0, nullptr);
+            if (M)
+                track_lk_kernel<T, false, true><<<blocks, kLkWarps * 32, smem, st>>>(
+                    P, d_q_at, f0, e - 1, d_points, d_tracked, d_status, d_flag, 0.0, nullptr, E);
+            else
+                track_lk_kernel<T, false><<<blocks, kLkWarps * 32, smem, st>>>(P, d_q_at, f0, e - 1, d_points,
+                                                                              d_tracked, d_status, d_flag, 0.0,
+                                                                              nullptr, E);
             g_launches += 1;
             if (back) {
                 track_lk_kernel<T, true><<<blocks, kLkWarps * 32, smem, st>>>(P, d_q_at, f0, e - 1, d_points,
                                                                              d_tracked, d_status, d_flag, ex.fb_max,
-                                                                             ex.d_fb);
+                                                                             ex.d_fb, E);
                 g_launches += 1;
             }
         }

@@ -235,15 +235,28 @@ struct TrackSelect {
     uint32_t* d_picks;           // scratch: per frame of a chunk, max_points pixel indices y * w + x
     int32_t* d_count;            // scratch: per frame of a chunk, the number of picks
 };
+// ---- the caller's mask (rssync_track_frames_masked_device) ---------------------------------------
+// The contract is stated at rssync_track_frames_masked_device in include/rssync_b200.h.  Row y of image j's
+// mask at mask + j * image_stride + y * pitch bytes (image_stride 0: one mask for every image).  The mask is
+// eroded by a (2 margin + 1)^2 square into eligibility planes of w0 * h0 bytes in d_elig: one plane when
+// image_stride is 0, else one per pyramid slot (image j in slot j % slots, eroded with its pyramid).
+constexpr int kTrackMaxMargin = 63;
+struct TrackMask {
+    const uint8_t* mask;
+    int64_t pitch, image_stride;
+    int margin;
+    uint8_t* d_elig;
+};
 // Options of launch_track_frames beyond forward tracking.  sel null: the query points are the
 // caller's (h_q_at known); otherwise the points of frame i are selected on image i into d_points (which
 // holds n_frames * max_points points) and d_q_at (written here, from d_q_at[0] = 0).  fb_max > 0: every
 // point kept forward is tracked back, its distance written to d_fb and its status set to 2 when the
-// backward pass loses it or the distance exceeds fb_max.
+// backward pass loses it or the distance exceeds fb_max.  mask null: no mask.
 struct TrackExtra {
     const TrackSelect* sel;
     double fb_max;
     double* d_fb;
+    const TrackMask* mask;
 };
 // Shared memory of one select_cells_kernel block staging `sample`-byte pixels
 size_t track_select_smem(int cell, int block, int sample);
@@ -251,8 +264,10 @@ size_t track_select_smem(int cell, int block, int sample);
 // image i + 1, for i in [0, n_frames).  The pyramids of `slots` (>= 2) images live in d_pyr at once
 // (slots * track_pyramid_floats floats): the images are processed in chunks, image j in slot j % slots,
 // each pyramid built once.  Per point: d_tracked (2 doubles) and d_status (1 = kept); *d_flag gets bit 0
-// when a query point is not finite.  ex: selection and the backward pass (TrackExtra); with ex.sel null
-// and ex.fb_max 0 the launches are the forward tracker's alone.  im.sample picks the kernels' pixel type.
+// when a query point is not finite.  ex: selection, the backward pass and the mask (TrackExtra); with
+// ex.sel and ex.mask null and ex.fb_max 0 the launches are the forward tracker's alone.  With a mask the
+// selection takes eligible candidates only, and a point the forward pass keeps gets status 3 instead of 1
+// when its query or tracked position is not eligible.  im.sample picks the kernels' pixel type.
 void launch_track_frames(const TrackImages& im, int n_frames, const int64_t* h_q_at, int64_t* d_q_at,
                          double* d_points, float* d_pyr, int slots, double* d_tracked, uint8_t* d_status,
                          unsigned* d_flag, const TrackExtra& ex, cudaStream_t st);

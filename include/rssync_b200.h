@@ -93,7 +93,8 @@ typedef struct rssync_lens {
  * [0, pi/2] overflows, and a non-finite or non-positive image_rows (RSSYNC_E_INVALID, "bad lens profile
  * or image height"); a non-finite frame timestamp, and a point that is not finite or whose
  * (x - cx) / fx, (y - cy) / fy or their squared norm is not (RSSYNC_E_NONFINITE, reported as the
- * ray buffer of its side: "non-finite numbers in rays_a" for points_a).  Either would give NaN rays. */
+ * ray buffer of its side: "non-finite numbers in rays_a" for points_a).  Either would give NaN rays.
+ * A frame id given more than once: the last occurrence wins. */
 int rssync_set_track_pixels(rssync_problem* p, size_t n_frames, const int64_t* frames,
                             const size_t* counts, const double* frame_ts_a, const double* frame_ts_b,
                             const double* points_a, const double* points_b, const rssync_lens* lens,
@@ -173,7 +174,8 @@ typedef struct rssync_track_params {
  * image_ts[0..n_frames) the a side) and a non-finite query point ("non-finite numbers in rays_a").
  * Ordering and borrowing as in the other _device forms: reads are ordered after `stream`, and the library
  * has finished with images and points when the call returns.  A multi-device problem ingests on its
- * primary; the replicas receive the arena at the next compute call. */
+ * primary; the replicas receive the arena at the next compute call.  A frame id given more than once: the last
+ * occurrence wins (its kept pairs are ingested; tracked_out and status_out still cover every point). */
 int rssync_track_frames_device(rssync_problem* p, size_t n_frames, const int64_t* frames, const size_t* counts,
                                const double* image_ts, const double* points, const uint8_t* images, size_t pitch,
                                int width, int height, const rssync_lens* lens, const rssync_track_params* params,

@@ -296,7 +296,7 @@ struct rssync_problem {
 
     // Grid scratch of every PreSync entry point: frame tables (the readout search's one per readout),
     // delays, per-task costs, the loss curves and their flag words (2 per curve).  d_pixframes holds the
-    // PixelFrame records of the host pixels ingest, of set_readout and of the readout search.  One set
+    // PixelFrame records of set_readout and of the readout search.  One set
     // serves all calls because each buffer is written and read only on `stream`: a call's use of it is
     // ordered after the previous call's, and every call that reads a result back synchronises that
     // stream before it returns.
@@ -306,9 +306,8 @@ struct rssync_problem {
     DevBuf<rs::PixelFrame> d_pixframes;
     DevBuf<uint64_t> d_frame_call;
     DevBuf<int> d_win_begin;
-    // pixel front end staging
-    PinBuf<double> h_pix;
-    DevBuf<double> d_pix, d_stage;
+    // staging of the bulk ingests
+    DevBuf<double> d_stage;
     PinBuf<double> h_stage;
     // sync: per-lane scratch (sync_batch_impl)
     std::vector<SyncLane> lanes;
@@ -471,6 +470,15 @@ int flush(rssync_problem* p, bool keep_in_flight = false) {
         p->pending.clear();
     }
     return RSSYNC_OK;
+}
+
+// The start of a bulk ingest on the problem's stream (every form but the chunked rssync_set_track_batch):
+// an earlier call's staging block is free again, and the ingest follows everything that writes the arena.
+// Frames set one by one before this call are older than it: their upload goes first.
+int begin_ingest(rssync_problem* p) {
+    CUDA_TRY(p, cudaSetDevice(p->device));
+    if (int rc = wait_arena_copies(p)) return rc;
+    return p->pending.empty() ? wait_in_flight(p) : flush(p);
 }
 
 // frames with begin <= id < end_exclusive, ascending id
@@ -1581,7 +1589,7 @@ void rssync_destroy(rssync_problem* p) {
     p->h_pos.release(); p->d_pos.release();
     p->d_frames.release(); p->d_delays.release(); p->d_framecost.release(); p->d_costs.release();
     p->d_frame_call.release(); p->d_win_begin.release();
-    p->h_pix.release(); p->d_pix.release(); p->d_pixframes.release(); p->d_stage.release();
+    p->d_pixframes.release(); p->d_stage.release();
     p->d_flags.release(); p->h_stage.release(); p->d_probe.release();
     p->d_gather.release(); p->h_gather.release();
     p->d_var_ts.release(); p->d_var_in.release(); p->d_var_q.release(); p->d_var_y.release(); p->d_var_rhs.release();
@@ -2281,6 +2289,10 @@ int check_pixel_args(rssync_problem* p, size_t n_frames, const size_t* counts, c
     return frame_offsets(p, n_frames, counts, at);
 }
 
+rs::LensDev lens_dev(const rssync_lens& l) {
+    return rs::LensDev{l.readout, l.fx, l.fy, l.cx, l.cy, l.k1, l.k2, l.k3, l.k4};
+}
+
 // the pixels forms' per-frame timestamps, checked before any point
 int check_frame_ts(rssync_problem* p, size_t n_frames, const double* frame_ts_a, const double* frame_ts_b) {
     if (!all_finite(frame_ts_a, n_frames)) { p->err = kMsgNonFinite[kTsA]; return RSSYNC_E_NONFINITE; }
@@ -2328,14 +2340,7 @@ struct DeviceStaging {
 int begin_device_staging(rssync_problem* p, const std::vector<size_t>& at, size_t data_doubles,
                          const double* frame_ts_a, const double* frame_ts_b, void* stream, DeviceStaging& s) {
     const size_t n = at.size() - 1;
-    CUDA_TRY(p, cudaSetDevice(p->device));
-    if (int rc = wait_arena_copies(p)) return rc;  // an earlier call's staging block is free again
-    // frames set one by one before this call are older than it: their upload goes first
-    if (!p->pending.empty()) {
-        if (int rc = flush(p)) return rc;
-    } else if (int rc = wait_in_flight(p)) {
-        return rc;
-    }
+    if (int rc = begin_ingest(p)) return rc;
     const size_t block = 10 * n + 1;
     CUDA_TRY(p, p->h_stage.reserve(block));
     CUDA_TRY(p, p->d_stage.reserve(block + data_doubles));
@@ -2383,6 +2388,48 @@ int reserve_rowq(rssync_problem* p) {
     CUDA_TRY(p, p->d_rowq.grow(2 * std::max<size_t>(p->d_orig.cap, 1), 2 * p->dev_used, p->stream));
     p->rowq_version++;
     return RSSYNC_OK;
+}
+
+// The bulk ingests on the problem's stream, once the first n frames have passed their checks: place the
+// last occurrence of each frame id among them (an ingest block per occurrence would write the same arena
+// range twice; the last one wins, as with rssync_set_track calls in order), fill its ingest record
+// (rec[0..k)) and make room in the device arena.  at: the frames' offsets in the staged data; info: their
+// timestamp bounds.  frame_ts_a / frame_ts_b (pixels and row-fractions forms, else null): the frames keep
+// them for re-timing, and the row-fraction plane grows with the arena.
+int place_frames(rssync_problem* p, size_t n, const int64_t* frames, const std::vector<size_t>& at,
+                 const rs::StageInfo* info, const double* frame_ts_a, const double* frame_ts_b, rs::PixelFrame* rec,
+                 size_t& k) {
+    std::vector<char> last(n, 1);
+    if (std::adjacent_find(frames, frames + n, std::greater_equal<int64_t>()) != frames + n) {  // not ascending
+        std::unordered_set<int64_t> seen;
+        for (size_t i = n; i-- > 0;) last[i] = seen.insert(frames[i]).second;
+    }
+    p->version++;
+    k = 0;
+    for (size_t i = 0; i < n; ++i) {
+        if (!last[i]) continue;
+        FrameDesc* fd = nullptr;
+        if (int rc = place_track(p, frames[i], at[i + 1] - at[i], &fd, /*host_mirror=*/false)) return rc;
+        fd->ts_lo = info[i].lo;
+        fd->ts_hi = info[i].hi;
+        rec[k++] = rs::PixelFrame{fd->off, fd->n, (int64_t)at[i], frame_ts_a ? frame_ts_a[i] : 0.0,
+                                  frame_ts_a ? frame_ts_b[i] : 0.0};
+        if (frame_ts_a) p->retime[frames[i]] = {frame_ts_a[i], frame_ts_b[i]};
+    }
+    if (int rc = reserve_device_arena(p)) return rc;
+    return frame_ts_a ? reserve_rowq(p) : RSSYNC_OK;
+}
+
+// the first of n frames whose check found a non-finite value (n: none)
+size_t first_bad(const rs::StageInfo* info, size_t n) {
+    size_t i = 0;
+    while (i < n && !info[i].bad) ++i;
+    return i;
+}
+// such a frame fails the call with the text of its first source buffer holding the value
+int fail_nonfinite(rssync_problem* p, const rs::StageInfo& info) {
+    p->err = kMsgNonFinite[__builtin_ctz(info.bad)];
+    return RSSYNC_E_NONFINITE;
 }
 
 // A plane that covers the whole device arena: frames a rays form appended since the last row fractions
@@ -2469,41 +2516,23 @@ int rssync_set_track_batch_device(rssync_problem* p, size_t n_frames, const int6
     rs::launch_stage_rays(s.d_at, (int)n_frames, (int64_t)total, rays_a, rays_b, ts_a, ts_b, s.d_data, s.d_info,
                           p->stream);
     if (int rc = read_stage_info(p, n_frames, s)) return rc;
-    size_t n_ok = n_frames;
-    for (size_t i = 0; i < n_frames; ++i)
-        if (s.h_info[i].bad) { n_ok = i; break; }
-    std::vector<char> last(n_ok, 0);  // the frame is the last occurrence of its id among the applied ones
-    {
-        std::unordered_set<int64_t> seen;
-        for (size_t i = n_ok; i-- > 0;) last[i] = seen.insert(frames[i]).second;
-    }
-    p->version++;
+    const size_t n_ok = first_bad(s.h_info, n_frames);
     size_t k = 0;
-    for (size_t i = 0; i < n_ok; ++i) {
-        if (!last[i]) continue;
-        FrameDesc* fd = nullptr;
-        if (int rc = place_track(p, frames[i], counts[i], &fd, /*host_mirror=*/false)) return rc;
-        fd->ts_lo = s.h_info[i].lo;
-        fd->ts_hi = s.h_info[i].hi;
-        s.h_rec[k++] = rs::PixelFrame{fd->off, fd->n, (int64_t)at[i], 0.0, 0.0};
-    }
+    if (int rc = place_frames(p, n_ok, frames, at, s.h_info, nullptr, nullptr, s.h_rec, k)) return rc;
     if (k) {
-        if (int rc = reserve_device_arena(p)) return rc;
         if (int rc = h2d(p, s.d_rec, s.h_rec, k * sizeof(rs::PixelFrame))) return rc;
         rs::launch_ingest_rays(s.d_rec, (int)k, s.d_data, s.d_data + total, s.d_data + 2 * total, s.d_data + 5 * total,
                                p->d_rays.ptr, p->d_orig.ptr, p->d_pos.ptr, p->stream);
         if (int rc = end_device_ingest(p)) return rc;
     }
-    if (n_ok < n_frames) {
-        p->err = kMsgNonFinite[__builtin_ctz(s.h_info[n_ok].bad)];
-        return RSSYNC_E_NONFINITE;
-    }
-    return RSSYNC_OK;
+    return n_ok < n_frames ? fail_nonfinite(p, s.h_info[n_ok]) : RSSYNC_OK;
 }
 
 // The per-frame tail of track_frames (core_testcode.cpp:134-161) on the device: pixel pairs in,
 // rays + rolling-shutter timestamps straight into the device arena (no host sort / transpose, half
-// the host->device bytes of the ray form).
+// the host->device bytes of the ray form).  One pass on the worker pool checks every frame while it copies
+// it into the pinned staging block and takes its timestamp bounds, then one upload and one ingest launch.
+// Staging block, in doubles: [records: 4 per frame][points_a 2n][points_b 2n].
 int rssync_set_track_pixels(rssync_problem* p, size_t n_frames, const int64_t* frames, const size_t* counts,
                             const double* frame_ts_a, const double* frame_ts_b, const double* points_a,
                             const double* points_b, const rssync_lens* lens, double image_rows) {
@@ -2511,27 +2540,26 @@ int rssync_set_track_pixels(rssync_problem* p, size_t n_frames, const int64_t* f
     if (!p) return RSSYNC_E_INVALID;
     if (n_frames == 0) return RSSYNC_OK;
     if (!frames || !counts || !frame_ts_a || !frame_ts_b || !points_a || !points_b || !lens) return RSSYNC_E_INVALID;
-    p->version++;
     std::vector<size_t> at;
     if (int rc = check_pixel_args(p, n_frames, counts, lens, image_rows, at)) return rc;
     const size_t total = at[n_frames];
     if (int rc = check_frame_ts(p, n_frames, frame_ts_a, frame_ts_b)) return rc;
-    if (int rc = wait_arena_copies(p)) return rc;
-    cudaSetDevice(p->device);
-    if (int rc = wait_in_flight(p)) return rc;  // this ingest runs on the problem's stream
-    CUDA_TRY(p, p->h_pix.reserve(4 * total + 1));
-    // per frame (worker pool): validate, copy into the pinned staging buffer, timestamp bounds with
+    if (int rc = begin_ingest(p)) return rc;
+    const size_t block = 4 * n_frames + 4 * total;
+    CUDA_TRY(p, p->h_stage.reserve(block + 1));
+    double* h_pa = p->h_stage.ptr + 4 * n_frames;
+    double* h_pb = h_pa + 2 * total;
+    // per frame (worker pool): validate, copy into the pinned staging block, timestamp bounds with
     // the device's expression (core_testcode.cpp:144-145)
-    std::vector<int> bad(n_frames, 0);
-    std::vector<double> lo(n_frames, 0.0), hi(n_frames, 0.0);
+    std::vector<rs::StageInfo> info(n_frames, rs::StageInfo{0u, 0u, 0.0, 0.0});
     parallel_frames(n_frames, [&](size_t i, size_t) {
         const double* a = points_a + 2 * at[i];
         const double* b = points_b + 2 * at[i];
         const size_t n = counts[i];
-        if (!points_ok(a, n, *lens)) { bad[i] = 1; return; }
-        if (!points_ok(b, n, *lens)) { bad[i] = 2; return; }
-        std::memcpy(p->h_pix.ptr + 2 * at[i], a, 2 * n * sizeof(double));
-        std::memcpy(p->h_pix.ptr + 2 * total + 2 * at[i], b, 2 * n * sizeof(double));
+        if (!points_ok(a, n, *lens)) { info[i].bad = 1u << kRaysA; return; }
+        if (!points_ok(b, n, *lens)) { info[i].bad = 1u << kRaysB; return; }
+        std::memcpy(h_pa + 2 * at[i], a, 2 * n * sizeof(double));
+        std::memcpy(h_pb + 2 * at[i], b, 2 * n * sizeof(double));
         double l = 0.0, h = 0.0;
         for (size_t k = 0; k < n; ++k) {
             const double ta = frame_ts_a[i] + lens->readout * (a[2 * k + 1] / image_rows);
@@ -2540,89 +2568,37 @@ int rssync_set_track_pixels(rssync_problem* p, size_t n_frames, const int64_t* f
             l = std::min(l, std::min(ta, tb));
             h = std::max(h, std::max(ta, tb));
         }
-        lo[i] = l;
-        hi[i] = h;
+        info[i].lo = l;
+        info[i].hi = h;
     });
-    for (size_t i = 0; i < n_frames; ++i)
-        if (bad[i]) {
-            p->err = kMsgNonFinite[bad[i] == 1 ? kRaysA : kRaysB];
-            return RSSYNC_E_NONFINITE;
-        }
-    std::vector<rs::PixelFrame> pf(n_frames);
-    for (size_t i = 0; i < n_frames; ++i) {
-        FrameDesc* fd = nullptr;
-        if (int rc = place_track(p, frames[i], counts[i], &fd, /*host_mirror=*/false)) return rc;
-        fd->ts_lo = lo[i];
-        fd->ts_hi = hi[i];
-        pf[i] = rs::PixelFrame{fd->off, fd->n, (int64_t)at[i], frame_ts_a[i], frame_ts_b[i]};
-    }
-    for (size_t i = 0; i < n_frames; ++i) p->retime[frames[i]] = {frame_ts_a[i], frame_ts_b[i]};
-    if (int rc = reserve_device_arena(p)) return rc;
-    if (int rc = reserve_rowq(p)) return rc;
-    CUDA_TRY(p, p->d_pix.reserve(4 * total + 1));
-    CUDA_TRY(p, p->d_pixframes.reserve(n_frames));
-    if (int rc = h2d(p, p->d_pix.ptr, p->h_pix.ptr, 4 * total * sizeof(double))) return rc;
-    if (int rc = h2d(p, p->d_pixframes.ptr, pf.data(), n_frames * sizeof(rs::PixelFrame))) return rc;
-    CUDA_TRY(p, cudaStreamSynchronize(p->stream));  // pf is a local; the pinned staging buffer is reused
-    rs::LensDev L{lens->readout, lens->fx, lens->fy, lens->cx, lens->cy, lens->k1, lens->k2, lens->k3, lens->k4};
-    rs::launch_ingest_pixels(p->d_pixframes.ptr, (int)n_frames, p->d_pix.ptr, p->d_pix.ptr + 2 * total, L,
-                             image_rows, p->d_rays.ptr, p->d_orig.ptr, p->d_pos.ptr, p->d_rowq.ptr, p->stream);
-    CUDA_TRY(p, cudaGetLastError());
-    p->dev_used = std::max(p->dev_used, p->used);
-    return RSSYNC_OK;
+    if (const size_t i = first_bad(info.data(), n_frames); i < n_frames) return fail_nonfinite(p, info[i]);
+    rs::PixelFrame* rec = reinterpret_cast<rs::PixelFrame*>(p->h_stage.ptr);
+    size_t k = 0;
+    if (int rc = place_frames(p, n_frames, frames, at, info.data(), frame_ts_a, frame_ts_b, rec, k)) return rc;
+    CUDA_TRY(p, p->d_stage.reserve(block + 1));
+    if (int rc = h2d(p, p->d_stage.ptr, p->h_stage.ptr, block * sizeof(double))) return rc;
+    const double* d_pa = p->d_stage.ptr + 4 * n_frames;
+    rs::launch_ingest_pixels(reinterpret_cast<const rs::PixelFrame*>(p->d_stage.ptr), (int)k, d_pa, d_pa + 2 * total,
+                             lens_dev(*lens), image_rows, p->d_rays.ptr, p->d_orig.ptr, p->d_pos.ptr, p->d_rowq.ptr,
+                             p->stream);
+    return end_device_ingest(p);
 }
 
 }  // extern "C"
 
 namespace {
 
-// Points that kernels on the problem's stream write during the call, with their frame offsets
-// (rssync_track_frames_device): `queue` enqueues the writers and the copies back of what the host needs,
-// and returns the offsets (device, n_frames + 1) for the stage kernel; `verdict`, after the round trip,
-// sets the host offsets or fails the call before anything is placed.
-struct DevicePointSource {
-    std::function<const int64_t*(const DeviceStaging&)> queue;
-    std::function<int(const DeviceStaging&, std::vector<size_t>&)> verdict;
-};
-
-// The body of rssync_set_track_pixels_device once its host checks have passed: the check, the timestamp
-// bounds and the copy into the staging buffer on the device (stage_tracks_kernel), the per-frame verdicts
-// back in the one round trip, then placement and ingest.  at: the frames' offsets in points_a / points_b;
-// the staging buffer holds at[n_frames] points per side.  src (or null): the points are written on the
-// device first, at offsets only known after the round trip (at then becomes those offsets).
-int ingest_pixels_device(rssync_problem* p, size_t n_frames, const int64_t* frames, std::vector<size_t>& at,
-                         const double* frame_ts_a, const double* frame_ts_b, const double* points_a,
-                         const double* points_b, const rssync_lens* lens, double image_rows, void* stream,
-                         const DevicePointSource* src = nullptr) {
-    const size_t total = at[n_frames];
-    DeviceStaging s;
-    if (int rc = begin_device_staging(p, at, 4 * total, frame_ts_a, frame_ts_b, stream, s)) return rc;
-    const int64_t* d_at = src ? src->queue(s) : s.d_at;
-    if (!d_at) return RSSYNC_E_CUDA;  // (p->err set by queue)
-    const rs::LensDev L{lens->readout, lens->fx, lens->fy, lens->cx, lens->cy, lens->k1, lens->k2, lens->k3, lens->k4};
-    rs::launch_stage_points(d_at, s.d_fts, (int)n_frames, (int64_t)total, points_a, points_b, L, image_rows,
-                            s.d_data, s.d_info, p->stream);
-    if (int rc = read_stage_info(p, n_frames, s)) return rc;
-    if (src)
-        if (int rc = src->verdict(s, at)) return rc;
-    for (size_t i = 0; i < n_frames; ++i)
-        if (s.h_info[i].bad) {
-            p->err = kMsgNonFinite[(s.h_info[i].bad & 1u) ? kRaysA : kRaysB];
-            return RSSYNC_E_NONFINITE;
-        }
-    p->version++;
-    for (size_t i = 0; i < n_frames; ++i) {
-        FrameDesc* fd = nullptr;
-        if (int rc = place_track(p, frames[i], at[i + 1] - at[i], &fd, /*host_mirror=*/false)) return rc;
-        fd->ts_lo = s.h_info[i].lo;
-        fd->ts_hi = s.h_info[i].hi;
-        s.h_rec[i] = rs::PixelFrame{fd->off, fd->n, (int64_t)at[i], frame_ts_a[i], frame_ts_b[i]};
-    }
-    for (size_t i = 0; i < n_frames; ++i) p->retime[frames[i]] = {frame_ts_a[i], frame_ts_b[i]};
-    if (int rc = reserve_device_arena(p)) return rc;
-    if (int rc = reserve_rowq(p)) return rc;
-    if (int rc = h2d(p, s.d_rec, s.h_rec, n_frames * sizeof(rs::PixelFrame))) return rc;
-    rs::launch_ingest_pixels(s.d_rec, (int)n_frames, s.d_data, s.d_data + 2 * total, L, image_rows, p->d_rays.ptr,
+// The device pixels forms once the per-frame verdicts are back (read_stage_info): the first frame holding a
+// non-finite value fails the call before anything is placed, else the frames are placed and their points,
+// staged at the offsets `at` of `total` points per side, ingested.
+int ingest_staged_pixels(rssync_problem* p, size_t n_frames, const int64_t* frames, const std::vector<size_t>& at,
+                         size_t total, const double* frame_ts_a, const double* frame_ts_b, const rs::LensDev& L,
+                         double image_rows, const DeviceStaging& s) {
+    if (const size_t i = first_bad(s.h_info, n_frames); i < n_frames) return fail_nonfinite(p, s.h_info[i]);
+    size_t k = 0;
+    if (int rc = place_frames(p, n_frames, frames, at, s.h_info, frame_ts_a, frame_ts_b, s.h_rec, k)) return rc;
+    if (int rc = h2d(p, s.d_rec, s.h_rec, k * sizeof(rs::PixelFrame))) return rc;
+    rs::launch_ingest_pixels(s.d_rec, (int)k, s.d_data, s.d_data + 2 * total, L, image_rows, p->d_rays.ptr,
                              p->d_orig.ptr, p->d_pos.ptr, p->d_rowq.ptr, p->stream);
     return end_device_ingest(p);
 }
@@ -2780,41 +2756,35 @@ int track_frames(rssync_problem* p, size_t n_frames, const int64_t* frames, cons
                              tp.window, tp.max_iters, (float)tp.epsilon, (float)tp.min_eig, (uint8_t)sample,
                              (uint8_t)shift};
     const rs::TrackExtra ex{select ? &sel : nullptr, fb_max, out.fb, mask ? &tm : nullptr};
-    DevicePointSource src;
-    // s.d_at holds the query offsets (begin_device_staging; in selection mode the bound, overwritten on
-    // the device by the selected offsets); s.h_at receives the kept ones
-    src.queue = [&](const DeviceStaging& s) -> const int64_t* {
-        cudaError_t e = cudaMemsetAsync(p->d_trk_flag.ptr, 0, sizeof(unsigned), p->stream);
-        if (e == cudaSuccess && out.fb && total) e = cudaMemsetAsync(out.fb, 0xff, total * sizeof(double), p->stream);
-        if (e == cudaSuccess && out.points && total && !select)
-            e = cudaMemcpyAsync(out.points, points, 2 * total * sizeof(double), cudaMemcpyDeviceToDevice, p->stream);
-        if (e != cudaSuccess) {
-            p->err = std::string("CUDA error: ") + cudaGetErrorString(e);
-            return nullptr;
-        }
-        rs::launch_track_frames(im, (int)n_frames, select ? nullptr : q_at.data(), s.d_at, d_points, p->d_trk_pyr.ptr,
-                                (int)slots, d_tracked, d_status, p->d_trk_flag.ptr, ex, p->stream);
-        rs::launch_track_compact(s.d_at, (int)n_frames, d_points, d_tracked, d_status, d_a, d_b, d_kept_at,
-                                 p->stream);
-        if (d2h(p, s.h_at, d_kept_at, (n_frames + 1) * sizeof(int64_t)) ||
-            d2h(p, p->h_trk_flag.ptr, p->d_trk_flag.ptr, sizeof(unsigned)) ||
-            (select && d2h(p, p->h_trk_qat.ptr, s.d_at, (n_frames + 1) * sizeof(int64_t))))
-            return nullptr;
-        return d_kept_at;
-    };
-    src.verdict = [&](const DeviceStaging& s, std::vector<size_t>& kept) {
-        if (*p->h_trk_flag.ptr) {
-            p->err = kMsgNonFinite[kRaysA];
-            return (int)RSSYNC_E_NONFINITE;
-        }
-        if (out.counts)
-            for (size_t i = 0; i < n_frames; ++i)
-                out.counts[i] = select ? (size_t)(p->h_trk_qat.ptr[i + 1] - p->h_trk_qat.ptr[i]) : counts[i];
-        for (size_t i = 0; i <= n_frames; ++i) kept[i] = (size_t)s.h_at[i];
-        return (int)RSSYNC_OK;
-    };
-    return ingest_pixels_device(p, n_frames, frames, at, image_ts, image_ts + 1, d_a, d_b, lens, (double)height,
-                                stream, &src);
+    // s.d_at holds the query offsets (in selection mode the bound, overwritten on the device by the selected
+    // offsets); the compacted pairs are staged at the kept offsets, which s.h_at receives
+    DeviceStaging s;
+    if (int rc = begin_device_staging(p, at, 4 * total, image_ts, image_ts + 1, stream, s)) return rc;
+    CUDA_TRY(p, cudaMemsetAsync(p->d_trk_flag.ptr, 0, sizeof(unsigned), p->stream));
+    if (out.fb && total) CUDA_TRY(p, cudaMemsetAsync(out.fb, 0xff, total * sizeof(double), p->stream));
+    if (out.points && total && !select)
+        CUDA_TRY(p, cudaMemcpyAsync(out.points, points, 2 * total * sizeof(double), cudaMemcpyDeviceToDevice,
+                                    p->stream));
+    rs::launch_track_frames(im, (int)n_frames, select ? nullptr : q_at.data(), s.d_at, d_points, p->d_trk_pyr.ptr,
+                            (int)slots, d_tracked, d_status, p->d_trk_flag.ptr, ex, p->stream);
+    rs::launch_track_compact(s.d_at, (int)n_frames, d_points, d_tracked, d_status, d_a, d_b, d_kept_at, p->stream);
+    if (int rc = d2h(p, s.h_at, d_kept_at, (n_frames + 1) * sizeof(int64_t))) return rc;
+    if (int rc = d2h(p, p->h_trk_flag.ptr, p->d_trk_flag.ptr, sizeof(unsigned))) return rc;
+    if (select)
+        if (int rc = d2h(p, p->h_trk_qat.ptr, s.d_at, (n_frames + 1) * sizeof(int64_t))) return rc;
+    const rs::LensDev L = lens_dev(*lens);
+    rs::launch_stage_points(d_kept_at, s.d_fts, (int)n_frames, (int64_t)total, d_a, d_b, L, (double)height, s.d_data,
+                            s.d_info, p->stream);
+    if (int rc = read_stage_info(p, n_frames, s)) return rc;
+    if (*p->h_trk_flag.ptr) {
+        p->err = kMsgNonFinite[kRaysA];
+        return RSSYNC_E_NONFINITE;
+    }
+    if (out.counts)
+        for (size_t i = 0; i < n_frames; ++i)
+            out.counts[i] = select ? (size_t)(p->h_trk_qat.ptr[i + 1] - p->h_trk_qat.ptr[i]) : counts[i];
+    for (size_t i = 0; i <= n_frames; ++i) at[i] = (size_t)s.h_at[i];
+    return ingest_staged_pixels(p, n_frames, frames, at, total, image_ts, image_ts + 1, L, (double)height, s);
 }
 
 // The ex entry points (rssync_track_frames_ex_device, rssync_track_frames16_device,
@@ -2857,12 +2827,17 @@ int rssync_set_track_pixels_device(rssync_problem* p, size_t n_frames, const int
     const size_t total = at[n_frames];
     if (int rc = check_device_buffers(p, {points_a, points_b}, total)) return rc;
     if (int rc = check_frame_ts(p, n_frames, frame_ts_a, frame_ts_b)) return rc;
-    return ingest_pixels_device(p, n_frames, frames, at, frame_ts_a, frame_ts_b, points_a, points_b, lens, image_rows,
-                                stream);
+    DeviceStaging s;
+    if (int rc = begin_device_staging(p, at, 4 * total, frame_ts_a, frame_ts_b, stream, s)) return rc;
+    const rs::LensDev L = lens_dev(*lens);
+    rs::launch_stage_points(s.d_at, s.d_fts, (int)n_frames, (int64_t)total, points_a, points_b, L, image_rows,
+                            s.d_data, s.d_info, p->stream);
+    if (int rc = read_stage_info(p, n_frames, s)) return rc;
+    return ingest_staged_pixels(p, n_frames, frames, at, total, frame_ts_a, frame_ts_b, L, image_rows, s);
 }
 
 // Sparse pyramidal Lucas-Kanade from image i to image i + 1 of the caller's luma planes, then the kept
-// pairs through rssync_set_track_pixels_device's ingest (ingest_pixels_device), compacted on the device.
+// pairs through rssync_set_track_pixels_device's ingest (ingest_staged_pixels), compacted on the device.
 int rssync_track_frames_device(rssync_problem* p, size_t n_frames, const int64_t* frames, const size_t* counts,
                                const double* image_ts, const double* points, const uint8_t* images, size_t pitch,
                                int width, int height, const rssync_lens* lens, const rssync_track_params* params,
@@ -2938,34 +2913,6 @@ int check_row_fraction_args(rssync_problem* p, size_t n_frames, const size_t* co
     return RSSYNC_OK;
 }
 
-// The row-fractions forms once every frame has passed its checks: place the last occurrence of each frame
-// id (an ingest block per occurrence would write the same arena range twice), fill its ingest record
-// (rec[0..k)), keep its frame timestamps for re-timing, and make room for the arena and the row-fraction
-// plane.  lo / hi: each frame's timestamp bounds.
-int place_row_fraction_frames(rssync_problem* p, size_t n_frames, const int64_t* frames, const size_t* counts,
-                              const std::vector<size_t>& at, const double* frame_ts_a, const double* frame_ts_b,
-                              const std::vector<double>& lo, const std::vector<double>& hi, rs::PixelFrame* rec,
-                              size_t& k) {
-    std::vector<char> last(n_frames, 0);
-    {
-        std::unordered_set<int64_t> seen;
-        for (size_t i = n_frames; i-- > 0;) last[i] = seen.insert(frames[i]).second;
-    }
-    p->version++;
-    k = 0;
-    for (size_t i = 0; i < n_frames; ++i) {
-        if (!last[i]) continue;
-        FrameDesc* fd = nullptr;
-        if (int rc = place_track(p, frames[i], counts[i], &fd, /*host_mirror=*/false)) return rc;
-        fd->ts_lo = lo[i];
-        fd->ts_hi = hi[i];
-        rec[k++] = rs::PixelFrame{fd->off, fd->n, (int64_t)at[i], frame_ts_a[i], frame_ts_b[i]};
-        p->retime[frames[i]] = {frame_ts_a[i], frame_ts_b[i]};
-    }
-    if (int rc = reserve_device_arena(p)) return rc;
-    return reserve_rowq(p);
-}
-
 }  // namespace
 
 extern "C" {
@@ -2991,22 +2938,14 @@ int rssync_set_track_row_fractions(rssync_problem* p, size_t n_frames, const int
     if (int rc = check_row_fraction_args(p, n_frames, counts, readout, at)) return rc;
     const size_t total = at[n_frames];
     if (int rc = check_frame_ts(p, n_frames, frame_ts_a, frame_ts_b)) return rc;
-    CUDA_TRY(p, cudaSetDevice(p->device));
-    if (int rc = wait_arena_copies(p)) return rc;  // an earlier call's staging block is free again
-    // frames set one by one before this call are older than it: their upload goes first
-    if (!p->pending.empty()) {
-        if (int rc = flush(p)) return rc;
-    } else if (int rc = wait_in_flight(p)) {
-        return rc;
-    }
+    if (int rc = begin_ingest(p)) return rc;
     const size_t block = 4 * n_frames + 8 * total;
     CUDA_TRY(p, p->h_stage.reserve(block + 1));
     double* h_fa = p->h_stage.ptr + 4 * n_frames;
     double* h_fb = h_fa + total;
     double* h_ra = h_fb + total;
     double* h_rb = h_ra + 3 * total;
-    std::vector<int> bad(n_frames, 0);  // 1 + the first buffer (kRaysA .. kTsB) holding a non-finite value
-    std::vector<double> lo(n_frames, 0.0), hi(n_frames, 0.0);
+    std::vector<rs::StageInfo> info(n_frames);
     parallel_frames(n_frames, [&](size_t i, size_t) {
         const size_t a0 = at[i], n = counts[i];
         const bool ok_ra = copy_checked(h_ra + 3 * a0, rays_a + 3 * a0, 3 * n, nullptr, nullptr);
@@ -3029,20 +2968,14 @@ int rssync_set_track_row_fractions(rssync_problem* p, size_t n_frames, const int
             l = tb < l ? tb : l;
             h = tb > h ? tb : h;
         }
-        lo[i] = l;
-        hi[i] = h;
-        // rssync_set_track_batch's order of checks (core_private.cpp:199-202)
-        bad[i] = !ok_ra ? 1 + kRaysA : !ok_rb ? 1 + kRaysB : !ok_ta ? 1 + kTsA : !ok_tb ? 1 + kTsB : 0;
+        // bit b: source buffer b (kRaysA .. kTsB) holds a non-finite value, as StageInfo::bad
+        const unsigned bad = (!ok_ra << kRaysA) | (!ok_rb << kRaysB) | (!ok_ta << kTsA) | (!ok_tb << kTsB);
+        info[i] = rs::StageInfo{bad, 0u, l, h};
     });
-    for (size_t i = 0; i < n_frames; ++i)
-        if (bad[i]) {
-            p->err = kMsgNonFinite[bad[i] - 1];
-            return RSSYNC_E_NONFINITE;
-        }
+    if (const size_t i = first_bad(info.data(), n_frames); i < n_frames) return fail_nonfinite(p, info[i]);
     rs::PixelFrame* rec = reinterpret_cast<rs::PixelFrame*>(p->h_stage.ptr);
     size_t k = 0;
-    if (int rc = place_row_fraction_frames(p, n_frames, frames, counts, at, frame_ts_a, frame_ts_b, lo, hi, rec, k))
-        return rc;
+    if (int rc = place_frames(p, n_frames, frames, at, info.data(), frame_ts_a, frame_ts_b, rec, k)) return rc;
     CUDA_TRY(p, p->d_stage.reserve(block + 1));
     if (int rc = h2d(p, p->d_stage.ptr, p->h_stage.ptr, block * sizeof(double))) return rc;
     const double* d_fa = p->d_stage.ptr + 4 * n_frames;
@@ -3076,18 +3009,9 @@ int rssync_set_track_row_fractions_device(rssync_problem* p, size_t n_frames, co
     rs::launch_stage_row_fractions(s.d_at, s.d_fts, (int)n_frames, (int64_t)total, rays_a, rays_b, frac_a, frac_b,
                                    readout, s.d_data, s.d_info, p->stream);
     if (int rc = read_stage_info(p, n_frames, s)) return rc;
-    std::vector<double> lo(n_frames), hi(n_frames);
-    for (size_t i = 0; i < n_frames; ++i) {
-        if (s.h_info[i].bad) {
-            p->err = kMsgNonFinite[__builtin_ctz(s.h_info[i].bad)];
-            return RSSYNC_E_NONFINITE;
-        }
-        lo[i] = s.h_info[i].lo;
-        hi[i] = s.h_info[i].hi;
-    }
+    if (const size_t i = first_bad(s.h_info, n_frames); i < n_frames) return fail_nonfinite(p, s.h_info[i]);
     size_t k = 0;
-    if (int rc = place_row_fraction_frames(p, n_frames, frames, counts, at, frame_ts_a, frame_ts_b, lo, hi, s.h_rec, k))
-        return rc;
+    if (int rc = place_frames(p, n_frames, frames, at, s.h_info, frame_ts_a, frame_ts_b, s.h_rec, k)) return rc;
     if (int rc = h2d(p, s.d_rec, s.h_rec, k * sizeof(rs::PixelFrame))) return rc;
     rs::launch_ingest_row_fractions(s.d_rec, (int)k, s.d_data, s.d_data + total, s.d_data + 2 * total,
                                     s.d_data + 5 * total, readout, p->d_rays.ptr, p->d_orig.ptr, p->d_pos.ptr,
